@@ -1,17 +1,19 @@
 #!/usr/bin/env python
 """bench.py -- DR env-steps/sec of the RandomCartPole-v0 hot path on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]                 # this framework (CUDA kernels)
-    python bench.py --impl reference [--gpus N] [--steps K] [--warmup W] # the reference's CPU path (oracle port)
-    torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...     # N > 1: one rank per GPU
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this framework (CUDA kernels)
+    python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]       # the reference's CPU path (oracle port)
+    torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...           # N > 1: one rank per GPU
 
 One "step" = one pass of the single-step kernel (RandomCartPoleEnv.step + TimeLimit + auto-reset + uniform DR
 resample on reset) over one batch of 2^20 envs -- BASELINE.json configs[1].  Per rank, 4 independent batches
-(248 MB > 126 MB L2) are stepped round-robin so every launch streams its working set from HBM.  The steps are
-captured in a CUDA graph (a 10 us kernel is otherwise bound by the Python/ctypes launch path); the graph
-holds the K steps ceil(400 / K) times over and is replayed until >= 200 x K steps and >= 50 ms have been timed, with a
-CUDA event after every replay: `ms_per_step` is the median replay / steps in the graph, the spread is reported beside it,
-and the eager public-API rate is reported as `value_eager`.
+(248 MB > 126 MB L2) are stepped round-robin so every launch streams its working set from HBM.  The K timed steps are
+captured in a CUDA graph (a 10 us kernel is otherwise bound by the Python/ctypes launch path); after W eager warm-up
+steps, the graph is replayed twice back to back and the second replay -- the K steps -- alone is timed between two CUDA
+events: `ms_per_step` is that replay / K.  The eager public-API rate over K steps is reported as `value_eager`.
+
+`--dump-outputs DIR` writes what the last timed step returned (obs, reward, done of the batch it stepped; rank 0) as
+DIR/<name>.npy.  Every input is seeded, so two builds run with the same arguments can be compared output for output.
 
 The reference arm (`--impl reference`) runs the REFERENCE's own RandomCartPoleEnv objects (oracle/_ref, see
 oracle/make_ref.py; the bit-exact port only if those copies are absent) on all host cores for >= 2 s whatever --steps is.
@@ -34,6 +36,7 @@ FLOPS_PER_STEP_ROLLOUT = 43                          # SURVEY.md section 8d: dyn
 SEARCH = [2.0, 20.0, 0.5, 3.0, 0.05, 0.3, 0.1, 1.0]  # random_cartpole.py:127-132 = BASELINE cfg 1/2 DR
 METRIC = "DR env-steps/sec (RandomCartPole-v0 single-step kernel, uniform DR resample on reset)"
 UNIT = "env-steps/s"
+SPIN_CYCLES = 400000                                 # torch.cuda._sleep before an event-timed region: ~200 us busy stream
 
 
 def parse_args():
@@ -49,9 +52,12 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--ref-seconds", type=float, default=4.0, help="wall time of the reference arm's timed region")
-    ap.add_argument("--min-replays", type=int, default=200)
-    ap.add_argument("--min-region-ms", type=float, default=50.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, <= 64 MB)")
+    args = ap.parse_args()
+    if args.impl == "b200" and args.steps < 1:
+        ap.error("--steps must be >= 1")
+    return args
 
 
 def workload_config(args, world):
@@ -171,6 +177,24 @@ def ncu_traffic(dtype):
         return None
 
 
+def dump_outputs(directory, arrays, limit_bytes=60 << 20):
+    """Write `arrays` (name -> tensor whose first dimension is the env) as DIR/<name>.npy.  If they hold more than
+    `limit_bytes` (60 MiB: the files stay below 64 MB), the same fixed, seeded sample of env rows is written from each,
+    with its row indices as env_index.npy."""
+    import numpy as np
+    import torch
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[0].numel() * a.element_size() for a in arrays.values())
+    if n * row_bytes > limit_bytes:
+        idx = np.sort(np.random.default_rng(0).choice(n, limit_bytes // (row_bytes + 8), replace=False))
+        rows = torch.from_numpy(idx)
+        arrays = {name: a.index_select(0, rows.to(a.device)) for name, a in arrays.items()}
+        arrays["env_index"] = torch.from_numpy(idx.astype(np.float64))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a.cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------------- b200 arm
 def run_b200(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -229,10 +253,6 @@ def run_b200(args):
 
     n, R, A = args.envs, args.batches, 8
     K = args.steps
-    # one captured graph holds K * reps_in_graph steps (>= 400): a 20-step graph is 0.23 ms of GPU work and its replay
-    # rate would measure the host's graph-launch gap, not the kernel
-    reps_in_graph = max(1, -(-400 // K))
-    G = K * reps_in_graph
 
     def make_batches(tile_ordering):
         envs, actions = [], []
@@ -251,10 +271,14 @@ def run_b200(args):
         torch.cuda.synchronize()
         return envs, actions
 
-    def stepper(envs, actions):
+    def stepper(envs, actions, returned=None):
+        """step_i(i) steps batch i % R; `returned[b]` keeps what the last step of batch b returned (views of the env's
+        buffers, refreshed in place by every later step, graph replays included)."""
         def step_i(i):
             b = i % R
-            envs[b].step(actions[b][(i // R) % A])
+            out = envs[b].step(actions[b][(i // R) % A])
+            if returned is not None:
+                returned[b] = out
         return step_i
 
     # the same K steps as one CUDA graph.  `chain`: one stream, launches in stream order.  `branches`: the R
@@ -267,42 +291,34 @@ def run_b200(args):
         with torch.cuda.stream(side):
             with torch.cuda.graph(g, stream=side):
                 if not parallel:
-                    for i in range(G):
+                    for i in range(K):
                         step_i(i)
                 else:
                     lanes = [torch.cuda.Stream(device=dev) for _ in range(R)]
                     for b, lane in enumerate(lanes):
                         lane.wait_stream(side)
                         with torch.cuda.stream(lane):
-                            for i in range(b, G, R):
+                            for i in range(b, K, R):
                                 step_i(i)
                     for lane in lanes:
                         side.wait_stream(lane)
         torch.cuda.current_stream().wait_stream(side)
-        g.replay()                                  # untimed: first launch uploads the graph
-        torch.cuda.synchronize()
         return g
 
-    def time_replays(graph, replays):
-        """`replays` back-to-back replays of a K-step graph with a CUDA event after each one (an event record does not
-        serialise anything): returns per-replay milliseconds (max over ranks of each percentile is taken by the caller)
-        and the whole region."""
-        ev = [torch.cuda.Event(enable_timing=True) for _ in range(replays + 1)]
+    def time_graph(graph):
+        """Two back-to-back replays of a K-step graph; the second alone is timed between two CUDA events (max over
+        ranks, milliseconds).  The first uploads the graph and keeps the GPU busy with the same K steps while the host
+        queues the second, and a spin kernel queued before both covers the host's launch latency: the events bracket
+        the K steps, not the host (a 20-step graph is only ~0.23 ms of GPU work) and not the ramp of an idle GPU."""
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier(); torch.cuda.synchronize()
-        ev[0].record()
-        for r in range(replays):
-            graph.replay()
-            ev[r + 1].record()
+        torch.cuda._sleep(SPIN_CYCLES)
+        graph.replay()
+        e0.record(); graph.replay(); e1.record()
         torch.cuda.synchronize(); barrier()
-        per = sorted(ev[r].elapsed_time(ev[r + 1]) for r in range(replays))
-        return per, ev[0].elapsed_time(ev[-1])
-
-    def pct(per, q):
-        return per[min(len(per) - 1, int(q * len(per)))]
+        return max_over_ranks(e0.elapsed_time(e1))
 
     bytes_per = BYTES_PER_STEP[args.dtype]
-    est_ms = G * n * bytes_per / 5.5e12 * 1e3                       # a first guess of one replay
-    replays = int(max(-(-args.min_replays // reps_in_graph), -(-args.min_region_ms // est_ms), 10))
 
     # ---- (1) the public API as a user drives it: default env (tile-granular step ordering at this size), ONE stream
     envs_t, actions_t = make_batches("auto")
@@ -310,48 +326,48 @@ def run_b200(args):
     for i in range(max(args.warmup, 3)):
         step_t(i)
     torch.cuda.synchronize()
-    k_eager = max(K, 400)
-    ms_eager = timed(lambda: [step_t(i) for i in range(k_eager)])
+    ms_eager = timed(lambda: [step_t(i) for i in range(K)])
     chain = capture(step_t, False)
-    per_chain, _ = time_replays(chain, replays)
-    ms_chain = max_over_ranks(pct(per_chain, 0.5))
+    ms_chain = time_graph(chain)
     del chain
 
     # ---- (2) the headline: grid-ordered launches, the R independent batches on R parallel graph branches
     envs, actions = make_batches(False)
-    step_g = stepper(envs, actions)
+    returned = {}
+    step_g = stepper(envs, actions, returned)
     for i in range(max(args.warmup, 3)):
         step_g(i)
     torch.cuda.synchronize()
     chain_g = capture(step_g, False)
-    per_chain_g, _ = time_replays(chain_g, replays)
-    ms_chain_g = max_over_ranks(pct(per_chain_g, 0.5))
+    ms_chain_g = time_graph(chain_g)
     del chain_g
     graph = capture(step_g, True)
 
     clocks = ClockSampler(local_rank).start() if rank == 0 else None
     t_wall0 = time.time()
-    per, region_ms = time_replays(graph, replays)
+    ms = time_graph(graph)
+    # what the last timed step returned, copied before anything steps these envs again
+    obs_last, reward_last, done_last, _ = returned[(K - 1) % R]
+    outputs = {"obs": obs_last.clone(memory_format=torch.contiguous_format), "reward": reward_last.clone(),
+               "done": done_last.to(torch.float32)}
     # keep the GPU under the same load for >= 0.5 s so that nvidia-smi gets samples of the timed workload
     while time.time() - t_wall0 < 0.6:
         graph.replay()
     torch.cuda.synchronize()
     t_wall1 = time.time()
     clock_info = clocks.stop(t_wall0, t_wall1) if clocks else None
-    ms = max_over_ranks(pct(per, 0.5))              # median replay of the K-step graph
-    region_ms = max_over_ranks(region_ms)
-    spread = {"graph_steps": G, "replays": replays, "steps_timed": G * replays, "region_ms": region_ms,
-              "p05_us_per_step": 1e3 * max_over_ranks(pct(per, 0.05)) / G, "p50_us_per_step": 1e3 * ms / G,
-              "p95_us_per_step": 1e3 * max_over_ranks(pct(per, 0.95)) / G, "mean_us_per_step": 1e3 * region_ms / (replays * G)}
-    value = world * n * G / (ms * 1e-3)
-    value_eager = world * n * k_eager / (ms_eager * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
+    del outputs
+    value = world * n * K / (ms * 1e-3)
+    value_eager = world * n * K / (ms_eager * 1e-3)
 
     # one launch in isolation (sync on both sides, the 4 batches rotating so that it streams from HBM): the number an
     # ncu launch list shows; the amortised figures above overlap consecutive launches
     def bracket(with_kernel, i):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize()
-        torch.cuda._sleep(400000)       # ~200 us of busy stream: what follows is queued before the GPU gets to it,
+        torch.cuda._sleep(SPIN_CYCLES)  # ~200 us of busy stream: what follows is queued before the GPU gets to it,
         e0.record()                     # so the events bracket the kernel and not the host's launch latency
         if with_kernel:
             step_g(i)
@@ -363,21 +379,21 @@ def run_b200(args):
     iso_us = 1e3 * max_over_ranks(iso[len(iso) // 2] - empty[len(empty) // 2])
 
     peak, peak_src = measured_peaks()
-    per_launch_ms = ms / G
+    per_launch_ms = ms / K
     achieved = bytes_per * n / (per_launch_ms * 1e-3) / 1e9
     roofline = {"bound": "hbm", "kernel": "cartpole_step_kernel<%s>" % ("float" if args.dtype == "float32" else "double"),
                 "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak, "peak_source": peak_src,
                 "bytes_per_env_step": bytes_per, "launch_us": per_launch_ms * 1e3, "isolated_launch_us": iso_us,
-                "launch_us_note": "launch_us = median graph replay / K with consecutive launches overlapping (amortised); "
+                "launch_us_note": "launch_us = graph replay / K with consecutive launches overlapping (amortised); "
                                   "isolated_launch_us = one launch alone on the GPU, nothing before or after it to overlap "
                                   "with (event pair behind a spin kernel minus the same pair with nothing in between; it still "
                                   "contains the launch ramp of a cold stream -- the ncu launch list under profiles/ has the "
                                   "kernel-only duration)",
                 "traffic": ncu_traffic(args.dtype)}
 
-    def roof(ms_g):
-        gbs = bytes_per * n / (ms_g / G * 1e-3) / 1e9
-        return {"launch_us": 1e3 * ms_g / G, "achieved": gbs, "frac": gbs / peak}
+    def roof(ms_k):
+        gbs = bytes_per * n / (ms_k / K * 1e-3) / 1e9
+        return {"launch_us": 1e3 * ms_k / K, "achieved": gbs, "frac": gbs / peak}
 
     # ---- end to end through the public host-buffer API: pinned H2D actions, D2H obs/reward/done every step.
     # The R env batches are stepped round-robin with one step in flight per batch (step_host_async / _wait), so
@@ -429,16 +445,15 @@ def run_b200(args):
     line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": args.warmup,
             "ms_per_step": per_launch_ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32" if args.dtype == "float32" else "f64", "data": "synthetic",
-            "config": workload_config(args, world), "clocks": clock_info, "e2e": e2e, "gpu_launches": G * replays,
-            "launch_mode": "one CUDA graph of %d cartpole_step_kernel launches (the K = %d steps x %d), the %d independent "
-                           "env batches on %d parallel graph branches (grid-ordered launches); the graph is replayed %d "
-                           "times back to back (%.0f ms), ms_per_step = median replay / %d"
-                           % (G, K, reps_in_graph, R, R, replays, region_ms, G),
-            "timing": spread,
-            "value_eager": value_eager, "value_graph_single_chain": world * n * G / (ms_chain * 1e-3),
+            "config": workload_config(args, world), "clocks": clock_info, "e2e": e2e, "gpu_launches": K,
+            "launch_mode": "one CUDA graph of the K = %d cartpole_step_kernel launches, the %d independent env batches on "
+                           "%d parallel graph branches (grid-ordered launches); one replay is timed (%.3f ms) directly "
+                           "after an untimed one, ms_per_step = replay / %d" % (K, R, R, ms, K),
+            "timing": {"steps_timed": K, "region_ms": ms},
+            "value_eager": value_eager, "value_graph_single_chain": world * n * K / (ms_chain * 1e-3),
             "single_stream": {"note": "the default env (tile-granular step ordering, include/renv.h progress) on ONE "
                                       "stream: what a plain step() loop over %d env batches gets" % R,
-                              "eager_python_loop": roof(ms_eager * G / k_eager), "graph_chain": roof(ms_chain),
+                              "eager_python_loop": roof(ms_eager), "graph_chain": roof(ms_chain),
                               "graph_chain_grid_ordered": roof(ms_chain_g)},
             "roofline_single_chain": roof(ms_chain),
             "roofline": roofline, "cpu_baseline": cpu_baseline, "extras": extras}

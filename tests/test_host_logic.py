@@ -13,7 +13,7 @@ import random_envs_b200 as random_envs
 from random_envs_b200 import gym
 from oracle import reference_loader as rl
 
-needs_ref = pytest.mark.skipif(not rl.available(), reason="/root/reference not mounted")
+needs_ref = pytest.mark.skipif(not rl.available(), reason=rl.UNAVAILABLE)
 SEARCH = [2, 20, 0.5, 3, 0.05, 0.3, 0.1, 1.0]
 
 

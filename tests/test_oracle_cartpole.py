@@ -12,7 +12,7 @@ import pytest
 
 from oracle import c_oracle, cartpole_port as port, reference_loader as rl
 
-needs_ref = pytest.mark.skipif(not rl.available(), reason="/root/reference not mounted")
+needs_ref = pytest.mark.skipif(not rl.available(), reason=rl.UNAVAILABLE)
 
 
 def _episodes(t):
@@ -109,10 +109,13 @@ def test_action_check_matches_gym_021():
             env.step(bad)
 
 
-def test_constants():
+def test_constants(golden_dir):
     assert port.THETA_THRESHOLD == 0.20943951023931953
     assert port.POLEMASS_LENGTH == 0.05
     assert port.SEARCH_BOUNDS == ((2.0, 20.0), (0.5, 3.0), (0.05, 0.3), (0.1, 1.0))
+    # the reference's own get_task_lower_bound(i), recorded by oracle/make_golden.py
+    ref_lb = np.load(os.path.join(golden_dir, "sampler_reference_draws.npz"))["truncnorm_lb"]
+    assert tuple(float(v) for v in ref_lb) == tuple(port.LOWER_BOUNDS)
 
 
 def test_philox_known_answers():

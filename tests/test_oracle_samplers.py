@@ -12,7 +12,7 @@ from scipy import stats
 
 from oracle import dr_port, reference_loader as rl
 
-needs_ref = pytest.mark.skipif(not rl.available(), reason="/root/reference not mounted")
+needs_ref = pytest.mark.skipif(not rl.available(), reason=rl.UNAVAILABLE)
 
 
 def _script(values):
@@ -95,7 +95,6 @@ def test_port_sample_task_shapes_and_errors():
         dr_port.sample_task(None, [1.0], [1.0])
 
 
-@needs_ref
 def test_truncnorm_rvs_is_inverse_cdf_of_one_uniform():
     """scipy's truncnorm.rvs == ppf(U): the GPU sampler's inverse-CDF design reproduces the same map."""
     import scipy.stats
