@@ -113,6 +113,25 @@ typedef struct renv_cartpole_env {
     uint64_t seed;               /* Philox key */
 } renv_cartpole_env;
 
+/* Episode log of a renv_cartpole_env (device pointers, T as there; row stride = the env's ld).  Every episode of env i
+ * that ENDS in a logged step or rollout -- terminated by the thresholds or truncated by the TimeLimit -- writes one
+ * record into slot j = count[i] mod capacity, then count[i] += 1: a per-env ring holding the latest
+ * min(count[i], capacity) episodes (count[i] - capacity, when positive, were overwritten).  Record slot j of env i is
+ * row j * ld + i of each field.  Written by the one thread that resets env i: no atomics, and the content does not
+ * depend on launch geometry, tile ordering or sharding; a K-step rollout at tick t logs what K steps at ticks
+ * t .. t+K-1 log.  A reset (renv_cartpole_reset_*) abandons running episodes without logging them. */
+typedef struct renv_episode_log {
+    void *xi;                    /* T (capacity, ld, 4) rows, 16-byte aligned: the task the episode ran under (before the
+                                    resample of its reset) */
+    void *final_state;           /* T (capacity, ld, 4) rows, 16-byte aligned: x, x_dot, theta, theta_dot after the step
+                                    that ended it -- what a step without auto-reset returns (terminal observation) */
+    int32_t *length;             /* (capacity, ld), 4-byte aligned: env-steps of the episode, across calls (= its return) */
+    uint8_t *truncated;          /* (capacity, ld): 1 when the TimeLimit ended it without meeting the thresholds */
+    int64_t *end_tick;           /* (capacity, ld), 8-byte aligned: step clock of the step that ended it */
+    int32_t *count;              /* (ld), 4-byte aligned: records written per env since the caller zeroed it */
+    int64_t capacity;            /* records per env, 1 <= capacity <= 2^31 - 1 */
+} renv_episode_log;
+
 int renv_abi_version(void);
 const char *renv_strerror(int code);
 
@@ -205,6 +224,23 @@ int renv_cartpole_rollout_noisy_f32(const renv_cartpole_env *env, const renv_obs
 int renv_cartpole_rollout_noisy_f64(const renv_cartpole_env *env, const renv_obs_noise *noise, const double w[4], double b,
                                     int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
                                     double *stats, unsigned long long *violations, void *stream);
+
+/* renv_cartpole_step_* with auto-reset (implied) and renv_cartpole_rollout_* (w == NULL: random policy), plus the
+ * episode log `log` (see renv_episode_log).  State, xi, counters, flags and stats are exactly those of the plain entry
+ * points.  log == NULL or a NULL field: RENV_E_NULL; capacity outside [1, 2^31 - 1]: RENV_E_SIZE; misaligned field:
+ * RENV_E_ALIGN. */
+int renv_cartpole_step_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log, const uint8_t *action,
+                                  float *reward, uint8_t *done, uint8_t *truncated, int integrator, int max_steps,
+                                  uint64_t tick, const renv_dr_cfg *dr, unsigned long long *counters, void *stream);
+int renv_cartpole_step_logged_f64(const renv_cartpole_env *env, const renv_episode_log *log, const uint8_t *action,
+                                  double *reward, uint8_t *done, uint8_t *truncated, int integrator, int max_steps,
+                                  uint64_t tick, const renv_dr_cfg *dr, unsigned long long *counters, void *stream);
+int renv_cartpole_rollout_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log, const double w[4], double b,
+                                     int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                     double *stats, unsigned long long *violations, void *stream);
+int renv_cartpole_rollout_logged_f64(const renv_cartpole_env *env, const renv_episode_log *log, const double w[4], double b,
+                                     int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                     double *stats, unsigned long long *violations, void *stream);
 
 /* The SCALAR drop-in env (gym.make('RandomCartPole-v0'): RandomCartPoleEnv.step / reset, random_cartpole.py:172-229,
  * one env, one host call per step) served by a resident one-warp kernel instead of one launch + synchronise per call.

@@ -45,9 +45,17 @@ class ObsNoise(ctypes.Structure):
     _fields_ = [("obs", ctypes.c_void_p), ("std", ctypes.c_double)]
 
 
+class EpisodeLog(ctypes.Structure):
+    """struct renv_episode_log (include/renv.h)."""
+    _fields_ = [("xi", ctypes.c_void_p), ("final_state", ctypes.c_void_p), ("length", ctypes.c_void_p),
+                ("truncated", ctypes.c_void_p), ("end_tick", ctypes.c_void_p), ("count", ctypes.c_void_p),
+                ("capacity", ctypes.c_int64)]
+
+
 _vp, _i64, _u64, _u32, _int, _dbl = (ctypes.c_void_p, ctypes.c_int64, ctypes.c_uint64, ctypes.c_uint32,
                                      ctypes.c_int, ctypes.c_double)
 _cfg_p, _env_p, _noise_p = ctypes.POINTER(DrCfg), ctypes.POINTER(CartpoleEnv), ctypes.POINTER(ObsNoise)
+_log_p = ctypes.POINTER(EpisodeLog)
 
 # name -> (restype, argtypes); must list every function declared in include/renv.h
 SIGNATURES = {
@@ -68,6 +76,10 @@ SIGNATURES = {
     "renv_cartpole_rollout_f64": (_int, [_env_p, ctypes.POINTER(_dbl), _dbl, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
     "renv_cartpole_rollout_noisy_f32": (_int, [_env_p, _noise_p, ctypes.POINTER(_dbl), _dbl, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
     "renv_cartpole_rollout_noisy_f64": (_int, [_env_p, _noise_p, ctypes.POINTER(_dbl), _dbl, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
+    "renv_cartpole_step_logged_f32": (_int, [_env_p, _log_p, _vp, _vp, _vp, _vp, _int, _int, _u64, _cfg_p, _vp, _vp]),
+    "renv_cartpole_step_logged_f64": (_int, [_env_p, _log_p, _vp, _vp, _vp, _vp, _int, _int, _u64, _cfg_p, _vp, _vp]),
+    "renv_cartpole_rollout_logged_f32": (_int, [_env_p, _log_p, ctypes.POINTER(_dbl), _dbl, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
+    "renv_cartpole_rollout_logged_f64": (_int, [_env_p, _log_p, ctypes.POINTER(_dbl), _dbl, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),
     "renv_random_actions_u8": (_int, [_vp, _i64, _u64, _u64, _u32, _vp]),
     "renv_pack_flags_u8": (_int, [_vp, _vp, _i64, _vp]),

@@ -93,6 +93,25 @@ template <typename T> int attach_noise(const renv_obs_noise *noise, EnvPtrs<T> *
     return RENV_OK;
 }
 
+template <typename T> int check_log(const renv_episode_log *log, LogPtrs<T> *out)
+{
+    if (log == nullptr || log->xi == nullptr || log->final_state == nullptr || log->length == nullptr ||
+        log->truncated == nullptr || log->end_tick == nullptr || log->count == nullptr)
+        return RENV_E_NULL;
+    if (log->capacity < 1 || log->capacity > 0x7fffffffLL) return RENV_E_SIZE;
+    if (!aligned(log->xi, 16) || !aligned(log->final_state, 16) || !aligned(log->length, 4) || !aligned(log->end_tick, 8) ||
+        !aligned(log->count, 4))
+        return RENV_E_ALIGN;
+    out->xi = static_cast<T *>(log->xi);
+    out->final_state = static_cast<T *>(log->final_state);
+    out->length = log->length;
+    out->truncated = log->truncated;
+    out->end_tick = log->end_tick;
+    out->count = log->count;
+    out->capacity = (uint32_t)log->capacity;
+    return RENV_OK;
+}
+
 inline int launch_status() { return (int)cudaGetLastError(); }
 
 #ifndef RENV_STEP_PDL
@@ -259,13 +278,16 @@ int cartpole_reset(const renv_cartpole_env *env, const renv_obs_noise *noise, co
 template <typename T, bool kLean>
 int cartpole_step(const renv_cartpole_env *env, const renv_obs_noise *noise, const uint8_t *action, T *reward,
                   uint8_t *done, uint8_t *truncated, int integrator, int max_steps, int auto_reset, uint64_t tick,
-                  const renv_dr_cfg *dr, unsigned long long *counters, void *stream)
+                  const renv_dr_cfg *dr, unsigned long long *counters, void *stream,
+                  const renv_episode_log *log = nullptr, bool logged = false)
 {
     StepArgs<T> a;
     int rc = check_env<T>(env, !auto_reset, &a.env, kLean ? kNeedElapsed16 : kNeedElapsed32);
     if (rc) return rc;
     rc = attach_noise<T>(noise, &a.env);
     if (rc) return rc;
+    LoggedStepArgs<T> la;
+    if (logged && (rc = check_log<T>(log, &la.log))) return rc;
     if (action == nullptr || done == nullptr) return RENV_E_NULL;
     if (reward == nullptr && !auto_reset) return RENV_E_NULL;      // only the auto-reset reward is the constant 1.0
     if (!aligned(action, 4) || !aligned(reward, 16) || !aligned(done, 4) || (truncated && !aligned(truncated, 4)))
@@ -285,6 +307,10 @@ int cartpole_step(const renv_cartpole_env *env, const renv_obs_noise *noise, con
     if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     const bool noisy = a.env.obs != nullptr;
+    if (logged) {
+        la.step = a;
+        return launch_pdl(cartpole_step_logged_kernel<T>, (unsigned)blocks, kStepThreads, st, la);
+    }
     if (kLean) return launch_pdl(cartpole_step_kernel<T, true, false, true>, (unsigned)blocks, kStepThreads, st, a);
     if (auto_reset && !noisy) return launch_pdl(cartpole_step_kernel<T, true, false>, (unsigned)blocks, kStepThreads, st, a);
     if (auto_reset) return launch_pdl(cartpole_step_kernel<T, true, true>, (unsigned)blocks, kStepThreads, st, a);
@@ -301,6 +327,14 @@ template <typename T> int launch_rollout_random(const RolloutArgs<T> &a, cudaStr
     if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
     if (a.euler) cartpole_rollout_kernel<T, true, false, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
     else cartpole_rollout_kernel<T, false, false, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
+    return launch_status();
+}
+template <typename T> int launch_rollout_random(const LoggedRolloutArgs<T> &a, cudaStream_t stream)
+{
+    const int64_t blocks = (a.roll.env.n + kRolloutThreads - 1) / kRolloutThreads;
+    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    if (a.roll.euler) cartpole_rollout_logged_kernel<T, true, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
+    else cartpole_rollout_logged_kernel<T, false, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
     return launch_status();
 }
 // Noisy variant (policy on the noisy observation): one env per thread for both element types.
@@ -339,17 +373,38 @@ int launch_rollout(const RolloutArgs<float> &a, cudaStream_t stream)
 #endif
     return launch_status();
 }
+// Logged linear-policy rollouts: the same kernel choice as above.
+int launch_rollout(const LoggedRolloutArgs<double> &a, cudaStream_t stream)
+{
+    const int64_t blocks = (a.roll.env.n + kRolloutThreads - 1) / kRolloutThreads;
+    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    if (a.roll.euler) cartpole_rollout_logged_kernel<double, true, false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
+    else cartpole_rollout_logged_kernel<double, false, false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
+    return launch_status();
+}
+int launch_rollout(const LoggedRolloutArgs<float> &a, cudaStream_t stream)
+{
+    const int64_t threads = (a.roll.env.n + kPairSlots - 1) / kPairSlots;
+    const int64_t blocks = (threads + kRolloutThreads - 1) / kRolloutThreads;
+    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    if (a.roll.euler) cartpole_rollout_pair_logged_kernel<true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
+    else cartpole_rollout_pair_logged_kernel<false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
+    return launch_status();
+}
 
 template <typename T>
 int cartpole_rollout(const renv_cartpole_env *env, const renv_obs_noise *noise, const double w[4], double b, int K,
                      int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
-                     unsigned long long *violations, void *stream)
+                     unsigned long long *violations, void *stream, const renv_episode_log *log = nullptr,
+                     bool logged = false)
 {
     RolloutArgs<T> a;
     int rc = check_env<T>(env, false, &a.env);
     if (rc) return rc;
     rc = attach_noise<T>(noise, &a.env);
     if (rc) return rc;
+    LoggedRolloutArgs<T> la;
+    if (logged && (rc = check_log<T>(log, &la.log))) return rc;
     if (stats == nullptr) return RENV_E_NULL;
     if (w == nullptr && noise != nullptr) return RENV_E_ARG;      // the random policy does not look at observations
     if (!aligned(stats, 8)) return RENV_E_ALIGN;
@@ -364,8 +419,13 @@ int cartpole_rollout(const renv_cartpole_env *env, const renv_obs_noise *noise, 
     a.tick = tick;
     a.stats = stats;
     a.violations = violations;
-    if (w == nullptr) return launch_rollout_random(a, static_cast<cudaStream_t>(stream));
-    return launch_rollout(a, static_cast<cudaStream_t>(stream));
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (logged) {
+        la.roll = a;
+        return w == nullptr ? launch_rollout_random(la, st) : launch_rollout(la, st);
+    }
+    if (w == nullptr) return launch_rollout_random(a, st);
+    return launch_rollout(a, st);
 }
 
 }  // namespace
@@ -475,6 +535,35 @@ int renv_cartpole_rollout_f64(const renv_cartpole_env *env, const double w[4], d
                               unsigned long long *violations, void *stream)
 {
     return cartpole_rollout<double>(env, nullptr, w, b, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+
+int renv_cartpole_step_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log, const uint8_t *action,
+                                  float *reward, uint8_t *done, uint8_t *truncated, int integrator, int max_steps,
+                                  uint64_t tick, const renv_dr_cfg *dr, unsigned long long *counters, void *stream)
+{
+    return cartpole_step<float, false>(env, nullptr, action, reward, done, truncated, integrator, max_steps, 1, tick, dr,
+                                       counters, stream, log, true);
+}
+int renv_cartpole_step_logged_f64(const renv_cartpole_env *env, const renv_episode_log *log, const uint8_t *action,
+                                  double *reward, uint8_t *done, uint8_t *truncated, int integrator, int max_steps,
+                                  uint64_t tick, const renv_dr_cfg *dr, unsigned long long *counters, void *stream)
+{
+    return cartpole_step<double, false>(env, nullptr, action, reward, done, truncated, integrator, max_steps, 1, tick, dr,
+                                        counters, stream, log, true);
+}
+int renv_cartpole_rollout_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log, const double w[4], double b,
+                                     int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                     double *stats, unsigned long long *violations, void *stream)
+{
+    return cartpole_rollout<float>(env, nullptr, w, b, K, integrator, max_steps, tick, dr, stats, violations, stream, log,
+                                   true);
+}
+int renv_cartpole_rollout_logged_f64(const renv_cartpole_env *env, const renv_episode_log *log, const double w[4], double b,
+                                     int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                     double *stats, unsigned long long *violations, void *stream)
+{
+    return cartpole_rollout<double>(env, nullptr, w, b, K, integrator, max_steps, tick, dr, stats, violations, stream, log,
+                                    true);
 }
 
 int renv_cartpole_rollout_noisy_f32(const renv_cartpole_env *env, const renv_obs_noise *noise, const double w[4], double b,

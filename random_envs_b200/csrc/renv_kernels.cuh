@@ -98,6 +98,33 @@ __device__ __forceinline__ unsigned reset_env(const EnvPtrs<T> &env, const DrCfg
     return viol;
 }
 
+// Episode log (include/renv.h renv_episode_log): a per-env ring of `capacity` records.  Record r of env i lives at
+// row (r mod capacity) * ld + i of every field; count[i] is the number of records env i has written.  Only the
+// thread that resets env i writes them, so no atomics are needed and the content is independent of launch geometry.
+template <typename T> struct LogPtrs {
+    T *xi; T *final_state; int32_t *length; uint8_t *truncated; int64_t *end_tick; int32_t *count;
+    uint32_t capacity;
+};
+
+// the termination test of dynamics() (:200-205), for a record whose episode ended: truncated = !this && length >= limit
+template <typename T> __device__ __forceinline__ bool beyond_thresholds(const State<T> &s)
+{
+    return s.x < -(T)kXThreshold || s.x > (T)kXThreshold || s.theta < -(T)kThetaThreshold || s.theta > (T)kThetaThreshold;
+}
+
+// Writes record number `count` of env i (the caller stores count + 1).
+template <typename T>
+__device__ __forceinline__ void log_episode(const LogPtrs<T> &log, int64_t ld, int64_t i, uint32_t count, const Xi<T> &xi,
+                                            const State<T> &s, int32_t length, bool truncated, uint64_t tick)
+{
+    const int64_t r = (int64_t)(count % log.capacity) * ld + i;
+    store_xi(log.xi, r, xi);
+    store_xi(log.final_state, r, Xi<T>{ s.x, s.x_dot, s.theta, s.theta_dot });      // the same 4-wide row layout
+    log.length[r] = length;
+    log.truncated[r] = truncated ? 1 : 0;
+    log.end_tick[r] = (int64_t)tick;
+}
+
 // ------------------------------------------------------------------------------------------------
 // Single step: RandomCartPoleEnv.step + TimeLimit.step + SyncVectorEnv auto-reset (+ set_random_task)
 // ------------------------------------------------------------------------------------------------
@@ -179,186 +206,28 @@ constexpr int kStepThreads = RENV_STEP_THREADS;
 //     streaming tiles through a shared-memory ring with cp.async.bulk (12.1 us in the best of 15 configurations, one
 //     of which hung), and CTAs that step 2 or 4 tiles (a loop makes ptxas spill the freshly loaded rows; straight-line
 //     copies blow the instruction cache: 16 us).
+//
+// kLog (cartpole_step_logged_kernel, auto-reset only): the thread that resets env i first writes the record of the
+// episode that ended -- the xi row before its resample, the state the owner stored, the length and truncated bit the
+// owner staged in s_len -- into the episode log.  All of it precedes the tile's release / the end of the grid.
 template <typename T, bool kAutoReset, bool kNoisy = false, bool kLean = false>
 __global__ void __launch_bounds__(kStepThreads, kNoisy ? (sizeof(T) == 8 ? 2 : 3) : RENV_STEP_MIN_CTAS(T)) cartpole_step_kernel(const __grid_constant__ StepArgs<T> a)
 {
-    using VT = VecTraits<T>;
-    constexpr int V = VT::V;
-    constexpr int kTile = kStepThreads * V;
-    __shared__ unsigned s_count;
-    __shared__ uint16_t s_list[kAutoReset ? kTile : 1];
-    const int64_t block0 = (int64_t)blockIdx.x * kTile;
-    const int64_t i0 = block0 + (int64_t)threadIdx.x * V;
-    const int64_t n = a.env.n, ld = a.env.ld;
-    const bool live = i0 < n;
-    const bool full = i0 + V <= n;
-    const bool tracked = a.env.progress != nullptr;
-    uint32_t ticket = 0;
+    constexpr bool kLog = false;
+    const LogPtrs<T> log = {};
+#include "renv_step_body.cuh"
+}
 
-    if (tracked) {
-        if (threadIdx.x == 0) {
-            uint32_t *const slot = a.env.progress + 2 * (size_t)blockIdx.x;
-            ticket = atomicAdd(slot, 1u);
-            uint32_t seen = ld_acquire_gpu(slot + 1);
-            for (int spin = 0; seen != ticket && spin < RENV_ORDER_SPINS; ++spin) {     // rare: the predecessor is still on this tile
-                __nanosleep(32);
-                seen = ld_acquire_gpu(slot + 1);
-            }
-            if (seen != ticket && a.counters) atomicAdd(a.counters + kCounterOrderTimeout, 1ull);
-            if (kAutoReset) s_count = 0;
-        } else if (RENV_TILE_PREFETCH && block0 + kTile <= n && threadIdx.x >= 32 && threadIdx.x < 39) {
-            // while thread 0 waits for its L2 round trip the tile is pulled from HBM into L2 (never stale: L2 is the
-            // point of coherence), so the loads below pay an L2 hit instead of a second DRAM latency
-            const int q = threadIdx.x - 32;
-            if (q < 4) prefetch_l2(a.env.state + q * ld + block0, kTile * sizeof(T));
-            else if (q == 4) prefetch_l2(a.env.xi + 4 * block0, kTile * 4 * sizeof(T));
-            else if (q == 5) { if (kLean) prefetch_l2(a.env.elapsed16 + block0, kTile * 2); else prefetch_l2(a.env.elapsed + block0, kTile * 4); }
-            else prefetch_l2(a.action + block0, kTile);
-        }
-        __syncthreads();            // thread 0 holds the ticket and has seen the predecessor's release
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    } else {
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-    }
+template <typename T> struct LoggedStepArgs { StepArgs<T> step; LogPtrs<T> log; };
 
-    T s[4][V];
-    Xi<T> p[V];
-    int32_t el[V];
-    uint8_t act[V];
-    if (full) {     // all ten 128-bit requests go out before anything waits (incl. the barrier below)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) vload<typename VT::Real>(s[c], a.env.state + c * ld + i0);
-#pragma unroll
-        for (int v = 0; v < V; ++v) p[v] = load_xi(a.env.xi, i0 + v);
-        if (kLean) {
-            uint16_t e16[V];
-            vload<typename VT::Half>(e16, a.env.elapsed16 + i0);
-#pragma unroll
-            for (int v = 0; v < V; ++v) el[v] = e16[v];
-        } else {
-            vload<typename VT::Int>(el, a.env.elapsed + i0);
-        }
-        vload<typename VT::Byte>(act, a.action + i0);
-    }
-    if (kAutoReset && !tracked) {
-        if (threadIdx.x == 0) s_count = 0;
-        __syncthreads();            // overlaps the loads' latency
-    }
-
-    if (live) {
-        if (!full) {
-#pragma unroll
-            for (int v = 0; v < V; ++v) {
-                const bool ok = i0 + v < n;
-#pragma unroll
-                for (int c = 0; c < 4; ++c) s[c][v] = ok ? a.env.state[c * ld + i0 + v] : T(0);
-                p[v] = ok ? load_xi(a.env.xi, i0 + v) : Xi<T>{ T(1), T(1), T(1), T(1) };
-                el[v] = !ok ? 0 : kLean ? (int32_t)a.env.elapsed16[i0 + v] : a.env.elapsed[i0 + v];
-                act[v] = ok ? a.action[i0 + v] : 0;
-            }
-        }
-
-        T rew[V];
-        uint8_t dn[V], tr[V];
-        const bool euler = a.euler != 0;
-        bool bad_action = false;            // Discrete(2).contains (:173-174): the host raises at its next sync
-#pragma unroll
-        for (int v = 0; v < V; ++v) {
-            bad_action = bad_action || act[v] > 1;
-            State<T> st = { s[0][v], s[1][v], s[2][v], s[3][v] };
-            const bool terminated = dynamics(st, p[v], derive(p[v]), act[v], euler);
-            s[0][v] = st.x; s[1][v] = st.x_dot; s[2][v] = st.theta; s[3][v] = st.theta_dot;
-            el[v] += 1;                                                    // TimeLimit.step
-            bool done = terminated, trunc = false;
-            if (a.max_steps > 0 && el[v] >= a.max_steps) { trunc = !terminated; done = true; }
-            T r = T(1);                                                    // :207-212
-            if (!kAutoReset && i0 + v < n && terminated) {
-                const int32_t b = a.env.beyond[i0 + v];                    // :213-222 (only reachable without auto-reset)
-                a.env.beyond[i0 + v] = b < 0 ? 0 : b + 1;
-                r = b < 0 ? T(1) : T(0);
-            }
-            rew[v] = r; dn[v] = done; tr[v] = trunc;
-            if (kAutoReset && done && i0 + v < n) {
-                el[v] = 0;
-                s_list[atomicAdd(&s_count, 1u)] = (uint16_t)(threadIdx.x * V + v);
-            }
-        }
-        if (bad_action && a.counters) atomicAdd(a.counters + kCounterBadAction, 1ull);
-
-        if (kNoisy) {       // obs = new state + std * N(0, I); a finished env's obs is overwritten by its reset below
-            T o[4][V];
-#pragma unroll
-            for (int v = 0; v < V; ++v) {
-                T ov[4];
-                add_obs_noise(State<T>{ s[0][v], s[1][v], s[2][v], s[3][v] }, a.env.noise_std, a.env.seed,
-                              a.env.env_id0 + (uint64_t)(i0 + v), a.tick, 0u, ov);
-#pragma unroll
-                for (int c = 0; c < 4; ++c) o[c][v] = ov[c];
-            }
-            if (full) {
-#pragma unroll
-                for (int c = 0; c < 4; ++c) vstore<typename VT::Real>(a.env.obs + c * ld + i0, o[c]);
-            } else {
-#pragma unroll
-                for (int v = 0; v < V; ++v)
-                    if (i0 + v < n) {
-#pragma unroll
-                        for (int c = 0; c < 4; ++c) a.env.obs[c * ld + i0 + v] = o[c][v];
-                    }
-            }
-        }
-
-        // (a): trigger AFTER the arithmetic: the dependent grid becomes launchable when every CTA of this one is about
-        // to store, so its CTAs spin in griddepcontrol.wait only briefly.  Triggering at kernel entry was 4 % faster
-        // for one stream but cost 4 independent graph branches 1 % (round 1).
-        if (!tracked) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-        if (full) {
-#pragma unroll
-            for (int c = 0; c < 4; ++c) vstore<typename VT::Real>(a.env.state + c * ld + i0, s[c]);
-            if (kLean) {
-                uint16_t e16[V];
-#pragma unroll
-                for (int v = 0; v < V; ++v) e16[v] = (uint16_t)el[v];
-                vstore<typename VT::Half>(a.env.elapsed16 + i0, e16);
-            } else {
-                vstore<typename VT::Int>(a.env.elapsed + i0, el);
-            }
-            if (a.reward) vstore<typename VT::Real>(a.reward + i0, rew);
-            vstore<typename VT::Byte>(a.done + i0, dn);
-            if (a.truncated) vstore<typename VT::Byte>(a.truncated + i0, tr);
-        } else {
-#pragma unroll
-            for (int v = 0; v < V; ++v) {
-                if (i0 + v < n) {
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) a.env.state[c * ld + i0 + v] = s[c][v];
-                    if (kLean) a.env.elapsed16[i0 + v] = (uint16_t)el[v];
-                    else a.env.elapsed[i0 + v] = el[v];
-                    if (a.reward) a.reward[i0 + v] = rew[v];
-                    a.done[i0 + v] = dn[v];
-                    if (a.truncated) a.truncated[i0 + v] = tr[v];
-                }
-            }
-        }
-    } else if (!tracked) {
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    }
-
-    if (kAutoReset) {
-        __syncthreads();                    // list complete; the owners' stores above are ordered before ours
-        const unsigned count = s_count;
-        unsigned viol = 0;
-        for (unsigned j = threadIdx.x; j < count; j += kStepThreads)
-            viol += reset_env(a.env, a.dr, block0 + s_list[j], a.tick, a.env.seed);
-        if (viol && a.counters) atomicAdd(a.counters + kCounterGaussian, (unsigned long long)viol);
-    }
-    if (tracked) {
-        __syncthreads();                    // every store of the CTA precedes (happens-before) thread 0's release
-        if (threadIdx.x == 0) {
-            st_release_gpu(a.env.progress + 2 * (size_t)blockIdx.x + 1, ticket + 1u);
-            asm volatile("griddepcontrol.wait;" ::: "memory");     // do not complete before the previous grid has
-        }
-    }
+// The plain auto-reset step plus the episode log (a kernel of its own: the plain one keeps its parameter layout).
+template <typename T>
+__global__ void __launch_bounds__(kStepThreads, RENV_STEP_MIN_CTAS(T)) cartpole_step_logged_kernel(const __grid_constant__ LoggedStepArgs<T> args)
+{
+    constexpr bool kAutoReset = true, kNoisy = false, kLean = false, kLog = true;
+    const StepArgs<T> &a = args.step;
+    const LogPtrs<T> &log = args.log;
+#include "renv_step_body.cuh"
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -607,74 +476,28 @@ __device__ __forceinline__ void rollout_reset(RolloutThread<T> &t, const Rollout
 __device__ __forceinline__ float pin(float v) { asm volatile("" : "+f"(v)); return v; }
 __device__ __forceinline__ double pin(double v) { asm volatile("" : "+d"(v)); return v; }
 
+#define RENV_ROLLOUT_CTAS(T, kNoisy, kRandom) (sizeof(T) == 4 ? 3 : ((kNoisy) || (kRandom)) ? 2 : RENV_ROLLOUT_F64_CTAS)
+
 template <typename T, bool kEuler, bool kNoisy = false, bool kRandom = false>
-__global__ void __launch_bounds__(kRolloutThreads, (sizeof(T) == 4 ? 3 : (kNoisy || kRandom) ? 2 : RENV_ROLLOUT_F64_CTAS))
+__global__ void __launch_bounds__(kRolloutThreads, RENV_ROLLOUT_CTAS(T, kNoisy, kRandom))
 cartpole_rollout_kernel(const __grid_constant__ RolloutArgs<T> a)
 {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int64_t ld = a.env.ld;
-    const bool live = i < a.env.n;
-    const int64_t il = live ? i : 0;        // dead lanes of the last warp shadow env 0 with zero steps to do
+    constexpr bool kLog = false;
+    const LogPtrs<T> log = {};
+#include "renv_rollout_body.cuh"
+}
 
-    // per-thread episode statistics (return == length here: reward is 1.0 on every step, :207-212)
-    RolloutThread<T> t;
-    t.sum_r = 0; t.sum_r2 = 0;
-    t.min_r = __int_as_float(0x7f800000); t.max_r = __int_as_float(0xff800000);
-    t.episodes = 0; t.sum_len = 0; t.viol = 0;
-    t.s = State<T>{ a.env.state[il], a.env.state[ld + il], a.env.state[2 * ld + il], a.env.state[3 * ld + il] };
-    t.p = load_xi(a.env.xi, il);
-    t.d = derive(t.p);
-    t.el = a.env.elapsed[il];
-    t.new_episodes = 0; t.xi_dirty = false; t.parked = -1;
-    t.obs_loaded = kNoisy; t.after_reset = 0u;
-    t.act.group = (uint32_t)a.tick >> 7; t.act.r = make_uint4(0, 0, 0, 0); t.refresh = false;
-    if (kRandom) t.act.r = draw_block(a.env.seed, a.env.env_id0 + (uint64_t)il, (uint64_t)t.act.group, kAction, 0);
-    if (kNoisy) t.obs0 = State<T>{ a.env.obs[il], a.env.obs[ld + il], a.env.obs[2 * ld + il], a.env.obs[3 * ld + il] };
-    else t.obs0 = t.s;
-    const uint64_t id = a.env.env_id0 + (uint64_t)il;
-    const int32_t limit = a.max_steps > 0 ? a.max_steps : 0x7fffffff;
-    t.remaining = live ? a.K : 0;
-    const Policy<T> policy = { pin(a.policy.w0), pin(a.policy.w1), pin(a.policy.w2), pin(a.policy.w3), pin(a.policy.b) };
+template <typename T> struct LoggedRolloutArgs { RolloutArgs<T> roll; LogPtrs<T> log; };
 
-    // Step 0 may start from a user-injected state with any angle; from step 1 on |theta| <= 0.2095 holds at
-    // every step start (an env beyond the threshold was just reset), so the sin/cos range check is dropped.
-    if (t.remaining > 0) rollout_step<T, kEuler, false, kNoisy, kRandom>(t, a, policy, limit, id);
-    for (;;) {
-        if (sizeof(T) == 4 && !kNoisy && !kRandom) {
-#pragma unroll
-            for (int u = 0; u < kStepsPerCheck; ++u)
-                if (t.remaining > 0) rollout_step<T, kEuler, true, kNoisy, kRandom>(t, a, policy, limit, id);
-        } else if (kRandom && sizeof(T) == 4) {
-#pragma unroll kRandomUnroll
-            for (int u = 0; u < RENV_RANDOM_STEPS_PER_CHECK; ++u)
-                if (t.remaining > 0) rollout_step<T, kEuler, true, kNoisy, kRandom>(t, a, policy, limit, id);
-        } else {            // the fp64 / noisy step is ~10x the code of the fp32 one: keep the loop body inside the i-cache
-#pragma unroll kUnrollF64
-            for (int u = 0; u < kStepsPerCheck; ++u)
-                if (t.remaining > 0) rollout_step<T, kEuler, true, kNoisy, kRandom>(t, a, policy, limit, id);
-        }
-        const unsigned parked = __ballot_sync(0xffffffffu, t.parked >= 0);
-        const unsigned running = __ballot_sync(0xffffffffu, t.remaining > 0);
-        if (parked != 0u && (__popc(parked) >= (kRandom && sizeof(T) == 4 ? RENV_RANDOM_RESET_BATCH : kResetBatch) || running == 0u)) {
-            if (t.parked >= 0) rollout_reset<T, kRandom>(t, a, id);
-            continue;                       // revived lanes may still have steps to do
-        }
-        if (running == 0u) break;           // nobody parked, nobody running
-    }
-
-    if (live) {
-        a.env.state[i] = t.s.x; a.env.state[ld + i] = t.s.x_dot; a.env.state[2 * ld + i] = t.s.theta;
-        a.env.state[3 * ld + i] = t.s.theta_dot;
-        if (t.xi_dirty) store_xi(a.env.xi, i, t.p);
-        a.env.elapsed[i] = t.el;
-        if (a.env.episode && t.new_episodes) a.env.episode[i] += t.new_episodes;
-        if (kNoisy) {       // leave the obs buffer as K calls of step() would: the observation of the last step / reset
-            T ov[4];
-            add_obs_noise(t.s, a.env.noise_std, a.env.seed, id, a.tick + (uint64_t)(a.K - 1), t.after_reset, ov);
-            a.env.obs[i] = ov[0]; a.env.obs[ld + i] = ov[1]; a.env.obs[2 * ld + i] = ov[2]; a.env.obs[3 * ld + i] = ov[3];
-        }
-    }
-    rollout_publish(a.stats, a.violations, t.episodes, t.sum_len, t.sum_r, t.sum_r2, t.min_r, t.max_r, t.viol);
+// The plain (not Noisy) rollout plus the episode log: fp64, and fp32 under the random policy.
+template <typename T, bool kEuler, bool kRandom>
+__global__ void __launch_bounds__(kRolloutThreads, RENV_ROLLOUT_CTAS(T, false, kRandom))
+cartpole_rollout_logged_kernel(const __grid_constant__ LoggedRolloutArgs<T> args)
+{
+    constexpr bool kNoisy = false, kLog = true;
+    const RolloutArgs<T> &a = args.roll;
+    const LogPtrs<T> &log = args.log;
+#include "renv_rollout_body.cuh"
 }
 
 // ------------------------------------------------------------------------------------------------

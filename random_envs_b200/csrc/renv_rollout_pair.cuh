@@ -35,6 +35,7 @@ struct PairSlot {
     float x, xd, th, thd;                       // state
     float ng, fot, pmlot, l43, nlpm;            // -gravity, F/M, pml/M, l*4/3, -(l*m_p/M)   (Derived<float>)
     int B, E, L, parked;                        // see the header comment; parked = env-steps done when parked, -1 = not
+    uint32_t log_count;                         // logged kernel only: episode-log records of the env (stored at exit)
 };
 
 __device__ __forceinline__ void slot_params(PairSlot &q, const Xi<float> &p)
@@ -97,9 +98,11 @@ __device__ __forceinline__ void pair_step(PairSlot &s0, PairSlot &s1, const Pair
 constexpr int kPairGroups = RENV_PAIR_GROUPS;    // env pairs per thread (independent packed chains: ILP)
 constexpr int kPairSlots = 2 * kPairGroups;
 
-template <bool kEuler>
-__global__ void __launch_bounds__(kRolloutThreads, RENV_PAIR_CTAS)
-cartpole_rollout_pair_kernel(const __grid_constant__ RolloutArgs<float> a)
+// kLog: on_event stores an ended episode's terminal state and length like a finished env's (one more use of a store
+// the hot loop already has), and reset_slot -- in the warp's reset pass, outside the loop -- reads them back with the
+// env's xi row (current in HBM: every reset stores it) and writes the episode-log record before the resample.
+template <bool kEuler, bool kLog>
+__device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, const LogPtrs<float> &log)
 {
     constexpr int S = kPairSlots;
     const int64_t i0 = S * ((int64_t)blockIdx.x * blockDim.x + threadIdx.x);
@@ -133,6 +136,7 @@ cartpole_rollout_pair_kernel(const __grid_constant__ RolloutArgs<float> a)
             episodes += 1; sum_r += (unsigned)el; sum_r2 += (unsigned long long)el * (unsigned)el;   // reward is 1.0/step
             min_r = fminf(min_r, ret); max_r = fmaxf(max_r, ret);
             s.parked = steps_done;
+            if (kLog) store_env(s, i, el);
         } else {
             store_env(s, i, el);
         }
@@ -142,6 +146,12 @@ cartpole_rollout_pair_kernel(const __grid_constant__ RolloutArgs<float> a)
     auto reset_slot = [&](PairSlot &s, int64_t i) {
         const uint64_t id = a.env.env_id0 + (uint64_t)i;
         const uint64_t tick = a.tick + (uint64_t)(s.parked - 1);
+        if (kLog) {
+            const State<float> fs = { a.env.state[i], a.env.state[ld + i], a.env.state[2 * ld + i], a.env.state[3 * ld + i] };
+            const int32_t len = a.env.elapsed[i];
+            log_episode(log, ld, i, s.log_count, load_xi(a.env.xi, i), fs, len, !beyond_thresholds(fs) && len >= limit, tick);
+            s.log_count += 1u;
+        }
         if (a.dr.dr_type != kDrNone) {
             Xi<float> p = { 0.0f, 0.0f, 0.0f, 0.0f };
             viol += sample_xi(p, a.dr, a.env.seed, id, tick);
@@ -175,6 +185,7 @@ cartpole_rollout_pair_kernel(const __grid_constant__ RolloutArgs<float> a)
             term0[k] = dynamics<false>(st, p, derive(p), policy_action(policy, st), kEuler);
             s.x = st.x; s.xd = st.x_dot; s.th = st.theta; s.thd = st.theta_dot;
             activate(s, 0, a.env.elapsed[i]);
+            if (kLog) s.log_count = (uint32_t)log.count[i];     // in a register: no DRAM round trip in the reset pass
         } else {
             deactivate(s);
         }
@@ -226,7 +237,26 @@ cartpole_rollout_pair_kernel(const __grid_constant__ RolloutArgs<float> a)
         }
         if (running == 0u) break;
     }
+    if (kLog) {
+#pragma unroll
+        for (int k = 0; k < S; ++k)
+            if (i0 + k < n) log.count[i0 + k] = (int32_t)q[k].log_count;
+    }
     rollout_publish(a.stats, a.violations, episodes, sum_r, sum_r, sum_r2, min_r, max_r, viol);
+}
+
+template <bool kEuler>
+__global__ void __launch_bounds__(kRolloutThreads, RENV_PAIR_CTAS)
+cartpole_rollout_pair_kernel(const __grid_constant__ RolloutArgs<float> a)
+{
+    rollout_pair_body<kEuler, false>(a, LogPtrs<float>{});
+}
+
+template <bool kEuler>
+__global__ void __launch_bounds__(kRolloutThreads, RENV_PAIR_CTAS)
+cartpole_rollout_pair_logged_kernel(const __grid_constant__ LoggedRolloutArgs<float> a)
+{
+    rollout_pair_body<kEuler, true>(a.roll, a.log);
 }
 
 }  // namespace renv

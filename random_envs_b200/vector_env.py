@@ -9,6 +9,7 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     get_task()     -> (N, 4)            set_task(Tensor(N, 4) | g, m_c, m_p, l)
     rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0])
     episode_stats()  -> dict            (returns of the episodes finished inside rollouts)
+    start_episode_log(R) -> EpisodeLog  (per-env record of every episode that ends in step / rollout)
 
 ``step`` fuses what the reference stack does in three Python layers: ``RandomCartPoleEnv.step``
 (random_cartpole.py:172-224), gym 0.21 ``TimeLimit.step`` (max_episode_steps=500, :294) and gym 0.21
@@ -26,6 +27,7 @@ import math
 import numpy as np
 
 from . import _device, _lib
+from .episode_log import EpisodeLog
 from .random_env import RandomEnv
 from .xi_tables import get_table
 
@@ -96,6 +98,7 @@ class RandomCartPoleVecEnv(RandomEnv):
         self.force_mag, self.tau = 10.0, 0.02
         self.polemass_length = 0.05     # frozen, as in the reference (:79 vs :157-166)
         self._buffers = None
+        self._episode_log = None        # EpisodeLog attached by start_episode_log
         self._cfg_cache = None
         self._cfg_key = None
         self._tick = 0                  # step clock: Philox episode key; +1 per reset/step, +K per rollout
@@ -165,8 +168,12 @@ class RandomCartPoleVecEnv(RandomEnv):
             b["noise"].obs, b["noise"].std = b["obs"].data_ptr(), math.sqrt(self.noise_level)
 
     def _entry(self, name):
-        """(function name, leading arguments): the *_noisy entry points take the obs-noise block after env."""
+        """(function name, leading arguments): the *_noisy entry points take the obs-noise block after env, the
+        *_logged ones (step and rollout while an episode log is attached) the log."""
         b = self._buffers
+        if self._episode_log is not None and name in ("step", "rollout"):
+            return "renv_cartpole_%s_logged_%s" % (name, self._suffix()), (ctypes.byref(b["env"]),
+                                                                          ctypes.byref(self._episode_log.struct))
         if self.noisy:
             b["noise"].std = math.sqrt(self.noise_level)      # noise_level is a plain attribute in the reference
             return "renv_cartpole_%s_noisy_%s" % (name, self._suffix()), (ctypes.byref(b["env"]), ctypes.byref(b["noise"]))
@@ -262,16 +269,18 @@ class RandomCartPoleVecEnv(RandomEnv):
         pointers of the persistent buffers and the views handed back.  Rebuilt when a layout-affecting attribute
         changes.  (A 2^20-env step is an 11 us kernel: per-call Python work has to stay below that.)"""
         b = self._buffers
-        key = (self.noisy, self.track_truncated, self._dtype_name, self.lean)
+        key = (self.noisy, self.track_truncated, self._dtype_name, self.lean, self._episode_log, self.auto_reset)
         plan = b.get("step_plan")
         if plan is not None and plan["key"] == key:
             return plan
         t = _device.torch()
         n = self.num_envs
+        if self._episode_log is not None:
+            self._check_log_supported()
         fn, head = self._entry("step_lean" if self.lean else "step")
         info = {"TimeLimit.truncated": b["truncated"][:n].view(t.bool)} if self.track_truncated else {}
         viol = self._violation_counter(b["device"])
-        plan = dict(key=key, fn=getattr(_lib.load(), fn), name=fn, head=head,
+        plan = dict(key=key, fn=getattr(_lib.load(), fn), name=fn, head=head, logged=self._episode_log is not None,
                     reward=_device.ptr(b["reward"]), done=_device.ptr(b["done"]),
                     truncated=_device.ptr(b["truncated"]) if self.track_truncated else None,
                     out=(self.obs, b["reward"][:n], b["done"][:n].view(t.bool)), info=info,
@@ -304,6 +313,10 @@ class RandomCartPoleVecEnv(RandomEnv):
         if self.lean:
             args = plan["head"] + (action_ptr, plan["done"], plan["truncated"], self._integrator(), self.max_episode_steps,
                                    self._tick, self._active_dr_cfg(), plan["viol"], ctypes.c_void_p(_device.raw_stream(idx)))
+        elif plan["logged"]:        # auto-reset is implied
+            args = plan["head"] + (action_ptr, plan["reward"], plan["done"], plan["truncated"],
+                                   self._integrator(), self.max_episode_steps, self._tick,
+                                   self._active_dr_cfg(), plan["viol"], ctypes.c_void_p(_device.raw_stream(idx)))
         else:
             args = plan["head"] + (action_ptr, plan["reward"], plan["done"], plan["truncated"],
                                    self._integrator(), self.max_episode_steps, int(self.auto_reset), self._tick,
@@ -350,6 +363,8 @@ class RandomCartPoleVecEnv(RandomEnv):
             w_arr = None
         else:
             w_arr = (ctypes.c_double * 4)(*[float(v) for v in w])
+        if self._episode_log is not None:
+            self._check_log_supported()
         viol = self._violation_counter(buf["device"])
         fn, head = self._entry("rollout")         # Noisy variant: the policy acts on the noisy observation
         with t.cuda.device(buf["device"]):
@@ -357,6 +372,34 @@ class RandomCartPoleVecEnv(RandomEnv):
                       int(num_steps), self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(),
                       _device.ptr(buf["stats"]), _device.ptr(viol), _device.stream_ptr(buf["device"]))
         self._tick += int(num_steps)
+
+    # ---- episode log ----------------------------------------------------------------------------------
+    def start_episode_log(self, capacity=1):
+        """Attach a fresh, zeroed episode log with ``capacity`` records per env and return it: from now on every
+        episode that ends in ``step()`` or ``rollout()`` (and so in ``step_host_*``) writes one record -- its task,
+        terminal state, length, truncated flag and step clock (see ``EpisodeLog``).  ``reset()`` abandons running
+        episodes without logging them.  Replaces a log attached before.  Plain auto-reset envs only (fp32, fp64)."""
+        self._check_log_supported()
+        b = self._alloc()
+        self._episode_log = EpisodeLog(self.num_envs, b["ld"], capacity, self.torch_dtype, b["device"], self.env_id0)
+        return self._episode_log
+
+    def stop_episode_log(self):
+        """Detach the episode log: later steps and rollouts write no records.  The EpisodeLog stays readable."""
+        if self._episode_log is None:
+            self._check_log_supported()
+        self._episode_log = None
+
+    def _check_log_supported(self):
+        """The logged entry points imply auto-reset and take no noise block: also checked at every step-plan rebuild
+        and rollout, since ``auto_reset`` and ``noisy`` are plain attributes a caller may change with a log attached."""
+        if self.lean or self.noisy or not self.auto_reset:
+            raise ValueError("the episode log needs an auto-reset env without lean=True or observation noise")
+
+    @property
+    def episode_log(self):
+        """The attached EpisodeLog, or None."""
+        return self._episode_log
 
     @property
     def stats_tensor(self):
