@@ -242,6 +242,43 @@ int renv_cartpole_rollout_logged_f64(const renv_cartpole_env *env, const renv_ep
                                      int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
                                      double *stats, unsigned long long *violations, void *stream);
 
+/* A trained MLP policy for the fp32 cart-pole entry points below:
+ *     Linear(4, h1) -> act -> Linear(h1, h2) -> act -> Linear(h2, o),  h1, h2 <= 64,  o = 1 or 2,  act = tanh or ReLU,
+ * action = argmax(l0, l1), a tie giving 0 (torch.argmax).  `params` is a DEVICE array of RENV_MLP_PARAM_FLOATS fp32,
+ * 16-byte aligned, holding the nn.Linear tensors (weight (out, in) row-major, then bias) padded to 64 units:
+ *     offset    0  W1 (64, 4)      offset  256  b1 (64)
+ *     offset  320  W2 (64, 64)     offset 4416  b2 (64)
+ *     offset 4480  W3 (2, 64)      offset 4608  b3 (2)      offset 4610  2 floats of padding (any value)
+ * Narrower layers are padded with zero rows / columns / biases (exact: tanh(0) = relu(0) = 0).  A 1-output head
+ * Linear(h2, 1) with weight w and bias c is stored as l0 = 0 (zero row 0, b3[0] = 0) and l1 = w.h + c, so that the
+ * action is [w.h + c > 0].  The contraction W2 h1 runs on the tensor cores split into TF32 head and tail (3 passes,
+ * fp32 accumulation); the logits agree with a float64 evaluation to 1e-5 * max(1, max |logit|). */
+#define RENV_MLP_HIDDEN 64
+#define RENV_MLP_PARAM_FLOATS 4612
+#define RENV_MLP_TANH 0
+#define RENV_MLP_RELU 1
+typedef struct renv_mlp_policy {
+    const void *params;          /* float[RENV_MLP_PARAM_FLOATS], device, 16-byte aligned */
+    int32_t activation;          /* RENV_MLP_TANH | RENV_MLP_RELU */
+} renv_mlp_policy;
+
+/* The policy's action for each of the env's n envs, from its SoA state: action[i] in {0, 1} (4-byte aligned);
+ * `logits` NULL or T (2, ld), 16-byte aligned: row 0 = l0, row 1 = l1.  Errors: NULL env / state / params / action
+ * RENV_E_NULL, misaligned RENV_E_ALIGN, unknown activation RENV_E_ARG. */
+int renv_cartpole_policy_actions_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, uint8_t *action,
+                                         float *logits, void *stream);
+/* renv_cartpole_rollout_f32 with the MLP policy in place of the linear one (the same K range, statistics, counters and
+ * argument checks; activation RENV_E_ARG, params as above).  Contract: rollout_mlp(K) at tick t equals K x
+ * { renv_cartpole_policy_actions_mlp_f32; renv_cartpole_step_f32 with auto-reset } at ticks t .. t+K-1, bit for bit --
+ * state, xi, elapsed, episode counters, stats and (the _logged form, see renv_episode_log) log records. */
+int renv_cartpole_rollout_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, int K, int integrator,
+                                  int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                                  unsigned long long *violations, void *stream);
+int renv_cartpole_rollout_mlp_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log,
+                                         const renv_mlp_policy *p, int K, int integrator, int max_steps, uint64_t tick,
+                                         const renv_dr_cfg *dr, double *stats, unsigned long long *violations,
+                                         void *stream);
+
 /* The SCALAR drop-in env (gym.make('RandomCartPole-v0'): RandomCartPoleEnv.step / reset, random_cartpole.py:172-229,
  * one env, one host call per step) served by a resident one-warp kernel instead of one launch + synchronise per call.
  * `ctrl` is PINNED, DEVICE-MAPPED HOST memory (zero-initialised once): the host rings a request in by writing

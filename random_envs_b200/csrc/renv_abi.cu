@@ -5,6 +5,7 @@
 #include <cmath>
 #include "renv_rollout_pair.cuh"
 #include "renv_fullgauss_tc.cuh"
+#include "renv_mlp_policy.cuh"
 #include "renv_scalar_server.cuh"
 #include <stdlib.h>
 
@@ -428,6 +429,88 @@ int cartpole_rollout(const renv_cartpole_env *env, const renv_obs_noise *noise, 
     return launch_rollout(a, st);
 }
 
+// MLP policy (renv_mlp_policy.cuh): the packed parameters and the activation.
+int check_mlp(const renv_mlp_policy *p)
+{
+    if (p == nullptr || p->params == nullptr) return RENV_E_NULL;
+    if (!aligned(p->params, 16)) return RENV_E_ALIGN;
+    if (p->activation != RENV_MLP_TANH && p->activation != RENV_MLP_RELU) return RENV_E_ARG;
+    return RENV_OK;
+}
+
+int sm_count(int *sms)
+{
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
+    return (int)e;
+}
+
+int policy_actions_mlp(const renv_cartpole_env *env, const renv_mlp_policy *p, uint8_t *action, float *logits, void *stream)
+{
+    if (env == nullptr || env->state == nullptr) return RENV_E_NULL;
+    int rc = check_mlp(p);
+    if (rc) return rc;
+    if (action == nullptr) return RENV_E_NULL;
+    if (env->n <= 0 || env->ld < env->n) return RENV_E_SIZE;
+    if (env->ld % 4 != 0 || !aligned(env->state, 16) || !aligned(action, 4) || !aligned(logits, 16)) return RENV_E_ALIGN;
+    MlpActionArgs a;
+    a.state = static_cast<const float *>(env->state);
+    a.n = env->n; a.ld = env->ld;
+    a.params = static_cast<const float *>(p->params);
+    a.action = action; a.logits = logits;
+    int sms = 0;
+    if ((rc = sm_count(&sms))) return rc;
+    const int64_t tiles = (env->n + kMlpThreads - 1) / kMlpThreads;
+    const int64_t grid = tiles < (int64_t)sms * RENV_MLP_CTAS ? tiles : (int64_t)sms * RENV_MLP_CTAS;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (p->activation == RENV_MLP_TANH) cartpole_policy_actions_mlp_kernel<kMlpTanh><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
+    else cartpole_policy_actions_mlp_kernel<kMlpRelu><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
+    return launch_status();
+}
+
+template <int kAct, bool kLog> void launch_rollout_mlp(const MlpRolloutArgs &a, unsigned blocks, cudaStream_t st)
+{
+    if (a.roll.euler) cartpole_rollout_mlp_kernel<kAct, true, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
+    else cartpole_rollout_mlp_kernel<kAct, false, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
+}
+
+int rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p, int K,
+                int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                unsigned long long *violations, void *stream)
+{
+    MlpRolloutArgs a;
+    int rc = check_env<float>(env, false, &a.roll.env);
+    if (rc) return rc;
+    if (logged && (rc = check_log<float>(log, &a.log))) return rc;
+    if (!logged) a.log = LogPtrs<float>{};
+    if ((rc = check_mlp(p))) return rc;
+    if (stats == nullptr) return RENV_E_NULL;
+    if (!aligned(stats, 8)) return RENV_E_ALIGN;
+    if (K <= 0 || K > (1 << 30)) return RENV_E_SIZE;      // the same range as the linear rollout
+    if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
+    if ((rc = to_cfg4<float>(dr, &a.roll.dr))) return rc;
+    a.roll.policy = Policy<float>{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
+    a.roll.K = K;
+    a.roll.euler = integrator == RENV_EULER;
+    a.roll.max_steps = max_steps;
+    a.roll.tick = tick;
+    a.roll.stats = stats;
+    a.roll.violations = violations;
+    a.params = static_cast<const float *>(p->params);
+    const int64_t blocks = (env->n + kMlpThreads - 1) / kMlpThreads;
+    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (p->activation == RENV_MLP_TANH) {
+        if (logged) launch_rollout_mlp<kMlpTanh, true>(a, (unsigned)blocks, st);
+        else launch_rollout_mlp<kMlpTanh, false>(a, (unsigned)blocks, st);
+    } else {
+        if (logged) launch_rollout_mlp<kMlpRelu, true>(a, (unsigned)blocks, st);
+        else launch_rollout_mlp<kMlpRelu, false>(a, (unsigned)blocks, st);
+    }
+    return launch_status();
+}
+
 }  // namespace
 
 extern "C" {
@@ -579,6 +662,25 @@ int renv_cartpole_rollout_noisy_f64(const renv_cartpole_env *env, const renv_obs
 {
     if (noise == nullptr) return RENV_E_NULL;
     return cartpole_rollout<double>(env, noise, w, b, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+
+int renv_cartpole_policy_actions_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, uint8_t *action,
+                                         float *logits, void *stream)
+{
+    return policy_actions_mlp(env, p, action, logits, stream);
+}
+int renv_cartpole_rollout_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, int K, int integrator,
+                                  int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                                  unsigned long long *violations, void *stream)
+{
+    return rollout_mlp(env, nullptr, false, p, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+int renv_cartpole_rollout_mlp_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log,
+                                         const renv_mlp_policy *p, int K, int integrator, int max_steps, uint64_t tick,
+                                         const renv_dr_cfg *dr, double *stats, unsigned long long *violations,
+                                         void *stream)
+{
+    return rollout_mlp(env, log, true, p, K, integrator, max_steps, tick, dr, stats, violations, stream);
 }
 
 int renv_cartpole_scalar_serve(renv_scalar_ctrl *ctrl, void *save, uint32_t lease_id, uint64_t lease_ns, void *stream)

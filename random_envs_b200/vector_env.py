@@ -7,7 +7,8 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     reset()        -> obs (N, 4)
     step(actions)  -> obs (N, 4), reward (N,), done (N,) bool, info {'TimeLimit.truncated': (N,) bool}
     get_task()     -> (N, 4)            set_task(Tensor(N, 4) | g, m_c, m_p, l)
-    rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0])
+    rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0] or of an MLPPolicy)
+    policy_actions(policy) -> (N,)      (the MLPPolicy's actions for the current observations, ready for step)
     episode_stats()  -> dict            (returns of the episodes finished inside rollouts)
     start_episode_log(R) -> EpisodeLog  (per-env record of every episode that ends in step / rollout)
 
@@ -28,6 +29,7 @@ import numpy as np
 
 from . import _device, _lib
 from .episode_log import EpisodeLog
+from .mlp_policy import MLPPolicy
 from .random_env import RandomEnv
 from .xi_tables import get_table
 
@@ -350,13 +352,62 @@ class RandomCartPoleVecEnv(RandomEnv):
                       self._tick & 0xFFFFFFFF, _device.stream_ptr(b["device"]))
         return self._own_action_view() if out is b["action"] else out
 
+    def _check_mlp_supported(self, policy, what):
+        if not isinstance(policy, MLPPolicy):
+            raise TypeError("%s takes an MLPPolicy (MLPPolicy.from_module(net, device))" % what)
+        if self._dtype_name != "float32" or self.noisy:
+            raise ValueError("%s with an MLPPolicy needs a float32 env without observation noise" % what)
+        if policy.device != self._alloc()["device"]:
+            raise ValueError("the MLPPolicy lives on %s, the env on %s" % (policy.device, self._buffers["device"]))
+
+    def policy_actions(self, policy, return_logits=False):
+        """The actions of ``policy`` (an MLPPolicy) for the current observations of every env, written into the env's
+        own action buffer: the returned (N,) uint8 view goes to ``step`` without a copy or a check, as
+        ``sample_actions()``'s does.  With ``return_logits``: (actions, logits (N, 2) float32), row i = (l0, l1) of
+        env i (overwritten by the next call).  A fused ``rollout(policy, K)`` equals K x step(policy_actions(policy))
+        bit for bit."""
+        self._check_mlp_supported(policy, "policy_actions()")
+        b = self._buffers
+        t = _device.torch()
+        logits = None
+        if return_logits:
+            logits = b.get("mlp_logits")
+            if logits is None:
+                logits = b["mlp_logits"] = t.empty((2, b["ld"]), dtype=t.float32, device=b["device"])
+        with t.cuda.device(b["device"]):
+            _lib.call("renv_cartpole_policy_actions_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(policy.struct),
+                      _device.ptr(b["action"]), _device.ptr(logits), _device.stream_ptr(b["device"]))
+        actions = self._own_action_view()
+        return (actions, logits[:, :self.num_envs].t()) if return_logits else actions
+
+    def _rollout_mlp(self, policy, b, num_steps):
+        self._check_mlp_supported(policy, "rollout()")
+        if float(b) != 0.0:
+            raise ValueError("an MLPPolicy carries its own biases: rollout(policy) takes no b")
+        buf = self._buffers
+        t = _device.torch()
+        head = (ctypes.byref(buf["env"]),)
+        fn = "renv_cartpole_rollout_mlp_f32"
+        if self._episode_log is not None:
+            self._check_log_supported()
+            fn, head = "renv_cartpole_rollout_mlp_logged_f32", head + (ctypes.byref(self._episode_log.struct),)
+        viol = self._violation_counter(buf["device"])
+        with t.cuda.device(buf["device"]):
+            _lib.call(fn, *head, ctypes.byref(policy.struct), int(num_steps), self._integrator(), self.max_episode_steps,
+                      self._tick, self._active_dr_cfg(), _device.ptr(buf["stats"]), _device.ptr(viol),
+                      _device.stream_ptr(buf["device"]))
+        self._tick += int(num_steps)
+
     def rollout(self, w, b=0.0, num_steps=MAX_EPISODE_STEPS):
-        """K fused env-steps under the in-kernel linear policy a = [w.s + b > 0] (auto-reset always on), or, with
-        ``w=None``, under the random policy ``action_space.sample()`` (test_random_policy.py:26)."""
+        """K fused env-steps under the in-kernel linear policy a = [w.s + b > 0] (auto-reset always on), with
+        ``w=None`` under the random policy ``action_space.sample()`` (test_random_policy.py:26), or with an
+        ``MLPPolicy`` in place of ``w`` under that network (float32 envs without observation noise; ``b`` must be 0)."""
         buf = self._alloc()
         t = _device.torch()
         if self.lean:
             raise ValueError("rollout() keeps the int32 TimeLimit counter: build the env without lean=True")
+        if isinstance(w, MLPPolicy):
+            return self._rollout_mlp(w, b, num_steps)
         if w is None:         # random policy: the fused equivalent of K x step(sample_actions())
             if self.noisy:
                 raise ValueError("the random policy ignores observations: use a noise-free env")
