@@ -28,7 +28,8 @@
  *       counters[2]  step CTAs whose tile-ordering wait (renv_cartpole_env.progress) timed out: the progress words
  *                    were not in the state the protocol leaves them in (see there); the step still ran.
  *     The host reads them at its next synchronisation point and raises the reference's exception.
- *   - RNG: counter-based Philox4x32-10, key = seed, counter = (global env id, tick, purpose|slot).  `tick` is
+ *   - RNG: counter-based Philox4x32-10, key = seed, counter = (global env id, tick, purpose|slot), purpose 0 initial
+ *     state, 1 xi, 2 random action, 3 sample_tasks, 4 observation noise, 5 MLP policy sample.  `tick` is
  *     the caller's step clock (48 bits used): pass a value that grows by 1 per reset/step call and by K per
  *     K-step rollout (step k of a rollout uses tick + k).  An env starts at most one episode per tick, so
  *     (seed, env_id0 + i, tick) names the episode; results never depend on launch geometry or sharding,
@@ -278,6 +279,47 @@ int renv_cartpole_rollout_mlp_logged_f32(const renv_cartpole_env *env, const ren
                                          const renv_mlp_policy *p, int K, int integrator, int max_steps, uint64_t tick,
                                          const renv_dr_cfg *dr, double *stats, unsigned long long *violations,
                                          void *stream);
+
+/* Stochastic actions of the MLP policy, for on-policy training.  With d = l1 - l0, env e (global id) acting at tick t:
+ *   sample = 1:  a = 1 iff u < sigmoid(d), sigmoid in fp32, u = the 24-bit uniform of word x of the Philox block
+ *                (seed, e, t, purpose 5, slot 0)  -- a ~ softmax(l0, l1);
+ *   sample = 0:  a = argmax(l0, l1), a tie giving 0 (renv_cartpole_policy_actions_mlp_f32's action);
+ *   logp = log pi(a | s) = log sigmoid(d) for a = 1, log sigmoid(-d) for a = 0 (in both modes).
+ * renv_cartpole_policy_actions_mlp_f32 plus the action rule above at tick `tick` (pass the tick of the step the actions
+ * go to): `logp` NULL or float (ld), 4-byte aligned.  Errors as there; `sample` outside {0, 1}: RENV_E_ARG. */
+int renv_cartpole_policy_logp_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, int sample, uint64_t tick,
+                                      uint8_t *action, float *logp, float *logits, void *stream);
+
+/* Per-step record of a collected trajectory (device pointers; row stride = the env's ld): step k of env i is row
+ * k * ld + i of every field, 0 <= k < K <= capacity. */
+typedef struct renv_trajectory {
+    float *obs;                  /* (capacity, ld, 4) rows, 16-byte aligned: x, x_dot, theta, theta_dot the action was
+                                    chosen from */
+    uint8_t *action;             /* (capacity, ld), 4-byte aligned: the action taken */
+    uint8_t *done;               /* (capacity, ld), 4-byte aligned: the step ended the episode (terminated or truncated) */
+    float *logp;                 /* (capacity, ld), 4-byte aligned, or NULL: log pi(action | obs) */
+    uint8_t *truncated;          /* (capacity, ld), 4-byte aligned, or NULL: the TimeLimit ended it (TimeLimit.truncated) */
+    float *final_obs;            /* (capacity, ld, 4) rows, 16-byte aligned, or NULL: the state after the step, written
+                                    only where done -- the terminal observation auto-reset replaces (the episode log's
+                                    final_state); elsewhere left untouched */
+    int32_t capacity;            /* steps the buffers hold */
+} renv_trajectory;
+
+/* renv_cartpole_rollout_mlp_f32 (_logged: renv_cartpole_rollout_mlp_logged_f32) that also records the trajectory:
+ * the reward is 1.0 on every step (:207-212) and is not stored.  Contract: collect(K) at tick t equals K x
+ * { record obs = the env's state; renv_cartpole_policy_logp_mlp_f32(sample, tick t + k);
+ *   renv_cartpole_step_f32 with auto-reset at tick t + k (done, truncated) }  for k = 0 .. K-1, bit for bit -- every
+ * trajectory row, state, xi, elapsed, episode counters, stats and (the _logged form) log records.  With sample = 0 the
+ * env, stats and log are exactly those renv_cartpole_rollout_mlp_f32 leaves.  Errors, all before any CUDA call: those of
+ * the rollout (K outside [1, 2^30] RENV_E_SIZE, ...); NULL traj / obs / action / done RENV_E_NULL; a misaligned field
+ * RENV_E_ALIGN; K > traj->capacity or `sample` outside {0, 1} RENV_E_ARG. */
+int renv_cartpole_collect_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, const renv_trajectory *traj,
+                                  int sample, int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                  double *stats, unsigned long long *violations, void *stream);
+int renv_cartpole_collect_mlp_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log,
+                                         const renv_mlp_policy *p, const renv_trajectory *traj, int sample, int K,
+                                         int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                         double *stats, unsigned long long *violations, void *stream);
 
 /* The SCALAR drop-in env (gym.make('RandomCartPole-v0'): RandomCartPoleEnv.step / reset, random_cartpole.py:172-229,
  * one env, one host call per step) served by a resident one-warp kernel instead of one launch + synchronise per call.

@@ -24,11 +24,12 @@ from .episode_log import EpisodeLog
 from .mlp_policy import MLPPolicy
 from .random_cartpole import RandomCartPoleEnv
 from .random_env import RandomEnv, TaskSampler
+from .trajectory import Trajectory
 from .vector_env import RandomCartPoleVecEnv
 from .gym_vector import RandomCartPoleGymVectorEnv
 from .xi_tables import HUMANOID_NOMINAL, XI_TABLES
 
-__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "XI_TABLES",
+__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "Trajectory", "XI_TABLES",
            "HUMANOID_NOMINAL", "shard_range", "combine_stats", "summarize_stats", "allgather_stats",
            "make_sharded_env", "load_library"]
 

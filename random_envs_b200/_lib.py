@@ -57,11 +57,19 @@ class MlpPolicy(ctypes.Structure):
     _fields_ = [("params", ctypes.c_void_p), ("activation", ctypes.c_int32)]
 
 
+class Trajectory(ctypes.Structure):
+    """struct renv_trajectory (include/renv.h)."""
+    _fields_ = [("obs", ctypes.c_void_p), ("action", ctypes.c_void_p), ("done", ctypes.c_void_p),
+                ("logp", ctypes.c_void_p), ("truncated", ctypes.c_void_p), ("final_obs", ctypes.c_void_p),
+                ("capacity", ctypes.c_int32)]
+
+
 _vp, _i64, _u64, _u32, _int, _dbl = (ctypes.c_void_p, ctypes.c_int64, ctypes.c_uint64, ctypes.c_uint32,
                                      ctypes.c_int, ctypes.c_double)
 _cfg_p, _env_p, _noise_p = ctypes.POINTER(DrCfg), ctypes.POINTER(CartpoleEnv), ctypes.POINTER(ObsNoise)
 _log_p = ctypes.POINTER(EpisodeLog)
 _mlp_p = ctypes.POINTER(MlpPolicy)
+_traj_p = ctypes.POINTER(Trajectory)
 
 # name -> (restype, argtypes); must list every function declared in include/renv.h
 SIGNATURES = {
@@ -89,6 +97,10 @@ SIGNATURES = {
     "renv_cartpole_policy_actions_mlp_f32": (_int, [_env_p, _mlp_p, _vp, _vp, _vp]),
     "renv_cartpole_rollout_mlp_f32": (_int, [_env_p, _mlp_p, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
     "renv_cartpole_rollout_mlp_logged_f32": (_int, [_env_p, _log_p, _mlp_p, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
+    "renv_cartpole_policy_logp_mlp_f32": (_int, [_env_p, _mlp_p, _int, _u64, _vp, _vp, _vp, _vp]),
+    "renv_cartpole_collect_mlp_f32": (_int, [_env_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
+    "renv_cartpole_collect_mlp_logged_f32": (_int, [_env_p, _log_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64, _cfg_p,
+                                                    _vp, _vp, _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),
     "renv_random_actions_u8": (_int, [_vp, _i64, _u64, _u64, _u32, _vp]),
     "renv_pack_flags_u8": (_int, [_vp, _vp, _i64, _vp]),

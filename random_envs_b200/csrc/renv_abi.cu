@@ -475,38 +475,119 @@ template <int kAct, bool kLog> void launch_rollout_mlp(const MlpRolloutArgs &a, 
     else cartpole_rollout_mlp_kernel<kAct, false, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
 }
 
-int rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p, int K,
-                int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
-                unsigned long long *violations, void *stream)
+// The argument checks and arguments shared by the MLP rollout and collect entry points.
+int prepare_rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p,
+                        int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                        unsigned long long *violations, MlpRolloutArgs *a)
 {
-    MlpRolloutArgs a;
-    int rc = check_env<float>(env, false, &a.roll.env);
+    int rc = check_env<float>(env, false, &a->roll.env);
     if (rc) return rc;
-    if (logged && (rc = check_log<float>(log, &a.log))) return rc;
-    if (!logged) a.log = LogPtrs<float>{};
+    if (logged && (rc = check_log<float>(log, &a->log))) return rc;
+    if (!logged) a->log = LogPtrs<float>{};
     if ((rc = check_mlp(p))) return rc;
     if (stats == nullptr) return RENV_E_NULL;
     if (!aligned(stats, 8)) return RENV_E_ALIGN;
     if (K <= 0 || K > (1 << 30)) return RENV_E_SIZE;      // the same range as the linear rollout
     if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
-    if ((rc = to_cfg4<float>(dr, &a.roll.dr))) return rc;
-    a.roll.policy = Policy<float>{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
-    a.roll.K = K;
-    a.roll.euler = integrator == RENV_EULER;
-    a.roll.max_steps = max_steps;
-    a.roll.tick = tick;
-    a.roll.stats = stats;
-    a.roll.violations = violations;
-    a.params = static_cast<const float *>(p->params);
+    if ((rc = to_cfg4<float>(dr, &a->roll.dr))) return rc;
+    a->roll.policy = Policy<float>{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
+    a->roll.K = K;
+    a->roll.euler = integrator == RENV_EULER;
+    a->roll.max_steps = max_steps;
+    a->roll.tick = tick;
+    a->roll.stats = stats;
+    a->roll.violations = violations;
+    a->params = static_cast<const float *>(p->params);
     const int64_t blocks = (env->n + kMlpThreads - 1) / kMlpThreads;
     if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    return RENV_OK;
+}
+
+int rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p, int K,
+                int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                unsigned long long *violations, void *stream)
+{
+    MlpRolloutArgs a;
+    const int rc = prepare_rollout_mlp(env, log, logged, p, K, integrator, max_steps, tick, dr, stats, violations, &a);
+    if (rc) return rc;
+    const unsigned blocks = (unsigned)((env->n + kMlpThreads - 1) / kMlpThreads);
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (p->activation == RENV_MLP_TANH) {
-        if (logged) launch_rollout_mlp<kMlpTanh, true>(a, (unsigned)blocks, st);
-        else launch_rollout_mlp<kMlpTanh, false>(a, (unsigned)blocks, st);
+        if (logged) launch_rollout_mlp<kMlpTanh, true>(a, blocks, st);
+        else launch_rollout_mlp<kMlpTanh, false>(a, blocks, st);
     } else {
-        if (logged) launch_rollout_mlp<kMlpRelu, true>(a, (unsigned)blocks, st);
-        else launch_rollout_mlp<kMlpRelu, false>(a, (unsigned)blocks, st);
+        if (logged) launch_rollout_mlp<kMlpRelu, true>(a, blocks, st);
+        else launch_rollout_mlp<kMlpRelu, false>(a, blocks, st);
+    }
+    return launch_status();
+}
+
+int policy_logp_mlp(const renv_cartpole_env *env, const renv_mlp_policy *p, int sample, uint64_t tick, uint8_t *action,
+                    float *logp, float *logits, void *stream)
+{
+    if (env == nullptr || env->state == nullptr) return RENV_E_NULL;
+    int rc = check_mlp(p);
+    if (rc) return rc;
+    if (action == nullptr) return RENV_E_NULL;
+    if (env->n <= 0 || env->ld < env->n) return RENV_E_SIZE;
+    if (env->ld % 4 != 0 || !aligned(env->state, 16) || !aligned(action, 4) || !aligned(logits, 16) || !aligned(logp, 4))
+        return RENV_E_ALIGN;
+    if (sample != 0 && sample != 1) return RENV_E_ARG;
+    MlpLogpArgs a;
+    a.act.state = static_cast<const float *>(env->state);
+    a.act.n = env->n; a.act.ld = env->ld;
+    a.act.params = static_cast<const float *>(p->params);
+    a.act.action = action; a.act.logits = logits;
+    a.logp = logp;
+    a.env_id0 = env->env_id0; a.seed = env->seed; a.tick = tick;
+    a.sample = sample;
+    int sms = 0;
+    if ((rc = sm_count(&sms))) return rc;
+    const int64_t tiles = (env->n + kMlpThreads - 1) / kMlpThreads;
+    const int64_t grid = tiles < (int64_t)sms * RENV_MLP_ROLLOUT_CTAS ? tiles : (int64_t)sms * RENV_MLP_ROLLOUT_CTAS;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (p->activation == RENV_MLP_TANH) cartpole_policy_logp_mlp_kernel<kMlpTanh><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
+    else cartpole_policy_logp_mlp_kernel<kMlpRelu><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
+    return launch_status();
+}
+
+int check_traj(const renv_trajectory *t, int K, MlpTrajPtrs *out)
+{
+    if (t == nullptr || t->obs == nullptr || t->action == nullptr || t->done == nullptr) return RENV_E_NULL;
+    if (!aligned(t->obs, 16) || !aligned(t->final_obs, 16) || !aligned(t->action, 4) || !aligned(t->done, 4) ||
+        !aligned(t->logp, 4) || !aligned(t->truncated, 4))
+        return RENV_E_ALIGN;
+    if (K > t->capacity) return RENV_E_ARG;
+    *out = MlpTrajPtrs{ t->obs, t->action, t->done, t->logp, t->truncated, t->final_obs };
+    return RENV_OK;
+}
+
+template <int kAct, bool kLog> void launch_collect_mlp(const MlpCollectArgs &a, unsigned blocks, cudaStream_t st)
+{
+    if (a.roll.euler) cartpole_collect_mlp_kernel<kAct, true, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
+    else cartpole_collect_mlp_kernel<kAct, false, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
+}
+
+int collect_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p,
+                const renv_trajectory *traj, int sample, int K, int integrator, int max_steps, uint64_t tick,
+                const renv_dr_cfg *dr, double *stats, unsigned long long *violations, void *stream)
+{
+    MlpRolloutArgs r;
+    int rc = prepare_rollout_mlp(env, log, logged, p, K, integrator, max_steps, tick, dr, stats, violations, &r);
+    if (rc) return rc;
+    MlpCollectArgs a;
+    if ((rc = check_traj(traj, K, &a.traj))) return rc;
+    if (sample != 0 && sample != 1) return RENV_E_ARG;
+    a.roll = r.roll; a.params = r.params; a.log = r.log;
+    a.sample = sample;
+    const unsigned blocks = (unsigned)((env->n + kMlpThreads - 1) / kMlpThreads);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (p->activation == RENV_MLP_TANH) {
+        if (logged) launch_collect_mlp<kMlpTanh, true>(a, blocks, st);
+        else launch_collect_mlp<kMlpTanh, false>(a, blocks, st);
+    } else {
+        if (logged) launch_collect_mlp<kMlpRelu, true>(a, blocks, st);
+        else launch_collect_mlp<kMlpRelu, false>(a, blocks, st);
     }
     return launch_status();
 }
@@ -681,6 +762,24 @@ int renv_cartpole_rollout_mlp_logged_f32(const renv_cartpole_env *env, const ren
                                          void *stream)
 {
     return rollout_mlp(env, log, true, p, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+int renv_cartpole_policy_logp_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, int sample, uint64_t tick,
+                                      uint8_t *action, float *logp, float *logits, void *stream)
+{
+    return policy_logp_mlp(env, p, sample, tick, action, logp, logits, stream);
+}
+int renv_cartpole_collect_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, const renv_trajectory *traj,
+                                  int sample, int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                  double *stats, unsigned long long *violations, void *stream)
+{
+    return collect_mlp(env, nullptr, false, p, traj, sample, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+int renv_cartpole_collect_mlp_logged_f32(const renv_cartpole_env *env, const renv_episode_log *log,
+                                         const renv_mlp_policy *p, const renv_trajectory *traj, int sample, int K,
+                                         int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                         double *stats, unsigned long long *violations, void *stream)
+{
+    return collect_mlp(env, log, true, p, traj, sample, K, integrator, max_steps, tick, dr, stats, violations, stream);
 }
 
 int renv_cartpole_scalar_serve(renv_scalar_ctrl *ctrl, void *save, uint32_t lease_id, uint64_t lease_ns, void *stream)

@@ -4,10 +4,11 @@
 //
 // act = tanh or ReLU, narrower nets zero-padded to 64 units on the host (exact: act(0) = 0).  fp32 envs only.
 //
-// mlp_logits() evaluates the policy for the 32 envs of a warp (one env per lane) and is the ONE implementation both
-// cartpole_policy_actions_mlp_kernel and cartpole_rollout_mlp_kernel call, so that a fused rollout equals K x
+// mlp_logits() evaluates the policy for the 32 envs of a warp (one env per lane) and is the ONE implementation all four
+// MLP kernels (policy_actions, policy_logp, rollout, collect) call, so that a fused rollout equals K x
 // {policy_actions; step} bit for bit by construction: the same instructions, the same head / tail split, the same
 // summation order.  Every floating-point operation is an explicit intrinsic, so no kernel can contract it differently.
+// mlp_pick() does the same for the sampled action and its log-probability (policy_logp and collect).
 //
 // Layer 2 (64 x 64, 8,192 of the ~9,000 FLOPs of an env-step) runs on the tensor cores as mma.sync m16n8k8 TF32
 // (HMMA.1688.F32.TF32): the warp's 32 envs are two M = 16 row tiles, the 64 outputs eight N = 8 column tiles, the 64
@@ -182,6 +183,37 @@ __device__ __forceinline__ void mlp_logits(const MlpSmem &sm, const State<float>
 // argmax(l0, l1) with torch.argmax's tie rule (the first index wins)
 __device__ __forceinline__ int mlp_action(float l0, float l1) { return l1 > l0 ? 1 : 0; }
 
+// The action of the softmax policy over (l0, l1) and its log-probability, for env `id` stepping at `tick`: the ONE
+// implementation both cartpole_policy_logp_mlp_kernel and cartpole_collect_mlp_kernel call.  With d = l1 - l0:
+//   sample: a = [u < sigmoid(d)], u = u01 of word x of block (seed, id, tick, purpose 5, slot 0) (include/renv.h);
+//   greedy: a = mlp_action(l0, l1);
+//   logp = log sigmoid(d) for a = 1, log sigmoid(-d) for a = 0, as -softplus(-/+d) = -(max(z, 0) + log1p(exp(-|d|))).
+// `sample` is warp-uniform in both kernels: the greedy path skips the Philox block.
+__device__ __forceinline__ int mlp_pick(float l0, float l1, bool sample, uint64_t seed, uint64_t id, uint64_t tick, float &logp)
+{
+    const float dl = __fsub_rn(l1, l0);
+    int action;
+    if (sample) {
+        const float u = u01(draw_block(seed, id, tick, kPolicySample, 0).x);
+        action = u < __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-dl))) ? 1 : 0;
+    } else {
+        action = mlp_action(l0, l1);
+    }
+    const float z = action ? -dl : dl;
+    logp = -__fadd_rn(fmaxf(z, 0.0f), log1pf(expf(-fabsf(dl))));
+    return action;
+}
+
+// Per-step trajectory record of cartpole_collect_mlp_kernel (include/renv.h renv_trajectory): row k * ld + i of each
+// field holds step k of env i.  logp, truncated and final_obs may be nullptr.
+struct MlpTrajPtrs {
+    float *obs;               // (capacity, ld, 4) rows: the observation the action was chosen from
+    uint8_t *action, *done;
+    float *logp;
+    uint8_t *truncated;
+    float *final_obs;         // (capacity, ld, 4) rows: the state after the step, written where done
+};
+
 // ------------------------------------------------------------------------------------------------
 // policy_actions: action[i] (and the logits) for every env, from the env's SoA state
 // ------------------------------------------------------------------------------------------------
@@ -216,6 +248,43 @@ cartpole_policy_actions_mlp_kernel(const __grid_constant__ MlpActionArgs a)
 }
 
 // ------------------------------------------------------------------------------------------------
+// policy_logp: the sampled (or greedy) action and its log-probability at one tick -- the step-loop twin of collect
+// ------------------------------------------------------------------------------------------------
+struct MlpLogpArgs {
+    MlpActionArgs act;        // state, n, ld, params, action, logits (nullptr: not written)
+    float *logp;              // (ld) or nullptr
+    uint64_t env_id0, seed, tick;
+    int sample;               // 0: argmax, 1: a ~ softmax(l0, l1)
+};
+
+// 3 CTAs per SM as the rollout: at 4 (128 registers) the Philox block and log1p beside mlp_logits spill 16 bytes (Tanh).
+template <int kAct>
+__global__ void __launch_bounds__(kMlpThreads, RENV_MLP_ROLLOUT_CTAS)
+cartpole_policy_logp_mlp_kernel(const __grid_constant__ MlpLogpArgs args)
+{
+    __shared__ MlpSmem sm;
+    const MlpActionArgs &a = args.act;
+    mlp_load_params(sm, a.params);
+    const int64_t ld = a.ld;
+    const bool sample = args.sample != 0;
+    for (int64_t base = (int64_t)blockIdx.x * kMlpThreads; base < a.n; base += (int64_t)gridDim.x * kMlpThreads) {
+        const int64_t i = base + threadIdx.x;
+        if (base + (threadIdx.x & ~31) >= a.n) break;           // the whole warp is past n (warp-uniform)
+        const bool live = i < a.n;
+        const State<float> s = live ? State<float>{ a.state[i], a.state[ld + i], a.state[2 * ld + i], a.state[3 * ld + i] }
+                                    : State<float>{ 0.0f, 0.0f, 0.0f, 0.0f };
+        float l0, l1;
+        mlp_logits<kAct>(sm, s, l0, l1);
+        if (live) {
+            float logp;
+            a.action[i] = (uint8_t)mlp_pick(l0, l1, sample, args.seed, args.env_id0 + (uint64_t)i, args.tick, logp);
+            if (args.logp) args.logp[i] = logp;
+            if (a.logits) { a.logits[i] = l0; a.logits[ld + i] = l1; }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // Fused K-step rollout under the MLP policy
 // ------------------------------------------------------------------------------------------------
 struct MlpRolloutArgs {
@@ -233,69 +302,37 @@ template <int kAct, bool kEuler, bool kLog>
 __global__ void __launch_bounds__(kMlpThreads, RENV_MLP_ROLLOUT_CTAS)
 cartpole_rollout_mlp_kernel(const __grid_constant__ MlpRolloutArgs args)
 {
-    __shared__ MlpSmem sm;
-    mlp_load_params(sm, args.params);
-    const RolloutArgs<float> &a = args.roll;
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int64_t ld = a.env.ld;
-    const bool live = i < a.env.n;
-    const int64_t il = live ? i : 0;
-    const uint64_t id = a.env.env_id0 + (uint64_t)il;
+    constexpr bool kCollect = false;
+    constexpr MlpTrajPtrs traj = {};
+    constexpr bool sample = false;
+#include "renv_mlp_rollout_body.cuh"
+}
 
-    State<float> s = live ? State<float>{ a.env.state[i], a.env.state[ld + i], a.env.state[2 * ld + i], a.env.state[3 * ld + i] }
-                          : State<float>{ 0.0f, 0.0f, 0.0f, 0.0f };      // lanes past n feed zero rows
-    Xi<float> p = load_xi(a.env.xi, il);
-    Derived<float> d = derive(p);
-    int32_t el = a.env.elapsed[il];
-    uint32_t log_count = kLog ? (uint32_t)args.log.count[il] : 0u;
-    unsigned episodes = 0, sum_len = 0, viol = 0;         // return == length (:207-212): sum_len is also sum R
-    unsigned long long sum_r2 = 0;
-    float min_r = __int_as_float(0x7f800000), max_r = __int_as_float(0xff800000);
-    bool xi_dirty = false;
+// ------------------------------------------------------------------------------------------------
+// Fused K-step trajectory collection: the rollout above plus the sampled action, its log-probability and the per-step
+// record a policy-gradient learner needs
+// ------------------------------------------------------------------------------------------------
+struct MlpCollectArgs {
+    RolloutArgs<float> roll;   // roll.policy is unused
+    const float *params;
+    LogPtrs<float> log;        // read only by the kLog instance
+    MlpTrajPtrs traj;
+    int sample;                // 0: argmax, 1: a ~ softmax(l0, l1)  (warp-uniform)
+};
 
-    if (__any_sync(0xffffffffu, live)) {                        // warp-uniform: a warp entirely past n only publishes
-        for (int k = 0; k < a.K; ++k) {
-            float l0, l1;
-            mlp_logits<kAct>(sm, s, l0, l1);
-            if (live) {
-                const int action = mlp_action(l0, l1);
-                // step 0 may start from an injected state at any angle; from step 1 on |theta| <= 0.2095 holds at
-                // every step start (an env beyond the threshold was just reset): the same bits without the range check
-                const bool terminated = k == 0 ? dynamics<false>(s, p, d, action, kEuler)
-                                               : dynamics<true>(s, p, d, action, kEuler);
-                el += 1;                                                   // TimeLimit.step
-                if (terminated || (a.max_steps > 0 && el >= a.max_steps)) {
-                    const uint64_t tick = a.tick + (uint64_t)k;
-                    const float ret = (float)el;
-                    episodes += 1; sum_len += (unsigned)el;
-                    sum_r2 += (unsigned long long)el * (unsigned)el;
-                    min_r = fminf(min_r, ret); max_r = fmaxf(max_r, ret);
-                    if (kLog) {
-                        log_episode(args.log, ld, i, log_count, p, s, el, !terminated, tick);
-                        log_count += 1u;
-                    }
-                    el = 0;
-                    if (a.dr.dr_type != kDrNone) {                         // reset_env: set_random_task, then reset
-                        p = Xi<float>{ 0.0f, 0.0f, 0.0f, 0.0f };
-                        viol += sample_xi(p, a.dr, a.env.seed, id, tick);
-                        d = derive(p);
-                        xi_dirty = true;
-                    }
-                    init_state(s, a.env.seed, id, tick);
-                }
-            }
-            __syncwarp();
-        }
-    }
-
-    if (live) {
-        a.env.state[i] = s.x; a.env.state[ld + i] = s.x_dot; a.env.state[2 * ld + i] = s.theta; a.env.state[3 * ld + i] = s.theta_dot;
-        if (xi_dirty) store_xi(a.env.xi, i, p);
-        a.env.elapsed[i] = el;
-        if (kLog) args.log.count[i] = (int32_t)log_count;
-        if (a.env.episode && episodes) a.env.episode[i] += episodes;      // one started per episode that ended
-    }
-    rollout_publish(a.stats, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
+// Step k of env i stores obs, action and logp before the dynamics, done and truncated after them, and final_obs where
+// the episode ended, before its reset; the env, the statistics and the log are handled exactly as in
+// cartpole_rollout_mlp_kernel (the same body).  The action comes from mlp_pick, which policy_logp also calls, so the
+// launch equals K x {record obs; renv_cartpole_policy_logp_mlp_f32; renv_cartpole_step_f32 (auto-reset)} bit for bit.
+// Greed / sampling is a runtime argument: one instance per (activation, integrator, log) as for the rollout.
+template <int kAct, bool kEuler, bool kLog>
+__global__ void __launch_bounds__(kMlpThreads, RENV_MLP_ROLLOUT_CTAS)
+cartpole_collect_mlp_kernel(const __grid_constant__ MlpCollectArgs args)
+{
+    constexpr bool kCollect = true;
+    const MlpTrajPtrs &traj = args.traj;
+    const bool sample = args.sample != 0;
+#include "renv_mlp_rollout_body.cuh"
 }
 
 }  // namespace renv

@@ -17,7 +17,7 @@
 
 namespace renv {
 
-enum Purpose : uint32_t { kInit = 0, kXi = 1, kAction = 2, kTasks = 3, kObs = 4 };
+enum Purpose : uint32_t { kInit = 0, kXi = 1, kAction = 2, kTasks = 3, kObs = 4, kPolicySample = 5 };
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
 {

@@ -9,6 +9,7 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     get_task()     -> (N, 4)            set_task(Tensor(N, 4) | g, m_c, m_p, l)
     rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0] or of an MLPPolicy)
     policy_actions(policy) -> (N,)      (the MLPPolicy's actions for the current observations, ready for step)
+    collect(policy, K) -> Trajectory    (K fused steps under the sampled policy, every step recorded for training)
     episode_stats()  -> dict            (returns of the episodes finished inside rollouts)
     start_episode_log(R) -> EpisodeLog  (per-env record of every episode that ends in step / rollout)
 
@@ -31,6 +32,7 @@ from . import _device, _lib
 from .episode_log import EpisodeLog
 from .mlp_policy import MLPPolicy
 from .random_env import RandomEnv
+from .trajectory import Trajectory
 from .xi_tables import get_table
 
 _TABLE = get_table("RandomCartPole-v0")
@@ -360,25 +362,84 @@ class RandomCartPoleVecEnv(RandomEnv):
         if policy.device != self._alloc()["device"]:
             raise ValueError("the MLPPolicy lives on %s, the env on %s" % (policy.device, self._buffers["device"]))
 
-    def policy_actions(self, policy, return_logits=False):
+    def policy_actions(self, policy, return_logits=False, *, sample=False, return_logp=False):
         """The actions of ``policy`` (an MLPPolicy) for the current observations of every env, written into the env's
         own action buffer: the returned (N,) uint8 view goes to ``step`` without a copy or a check, as
-        ``sample_actions()``'s does.  With ``return_logits``: (actions, logits (N, 2) float32), row i = (l0, l1) of
-        env i (overwritten by the next call).  A fused ``rollout(policy, K)`` equals K x step(policy_actions(policy))
-        bit for bit."""
+        ``sample_actions()``'s does.  By default the action is argmax(l0, l1); with ``sample=True`` it is drawn from
+        softmax(l0, l1) with the Philox stream of the env's current step clock, i.e. of the ``step`` it goes to
+        (include/renv.h renv_cartpole_policy_logp_mlp_f32).  Returns ``actions``, then ``logits`` (N, 2) float32
+        (row i = (l0, l1) of env i) with ``return_logits``, then ``logp`` (N,) float32 = log pi(action | obs) with
+        ``return_logp``; the tensors are overwritten by the next call.  A fused ``rollout(policy, K)`` equals K x
+        step(policy_actions(policy)) bit for bit, and ``collect(policy, K, sample)`` records K x
+        step(policy_actions(policy, sample=sample, return_logp=True))."""
         self._check_mlp_supported(policy, "policy_actions()")
         b = self._buffers
         t = _device.torch()
-        logits = None
+        n = self.num_envs
+        logits = logp = None
         if return_logits:
             logits = b.get("mlp_logits")
             if logits is None:
                 logits = b["mlp_logits"] = t.empty((2, b["ld"]), dtype=t.float32, device=b["device"])
+        if return_logp:
+            logp = b.get("mlp_logp")
+            if logp is None:
+                logp = b["mlp_logp"] = t.empty(b["ld"], dtype=t.float32, device=b["device"])
         with t.cuda.device(b["device"]):
-            _lib.call("renv_cartpole_policy_actions_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(policy.struct),
-                      _device.ptr(b["action"]), _device.ptr(logits), _device.stream_ptr(b["device"]))
-        actions = self._own_action_view()
-        return (actions, logits[:, :self.num_envs].t()) if return_logits else actions
+            if sample or return_logp:
+                _lib.call("renv_cartpole_policy_logp_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(policy.struct),
+                          int(bool(sample)), self._tick, _device.ptr(b["action"]), _device.ptr(logp), _device.ptr(logits),
+                          _device.stream_ptr(b["device"]))
+            else:
+                _lib.call("renv_cartpole_policy_actions_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(policy.struct),
+                          _device.ptr(b["action"]), _device.ptr(logits), _device.stream_ptr(b["device"]))
+        out = (self._own_action_view(),) + ((logits[:, :n].t(),) if return_logits else ()) + \
+            ((logp[:n],) if return_logp else ())
+        return out if len(out) > 1 else out[0]
+
+    def trajectory_buffer(self, capacity, logp=True, final_obs=True):
+        """A ``Trajectory`` of up to ``capacity`` steps of this env's N envs for ``collect(..., out=buf)``: allocate it
+        once and reuse it (2^20 envs x 256 steps with final_obs is ~10 GB).  ``logp`` / ``final_obs`` False: those
+        fields are neither allocated nor written."""
+        b = self._alloc()
+        return Trajectory(self.num_envs, b["ld"], capacity, b["device"], logp=logp, final_obs=final_obs)
+
+    def collect(self, policy, num_steps, sample=True, out=None):
+        """``num_steps`` fused env-steps under ``policy`` (an MLPPolicy), recording every step: returns a
+        ``Trajectory`` (``out``, or a new buffer when None) with obs, actions, logp, dones, truncated and final_obs
+        of each step.  ``sample=True`` draws a ~ softmax(l0, l1) (on-policy data for PPO / A2C-style training),
+        ``sample=False`` takes argmax and leaves the env, statistics and episode log exactly as ``rollout(policy, K)``.
+        One kernel; bit for bit the K x {obs; policy_actions(policy, sample=sample, return_logp=True); step} loop.
+        Advances the step clock by K; afterwards ``obs`` is the observation after the last step (the bootstrap
+        observation).  float32 envs without observation noise or lean=True only."""
+        buf = self._alloc()
+        t = _device.torch()
+        if self.lean:
+            raise ValueError("collect() keeps the int32 TimeLimit counter: build the env without lean=True")
+        self._check_mlp_supported(policy, "collect()")
+        K = int(num_steps)
+        if K < 1:
+            raise ValueError("num_steps must be >= 1, got %d" % K)
+        if out is None:
+            out = self.trajectory_buffer(K)
+        elif not isinstance(out, Trajectory) or out.num_envs != self.num_envs or out.ld != buf["ld"] \
+                or out.device != buf["device"]:
+            raise ValueError("out is not a trajectory buffer of this env's shape and device: use trajectory_buffer()")
+        elif out.capacity < K:
+            raise ValueError("out holds %d steps, collect() was asked for %d" % (out.capacity, K))
+        head = (ctypes.byref(buf["env"]),)
+        fn = "renv_cartpole_collect_mlp_f32"
+        if self._episode_log is not None:
+            self._check_log_supported()
+            fn, head = "renv_cartpole_collect_mlp_logged_f32", head + (ctypes.byref(self._episode_log.struct),)
+        viol = self._violation_counter(buf["device"])
+        with t.cuda.device(buf["device"]):
+            _lib.call(fn, *head, ctypes.byref(policy.struct), ctypes.byref(out.struct), int(bool(sample)), K,
+                      self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(),
+                      _device.ptr(buf["stats"]), _device.ptr(viol), _device.stream_ptr(buf["device"]))
+        out.tick0, out.num_steps = self._tick, K
+        self._tick += K
+        return out
 
     def _rollout_mlp(self, policy, b, num_steps):
         self._check_mlp_supported(policy, "rollout()")
