@@ -321,6 +321,26 @@ int renv_cartpole_collect_mlp_logged_f32(const renv_cartpole_env *env, const ren
                                          int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
                                          double *stats, unsigned long long *violations, void *stream);
 
+/* Advantage estimation (GAE) under an MLP critic, for the trajectory renv_cartpole_collect_mlp_f32 has just written.
+ * `critic` is a packed 1-output net (l0 = 0): V(s) = l1, the bits renv_cartpole_policy_actions_mlp_f32 returns in logits
+ * row 1 for state s.  env->state must be s_K, the state after the collect's last step; only env->state, n and ld are
+ * read.  The reward is 1.0 on every step.  For every env i, from k = K-1 down to 0, in fp32 with every operation
+ * rounded on its own (no FMA contraction):
+ *     v_k   = V(obs[k])
+ *     nv_k  = done[k] ? (truncated[k] ? V(final_obs[k]) : 0) : (k + 1 < K ? v_{k+1} : V(s_K))
+ *     delta = (1 + gamma * nv_k) - v_k
+ *     A_k   = done[k] ? delta : delta + (gamma * lambda) * A_{k+1},   A_K = 0
+ *     R_k   = A_k + v_k
+ * -- a terminated step bootstraps nothing, a truncated one bootstraps from its terminal observation, and both cut the
+ * trace.  final_obs is read only where truncated.  values[k * ld + i] = v_k, advantages[..] = A_k, returns[..] = R_k:
+ * (capacity, ld) float arrays, 4-byte aligned.  Errors, all before any CUDA call: NULL env / state / critic / params /
+ * traj / obs / done / truncated / final_obs / output RENV_E_NULL; n <= 0, ld < n or K <= 0 RENV_E_SIZE; a misaligned
+ * pointer or ld RENV_E_ALIGN; K > traj->capacity, gamma or lambda outside [0, 1] (or NaN), an unknown activation
+ * RENV_E_ARG. */
+int renv_cartpole_gae_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *critic, const renv_trajectory *traj,
+                              int K, float gamma, float lambda, float *values, float *advantages, float *returns,
+                              void *stream);
+
 /* The SCALAR drop-in env (gym.make('RandomCartPole-v0'): RandomCartPoleEnv.step / reset, random_cartpole.py:172-229,
  * one env, one host call per step) served by a resident one-warp kernel instead of one launch + synchronise per call.
  * `ctrl` is PINNED, DEVICE-MAPPED HOST memory (zero-initialised once): the host rings a request in by writing

@@ -66,6 +66,7 @@ class Trajectory(ctypes.Structure):
 
 _vp, _i64, _u64, _u32, _int, _dbl = (ctypes.c_void_p, ctypes.c_int64, ctypes.c_uint64, ctypes.c_uint32,
                                      ctypes.c_int, ctypes.c_double)
+_flt = ctypes.c_float
 _cfg_p, _env_p, _noise_p = ctypes.POINTER(DrCfg), ctypes.POINTER(CartpoleEnv), ctypes.POINTER(ObsNoise)
 _log_p = ctypes.POINTER(EpisodeLog)
 _mlp_p = ctypes.POINTER(MlpPolicy)
@@ -101,6 +102,7 @@ SIGNATURES = {
     "renv_cartpole_collect_mlp_f32": (_int, [_env_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
     "renv_cartpole_collect_mlp_logged_f32": (_int, [_env_p, _log_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64, _cfg_p,
                                                     _vp, _vp, _vp]),
+    "renv_cartpole_gae_mlp_f32": (_int, [_env_p, _mlp_p, _traj_p, _int, _flt, _flt, _vp, _vp, _vp, _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),
     "renv_random_actions_u8": (_int, [_vp, _i64, _u64, _u64, _u32, _vp]),
     "renv_pack_flags_u8": (_int, [_vp, _vp, _i64, _vp]),

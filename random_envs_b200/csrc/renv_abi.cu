@@ -6,6 +6,7 @@
 #include "renv_rollout_pair.cuh"
 #include "renv_fullgauss_tc.cuh"
 #include "renv_mlp_policy.cuh"
+#include "renv_mlp_gae.cuh"
 #include "renv_scalar_server.cuh"
 #include <stdlib.h>
 
@@ -592,6 +593,39 @@ int collect_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool 
     return launch_status();
 }
 
+int gae_mlp(const renv_cartpole_env *env, const renv_mlp_policy *critic, const renv_trajectory *traj, int K, float gamma,
+            float lambda, float *values, float *advantages, float *returns, void *stream)
+{
+    if (env == nullptr || env->state == nullptr) return RENV_E_NULL;
+    int rc = check_mlp(critic);
+    if (rc) return rc;
+    if (traj == nullptr || traj->obs == nullptr || traj->done == nullptr || traj->truncated == nullptr ||
+        traj->final_obs == nullptr || values == nullptr || advantages == nullptr || returns == nullptr)
+        return RENV_E_NULL;
+    if (env->n <= 0 || env->ld < env->n) return RENV_E_SIZE;
+    if (env->ld % 4 != 0 || !aligned(env->state, 16) || !aligned(traj->obs, 16) || !aligned(traj->final_obs, 16) ||
+        !aligned(traj->done, 4) || !aligned(traj->truncated, 4) || !aligned(values, 4) || !aligned(advantages, 4) ||
+        !aligned(returns, 4))
+        return RENV_E_ALIGN;
+    if (K <= 0) return RENV_E_SIZE;
+    if (K > traj->capacity) return RENV_E_ARG;
+    if (!(gamma >= 0.0f && gamma <= 1.0f) || !(lambda >= 0.0f && lambda <= 1.0f)) return RENV_E_ARG;   // NaN fails too
+    const int64_t blocks = (env->n + kMlpThreads - 1) / kMlpThreads;
+    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    MlpGaeArgs a;
+    a.state = static_cast<const float *>(env->state);
+    a.n = env->n; a.ld = env->ld;
+    a.params = static_cast<const float *>(critic->params);
+    a.obs = traj->obs; a.final_obs = traj->final_obs;
+    a.done = traj->done; a.truncated = traj->truncated;
+    a.values = values; a.advantages = advantages; a.returns = returns;
+    a.K = K; a.gamma = gamma; a.lambda = lambda;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (critic->activation == RENV_MLP_TANH) cartpole_gae_mlp_kernel<kMlpTanh><<<(unsigned)blocks, kMlpThreads, 0, st>>>(a);
+    else cartpole_gae_mlp_kernel<kMlpRelu><<<(unsigned)blocks, kMlpThreads, 0, st>>>(a);
+    return launch_status();
+}
+
 }  // namespace
 
 extern "C" {
@@ -780,6 +814,12 @@ int renv_cartpole_collect_mlp_logged_f32(const renv_cartpole_env *env, const ren
                                          double *stats, unsigned long long *violations, void *stream)
 {
     return collect_mlp(env, log, true, p, traj, sample, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+int renv_cartpole_gae_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *critic, const renv_trajectory *traj,
+                              int K, float gamma, float lambda, float *values, float *advantages, float *returns,
+                              void *stream)
+{
+    return gae_mlp(env, critic, traj, K, gamma, lambda, values, advantages, returns, stream);
 }
 
 int renv_cartpole_scalar_serve(renv_scalar_ctrl *ctrl, void *save, uint32_t lease_id, uint64_t lease_ns, void *stream)

@@ -9,6 +9,9 @@ places, ``o`` = 1 or 2 outputs.  The action is ``argmax(l0, l1)`` with ties goin
 head is taken as ``l0 = 0, l1 = l``, i.e. ``a = [l > 0]``.  The padding is exact: the added units have zero weights and
 biases and ``tanh(0) = relu(0) = 0``.  The kernels evaluate the net with fp32-class accuracy (the 64 x 64 layer on the
 tensor cores as 3xTF32): ``max |logit - float64 logit| <= 1e-5 * max(1, max |float64 logit|)``.
+
+A 1-output net packed the same way is a critic: ``V(s) = l1`` (``outputs == 1``), which
+``RandomCartPoleVecEnv.gae(traj, critic)`` evaluates on a collected trajectory.
 """
 import numpy as np
 
@@ -85,11 +88,15 @@ def reference_logits(params, activation, obs):
 
 
 class MLPPolicy:
-    """Packed device parameters of a supported ``nn.Sequential`` policy (see the module docstring)."""
+    """Packed device parameters of a supported ``nn.Sequential`` policy (see the module docstring).  ``outputs`` is
+    the width of the net's head, 1 or 2 (``from_module`` reads it from the net)."""
 
-    def __init__(self, params, activation, device):
+    def __init__(self, params, activation, device, outputs=2):
         t = _device.torch()
+        if outputs not in (1, 2):
+            raise ValueError("outputs must be 1 or 2, got %r" % (outputs,))
         self.activation = int(activation)
+        self.outputs = int(outputs)     # width of the head: 1 for a critic V(s) = l1 (``RandomCartPoleVecEnv.gae``)
         self.device = t.device(device)
         self.params = t.as_tensor(params, dtype=t.float32).to(self.device).contiguous()    # 16-byte aligned allocation
         s = _lib.MlpPolicy()
@@ -100,7 +107,7 @@ class MLPPolicy:
     def from_module(cls, module, device=None):
         """Validate and pack ``module``.  Raises ValueError for anything but the supported architecture."""
         params, act = pack(module)
-        return cls(params, act, _device.require_cuda(device))
+        return cls(params, act, _device.require_cuda(device), outputs=list(module)[4].out_features)
 
     def reference_logits(self, obs):
         """float64 logits of the packed (padded) net for (N, 4) observations."""

@@ -8,6 +8,12 @@ Step k of env i is row ``[k, i]`` of every field: ``obs`` is the observation the
 ``log pi(action | obs)``, ``dones`` / ``truncated`` are what ``step()`` returned for that step, and ``final_obs`` holds,
 where ``dones``, the observation after the step that auto-reset replaced (the value to bootstrap a truncated episode
 from; elsewhere it is stale).  After ``collect`` the env's ``obs`` is the observation that follows the last step.
+
+    venv.gae(traj, critic, gamma=0.99, lam=0.95)         # one kernel: V under a 1-output MLPPolicy, GAE, returns
+    traj.values, traj.advantages, traj.returns
+
+``gae`` fills ``values`` (V(obs[k])), ``advantages`` and ``returns`` (``advantages + values``), each (K, N) float32;
+they are None until ``gae()`` has run on the current collect.
 """
 from . import _device, _lib
 
@@ -34,11 +40,54 @@ class Trajectory:
         s.final_obs = self._final_obs.data_ptr() if final_obs else None
         s.capacity = capacity
         self.struct = s
+        self._values = self._advantages = self._returns = None      # (capacity, ld) float32, allocated by gae()
         self.tick0 = None           # step clock of step 0 of the last collect
         self.num_steps = 0          # steps the last collect wrote
 
+    @property
+    def tick0(self):
+        """Step clock of step 0 of the last collect (None before the first)."""
+        return self._tick0
+
+    @tick0.setter
+    def tick0(self, tick):
+        self._tick0 = tick
+        self._gae_tick0 = None      # a new collect (even one at the same clock, after seed()): the values, advantages
+                                    # and returns no longer belong to the data
+
+    def _gae_storage(self):
+        """The (capacity, ld) value / advantage / return arrays, allocated on the first ``gae()`` and then reused."""
+        if self._values is None:
+            t = _device.torch()
+            self._values, self._advantages, self._returns = (
+                t.empty((self.capacity, self.ld), dtype=t.float32, device=self.device) for _ in range(3))
+        return self._values, self._advantages, self._returns
+
+    def _gae_done(self):
+        """Record that ``gae()`` has filled the arrays for the current collect."""
+        self._gae_tick0 = self._tick0
+
     def _view(self, buf):
         return None if buf is None else buf[:self.num_steps, :self.num_envs]
+
+    def _gae_view(self, buf):
+        return self._view(buf) if self._gae_tick0 is not None else None
+
+    @property
+    def values(self):
+        """(K, N) float32 V(obs[k]) of the critic of the last ``gae()``, or None unless ``gae()`` ran on this collect."""
+        return self._gae_view(self._values)
+
+    @property
+    def advantages(self):
+        """(K, N) float32 GAE advantages of the last ``gae()``, or None unless ``gae()`` ran on this collect."""
+        return self._gae_view(self._advantages)
+
+    @property
+    def returns(self):
+        """(K, N) float32 ``advantages + values`` (the critic's regression target), or None unless ``gae()`` ran on
+        this collect."""
+        return self._gae_view(self._returns)
 
     @property
     def obs(self):

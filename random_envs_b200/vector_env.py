@@ -10,6 +10,7 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0] or of an MLPPolicy)
     policy_actions(policy) -> (N,)      (the MLPPolicy's actions for the current observations, ready for step)
     collect(policy, K) -> Trajectory    (K fused steps under the sampled policy, every step recorded for training)
+    gae(traj, critic) -> Trajectory     (values, GAE advantages and returns of that trajectory under an MLP critic)
     episode_stats()  -> dict            (returns of the episodes finished inside rollouts)
     start_episode_log(R) -> EpisodeLog  (per-env record of every episode that ends in step / rollout)
 
@@ -440,6 +441,44 @@ class RandomCartPoleVecEnv(RandomEnv):
         out.tick0, out.num_steps = self._tick, K
         self._tick += K
         return out
+
+    def gae(self, traj, critic, gamma=0.99, lam=0.95):
+        """Values, GAE(gamma, lam) advantages and returns of ``traj``, the trajectory this env's last ``collect`` wrote,
+        under ``critic`` (a 1-output MLPPolicy, V(s) = its head): one kernel on the env's stream, which fills
+        ``traj.values``, ``traj.advantages`` and ``traj.returns`` ((K, N) float32) and returns ``traj``.
+
+        The reward is 1 on every step.  A terminated step bootstraps nothing, a truncated one bootstraps from
+        V(final_obs), and both cut the trace; the last step bootstraps from V(obs), the observation after it.  gamma
+        and lam are rounded to float32 and must lie in [0, 1]; the recurrence is that of include/renv.h
+        ``renv_cartpole_gae_mlp_f32``.  Raises ValueError unless the env's clock stands where that collect left it
+        (any step, reset, rollout or collect since then moved it); a ``set_state()`` in between is not detected and is
+        the caller's responsibility.  ``traj`` must have been made with ``final_obs=True``."""
+        self._check_mlp_supported(critic, "gae()")
+        if critic.outputs != 1:
+            raise ValueError("gae() takes a 1-output critic V(s), got a %d-output net" % critic.outputs)
+        b = self._buffers
+        if not isinstance(traj, Trajectory) or traj.num_envs != self.num_envs or traj.ld != b["ld"] \
+                or traj.device != b["device"]:
+            raise ValueError("traj is not a trajectory buffer of this env's shape and device")
+        if traj._final_obs is None:
+            raise ValueError("gae() bootstraps truncated episodes from final_obs: use trajectory_buffer(final_obs=True)")
+        if traj.num_steps == 0:
+            raise ValueError("traj holds no collected steps")
+        g, lm = np.float32(gamma), np.float32(lam)
+        if not (0 <= g <= 1 and 0 <= lm <= 1):
+            raise ValueError("gamma and lam must lie in [0, 1], got %r and %r" % (gamma, lam))
+        if traj.tick0 + traj.num_steps != self._tick:
+            raise ValueError("the env has moved since this trajectory was collected (clock %d, the collect ended at %d): "
+                             "obs is no longer the observation after its last step" % (self._tick,
+                                                                                       traj.tick0 + traj.num_steps))
+        t = _device.torch()
+        values, advantages, returns = traj._gae_storage()
+        with t.cuda.device(b["device"]):
+            _lib.call("renv_cartpole_gae_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(critic.struct),
+                      ctypes.byref(traj.struct), traj.num_steps, float(g), float(lm), _device.ptr(values),
+                      _device.ptr(advantages), _device.ptr(returns), _device.stream_ptr(b["device"]))
+        traj._gae_done()
+        return traj
 
     def _rollout_mlp(self, policy, b, num_steps):
         self._check_mlp_supported(policy, "rollout()")
