@@ -9,10 +9,7 @@
 #include "renv_mlp_gae.cuh"
 #include "renv_scalar_server.cuh"
 #include <stdlib.h>
-
-#ifndef RENV_ROLLOUT_F32_PAIR
-#define RENV_ROLLOUT_F32_PAIR 1     // 0: one env per thread (scalar FFMA) for A/B timing
-#endif
+#include <type_traits>
 
 using namespace renv;
 
@@ -116,6 +113,53 @@ template <typename T> int check_log(const renv_episode_log *log, LogPtrs<T> *out
 
 inline int launch_status() { return (int)cudaGetLastError(); }
 
+// Blocks of `per_block` items each for n items; RENV_E_SIZE when the grid does not fit in a launch.
+inline int grid_for(int64_t n, int64_t per_block, unsigned *blocks)
+{
+    const int64_t g = (n + per_block - 1) / per_block;
+    if (g > 0x7fffffffLL) return RENV_E_SIZE;
+    *blocks = (unsigned)g;
+    return RENV_OK;
+}
+
+int sm_count(int *sms)
+{
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
+    return (int)e;
+}
+
+// One wave of persistent CTAs over tiles of `per_cta` items: min(tiles, SMs x ctas_per_sm).
+int persistent_grid(int64_t n, int per_cta, int ctas_per_sm, unsigned *grid)
+{
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc) return rc;
+    const int64_t tiles = (n + per_cta - 1) / per_cta;
+    *grid = (unsigned)(tiles < (int64_t)sms * ctas_per_sm ? tiles : (int64_t)sms * ctas_per_sm);
+    return RENV_OK;
+}
+
+// A runtime choice as a template argument: f(std::integral_constant<...>{}) for the value given.
+template <typename F> void with_flag(bool b, F &&f)
+{
+    if (b) f(std::true_type{});
+    else f(std::false_type{});
+}
+template <typename F> void with_activation(int activation, F &&f)
+{
+    if (activation == RENV_MLP_TANH) f(std::integral_constant<int, kMlpTanh>{});
+    else f(std::integral_constant<int, kMlpRelu>{});
+}
+// The 8 instances of the MLP rollout and collect kernels: f(activation, euler, logged).
+template <typename F> void with_mlp_instance(int activation, bool euler, bool logged, F &&f)
+{
+    with_activation(activation, [&](auto act) {
+        with_flag(euler, [&](auto eu) { with_flag(logged, [&](auto lg) { f(act, eu, lg); }); });
+    });
+}
+
 #ifndef RENV_STEP_PDL
 #define RENV_STEP_PDL 1
 #endif
@@ -174,19 +218,15 @@ bool launch_fullgaussian_tc(float *out, int64_t n, const FullGaussCfg<float> &g,
 {
     const char *knob = getenv("RENV_FULLGAUSS_TENSOR");           // "0": CUDA-core kernel (tests compare the two)
     if (knob && knob[0] == '0') return false;
-    int dev = 0, sms = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e != cudaSuccess) { *rc = (int)e; return true; }
-    const int64_t tiles = (n + kFgTile - 1) / kFgTile;
-    const int64_t grid = tiles < (int64_t)sms * RENV_FG_TC_CTAS ? tiles : (int64_t)sms * RENV_FG_TC_CTAS;
+    unsigned grid = 0;
+    if ((*rc = persistent_grid(n, kFgTile, RENV_FG_TC_CTAS, &grid))) return true;
     FullGaussCfg<float> gt = g;
     for (int k = 0; k < 32; ++k) {      // the kernel's epilogue takes the WIDTH hi - lo (rounded once, as denormalize does) and mean / 4 (exact)
         gt.hi[k] = g.hi[k] - g.lo[k];
         gt.mean[k] = 0.25f * g.mean[k];
     }
     const PhiloxKeys ks = philox_keys((uint32_t)seed, (uint32_t)(seed >> 32));
-    dr_sample_fullgaussian_tc_kernel<<<(unsigned)grid, kFgThreads, kFgPadSmem, st>>>(out, n, gt, ks, sample_id0, call, counters);
+    dr_sample_fullgaussian_tc_kernel<<<grid, kFgThreads, kFgPadSmem, st>>>(out, n, gt, ks, sample_id0, call, counters);
     *rc = launch_status();
     return true;
 }
@@ -211,14 +251,14 @@ int dr_sample(T *out, int64_t n, const renv_dr_cfg *cfg, uint64_t seed, uint64_t
         for (int k = 0; k < 32; ++k)                 // transposed, zero-padded: ft[k][d] = F[d][k]
             for (int d = 0; d < 32; ++d)
                 g.ft[k * 32 + d] = (k < cfg->dim && d < cfg->dim) ? (T)cfg->factor[d * cfg->dim + k] : T(0);
-        const int64_t gblocks = (n + kFullGaussThreads - 1) / kFullGaussThreads;
-        if (gblocks > 0x7fffffffLL) return RENV_E_SIZE;
+        unsigned gblocks = 0;
+        if (const int rc = grid_for(n, kFullGaussThreads, &gblocks)) return rc;
         const cudaStream_t gst = static_cast<cudaStream_t>(stream);
         if (cfg->dim > 16 && launch_fullgaussian_tc(out, n, g, seed, sample_id0, call, violations, gst, &rc_tc)) return rc_tc;
-        if (cfg->dim <= 4) dr_sample_fullgaussian_kernel<T, 4><<<(unsigned)gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
-        else if (cfg->dim <= 8) dr_sample_fullgaussian_kernel<T, 8><<<(unsigned)gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
-        else if (cfg->dim <= 16) dr_sample_fullgaussian_kernel<T, 16><<<(unsigned)gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
-        else dr_sample_fullgaussian_kernel<T, 32><<<(unsigned)gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
+        if (cfg->dim <= 4) dr_sample_fullgaussian_kernel<T, 4><<<gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
+        else if (cfg->dim <= 8) dr_sample_fullgaussian_kernel<T, 8><<<gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
+        else if (cfg->dim <= 16) dr_sample_fullgaussian_kernel<T, 16><<<gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
+        else dr_sample_fullgaussian_kernel<T, 32><<<gblocks, kFullGaussThreads, 0, gst>>>(out, n, g, seed, sample_id0, call);
         return launch_status();
     }
     // host-side image of renv_dr.cuh load_dim_block: same conversions, same order, done once per launch
@@ -239,13 +279,13 @@ int dr_sample(T *out, int64_t n, const renv_dr_cfg *cfg, uint64_t seed, uint64_t
     }
     const int items = sampler_items<T>(n, cfg->dim);
     const int kTile = tile_samples<T>(cfg->dim, items);
-    const int64_t blocks = (n + kTile - 1) / kTile;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    unsigned blocks = 0;
+    if (const int rc = grid_for(n, kTile, &blocks)) return rc;
     // store width follows the row alignment: whole 128-bit blocks, float pairs (e.g. the 30-dim humanoid), scalars
     constexpr int P = Pack<T>::kPerBlock;
     const int store = cfg->dim % P == 0 ? 0 : (sizeof(T) == 4 && cfg->dim % 2 == 0 ? 1 : 2);
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
-#define RENV_LAUNCH_SAMPLER(TYPE, STORE) launch_sampler<TYPE, STORE>(out, n, c, seed, sample_id0, call, violations, items, (unsigned)blocks, st)
+#define RENV_LAUNCH_SAMPLER(TYPE, STORE) launch_sampler<TYPE, STORE>(out, n, c, seed, sample_id0, call, violations, items, blocks, st)
 #define RENV_LAUNCH_SAMPLER_TYPE(TYPE) \
     do { if (store == 0) RENV_LAUNCH_SAMPLER(TYPE, 0); else if (store == 1) RENV_LAUNCH_SAMPLER(TYPE, 1); \
          else RENV_LAUNCH_SAMPLER(TYPE, 2); } while (0)
@@ -271,9 +311,9 @@ int cartpole_reset(const renv_cartpole_env *env, const renv_obs_noise *noise, co
     a.mask = mask;
     a.tick = tick;
     a.violations = violations;
-    const int64_t blocks = (env->n + 255) / 256;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    cartpole_reset_kernel<T><<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    unsigned blocks = 0;
+    if ((rc = grid_for(env->n, 256, &blocks))) return rc;
+    cartpole_reset_kernel<T><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
     return launch_status();
 }
 
@@ -304,93 +344,70 @@ int cartpole_step(const renv_cartpole_env *env, const renv_obs_noise *noise, con
     a.max_steps = max_steps;
     a.tick = tick;
     a.counters = counters;
-    constexpr int64_t per_block = (int64_t)kStepThreads * VecTraits<T>::V;
-    const int64_t blocks = (env->n + per_block - 1) / per_block;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    unsigned blocks = 0;
+    if ((rc = grid_for(env->n, (int64_t)kStepThreads * VecTraits<T>::V, &blocks))) return rc;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     const bool noisy = a.env.obs != nullptr;
     if (logged) {
         la.step = a;
-        return launch_pdl(cartpole_step_logged_kernel<T>, (unsigned)blocks, kStepThreads, st, la);
+        return launch_pdl(cartpole_step_logged_kernel<T>, blocks, kStepThreads, st, la);
     }
-    if (kLean) return launch_pdl(cartpole_step_kernel<T, true, false, true>, (unsigned)blocks, kStepThreads, st, a);
-    if (auto_reset && !noisy) return launch_pdl(cartpole_step_kernel<T, true, false>, (unsigned)blocks, kStepThreads, st, a);
-    if (auto_reset) return launch_pdl(cartpole_step_kernel<T, true, true>, (unsigned)blocks, kStepThreads, st, a);
-    if (!noisy) return launch_pdl(cartpole_step_kernel<T, false, false>, (unsigned)blocks, kStepThreads, st, a);
-    return launch_pdl(cartpole_step_kernel<T, false, true>, (unsigned)blocks, kStepThreads, st, a);
+    if (kLean) return launch_pdl(cartpole_step_kernel<T, true, false, true>, blocks, kStepThreads, st, a);
+    if (auto_reset && !noisy) return launch_pdl(cartpole_step_kernel<T, true, false>, blocks, kStepThreads, st, a);
+    if (auto_reset) return launch_pdl(cartpole_step_kernel<T, true, true>, blocks, kStepThreads, st, a);
+    if (!noisy) return launch_pdl(cartpole_step_kernel<T, false, false>, blocks, kStepThreads, st, a);
+    return launch_pdl(cartpole_step_kernel<T, false, true>, blocks, kStepThreads, st, a);
 }
 
-// Random policy (w == NULL): one env per thread for both element types (an env draws one Philox block per 128 env-steps
-// for its action bits).  The fp32 env-PAIR kernel was tried for it and is slower (1.4e11 vs 2.4e11 env-steps/s at the time, 3.2e11 now): with
-// ~27-step episodes a pair spends most packed steps with one slot parked for its reset.
-template <typename T> int launch_rollout_random(const RolloutArgs<T> &a, cudaStream_t stream)
+// The checks and arguments every fused rollout shares (linear policy, MLP policy, collect), after the caller's checks
+// of the env, the log, the policy and stats == NULL (the linear rollout checks its policy between that and the
+// alignment of stats).
+template <typename T>
+int check_rollout(double *stats, int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                  unsigned long long *violations, const Policy<T> &policy, RolloutArgs<T> *a)
 {
-    const int64_t blocks = (a.env.n + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.euler) cartpole_rollout_kernel<T, true, false, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_kernel<T, false, false, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    return launch_status();
+    if (!aligned(stats, 8)) return RENV_E_ALIGN;
+    if (K <= 0 || K > (1 << 30)) return RENV_E_SIZE;      // per-thread step counters are 32-bit
+    if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
+    const int rc = to_cfg4<T>(dr, &a->dr);
+    if (rc) return rc;
+    a->policy = policy;
+    a->K = K;
+    a->euler = integrator == RENV_EULER;
+    a->max_steps = max_steps;
+    a->tick = tick;
+    a->stats = stats;
+    a->violations = violations;
+    return RENV_OK;
 }
-template <typename T> int launch_rollout_random(const LoggedRolloutArgs<T> &a, cudaStream_t stream)
+
+// The linear-policy rollout kernels (la.log is read only when logged).  One env per thread, except the fp32 linear
+// policy on the true state: an env PAIR per thread on the packed FFMA2 pipe (renv_rollout_pair.cuh).  The random
+// policy keeps one env per thread for both element types (an env draws one Philox block per 128 env-steps for its
+// action bits): the pair kernel was tried for it and is slower (1.4e11 vs 2.4e11 env-steps/s at the time, 3.2e11
+// now), because with ~27-step episodes a pair spends most packed steps with one slot parked for its reset.
+template <typename T> int launch_rollout(const LoggedRolloutArgs<T> &la, bool logged, bool random, cudaStream_t st)
 {
-    const int64_t blocks = (a.roll.env.n + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.roll.euler) cartpole_rollout_logged_kernel<T, true, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_logged_kernel<T, false, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    return launch_status();
-}
-// Noisy variant (policy on the noisy observation): one env per thread for both element types.
-template <typename T> int launch_rollout_noisy(const RolloutArgs<T> &a, cudaStream_t stream)
-{
-    const int64_t blocks = (a.env.n + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.euler) cartpole_rollout_kernel<T, true, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_kernel<T, false, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    return launch_status();
-}
-// fp64: one env per thread.  fp32: an env PAIR per thread on the packed FFMA2 pipe (renv_rollout_pair.cuh).
-int launch_rollout(const RolloutArgs<double> &a, cudaStream_t stream)
-{
-    if (a.env.obs) return launch_rollout_noisy(a, stream);
-    const int64_t blocks = (a.env.n + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.euler) cartpole_rollout_kernel<double, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_kernel<double, false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    return launch_status();
-}
-int launch_rollout(const RolloutArgs<float> &a, cudaStream_t stream)
-{
-    if (a.env.obs) return launch_rollout_noisy(a, stream);
-#if RENV_ROLLOUT_F32_PAIR
-    const int64_t threads = (a.env.n + kPairSlots - 1) / kPairSlots;
-    const int64_t blocks = (threads + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.euler) cartpole_rollout_pair_kernel<true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_pair_kernel<false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-#else
-    const int64_t blocks = (a.env.n + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.euler) cartpole_rollout_kernel<float, true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_kernel<float, false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-#endif
-    return launch_status();
-}
-// Logged linear-policy rollouts: the same kernel choice as above.
-int launch_rollout(const LoggedRolloutArgs<double> &a, cudaStream_t stream)
-{
-    const int64_t blocks = (a.roll.env.n + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.roll.euler) cartpole_rollout_logged_kernel<double, true, false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_logged_kernel<double, false, false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    return launch_status();
-}
-int launch_rollout(const LoggedRolloutArgs<float> &a, cudaStream_t stream)
-{
-    const int64_t threads = (a.roll.env.n + kPairSlots - 1) / kPairSlots;
-    const int64_t blocks = (threads + kRolloutThreads - 1) / kRolloutThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    if (a.roll.euler) cartpole_rollout_pair_logged_kernel<true><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
-    else cartpole_rollout_pair_logged_kernel<false><<<(unsigned)blocks, kRolloutThreads, 0, stream>>>(a);
+    const RolloutArgs<T> &a = la.roll;
+    const bool noisy = a.env.obs != nullptr;
+    const bool pair = std::is_same<T, float>::value && !random && !noisy;
+    unsigned blocks = 0;
+    const int rc = grid_for(pair ? (a.env.n + kPairSlots - 1) / kPairSlots : a.env.n, kRolloutThreads, &blocks);
+    if (rc) return rc;
+    with_flag(a.euler, [&](auto euler) {
+        if (random) {
+            if (logged) cartpole_rollout_logged_kernel<T, euler, true><<<blocks, kRolloutThreads, 0, st>>>(la);
+            else cartpole_rollout_kernel<T, euler, false, true><<<blocks, kRolloutThreads, 0, st>>>(a);
+        } else if (noisy) {       // the logged entry points take no noise block
+            cartpole_rollout_kernel<T, euler, true><<<blocks, kRolloutThreads, 0, st>>>(a);
+        } else if constexpr (std::is_same<T, float>::value) {
+            if (logged) cartpole_rollout_pair_logged_kernel<euler><<<blocks, kRolloutThreads, 0, st>>>(la);
+            else cartpole_rollout_pair_kernel<euler><<<blocks, kRolloutThreads, 0, st>>>(a);
+        } else {
+            if (logged) cartpole_rollout_logged_kernel<T, euler, false><<<blocks, kRolloutThreads, 0, st>>>(la);
+            else cartpole_rollout_kernel<T, euler><<<blocks, kRolloutThreads, 0, st>>>(a);
+        }
+    });
     return launch_status();
 }
 
@@ -400,34 +417,18 @@ int cartpole_rollout(const renv_cartpole_env *env, const renv_obs_noise *noise, 
                      unsigned long long *violations, void *stream, const renv_episode_log *log = nullptr,
                      bool logged = false)
 {
-    RolloutArgs<T> a;
-    int rc = check_env<T>(env, false, &a.env);
-    if (rc) return rc;
-    rc = attach_noise<T>(noise, &a.env);
-    if (rc) return rc;
     LoggedRolloutArgs<T> la;
+    int rc = check_env<T>(env, false, &la.roll.env);
+    if (rc) return rc;
+    rc = attach_noise<T>(noise, &la.roll.env);
+    if (rc) return rc;
     if (logged && (rc = check_log<T>(log, &la.log))) return rc;
     if (stats == nullptr) return RENV_E_NULL;
     if (w == nullptr && noise != nullptr) return RENV_E_ARG;      // the random policy does not look at observations
-    if (!aligned(stats, 8)) return RENV_E_ALIGN;
-    if (K <= 0 || K > (1 << 30)) return RENV_E_SIZE;      // per-thread step counters are 32-bit
-    if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
-    rc = to_cfg4<T>(dr, &a.dr);
+    const Policy<T> policy = w ? Policy<T>{ (T)w[0], (T)w[1], (T)w[2], (T)w[3], (T)b } : Policy<T>{ T(0), T(0), T(0), T(0), T(0) };
+    rc = check_rollout<T>(stats, K, integrator, max_steps, tick, dr, violations, policy, &la.roll);
     if (rc) return rc;
-    a.policy = w ? Policy<T>{ (T)w[0], (T)w[1], (T)w[2], (T)w[3], (T)b } : Policy<T>{ T(0), T(0), T(0), T(0), T(0) };
-    a.K = K;
-    a.euler = integrator == RENV_EULER;
-    a.max_steps = max_steps;
-    a.tick = tick;
-    a.stats = stats;
-    a.violations = violations;
-    const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (logged) {
-        la.roll = a;
-        return w == nullptr ? launch_rollout_random(la, st) : launch_rollout(la, st);
-    }
-    if (w == nullptr) return launch_rollout_random(a, st);
-    return launch_rollout(a, st);
+    return launch_rollout(la, logged, w == nullptr, static_cast<cudaStream_t>(stream));
 }
 
 // MLP policy (renv_mlp_policy.cuh): the packed parameters and the activation.
@@ -439,92 +440,10 @@ int check_mlp(const renv_mlp_policy *p)
     return RENV_OK;
 }
 
-int sm_count(int *sms)
-{
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
-    return (int)e;
-}
-
-int policy_actions_mlp(const renv_cartpole_env *env, const renv_mlp_policy *p, uint8_t *action, float *logits, void *stream)
-{
-    if (env == nullptr || env->state == nullptr) return RENV_E_NULL;
-    int rc = check_mlp(p);
-    if (rc) return rc;
-    if (action == nullptr) return RENV_E_NULL;
-    if (env->n <= 0 || env->ld < env->n) return RENV_E_SIZE;
-    if (env->ld % 4 != 0 || !aligned(env->state, 16) || !aligned(action, 4) || !aligned(logits, 16)) return RENV_E_ALIGN;
-    MlpActionArgs a;
-    a.state = static_cast<const float *>(env->state);
-    a.n = env->n; a.ld = env->ld;
-    a.params = static_cast<const float *>(p->params);
-    a.action = action; a.logits = logits;
-    int sms = 0;
-    if ((rc = sm_count(&sms))) return rc;
-    const int64_t tiles = (env->n + kMlpThreads - 1) / kMlpThreads;
-    const int64_t grid = tiles < (int64_t)sms * RENV_MLP_CTAS ? tiles : (int64_t)sms * RENV_MLP_CTAS;
-    const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (p->activation == RENV_MLP_TANH) cartpole_policy_actions_mlp_kernel<kMlpTanh><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
-    else cartpole_policy_actions_mlp_kernel<kMlpRelu><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
-    return launch_status();
-}
-
-template <int kAct, bool kLog> void launch_rollout_mlp(const MlpRolloutArgs &a, unsigned blocks, cudaStream_t st)
-{
-    if (a.roll.euler) cartpole_rollout_mlp_kernel<kAct, true, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
-    else cartpole_rollout_mlp_kernel<kAct, false, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
-}
-
-// The argument checks and arguments shared by the MLP rollout and collect entry points.
-int prepare_rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p,
-                        int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
-                        unsigned long long *violations, MlpRolloutArgs *a)
-{
-    int rc = check_env<float>(env, false, &a->roll.env);
-    if (rc) return rc;
-    if (logged && (rc = check_log<float>(log, &a->log))) return rc;
-    if (!logged) a->log = LogPtrs<float>{};
-    if ((rc = check_mlp(p))) return rc;
-    if (stats == nullptr) return RENV_E_NULL;
-    if (!aligned(stats, 8)) return RENV_E_ALIGN;
-    if (K <= 0 || K > (1 << 30)) return RENV_E_SIZE;      // the same range as the linear rollout
-    if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
-    if ((rc = to_cfg4<float>(dr, &a->roll.dr))) return rc;
-    a->roll.policy = Policy<float>{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
-    a->roll.K = K;
-    a->roll.euler = integrator == RENV_EULER;
-    a->roll.max_steps = max_steps;
-    a->roll.tick = tick;
-    a->roll.stats = stats;
-    a->roll.violations = violations;
-    a->params = static_cast<const float *>(p->params);
-    const int64_t blocks = (env->n + kMlpThreads - 1) / kMlpThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    return RENV_OK;
-}
-
-int rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p, int K,
-                int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
-                unsigned long long *violations, void *stream)
-{
-    MlpRolloutArgs a;
-    const int rc = prepare_rollout_mlp(env, log, logged, p, K, integrator, max_steps, tick, dr, stats, violations, &a);
-    if (rc) return rc;
-    const unsigned blocks = (unsigned)((env->n + kMlpThreads - 1) / kMlpThreads);
-    const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (p->activation == RENV_MLP_TANH) {
-        if (logged) launch_rollout_mlp<kMlpTanh, true>(a, blocks, st);
-        else launch_rollout_mlp<kMlpTanh, false>(a, blocks, st);
-    } else {
-        if (logged) launch_rollout_mlp<kMlpRelu, true>(a, blocks, st);
-        else launch_rollout_mlp<kMlpRelu, false>(a, blocks, st);
-    }
-    return launch_status();
-}
-
-int policy_logp_mlp(const renv_cartpole_env *env, const renv_mlp_policy *p, int sample, uint64_t tick, uint8_t *action,
-                    float *logp, float *logits, void *stream)
+// renv_cartpole_policy_logp_mlp_f32 (with_logp) and renv_cartpole_policy_actions_mlp_f32 (argmax only: sample 0, no
+// logp), each on its own kernel.
+int policy_mlp(const renv_cartpole_env *env, const renv_mlp_policy *p, bool with_logp, int sample, uint64_t tick,
+               uint8_t *action, float *logp, float *logits, void *stream)
 {
     if (env == nullptr || env->state == nullptr) return RENV_E_NULL;
     int rc = check_mlp(p);
@@ -542,13 +461,47 @@ int policy_logp_mlp(const renv_cartpole_env *env, const renv_mlp_policy *p, int 
     a.logp = logp;
     a.env_id0 = env->env_id0; a.seed = env->seed; a.tick = tick;
     a.sample = sample;
-    int sms = 0;
-    if ((rc = sm_count(&sms))) return rc;
-    const int64_t tiles = (env->n + kMlpThreads - 1) / kMlpThreads;
-    const int64_t grid = tiles < (int64_t)sms * RENV_MLP_ROLLOUT_CTAS ? tiles : (int64_t)sms * RENV_MLP_ROLLOUT_CTAS;
+    unsigned grid = 0;
+    if ((rc = persistent_grid(env->n, kMlpThreads, with_logp ? RENV_MLP_ROLLOUT_CTAS : RENV_MLP_CTAS, &grid))) return rc;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (p->activation == RENV_MLP_TANH) cartpole_policy_logp_mlp_kernel<kMlpTanh><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
-    else cartpole_policy_logp_mlp_kernel<kMlpRelu><<<(unsigned)grid, kMlpThreads, 0, st>>>(a);
+    with_activation(p->activation, [&](auto act) {
+        if (with_logp) cartpole_policy_logp_mlp_kernel<act><<<grid, kMlpThreads, 0, st>>>(a);
+        else cartpole_policy_actions_mlp_kernel<act><<<grid, kMlpThreads, 0, st>>>(a.act);
+    });
+    return launch_status();
+}
+
+// The argument checks and arguments shared by the MLP rollout and collect entry points (A: MlpRolloutArgs or
+// MlpCollectArgs).
+template <typename A>
+int prepare_rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p,
+                        int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                        unsigned long long *violations, A *a, unsigned *blocks)
+{
+    int rc = check_env<float>(env, false, &a->roll.env);
+    if (rc) return rc;
+    if (logged && (rc = check_log<float>(log, &a->log))) return rc;
+    if (!logged) a->log = LogPtrs<float>{};
+    if ((rc = check_mlp(p))) return rc;
+    if (stats == nullptr) return RENV_E_NULL;
+    const Policy<float> unused{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
+    if ((rc = check_rollout<float>(stats, K, integrator, max_steps, tick, dr, violations, unused, &a->roll))) return rc;
+    a->params = static_cast<const float *>(p->params);
+    return grid_for(env->n, kMlpThreads, blocks);
+}
+
+int rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p, int K,
+                int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                unsigned long long *violations, void *stream)
+{
+    MlpRolloutArgs a;
+    unsigned blocks = 0;
+    const int rc = prepare_rollout_mlp(env, log, logged, p, K, integrator, max_steps, tick, dr, stats, violations, &a, &blocks);
+    if (rc) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_mlp_instance(p->activation, a.roll.euler, logged, [&](auto act, auto euler, auto lg) {
+        cartpole_rollout_mlp_kernel<act, euler, lg><<<blocks, kMlpThreads, 0, st>>>(a);
+    });
     return launch_status();
 }
 
@@ -563,33 +516,21 @@ int check_traj(const renv_trajectory *t, int K, MlpTrajPtrs *out)
     return RENV_OK;
 }
 
-template <int kAct, bool kLog> void launch_collect_mlp(const MlpCollectArgs &a, unsigned blocks, cudaStream_t st)
-{
-    if (a.roll.euler) cartpole_collect_mlp_kernel<kAct, true, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
-    else cartpole_collect_mlp_kernel<kAct, false, kLog><<<blocks, kMlpThreads, 0, st>>>(a);
-}
-
 int collect_mlp(const renv_cartpole_env *env, const renv_episode_log *log, bool logged, const renv_mlp_policy *p,
                 const renv_trajectory *traj, int sample, int K, int integrator, int max_steps, uint64_t tick,
                 const renv_dr_cfg *dr, double *stats, unsigned long long *violations, void *stream)
 {
-    MlpRolloutArgs r;
-    int rc = prepare_rollout_mlp(env, log, logged, p, K, integrator, max_steps, tick, dr, stats, violations, &r);
-    if (rc) return rc;
     MlpCollectArgs a;
+    unsigned blocks = 0;
+    int rc = prepare_rollout_mlp(env, log, logged, p, K, integrator, max_steps, tick, dr, stats, violations, &a, &blocks);
+    if (rc) return rc;
     if ((rc = check_traj(traj, K, &a.traj))) return rc;
     if (sample != 0 && sample != 1) return RENV_E_ARG;
-    a.roll = r.roll; a.params = r.params; a.log = r.log;
     a.sample = sample;
-    const unsigned blocks = (unsigned)((env->n + kMlpThreads - 1) / kMlpThreads);
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (p->activation == RENV_MLP_TANH) {
-        if (logged) launch_collect_mlp<kMlpTanh, true>(a, blocks, st);
-        else launch_collect_mlp<kMlpTanh, false>(a, blocks, st);
-    } else {
-        if (logged) launch_collect_mlp<kMlpRelu, true>(a, blocks, st);
-        else launch_collect_mlp<kMlpRelu, false>(a, blocks, st);
-    }
+    with_mlp_instance(p->activation, a.roll.euler, logged, [&](auto act, auto euler, auto lg) {
+        cartpole_collect_mlp_kernel<act, euler, lg><<<blocks, kMlpThreads, 0, st>>>(a);
+    });
     return launch_status();
 }
 
@@ -610,8 +551,8 @@ int gae_mlp(const renv_cartpole_env *env, const renv_mlp_policy *critic, const r
     if (K <= 0) return RENV_E_SIZE;
     if (K > traj->capacity) return RENV_E_ARG;
     if (!(gamma >= 0.0f && gamma <= 1.0f) || !(lambda >= 0.0f && lambda <= 1.0f)) return RENV_E_ARG;   // NaN fails too
-    const int64_t blocks = (env->n + kMlpThreads - 1) / kMlpThreads;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
+    unsigned blocks = 0;
+    if ((rc = grid_for(env->n, kMlpThreads, &blocks))) return rc;
     MlpGaeArgs a;
     a.state = static_cast<const float *>(env->state);
     a.n = env->n; a.ld = env->ld;
@@ -621,8 +562,9 @@ int gae_mlp(const renv_cartpole_env *env, const renv_mlp_policy *critic, const r
     a.values = values; a.advantages = advantages; a.returns = returns;
     a.K = K; a.gamma = gamma; a.lambda = lambda;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (critic->activation == RENV_MLP_TANH) cartpole_gae_mlp_kernel<kMlpTanh><<<(unsigned)blocks, kMlpThreads, 0, st>>>(a);
-    else cartpole_gae_mlp_kernel<kMlpRelu><<<(unsigned)blocks, kMlpThreads, 0, st>>>(a);
+    with_activation(critic->activation, [&](auto act) {
+        cartpole_gae_mlp_kernel<act><<<blocks, kMlpThreads, 0, st>>>(a);
+    });
     return launch_status();
 }
 
@@ -782,7 +724,7 @@ int renv_cartpole_rollout_noisy_f64(const renv_cartpole_env *env, const renv_obs
 int renv_cartpole_policy_actions_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, uint8_t *action,
                                          float *logits, void *stream)
 {
-    return policy_actions_mlp(env, p, action, logits, stream);
+    return policy_mlp(env, p, false, 0, 0, action, nullptr, logits, stream);
 }
 int renv_cartpole_rollout_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, int K, int integrator,
                                   int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
@@ -800,7 +742,7 @@ int renv_cartpole_rollout_mlp_logged_f32(const renv_cartpole_env *env, const ren
 int renv_cartpole_policy_logp_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, int sample, uint64_t tick,
                                       uint8_t *action, float *logp, float *logits, void *stream)
 {
-    return policy_logp_mlp(env, p, sample, tick, action, logp, logits, stream);
+    return policy_mlp(env, p, true, sample, tick, action, logp, logits, stream);
 }
 int renv_cartpole_collect_mlp_f32(const renv_cartpole_env *env, const renv_mlp_policy *p, const renv_trajectory *traj,
                                   int sample, int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
@@ -837,10 +779,9 @@ int renv_random_actions_u8(uint8_t *action, int64_t n, uint64_t env_id0, uint64_
     if (action == nullptr) return RENV_E_NULL;
     if (n <= 0) return RENV_E_SIZE;
     if (!aligned(action, 4)) return RENV_E_ALIGN;
-    const int64_t threads = (n + 3) / 4;
-    const int64_t blocks = (threads + 255) / 256;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    random_actions_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(action, n, env_id0, seed, step);
+    unsigned blocks = 0;
+    if (const int rc = grid_for((n + 3) / 4, 256, &blocks)) return rc;
+    random_actions_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(action, n, env_id0, seed, step);
     return launch_status();
 }
 
@@ -849,10 +790,9 @@ int renv_pack_flags_u8(const uint8_t *flags, uint32_t *bits, int64_t n, void *st
     if (flags == nullptr || bits == nullptr) return RENV_E_NULL;
     if (n <= 0) return RENV_E_SIZE;
     if (!aligned(flags, 4) || !aligned(bits, 4)) return RENV_E_ALIGN;
-    const int64_t threads = (n + 31) / 32;
-    const int64_t blocks = (threads + 255) / 256;
-    if (blocks > 0x7fffffffLL) return RENV_E_SIZE;
-    pack_flags_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(flags, bits, n);
+    unsigned blocks = 0;
+    if (const int rc = grid_for((n + 31) / 32, 256, &blocks)) return rc;
+    pack_flags_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(flags, bits, n);
     return launch_status();
 }
 

@@ -41,6 +41,9 @@ NOMINAL_TASK = (9.8, 1.0, 0.1, 0.5)                 # random_cartpole.py:74-78
 THETA_THRESHOLD_RADIANS = 12 * 2 * math.pi / 360   # :85
 X_THRESHOLD = 2.4                                  # :86
 MAX_EPISODE_STEPS = 500                            # :294
+# entry points that end episodes: a _logged variant (taking the log after env) runs them while a log is attached
+_LOGGED_ENTRIES = ("step", "step_lean", "rollout", "rollout_mlp", "collect_mlp")
+_NOISY_ENTRIES = ("reset", "step", "rollout")       # a _noisy variant takes the obs-noise block after env
 
 
 def _round_up(x, m):
@@ -172,20 +175,26 @@ class RandomCartPoleVecEnv(RandomEnv):
             b["noise"] = _lib.ObsNoise()
             b["noise"].obs, b["noise"].std = b["obs"].data_ptr(), math.sqrt(self.noise_level)
 
-    def _entry(self, name):
-        """(function name, leading arguments): the *_noisy entry points take the obs-noise block after env, the
-        *_logged ones (step and rollout while an episode log is attached) the log."""
+    def _resolve(self, name):
+        """(C function, leading arguments) of the entry point ``name`` ("reset", "step", "rollout_mlp", ...) for this
+        env: the _logged variant while an episode log is attached, the _noisy one for a noisy env, else the plain
+        one, each for the env's dtype."""
         b = self._buffers
-        if self._episode_log is not None and name in ("step", "rollout"):
-            return "renv_cartpole_%s_logged_%s" % (name, self._suffix()), (ctypes.byref(b["env"]),
-                                                                          ctypes.byref(self._episode_log.struct))
-        if self.noisy:
+        head = (ctypes.byref(b["env"]),)
+        suffix = "f32" if self._dtype_name == "float32" else "f64"
+        if self._episode_log is not None and name in _LOGGED_ENTRIES:
+            self._check_log_supported()
+            return "renv_cartpole_%s_logged_%s" % (name, suffix), head + (ctypes.byref(self._episode_log.struct),)
+        if self.noisy and name in _NOISY_ENTRIES:
             b["noise"].std = math.sqrt(self.noise_level)      # noise_level is a plain attribute in the reference
-            return "renv_cartpole_%s_noisy_%s" % (name, self._suffix()), (ctypes.byref(b["env"]), ctypes.byref(b["noise"]))
-        return "renv_cartpole_%s_%s" % (name, self._suffix()), (ctypes.byref(b["env"]),)
+            return "renv_cartpole_%s_noisy_%s" % (name, suffix), head + (ctypes.byref(b["noise"]),)
+        return "renv_cartpole_%s_%s" % (name, suffix), head
 
-    def _suffix(self):
-        return "f32" if self._dtype_name == "float32" else "f64"
+    def _launch(self, fn, *args):
+        """Call the C function ``fn`` with ``args`` on the env's device and current stream (the last argument)."""
+        dev = self._buffers["device"]
+        with _device.torch().cuda.device(dev):
+            _lib.call(fn, *args, _device.stream_ptr(dev))
 
     def _integrator(self):
         return _lib.EULER if self.kinematics_integrator == "euler" else _lib.SEMI_IMPLICIT   # :187-196
@@ -228,10 +237,8 @@ class RandomCartPoleVecEnv(RandomEnv):
             assert mask.shape == (self.num_envs,)
             mask_ptr = _device.ptr(mask)
         viol = self._violation_counter(b["device"])
-        fn, head = self._entry("reset")
-        with t.cuda.device(b["device"]):
-            _lib.call(fn, *head, mask_ptr, self._tick,
-                      self._active_dr_cfg(), _device.ptr(viol), _device.stream_ptr(b["device"]))
+        fn, head = self._resolve("reset")
+        self._launch(fn, *head, mask_ptr, self._tick, self._active_dr_cfg(), _device.ptr(viol))
         self._tick += 1
         return self.obs
 
@@ -280,9 +287,7 @@ class RandomCartPoleVecEnv(RandomEnv):
             return plan
         t = _device.torch()
         n = self.num_envs
-        if self._episode_log is not None:
-            self._check_log_supported()
-        fn, head = self._entry("step_lean" if self.lean else "step")
+        fn, head = self._resolve("step_lean" if self.lean else "step")
         info = {"TimeLimit.truncated": b["truncated"][:n].view(t.bool)} if self.track_truncated else {}
         viol = self._violation_counter(b["device"])
         plan = dict(key=key, fn=getattr(_lib.load(), fn), name=fn, head=head, logged=self._episode_log is not None,
@@ -348,11 +353,9 @@ class RandomCartPoleVecEnv(RandomEnv):
     def sample_actions(self, out=None):
         """``action_space.sample()`` for every env: (N,) uint8 Bernoulli(1/2), Philox keyed by the step clock."""
         b = self._alloc()
-        t = _device.torch()
         out = b["action"] if out is None else out
-        with t.cuda.device(b["device"]):
-            _lib.call("renv_random_actions_u8", _device.ptr(out), self.num_envs, self.env_id0, self._seed,
-                      self._tick & 0xFFFFFFFF, _device.stream_ptr(b["device"]))
+        self._launch("renv_random_actions_u8", _device.ptr(out), self.num_envs, self.env_id0, self._seed,
+                     self._tick & 0xFFFFFFFF)
         return self._own_action_view() if out is b["action"] else out
 
     def _check_mlp_supported(self, policy, what):
@@ -386,14 +389,13 @@ class RandomCartPoleVecEnv(RandomEnv):
             logp = b.get("mlp_logp")
             if logp is None:
                 logp = b["mlp_logp"] = t.empty(b["ld"], dtype=t.float32, device=b["device"])
-        with t.cuda.device(b["device"]):
-            if sample or return_logp:
-                _lib.call("renv_cartpole_policy_logp_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(policy.struct),
-                          int(bool(sample)), self._tick, _device.ptr(b["action"]), _device.ptr(logp), _device.ptr(logits),
-                          _device.stream_ptr(b["device"]))
-            else:
-                _lib.call("renv_cartpole_policy_actions_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(policy.struct),
-                          _device.ptr(b["action"]), _device.ptr(logits), _device.stream_ptr(b["device"]))
+        if sample or return_logp:
+            fn, head = self._resolve("policy_logp_mlp")
+            self._launch(fn, *head, ctypes.byref(policy.struct), int(bool(sample)), self._tick, _device.ptr(b["action"]),
+                         _device.ptr(logp), _device.ptr(logits))
+        else:
+            fn, head = self._resolve("policy_actions_mlp")
+            self._launch(fn, *head, ctypes.byref(policy.struct), _device.ptr(b["action"]), _device.ptr(logits))
         out = (self._own_action_view(),) + ((logits[:, :n].t(),) if return_logits else ()) + \
             ((logp[:n],) if return_logp else ())
         return out if len(out) > 1 else out[0]
@@ -414,7 +416,6 @@ class RandomCartPoleVecEnv(RandomEnv):
         Advances the step clock by K; afterwards ``obs`` is the observation after the last step (the bootstrap
         observation).  float32 envs without observation noise or lean=True only."""
         buf = self._alloc()
-        t = _device.torch()
         if self.lean:
             raise ValueError("collect() keeps the int32 TimeLimit counter: build the env without lean=True")
         self._check_mlp_supported(policy, "collect()")
@@ -428,16 +429,11 @@ class RandomCartPoleVecEnv(RandomEnv):
             raise ValueError("out is not a trajectory buffer of this env's shape and device: use trajectory_buffer()")
         elif out.capacity < K:
             raise ValueError("out holds %d steps, collect() was asked for %d" % (out.capacity, K))
-        head = (ctypes.byref(buf["env"]),)
-        fn = "renv_cartpole_collect_mlp_f32"
-        if self._episode_log is not None:
-            self._check_log_supported()
-            fn, head = "renv_cartpole_collect_mlp_logged_f32", head + (ctypes.byref(self._episode_log.struct),)
+        fn, head = self._resolve("collect_mlp")
         viol = self._violation_counter(buf["device"])
-        with t.cuda.device(buf["device"]):
-            _lib.call(fn, *head, ctypes.byref(policy.struct), ctypes.byref(out.struct), int(bool(sample)), K,
-                      self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(),
-                      _device.ptr(buf["stats"]), _device.ptr(viol), _device.stream_ptr(buf["device"]))
+        self._launch(fn, *head, ctypes.byref(policy.struct), ctypes.byref(out.struct), int(bool(sample)), K,
+                     self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(),
+                     _device.ptr(buf["stats"]), _device.ptr(viol))
         out.tick0, out.num_steps = self._tick, K
         self._tick += K
         return out
@@ -471,57 +467,34 @@ class RandomCartPoleVecEnv(RandomEnv):
             raise ValueError("the env has moved since this trajectory was collected (clock %d, the collect ended at %d): "
                              "obs is no longer the observation after its last step" % (self._tick,
                                                                                        traj.tick0 + traj.num_steps))
-        t = _device.torch()
         values, advantages, returns = traj._gae_storage()
-        with t.cuda.device(b["device"]):
-            _lib.call("renv_cartpole_gae_mlp_f32", ctypes.byref(b["env"]), ctypes.byref(critic.struct),
-                      ctypes.byref(traj.struct), traj.num_steps, float(g), float(lm), _device.ptr(values),
-                      _device.ptr(advantages), _device.ptr(returns), _device.stream_ptr(b["device"]))
+        fn, head = self._resolve("gae_mlp")
+        self._launch(fn, *head, ctypes.byref(critic.struct), ctypes.byref(traj.struct), traj.num_steps, float(g), float(lm),
+                     _device.ptr(values), _device.ptr(advantages), _device.ptr(returns))
         traj._gae_done()
         return traj
-
-    def _rollout_mlp(self, policy, b, num_steps):
-        self._check_mlp_supported(policy, "rollout()")
-        if float(b) != 0.0:
-            raise ValueError("an MLPPolicy carries its own biases: rollout(policy) takes no b")
-        buf = self._buffers
-        t = _device.torch()
-        head = (ctypes.byref(buf["env"]),)
-        fn = "renv_cartpole_rollout_mlp_f32"
-        if self._episode_log is not None:
-            self._check_log_supported()
-            fn, head = "renv_cartpole_rollout_mlp_logged_f32", head + (ctypes.byref(self._episode_log.struct),)
-        viol = self._violation_counter(buf["device"])
-        with t.cuda.device(buf["device"]):
-            _lib.call(fn, *head, ctypes.byref(policy.struct), int(num_steps), self._integrator(), self.max_episode_steps,
-                      self._tick, self._active_dr_cfg(), _device.ptr(buf["stats"]), _device.ptr(viol),
-                      _device.stream_ptr(buf["device"]))
-        self._tick += int(num_steps)
 
     def rollout(self, w, b=0.0, num_steps=MAX_EPISODE_STEPS):
         """K fused env-steps under the in-kernel linear policy a = [w.s + b > 0] (auto-reset always on), with
         ``w=None`` under the random policy ``action_space.sample()`` (test_random_policy.py:26), or with an
         ``MLPPolicy`` in place of ``w`` under that network (float32 envs without observation noise; ``b`` must be 0)."""
         buf = self._alloc()
-        t = _device.torch()
         if self.lean:
             raise ValueError("rollout() keeps the int32 TimeLimit counter: build the env without lean=True")
         if isinstance(w, MLPPolicy):
-            return self._rollout_mlp(w, b, num_steps)
-        if w is None:         # random policy: the fused equivalent of K x step(sample_actions())
-            if self.noisy:
-                raise ValueError("the random policy ignores observations: use a noise-free env")
-            w_arr = None
+            self._check_mlp_supported(w, "rollout()")
+            if float(b) != 0.0:
+                raise ValueError("an MLPPolicy carries its own biases: rollout(policy) takes no b")
+            name, policy_args = "rollout_mlp", (ctypes.byref(w.struct),)
         else:
-            w_arr = (ctypes.c_double * 4)(*[float(v) for v in w])
-        if self._episode_log is not None:
-            self._check_log_supported()
+            if w is None and self.noisy:        # random policy: the fused equivalent of K x step(sample_actions())
+                raise ValueError("the random policy ignores observations: use a noise-free env")
+            w_arr = None if w is None else (ctypes.c_double * 4)(*[float(v) for v in w])
+            name, policy_args = "rollout", (w_arr, float(b))    # Noisy variant: the policy acts on the noisy observation
+        fn, head = self._resolve(name)
         viol = self._violation_counter(buf["device"])
-        fn, head = self._entry("rollout")         # Noisy variant: the policy acts on the noisy observation
-        with t.cuda.device(buf["device"]):
-            _lib.call(fn, *head, w_arr, float(b),
-                      int(num_steps), self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(),
-                      _device.ptr(buf["stats"]), _device.ptr(viol), _device.stream_ptr(buf["device"]))
+        self._launch(fn, *head, *policy_args, int(num_steps), self._integrator(), self.max_episode_steps, self._tick,
+                     self._active_dr_cfg(), _device.ptr(buf["stats"]), _device.ptr(viol))
         self._tick += int(num_steps)
 
     # ---- episode log ----------------------------------------------------------------------------------
@@ -542,8 +515,8 @@ class RandomCartPoleVecEnv(RandomEnv):
         self._episode_log = None
 
     def _check_log_supported(self):
-        """The logged entry points imply auto-reset and take no noise block: also checked at every step-plan rebuild
-        and rollout, since ``auto_reset`` and ``noisy`` are plain attributes a caller may change with a log attached."""
+        """The logged entry points imply auto-reset and take no noise block: also checked whenever ``_resolve`` picks
+        one, since ``auto_reset`` and ``noisy`` are plain attributes a caller may change with a log attached."""
         if self.lean or self.noisy or not self.auto_reset:
             raise ValueError("the episode log needs an auto-reset env without lean=True or observation noise")
 

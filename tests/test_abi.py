@@ -5,6 +5,7 @@ import re
 
 import pytest
 
+from abi_support import fake_env, gcc_layout
 from random_envs_b200 import _lib, build
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -54,10 +55,8 @@ def test_strerror_and_argument_validation_without_a_gpu():
     assert lib.renv_dr_sample_f32(ctypes.c_void_p(256), 8, ctypes.byref(cfg), 0, 0, 0, None, None) == -4
     cfg.dim, cfg.dr_type = 4, 9
     assert lib.renv_dr_sample_f32(ctypes.c_void_p(256), 8, ctypes.byref(cfg), 0, 0, 0, None, None) == -5
-    env = _lib.CartpoleEnv()
-    assert lib.renv_cartpole_reset_f32(ctypes.byref(env), None, 0, None, None, None) == -1
-    env.state = env.xi = env.elapsed = env.episode = 4096
-    env.n, env.ld = 10, 8
+    assert lib.renv_cartpole_reset_f32(ctypes.byref(_lib.CartpoleEnv()), None, 0, None, None, None) == -1
+    env = fake_env(ld=8)
     assert lib.renv_cartpole_reset_f32(ctypes.byref(env), None, 0, None, None, None) == -3             # ld < n
     env.ld = 10
     assert lib.renv_cartpole_reset_f32(ctypes.byref(env), None, 0, None, None, None) == -2             # ld % 4
@@ -79,9 +78,7 @@ def test_unknown_dr_type_raises_reference_message():
 
 def test_noisy_and_rollout_argument_validation_without_a_gpu():
     lib = _lib.load()
-    env = _lib.CartpoleEnv()
-    env.state = env.xi = env.elapsed = env.episode = env.beyond = 4096
-    env.n, env.ld = 10, 12
+    env = fake_env(beyond=4096)
     w = (ctypes.c_double * 4)(0, 0, 1, 0)
     noise = _lib.ObsNoise()
     assert lib.renv_cartpole_step_noisy_f32(ctypes.byref(env), None, 4096, 4096, 4096, None, 0, 500, 1, 0, None, None, None) == -1
@@ -107,22 +104,11 @@ def test_noisy_and_rollout_argument_validation_without_a_gpu():
 def test_scalar_ctrl_offsets_in_python_match_the_header(tmp_path):
     """random_cartpole._ResidentScalarCore addresses struct renv_scalar_ctrl by byte offset (the block is shared with a
     running kernel through pinned host memory): the offsets must be the C compiler's."""
-    import shutil
-    import subprocess
-    gcc = shutil.which("gcc")
-    if gcc is None:
-        pytest.skip("no gcc")
     fields = ["request", "arg", "arg_u64", "state", "obs", "xi", "reward", "done", "beyond", "violations", "ack",
               "exited", "next", "next_seq"]
-    src = tmp_path / "offsets.c"
-    src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "renv.h"\nint main(void) {\n' +
-                   "".join('  printf("%s %%zu\\n", offsetof(renv_scalar_ctrl, %s));\n' % (f, f) for f in fields) +
-                   '  printf("sizeof %zu\\n", sizeof(renv_scalar_ctrl));\n'
-                   '  printf("stride %zu\\n", sizeof(struct renv_scalar_outcome));\n'
-                   '  printf("outcome_reward %zu\\n", offsetof(struct renv_scalar_outcome, reward));\n  return 0;\n}\n')
-    exe = tmp_path / "offsets"
-    subprocess.run([gcc, "-I", os.path.dirname(HEADER), "-o", str(exe), str(src)], check=True)
-    got = dict(line.split() for line in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.splitlines())
+    got = gcc_layout(tmp_path, "renv_scalar_ctrl", fields,
+                     [("stride", "%zu", "sizeof(struct renv_scalar_outcome)"),
+                      ("outcome_reward", "%zu", "offsetof(struct renv_scalar_outcome, reward)")])
     from random_envs_b200.random_cartpole import _ResidentScalarCore as C
     want = dict(request=C.OFF_REQUEST, arg=C.OFF_ARG, arg_u64=C.OFF_ARG_U64, state=C.OFF_STATE, obs=C.OFF_OBS, xi=C.OFF_XI,
                 reward=C.OFF_REWARD, done=C.OFF_DONE, beyond=C.OFF_BEYOND, violations=C.OFF_VIOL, ack=C.OFF_ACK,

@@ -12,6 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "profiles"))
 import sass_stats  # noqa: E402
 
+from abi_support import ptxas_blocks  # noqa: E402
 from random_envs_b200 import build as lib_build  # noqa: E402
 
 
@@ -84,15 +85,10 @@ def test_fullgaussian_contraction_runs_on_tcgen05(sass):
 
 def test_no_register_spills_in_any_kernel():
     """Every kernel of the library: zero spill stores / loads (ptxas -v log written by the build)."""
-    path = os.path.join(ROOT, "random_envs_b200", "librenv_b200.ptxas.log")
-    if not os.path.isfile(path):
-        lib_build.build(force=True)         # the log is written by the build (it is not tracked)
-    log = open(path).read()
-    blocks = re.split(r"ptxas info\s+: Compiling entry function '", log)[1:]
+    blocks = ptxas_blocks()
     assert len(blocks) >= 45
     seen = set()
-    for b in blocks:
-        name = b.split("'")[0]
+    for name, b in blocks.items():
         for st, ld in re.findall(r"(\d+) bytes spill stores, (\d+) bytes spill loads", b):
             assert st == "0" and ld == "0", (name, st, ld)
         regs = int(re.search(r"Used (\d+) registers", b).group(1))

@@ -3,63 +3,29 @@ collect and policy_logp entry points, the compiled form of the new kernels, and 
 import ctypes
 import os
 import re
-import shutil
-import subprocess
 import sys
 
 import pytest
 import torch
 
+from abi_support import ROOT, fake_env as _env, fake_log, fake_policy as _policy, fake_traj as _traj, gcc_layout, \
+    ptxas_blocks
 from random_envs_b200 import Trajectory, _lib, build as lib_build
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HEADER = os.path.join(ROOT, "include", "renv.h")
 FIELDS = ["obs", "action", "done", "logp", "truncated", "final_obs", "capacity"]
 
 
 def test_trajectory_struct_offsets_in_python_match_the_header(tmp_path):
-    gcc = shutil.which("gcc")
-    if gcc is None:
-        pytest.skip("no gcc")
-    src = tmp_path / "offsets.c"
-    src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "renv.h"\nint main(void) {\n' +
-                   "".join('  printf("%s %%zu\\n", offsetof(renv_trajectory, %s));\n' % (f, f) for f in FIELDS) +
-                   '  printf("sizeof %zu\\n", sizeof(renv_trajectory));\n  return 0;\n}\n')
-    exe = tmp_path / "offsets"
-    subprocess.run([gcc, "-I", os.path.dirname(HEADER), "-o", str(exe), str(src)], check=True)
-    got = dict(line.split() for line in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.splitlines())
+    got = gcc_layout(tmp_path, "renv_trajectory", FIELDS)
     want = {f: getattr(_lib.Trajectory, f).offset for f in FIELDS}
     want["sizeof"] = ctypes.sizeof(_lib.Trajectory)
     assert {k: int(v) for k, v in got.items()} == want
 
 
-def _env():
-    env = _lib.CartpoleEnv()
-    env.state = env.xi = env.elapsed = env.episode = 4096
-    env.n, env.ld = 10, 12
-    return env
-
-
-def _policy(params=4096, act=0):
-    p = _lib.MlpPolicy()
-    p.params, p.activation = params, act
-    return p
-
-
-def _traj(**kw):
-    t = _lib.Trajectory()
-    t.obs, t.action, t.done, t.logp, t.truncated, t.final_obs, t.capacity = 4096, 8192, 8448, 8704, 8960, 12288, 8
-    for k, v in kw.items():
-        setattr(t, k, v)
-    return t
-
-
 def _rcs(env=None, pol="ok", traj="ok", sample=1, K=5, integrator=0, dr=None, stats=4096):
     """Status of the plain and the logged collect entry point for the same arguments."""
     lib = _lib.load()
-    log = _lib.EpisodeLog()
-    log.xi, log.final_state, log.length, log.truncated, log.end_tick, log.count = 8192, 12288, 16384, 20480, 24576, 28672
-    log.capacity = 2
+    log = fake_log()
     env = _env() if env is None else env
     pol = _policy() if pol == "ok" else pol
     traj = _traj() if traj == "ok" else traj
@@ -121,13 +87,6 @@ def test_policy_logp_validates_arguments_before_any_cuda_call():
     assert f(ctypes.byref(bad_env), p, 0, 0, 4096, None, None, None) == -3
 
 
-def _ptxas_blocks():
-    path = os.path.join(ROOT, "random_envs_b200", "librenv_b200.ptxas.log")
-    if not os.path.isfile(path):
-        lib_build.build(force=True)         # the log is written by the build (it is not tracked)
-    return {b.split("'")[0]: b for b in re.split(r"ptxas info\s+: Compiling entry function '", open(path).read())[1:]}
-
-
 def test_collect_and_policy_logp_kernels_keep_the_mlp_budgets():
     sys.path.insert(0, os.path.join(ROOT, "profiles"))
     import sass_stats
@@ -142,7 +101,7 @@ def test_collect_and_policy_logp_kernels_keep_the_mlp_budgets():
         assert not any(o.startswith("MUFU.TANH") for o in ops), name
     for name in logp:                                                    # no local memory at all
         assert not any(op.startswith(("LDL", "STL")) for _, op, _ in sass[name]), name
-    blocks = _ptxas_blocks()
+    blocks = ptxas_blocks()
     for name in collect + logp:
         b = blocks[name]
         assert re.search(r"\b0 bytes spill stores, 0 bytes spill loads", b), name

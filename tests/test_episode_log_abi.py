@@ -3,48 +3,22 @@ points, the Python-side rejection of unsupported env variants, and the compiled 
 import ctypes
 import os
 import re
-import shutil
-import subprocess
 import sys
 
 import pytest
 
+from abi_support import ROOT, fake_env as _env, fake_log as _log, gcc_layout, ptxas_blocks
 from random_envs_b200 import _lib, build as lib_build
 import random_envs_b200 as random_envs
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HEADER = os.path.join(ROOT, "include", "renv.h")
 FIELDS = ["xi", "final_state", "length", "truncated", "end_tick", "count", "capacity"]
 
 
 def test_episode_log_struct_offsets_in_python_match_the_header(tmp_path):
-    gcc = shutil.which("gcc")
-    if gcc is None:
-        pytest.skip("no gcc")
-    src = tmp_path / "offsets.c"
-    src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "renv.h"\nint main(void) {\n' +
-                   "".join('  printf("%s %%zu\\n", offsetof(renv_episode_log, %s));\n' % (f, f) for f in FIELDS) +
-                   '  printf("sizeof %zu\\n", sizeof(renv_episode_log));\n  return 0;\n}\n')
-    exe = tmp_path / "offsets"
-    subprocess.run([gcc, "-I", os.path.dirname(HEADER), "-o", str(exe), str(src)], check=True)
-    got = dict(line.split() for line in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.splitlines())
+    got = gcc_layout(tmp_path, "renv_episode_log", FIELDS)
     want = {f: getattr(_lib.EpisodeLog, f).offset for f in FIELDS}
     want["sizeof"] = ctypes.sizeof(_lib.EpisodeLog)
     assert {k: int(v) for k, v in got.items()} == want
-
-
-def _env():
-    env = _lib.CartpoleEnv()
-    env.state = env.xi = env.elapsed = env.episode = 4096
-    env.n, env.ld = 10, 12
-    return env
-
-
-def _log():
-    log = _lib.EpisodeLog()
-    log.xi, log.final_state, log.length, log.truncated, log.end_tick, log.count = 8192, 12288, 16384, 20480, 24576, 28672
-    log.capacity = 2
-    return log
 
 
 def _calls(env, log):
@@ -92,18 +66,8 @@ def test_start_episode_log_rejects_unsupported_envs_before_touching_cuda(kw):
     assert env._buffers is None
 
 
-def _ptxas_blocks():
-    path = os.path.join(ROOT, "random_envs_b200", "librenv_b200.ptxas.log")
-    if lib_build.is_stale() or not os.path.isfile(path):
-        lib_build.build(force=True)
-    blocks = {}
-    for b in re.split(r"ptxas info\s+: Compiling entry function '", open(path).read())[1:]:
-        blocks[b.split("'")[0]] = b
-    return blocks
-
-
 def test_logged_kernels_have_no_spills_and_keep_their_occupancy():
-    logged = {name: b for name, b in _ptxas_blocks().items() if "logged_kernel" in name}
+    logged = {name: b for name, b in ptxas_blocks().items() if "logged_kernel" in name}
     assert len(logged) == 10, sorted(logged)      # step f32/f64, pair x2, generic (fp64 x2 policies, fp32 random) x2
     for name, b in logged.items():
         for st, ld in re.findall(r"(\d+) bytes spill stores, (\d+) bytes spill loads", b):

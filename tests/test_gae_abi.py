@@ -11,32 +11,8 @@ import torch
 from torch import nn
 
 import random_envs_b200 as random_envs
+from abi_support import ROOT, fake_env as _env, fake_policy as _critic, fake_traj as _traj, ptxas_blocks
 from random_envs_b200 import MLPPolicy, Trajectory, _device, _lib, build as lib_build
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _env(**kw):
-    env = _lib.CartpoleEnv()
-    env.state = env.xi = env.elapsed = env.episode = 4096
-    env.n, env.ld = 10, 12
-    for k, v in kw.items():
-        setattr(env, k, v)
-    return env
-
-
-def _critic(params=4096, act=0):
-    p = _lib.MlpPolicy()
-    p.params, p.activation = params, act
-    return p
-
-
-def _traj(**kw):
-    t = _lib.Trajectory()
-    t.obs, t.action, t.done, t.logp, t.truncated, t.final_obs, t.capacity = 4096, 8192, 8448, 8704, 8960, 12288, 8
-    for k, v in kw.items():
-        setattr(t, k, v)
-    return t
 
 
 def _rc(env="ok", critic="ok", traj="ok", K=5, gamma=0.99, lam=0.95, values=16384, advantages=20480, returns=24576):
@@ -89,13 +65,6 @@ def test_gae_entry_point_is_bound_with_float_gamma_and_lambda():
     assert _lib.load().renv_cartpole_gae_mlp_f32.argtypes == argtypes
 
 
-def _ptxas_blocks():
-    path = os.path.join(ROOT, "random_envs_b200", "librenv_b200.ptxas.log")
-    if not os.path.isfile(path):
-        lib_build.build(force=True)         # the log is written by the build (it is not tracked)
-    return {b.split("'")[0]: b for b in re.split(r"ptxas info\s+: Compiling entry function '", open(path).read())[1:]}
-
-
 def test_gae_kernels_use_the_tensor_cores_without_spills_or_local_memory():
     sys.path.insert(0, os.path.join(ROOT, "profiles"))
     import sass_stats
@@ -103,7 +72,7 @@ def test_gae_kernels_use_the_tensor_cores_without_spills_or_local_memory():
     sass = sass_stats.functions(lib_build.LIB_PATH)
     names = [n for n in sass if "cartpole_gae_mlp_kernel" in n]
     assert len(names) == 2, names                                       # Tanh and ReLU
-    blocks = _ptxas_blocks()
+    blocks = ptxas_blocks()
     for name in names:
         ops = [op for _, op, _ in sass[name]]
         hmma = sum(o.startswith("HMMA.1688.F32.TF32") for o in ops)

@@ -3,8 +3,6 @@ rejection of unsupported networks, exactness of the 64-unit padding, and the com
 import ctypes
 import os
 import re
-import shutil
-import subprocess
 import sys
 
 import numpy as np
@@ -12,27 +10,14 @@ import pytest
 import torch
 from torch import nn
 
+from abi_support import ROOT, fake_env as _env, fake_log, fake_policy as _policy, gcc_layout, ptxas_blocks
 from random_envs_b200 import _lib, build as lib_build, mlp_policy
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HEADER = os.path.join(ROOT, "include", "renv.h")
 
 
 def test_mlp_policy_struct_offsets_in_python_match_the_header(tmp_path):
-    gcc = shutil.which("gcc")
-    if gcc is None:
-        pytest.skip("no gcc")
-    src = tmp_path / "offsets.c"
-    src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "renv.h"\nint main(void) {\n'
-                   '  printf("params %zu\\n", offsetof(renv_mlp_policy, params));\n'
-                   '  printf("activation %zu\\n", offsetof(renv_mlp_policy, activation));\n'
-                   '  printf("sizeof %zu\\n", sizeof(renv_mlp_policy));\n'
-                   '  printf("floats %d\\n", RENV_MLP_PARAM_FLOATS);\n'
-                   '  printf("hidden %d\\n", RENV_MLP_HIDDEN);\n'
-                   '  printf("tanh %d\\n", RENV_MLP_TANH);\n  printf("relu %d\\n", RENV_MLP_RELU);\n  return 0;\n}\n')
-    exe = tmp_path / "offsets"
-    subprocess.run([gcc, "-I", os.path.dirname(HEADER), "-o", str(exe), str(src)], check=True)
-    got = dict(line.split() for line in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.splitlines())
+    got = gcc_layout(tmp_path, "renv_mlp_policy", ["params", "activation"],
+                     [("floats", "%d", "RENV_MLP_PARAM_FLOATS"), ("hidden", "%d", "RENV_MLP_HIDDEN"),
+                      ("tanh", "%d", "RENV_MLP_TANH"), ("relu", "%d", "RENV_MLP_RELU")])
     want = dict(params=_lib.MlpPolicy.params.offset, activation=_lib.MlpPolicy.activation.offset,
                 sizeof=ctypes.sizeof(_lib.MlpPolicy), floats=mlp_policy.PARAM_FLOATS, hidden=mlp_policy.HIDDEN,
                 tanh=mlp_policy.TANH, relu=mlp_policy.RELU)
@@ -40,24 +25,9 @@ def test_mlp_policy_struct_offsets_in_python_match_the_header(tmp_path):
     assert mlp_policy.PARAM_FLOATS == 4612 and (64 * 4 + 64 + 64 * 64 + 64 + 2 * 64 + 2 + 3) // 4 * 4 == 4612
 
 
-def _env():
-    env = _lib.CartpoleEnv()
-    env.state = env.xi = env.elapsed = env.episode = 4096
-    env.n, env.ld = 10, 12
-    return env
-
-
-def _policy(params=4096, act=0):
-    p = _lib.MlpPolicy()
-    p.params, p.activation = params, act
-    return p
-
-
 def _rcs(env, pol, K=5, integrator=0, dr=None, stats=4096):
     lib = _lib.load()
-    log = _lib.EpisodeLog()
-    log.xi, log.final_state, log.length, log.truncated, log.end_tick, log.count = 8192, 12288, 16384, 20480, 24576, 28672
-    log.capacity = 2
+    log = fake_log()
     pp = ctypes.byref(pol) if pol is not None else None
     e = ctypes.byref(env)
     return [lib.renv_cartpole_rollout_mlp_f32(e, pp, K, integrator, 500, 0, dr, stats, None, None),
@@ -173,8 +143,7 @@ def test_mlp_kernels_run_layer_2_on_the_tensor_cores_without_spills():
         assert not any(o.startswith("MUFU.TANH") for o in ops), name        # the accurate tanh, not tanh.approx
     for name in actions:                                                     # no local memory at all
         assert not any(op.startswith(("LDL", "STL")) for _, op, _ in sass[name]), name
-    path = os.path.join(ROOT, "random_envs_b200", "librenv_b200.ptxas.log")
-    blocks = {b.split("'")[0]: b for b in re.split(r"ptxas info\s+: Compiling entry function '", open(path).read())[1:]}
+    blocks = ptxas_blocks()
     for name in rollout + actions:
         b = blocks[name]
         assert re.search(r"\b0 bytes spill stores, 0 bytes spill loads", b), name
