@@ -341,6 +341,41 @@ int renv_cartpole_gae_mlp_f32(const renv_cartpole_env *env, const renv_mlp_polic
                               int K, float gamma, float lambda, float *values, float *advantages, float *returns,
                               void *stream);
 
+/* Recorded cart-pole transitions for offline DR fitting (device pointers): transition i is (obs[i], action[i],
+ * next_obs[i]), and `window` lists the W start indices t that are scored (t + lam <= T; windows crossing an episode
+ * boundary are the caller's to leave out). */
+typedef struct renv_transitions {
+    const double *obs;           /* (T, 4) rows x, x_dot, theta, theta_dot, 16-byte aligned */
+    const double *next_obs;      /* (T, 4) rows, 16-byte aligned: the observation after action[i] */
+    const uint8_t *action;       /* (T) in {0, 1} */
+    const int32_t *window;       /* (W) start indices, 4-byte aligned */
+    int64_t T;
+    int32_t W;
+} renv_transitions;
+
+/* Log-likelihood of C candidate task distributions on recorded transitions, the objective DROPO-style offline DR
+ * fitting maximises (it replaces set_task / state assignment / step, random_cartpole.py:157-166,172-205, called once per
+ * candidate, transition, sample and step).  Candidate c is given by M >= 2 task samples xi (C, M, 4) rows, 16-byte
+ * aligned (gravity, cart_mass, pole_mass, pole_length).  For window w with start t and sample m:
+ *     s_m = lam applications of RandomCartPoleEnv's dynamics (:176-196, the fp64 parity arithmetic of step; termination
+ *           is ignored: no TimeLimit, no reset) under xi[c, m] and actions action[t .. t+lam-1], from obs[t]
+ *     y = next_obs[t+lam-1],  mu = mean_m s_m,  Sigma = 1/(M-1) sum_m (s_m - mu)(s_m - mu)' (numpy cov, ddof 1)
+ *     S = Sigma + diag(eps)
+ *     loglik[c * W + w] = -1/2 (y - mu)' S^-1 (y - mu) - 1/2 log det S - 2 log(2 pi)
+ *                         (= scipy.stats.multivariate_normal.logpdf(y, mu, S));
+ *                         -inf when the Cholesky factorisation of S meets a pivot <= 0 or NaN;
+ *                         NaN when t < 0 or t + lam > T (a device-side guard; validate windows on the host)
+ *     total[c] = sum_w loglik[c, w]  (fixed order, compensated: within a few ulp of the exact sum of the values)
+ * eps (4 doubles, host) >= 0, per dimension: under Euler with lam = 1 the rows x and theta of s_m do not depend on xi,
+ * so two rows of Sigma are exactly zero and S is singular without it; with observation noise of std sigma in obs and
+ * next_obs, eps = 2 sigma^2 is the natural floor.  loglik (C, W) and total (C) are device doubles, 8-byte aligned.
+ * Bitwise reproducible: loglik[c, .] and total[c] depend only on (data, windows, xi[c], eps, lam, integrator), not on C,
+ * the other candidates or the launch, and two identical calls give identical bits.  Errors, all before any CUDA call:
+ * NULL data / pointer RENV_E_NULL; a misaligned pointer RENV_E_ALIGN; T, W, C < 1, M < 2, lam < 1 or lam > T
+ * RENV_E_SIZE; an unknown integrator RENV_E_INTEGRATOR; eps < 0 or not finite RENV_E_ARG. */
+int renv_cartpole_transition_loglik_f64(const renv_transitions *data, int lam, int integrator, const double *xi, int C,
+                                        int M, const double eps[4], double *loglik, double *total, void *stream);
+
 /* The SCALAR drop-in env (gym.make('RandomCartPole-v0'): RandomCartPoleEnv.step / reset, random_cartpole.py:172-229,
  * one env, one host call per step) served by a resident one-warp kernel instead of one launch + synchronise per call.
  * `ctrl` is PINNED, DEVICE-MAPPED HOST memory (zero-initialised once): the host rings a request in by writing

@@ -13,6 +13,11 @@ and the batched variant of the same calls::
     venv = random_envs.RandomCartPoleVecEnv(1 << 20)        # torch CUDA tensors in / out
     obs = venv.reset(); obs, reward, done, info = venv.step(actions)
 
+and offline DR fitting on recorded transitions::
+
+    data = random_envs.TransitionDataset(obs, actions, next_obs, episode_starts=starts)
+    ll = data.dr_log_likelihood("truncnorm", candidates, num_samples=1024)     # one log-likelihood per candidate
+
 All compute is in hand-written sm_100a CUDA kernels behind the C ABI of include/renv.h
 (librenv_b200.so, loaded with ctypes).  There is no CPU fallback: without the library or without a
 GPU the compute entry points raise.
@@ -22,6 +27,7 @@ from . import _lib
 from .distributed import allgather_stats, combine_stats, make_sharded_env, shard_range, summarize_stats
 from .episode_log import EpisodeLog
 from .mlp_policy import MLPPolicy
+from .offline_dr import TransitionDataset
 from .random_cartpole import RandomCartPoleEnv
 from .random_env import RandomEnv, TaskSampler
 from .trajectory import Trajectory
@@ -29,7 +35,7 @@ from .vector_env import RandomCartPoleVecEnv
 from .gym_vector import RandomCartPoleGymVectorEnv
 from .xi_tables import HUMANOID_NOMINAL, XI_TABLES
 
-__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "Trajectory", "XI_TABLES",
+__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "Trajectory", "TransitionDataset", "XI_TABLES",
            "HUMANOID_NOMINAL", "shard_range", "combine_stats", "summarize_stats", "allgather_stats",
            "make_sharded_env", "load_library"]
 

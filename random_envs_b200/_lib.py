@@ -64,6 +64,12 @@ class Trajectory(ctypes.Structure):
                 ("capacity", ctypes.c_int32)]
 
 
+class Transitions(ctypes.Structure):
+    """struct renv_transitions (include/renv.h)."""
+    _fields_ = [("obs", ctypes.c_void_p), ("next_obs", ctypes.c_void_p), ("action", ctypes.c_void_p),
+                ("window", ctypes.c_void_p), ("T", ctypes.c_int64), ("W", ctypes.c_int32)]
+
+
 _vp, _i64, _u64, _u32, _int, _dbl = (ctypes.c_void_p, ctypes.c_int64, ctypes.c_uint64, ctypes.c_uint32,
                                      ctypes.c_int, ctypes.c_double)
 _flt = ctypes.c_float
@@ -71,6 +77,7 @@ _cfg_p, _env_p, _noise_p = ctypes.POINTER(DrCfg), ctypes.POINTER(CartpoleEnv), c
 _log_p = ctypes.POINTER(EpisodeLog)
 _mlp_p = ctypes.POINTER(MlpPolicy)
 _traj_p = ctypes.POINTER(Trajectory)
+_trans_p = ctypes.POINTER(Transitions)
 
 # name -> (restype, argtypes); must list every function declared in include/renv.h
 SIGNATURES = {
@@ -103,6 +110,8 @@ SIGNATURES = {
     "renv_cartpole_collect_mlp_logged_f32": (_int, [_env_p, _log_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64, _cfg_p,
                                                     _vp, _vp, _vp]),
     "renv_cartpole_gae_mlp_f32": (_int, [_env_p, _mlp_p, _traj_p, _int, _flt, _flt, _vp, _vp, _vp, _vp]),
+    "renv_cartpole_transition_loglik_f64": (_int, [_trans_p, _int, _int, _vp, _int, _int, ctypes.POINTER(_dbl), _vp, _vp,
+                                                   _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),
     "renv_random_actions_u8": (_int, [_vp, _i64, _u64, _u64, _u32, _vp]),
     "renv_pack_flags_u8": (_int, [_vp, _vp, _i64, _vp]),

@@ -15,7 +15,7 @@ CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_PATH = os.path.join(_HERE, "librenv_b200.so")
 SOURCES = ["renv_abi.cu"]
-HEADERS = ["renv_philox.cuh", "renv_dr.cuh", "renv_cartpole.cuh", "renv_kernels.cuh", "renv_rollout_pair.cuh", "renv_pack.cuh", "renv_fullgauss_tc.cuh", "renv_scalar_server.cuh", "renv_step_body.cuh", "renv_rollout_body.cuh", "renv_mlp_policy.cuh", "renv_mlp_rollout_body.cuh", "renv_mlp_gae.cuh"]
+HEADERS = ["renv_philox.cuh", "renv_dr.cuh", "renv_cartpole.cuh", "renv_kernels.cuh", "renv_rollout_pair.cuh", "renv_pack.cuh", "renv_fullgauss_tc.cuh", "renv_scalar_server.cuh", "renv_step_body.cuh", "renv_rollout_body.cuh", "renv_mlp_policy.cuh", "renv_mlp_rollout_body.cuh", "renv_mlp_gae.cuh", "renv_transition_loglik.cuh"]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17",

@@ -7,6 +7,7 @@
 #include "renv_fullgauss_tc.cuh"
 #include "renv_mlp_policy.cuh"
 #include "renv_mlp_gae.cuh"
+#include "renv_transition_loglik.cuh"
 #include "renv_scalar_server.cuh"
 #include <stdlib.h>
 #include <type_traits>
@@ -568,6 +569,39 @@ int gae_mlp(const renv_cartpole_env *env, const renv_mlp_policy *critic, const r
     return launch_status();
 }
 
+int check_transition_loglik(const renv_transitions *data, int lam, int integrator, const double *xi, int C, int M,
+                            const double *eps, double *loglik, double *total, LoglikArgs *a, unsigned *blocks)
+{
+    if (data == nullptr || data->obs == nullptr || data->next_obs == nullptr || data->action == nullptr ||
+        data->window == nullptr || xi == nullptr || eps == nullptr || loglik == nullptr || total == nullptr)
+        return RENV_E_NULL;
+    if (!aligned(data->obs, 16) || !aligned(data->next_obs, 16) || !aligned(data->window, 4) || !aligned(xi, 16) ||
+        !aligned(loglik, 8) || !aligned(total, 8))
+        return RENV_E_ALIGN;
+    if (data->T < 1 || data->W < 1 || C < 1 || M < 2 || lam < 1 || lam > data->T) return RENV_E_SIZE;
+    if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
+    for (int k = 0; k < 4; ++k)
+        if (!(eps[k] >= 0.0) || !std::isfinite(eps[k])) return RENV_E_ARG;
+    *a = LoglikArgs{ data->obs, data->next_obs, data->action, data->window, xi, loglik, data->T, data->W, C, M, lam,
+                     (data->W + kLlWindowsPerCta - 1) / kLlWindowsPerCta, { eps[0], eps[1], eps[2], eps[3] } };
+    return grid_for((int64_t)C * a->tiles, 1, blocks);
+}
+
+int transition_loglik(const renv_transitions *data, int lam, int integrator, const double *xi, int C, int M,
+                      const double *eps, double *loglik, double *total, void *stream)
+{
+    LoglikArgs a;
+    unsigned blocks = 0;
+    const int rc = check_transition_loglik(data, lam, integrator, xi, C, M, eps, loglik, total, &a, &blocks);
+    if (rc) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_flag(integrator == RENV_EULER, [&](auto euler) {
+        cartpole_transition_loglik_kernel<euler><<<blocks, kLlThreads, 0, st>>>(a);
+    });
+    loglik_total_kernel<<<C, kLlSumThreads, 0, st>>>(loglik, data->W, total);
+    return launch_status();
+}
+
 }  // namespace
 
 extern "C" {
@@ -762,6 +796,12 @@ int renv_cartpole_gae_mlp_f32(const renv_cartpole_env *env, const renv_mlp_polic
                               void *stream)
 {
     return gae_mlp(env, critic, traj, K, gamma, lambda, values, advantages, returns, stream);
+}
+
+int renv_cartpole_transition_loglik_f64(const renv_transitions *data, int lam, int integrator, const double *xi, int C,
+                                        int M, const double eps[4], double *loglik, double *total, void *stream)
+{
+    return transition_loglik(data, lam, integrator, xi, C, M, eps, loglik, total, stream);
 }
 
 int renv_cartpole_scalar_serve(renv_scalar_ctrl *ctrl, void *save, uint32_t lease_id, uint64_t lease_ns, void *stream)
