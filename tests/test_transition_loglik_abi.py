@@ -191,6 +191,62 @@ def test_oracle_matches_scipy_multivariate_normal():
     assert np.isfinite(ll[0, :2]).all() and np.isnan(ll[0, 2:]).all() and np.isnan(total[0])
 
 
+def _fraction_logpdf(y, pred, eps):
+    """The whole objective in rational arithmetic from the float64 predictions: mu, Sigma, S = Sigma + diag(eps),
+    r' S^-1 r and det S exact (Gaussian elimination); only the final quad form and log det are rounded."""
+    from fractions import Fraction
+    M = len(pred)
+    P = [[Fraction(float(v)) for v in row] for row in pred]
+    mu = [sum(row[i] for row in P) / M for i in range(4)]
+    A = [[sum((row[i] - mu[i]) * (row[j] - mu[j]) for row in P) / (M - 1) + (Fraction(float(eps[i])) if i == j else 0)
+          for j in range(4)] + [Fraction(float(y[i])) - mu[i]] for i in range(4)]
+    r = [A[i][4] for i in range(4)]
+    det = Fraction(1)
+    for k in range(4):
+        det *= A[k][k]
+        for i in range(k + 1, 4):
+            f = A[i][k] / A[k][k]
+            for j in range(k, 5):
+                A[i][j] -= f * A[k][j]
+    z = [Fraction(0)] * 4
+    for i in reversed(range(4)):
+        z[i] = (A[i][4] - sum(A[i][j] * z[j] for j in range(i + 1, 4))) / A[i][i]
+    quad = sum(r[i] * z[i] for i in range(4))
+    return -0.5 * float(quad) - 0.5 * (math.log(det.numerator) - math.log(det.denominator)) - 2.0 * oracle.LOG_2PI
+
+
+def test_exact_oracle_matches_scipy_and_keeps_its_accuracy_far_from_the_origin():
+    stats = pytest.importorskip("scipy.stats")
+    rs = np.random.RandomState(4)
+    obs = rs.uniform(-0.1, 0.1, (20, 4))
+    act = rs.randint(0, 2, 20)
+    nxt = obs + rs.normal(0, 0.01, (20, 4))
+    xi = np.array([5.0, 0.5, 0.05, 0.3]) + np.array([10.0, 1.5, 0.25, 0.7]) * rs.uniform(size=(2, 40, 4))
+    eps = np.array([1e-4, 2e-4, 3e-4, 4e-4])
+    for euler, lam in ((True, 1), (False, 1), (True, 3), (False, 4)):
+        windows = oracle.window_starts(20, lam)[:6]
+        ll, total = oracle.loglik(obs, act, nxt, windows, xi, lam, eps, euler, exact=True)
+        for c in range(2):
+            for w, t in enumerate(windows):
+                pred = oracle.predict(obs, act, int(t), lam, xi[c], euler)
+                ref = stats.multivariate_normal.logpdf(nxt[t + lam - 1], pred.mean(0), np.cov(pred.T) + np.diag(eps))
+                assert abs(ll[c, w] - ref) <= 1e-12 * max(1.0, abs(ref)), (euler, lam, c, w)
+            assert total[c] == math.fsum(ll[c])
+    assert np.all(oracle.loglik(obs, act, nxt, [0, 1], xi, 1, 0.0, True, exact=True)[0] == -np.inf)
+
+    # x = 1e6 with a spread of ~1e-4 (x does not enter the dynamics; the spread comes from x_dot): the exact moments
+    # keep l within 1e-13 of the rational value, np.cov's float64 moments do not
+    xi = np.array([12.0, 1.5, 0.2, 0.7]) * (1.0 + 0.05 * rs.uniform(-1.0, 1.0, (300, 4)))
+    start = np.array([[1e6 + 0.01, 0.05, 0.02, -0.1]] * 2)
+    pred = oracle.predict(start, [1, 0], 0, 2, xi, False)
+    y = pred.mean(0) + pred.std(0) * np.array([0.5, -0.3, 0.8, 0.1])
+    eps = np.full(4, 1e-8)
+    ref = _fraction_logpdf(y, pred, eps)
+    assert 10.0 < ref < 50.0
+    assert abs(oracle.gauss_logpdf_exact(y, pred, eps) - ref) <= 1e-13 * abs(ref)
+    assert abs(oracle.gauss_logpdf(y, pred, eps) - ref) > 1e-10 * abs(ref)
+
+
 @pytest.mark.reference
 @pytest.mark.skipif(not rl.available(), reason=rl.UNAVAILABLE)
 def test_oracle_predictions_against_the_live_reference():
