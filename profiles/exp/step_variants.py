@@ -1,6 +1,6 @@
 """A/B timing of the fp32 auto-reset step kernel: grid- vs tile-granular step ordering; 62 B vs lean 54 B.
 
-    python profiles/exp/step_variants.py [--lib path/to/variant.so] [--tag name]
+    python profiles/exp/step_variants.py [--tag name]
 
 Prints one JSON object per (kernel, mode).  Modes: `chain` = one CUDA graph of K launches on ONE stream over 4 rotating
 2^20-env batches (what a plain step() loop does, minus the Python launch path); `branches` = the same with the 4
@@ -15,25 +15,18 @@ import sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 
 ap = argparse.ArgumentParser()
-ap.add_argument("--lib", default=None)
 ap.add_argument("--tag", default="default")
 ap.add_argument("--K", type=int, default=400)
 ap.add_argument("--reps", type=int, default=5)
 ap.add_argument("--batches", type=int, default=4)
 ap.add_argument("--modes", default="chain,branches,eager,lone,big")
 ap.add_argument("--kernels", default="grid,tile,grid_lean,tile_lean")
-ap.add_argument("--tile-envs", type=int, default=0, help="envs per step CTA of the variant library (RENV_STEP_THREADS * 4)")
 args = ap.parse_args()
-if args.lib:
-    os.environ["RENV_B200_LIB"] = os.path.abspath(args.lib)
 
 import torch  # noqa: E402
 
 import random_envs_b200 as renv  # noqa: E402
 from random_envs_b200 import _device, _lib  # noqa: E402
-
-if args.tile_envs:
-    _lib.TILE_ENVS["float32"] = args.tile_envs      # sizes the `progress` array of the tile-ordered step
 
 SEARCH = [2.0, 20.0, 0.5, 3.0, 0.05, 0.3, 0.1, 1.0]
 dev = torch.device("cuda", 0)

@@ -1,6 +1,6 @@
-"""A/B timing of the fused-rollout kernels: RENV_B200_LIB=build/variants/librenv_<name>.so python profiles/exp/time_rollout.py
+"""Timing of the fused-rollout kernels of the built library: python profiles/exp/time_rollout.py
 Prints env-steps/s for the three bench policies (survive, reset-heavy, random) plus a fingerprint of the final device
-state, so that variants can be checked against each other (the trajectories must be bit-identical)."""
+state, so that two builds can be checked against each other (the trajectories must be bit-identical)."""
 import argparse
 import json
 import os
@@ -57,7 +57,7 @@ def main():
     ap.add_argument("--only", default="")
     a = ap.parse_args()
     n = 1 << a.log2n
-    out = {"lib": os.environ.get("RENV_B200_LIB", "default"), "n": n, "K": a.K}
+    out = {"n": n, "K": a.K}
     for name, w in (("survive", [0.1, 0.1, 1.0, 0.3]), ("resetheavy", [0.0, 0.0, 1.0, 0.0]), ("random", None)):
         if a.only and name not in a.only.split(","):
             continue

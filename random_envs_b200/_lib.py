@@ -7,7 +7,7 @@ import ctypes
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("RENV_B200_LIB", os.path.join(_HERE, "librenv_b200.so"))   # override: kernel experiments
+LIB_PATH = os.path.join(_HERE, "librenv_b200.so")
 
 ABI_VERSION = 6
 MAX_DIM = 32

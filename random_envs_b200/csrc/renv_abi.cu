@@ -161,9 +161,6 @@ template <typename F> void with_mlp_instance(int activation, bool euler, bool lo
     });
 }
 
-#ifndef RENV_STEP_PDL
-#define RENV_STEP_PDL 1
-#endif
 // Launch with programmatic stream serialization: the kernel may start while its predecessor in the stream drains and
 // synchronises itself with griddepcontrol.wait (see cartpole_step_kernel).  Captured into CUDA graphs as a
 // programmatic dependency edge.
@@ -179,7 +176,7 @@ int launch_pdl(void (*kernel)(const Args), unsigned blocks, unsigned threads, cu
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = RENV_STEP_PDL ? 1 : 0;
+    cfg.numAttrs = 1;
     const cudaError_t rc = cudaLaunchKernelEx(&cfg, kernel, args);
     return rc != cudaSuccess ? (int)rc : launch_status();
 }
@@ -220,14 +217,14 @@ bool launch_fullgaussian_tc(float *out, int64_t n, const FullGaussCfg<float> &g,
     const char *knob = getenv("RENV_FULLGAUSS_TENSOR");           // "0": CUDA-core kernel (tests compare the two)
     if (knob && knob[0] == '0') return false;
     unsigned grid = 0;
-    if ((*rc = persistent_grid(n, kFgTile, RENV_FG_TC_CTAS, &grid))) return true;
+    if ((*rc = persistent_grid(n, kFgTile, kFgCtas, &grid))) return true;
     FullGaussCfg<float> gt = g;
     for (int k = 0; k < 32; ++k) {      // the kernel's epilogue takes the WIDTH hi - lo (rounded once, as denormalize does) and mean / 4 (exact)
         gt.hi[k] = g.hi[k] - g.lo[k];
         gt.mean[k] = 0.25f * g.mean[k];
     }
     const PhiloxKeys ks = philox_keys((uint32_t)seed, (uint32_t)(seed >> 32));
-    dr_sample_fullgaussian_tc_kernel<<<grid, kFgThreads, kFgPadSmem, st>>>(out, n, gt, ks, sample_id0, call, counters);
+    dr_sample_fullgaussian_tc_kernel<<<grid, kFgThreads, 0, st>>>(out, n, gt, ks, sample_id0, call, counters);
     *rc = launch_status();
     return true;
 }
@@ -317,6 +314,11 @@ int cartpole_reset(const renv_cartpole_env *env, const renv_obs_noise *noise, co
     cartpole_reset_kernel<T><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
     return launch_status();
 }
+
+// A step CTA covers one tile of envs, the granule of renv_cartpole_env.progress: callers size that array from the
+// header's tile sizes, so the kernels must use the same ones.
+static_assert(kStepThreads * VecTraits<float>::V == RENV_TILE_ENVS_F32, "fp32 step tile differs from include/renv.h");
+static_assert(kStepThreads * VecTraits<double>::V == RENV_TILE_ENVS_F64, "fp64 step tile differs from include/renv.h");
 
 template <typename T, bool kLean>
 int cartpole_step(const renv_cartpole_env *env, const renv_obs_noise *noise, const uint8_t *action, T *reward,
@@ -463,7 +465,7 @@ int policy_mlp(const renv_cartpole_env *env, const renv_mlp_policy *p, bool with
     a.env_id0 = env->env_id0; a.seed = env->seed; a.tick = tick;
     a.sample = sample;
     unsigned grid = 0;
-    if ((rc = persistent_grid(env->n, kMlpThreads, with_logp ? RENV_MLP_ROLLOUT_CTAS : RENV_MLP_CTAS, &grid))) return rc;
+    if ((rc = persistent_grid(env->n, kMlpThreads, with_logp ? kMlpRolloutCtas : kMlpCtas, &grid))) return rc;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     with_activation(p->activation, [&](auto act) {
         if (with_logp) cartpole_policy_logp_mlp_kernel<act><<<grid, kMlpThreads, 0, st>>>(a);

@@ -8,7 +8,7 @@
 // sample; a 256-thread variant in which threads t and t + 128 share TMEM lane t and split the k / d range in halves
 // was measured slower: 1.17 vs 1.03 ms for 2^24 x 30 -- the work per sample is the same and the barriers double):
 //
-//   1. the thread(s) of sample t draw its 32 normals (the SAME Philox blocks and Box-Muller as the CUDA-core
+//   1. the thread of sample t draws its 32 normals (the SAME Philox blocks and Box-Muller as the CUDA-core
 //      kernel: draw_block(seed, id, call, kTasks, j), j = 0..7) and write them -- split into a TF32 head and a TF32
 //      tail, z = z_hi + z_lo -- straight from registers into TENSOR MEMORY with tcgen05.st: row t of the A operand
 //      is TMEM lane t, element k is column k.  Z never touches shared or global memory.
@@ -21,7 +21,9 @@
 //      contiguous span.  The accumulator is double-buffered: the epilogue of tile i-1 runs while the tensor core
 //      works on tile i, and the wait for tile i's MMAs sits after the NEXT tile's normals have been drawn.
 //
-// TMEM per CTA: 32 (Z_hi) + 32 (Z_lo) + 2 x 32 (D) = 128 columns: 4 CTAs per SM share the 512 columns.
+// TMEM per CTA: 32 (Z_hi) + 32 (Z_lo) + 2 x 32 (D) = 128 columns: 4 CTAs per SM share the 512 columns.  (One
+// accumulator, 64 + 32 columns and 5 CTAs per SM, measured 0.928 vs 0.939 ms for 2^24 x 30, +1 %: occupancy is not what
+// holds the kernel back.)
 // Tolerance against the fp32 FMA-chain kernel (same draws): <= 4e-6 of the search-bound width (tests/test_gpu_fullgaussian.py).
 #pragma once
 #include "renv_kernels.cuh"
@@ -29,31 +31,10 @@
 namespace renv {
 
 constexpr int kFgTile = 128;            // samples per tile = MMA M = TMEM lanes
-#ifndef RENV_FG_TC_THREADS
-#define RENV_FG_TC_THREADS 128
-#endif
-constexpr int kFgThreads = RENV_FG_TC_THREADS;      // 128: one thread per sample; 256: two (k / d halves), see below
-constexpr int kFgSplit = kFgThreads / 128;          // threads per sample
-constexpr int kFgPer = 32 / kFgSplit;               // normals / outputs per thread
-static_assert(kFgThreads == 128 || kFgThreads == 256, "one or two threads per sample");
+constexpr int kFgThreads = 128;         // one thread per sample
+constexpr int kFgCtas = 4;              // resident CTAs per SM: 4 x 128 TMEM columns
 constexpr int kFgTmemCols = 128;        // Z_hi 32 + Z_lo 32 + two accumulators of 32
 constexpr uint32_t kFgColZhi = 0, kFgColZlo = 32, kFgColD = 64;
-#ifndef RENV_FG_EXP_PASSES
-#define RENV_FG_EXP_PASSES 3        // experiment knobs (profiles/exp): 1 = head x head only; NOGEN = no Philox / Box-Muller
-#endif
-#ifndef RENV_FG_EXP_NOGEN
-#define RENV_FG_EXP_NOGEN 0
-#endif
-#ifndef RENV_FG_TC_SINGLE_D
-#define RENV_FG_TC_SINGLE_D 0       // 1: ONE accumulator, TMEM taken as 64 (Z) + 32 (D) columns -> 5 CTAs per SM; measured 0.928 vs
-                                    //    0.939 ms for 2^24 x 30 (+1 %): occupancy is not what holds the kernel back, left off
-#endif
-#ifndef RENV_FG_TC_CTAS
-#define RENV_FG_TC_CTAS (RENV_FG_TC_SINGLE_D ? 5 : 4)
-#endif
-// SINGLE_D: with two allocations per CTA a sixth resident CTA could take 64 columns and then wait for ever-busy 32;
-// the launcher pads the dynamic shared memory so that exactly five CTAs fit an SM.
-constexpr int kFgPadSmem = RENV_FG_TC_SINGLE_D ? 14848 : 0;
 
 struct __align__(128) FgTcSmem {
     float b_hi[32 * 32];                // F as the B operand, K-major core-matrix layout (see fg_b_index)
@@ -61,7 +42,6 @@ struct __align__(128) FgTcSmem {
     float stage[kFgTile * 32];          // per lane quadrant: 32 rows of `dim` values, contiguous
     unsigned long long mbar;
     uint32_t tmem_base;
-    uint32_t tmem_base_d;               // SINGLE_D: the accumulator's own 32-column allocation
     uint32_t failed;
 };
 
@@ -109,20 +89,7 @@ __device__ __forceinline__ void fg_tmem_ld32(uint32_t taddr, float *v)
 #pragma unroll
     for (int k = 0; k < 32; ++k) v[k] = __uint_as_float(r[k]);
 }
-__device__ __forceinline__ void fg_tmem_ld16(uint32_t taddr, float *v)
-{
-    uint32_t r[16];
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-                 "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                   "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                 : "r"(taddr) : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int k = 0; k < 16; ++k) v[k] = __uint_as_float(r[k]);
-}
-
-__global__ void __launch_bounds__(kFgThreads, RENV_FG_TC_CTAS)
+__global__ void __launch_bounds__(kFgThreads, kFgCtas)
 dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __grid_constant__ FullGaussCfg<float> cfg,
                                  const __grid_constant__ PhiloxKeys ks, uint64_t sample_id0, uint32_t call,
                                  unsigned long long *counters)
@@ -145,15 +112,8 @@ dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __gri
         sm.failed = 0;
     }
     if (warp == 0) {
-#if RENV_FG_TC_SINGLE_D
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 64;"
-                     :: "r"((uint32_t)__cvta_generic_to_shared(&sm.tmem_base)) : "memory");
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 32;"
-                     :: "r"((uint32_t)__cvta_generic_to_shared(&sm.tmem_base_d)) : "memory");
-#else
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
                      :: "r"((uint32_t)__cvta_generic_to_shared(&sm.tmem_base)), "n"(kFgTmemCols) : "memory");
-#endif
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");           // B was written through the generic proxy
@@ -161,12 +121,8 @@ dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __gri
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = sm.tmem_base;
-#if RENV_FG_TC_SINGLE_D
-    const uint32_t tmem_d = sm.tmem_base_d;                                // one accumulator, its own allocation
-#else
     const uint32_t tmem_d = tmem + kFgColD;                                // two accumulators behind Z
-#endif
-    const int quad = warp & 3, half = warp >> 2;                           // TMEM lane quadrant / which 16 of the 32 k, d
+    const int quad = warp;                                                 // TMEM lane quadrant
     const uint32_t lane_base = tmem + ((uint32_t)(quad * 32) << 16);       // this warp's 32 TMEM lanes
     const uint32_t lane_base_d = tmem_d + ((uint32_t)(quad * 32) << 16);
     const uint64_t desc_hi = fg_smem_desc(sm.b_hi), desc_lo = fg_smem_desc(sm.b_lo);
@@ -182,33 +138,29 @@ dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __gri
     };
     // rows of tile `tile` out of accumulator `buf`: clip, denormalise, and write the quadrant's 32 rows as one span
     auto epilogue = [&](int64_t tile, int buf) {
-        float x[kFgPer];
-        if (kFgSplit == 1) fg_tmem_ld32(lane_base_d + 32 * buf, x);
-        else fg_tmem_ld16(lane_base_d + 32 * buf + 16 * half, x);
+        float x[32];
+        fg_tmem_ld32(lane_base_d + 32 * buf, x);
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         float *rows = sm.stage + quad * 32 * 32;
-        float *row = rows + lane * dim + kFgPer * half;
+        float *row = rows + lane * dim;
 #pragma unroll
-        for (int q = 0; q < kFgPer; ++q) {
-            const int d = kFgPer * half + q;
+        for (int d = 0; d < 32; ++d) {
             // (clip(mean + x, 0, 4) * width) / 4 + lo (random_env.py:194-198, 205-220) in two instructions: scaling by
             // 1/4 is exact and commutes with rounding, so sat(x / 4 + mean / 4) == clip(fl(mean + x), 0, 4) / 4 and
             // fl(q * width) == fl(p * width) / 4 bit for bit; the host passes mean / 4 and width = hi - lo
-            const float q4 = __saturatef(fmaf(x[q], 0.25f, cfg.mean[d]));
-            if (d < dim) row[q] = fmaf(q4, cfg.hi[d], cfg.lo[d]);
+            const float q4 = __saturatef(fmaf(x[d], 0.25f, cfg.mean[d]));
+            if (d < dim) row[d] = fmaf(q4, cfg.hi[d], cfg.lo[d]);
         }
-        if (kFgSplit == 1) __syncwarp();
-        else asm volatile("bar.sync %0, 64;" :: "r"(1 + quad) : "memory");    // both halves of the quadrant have written
+        __syncwarp();
         const int64_t quad_first = tile * kFgTile + quad * 32;
         const int nrows = (int)max((int64_t)0, min((int64_t)32, n - quad_first));
         const int total = nrows * dim;
         float *dst = out + quad_first * dim;                        // 32 * dim * 4 bytes is a multiple of 128
-        const int nvec = total / 4, t0 = half * 32 + lane;
-        for (int q = t0; q < nvec; q += 32 * kFgSplit)
+        const int nvec = total / 4;
+        for (int q = lane; q < nvec; q += 32)
             reinterpret_cast<uint4 *>(dst)[q] = reinterpret_cast<const uint4 *>(rows)[q];
-        for (int q = nvec * 4 + t0; q < total; q += 32 * kFgSplit) dst[q] = rows[q];
-        if (kFgSplit == 1) __syncwarp();
-        else asm volatile("bar.sync %0, 64;" :: "r"(1 + quad) : "memory");    // the stage may be rewritten
+        for (int q = nvec * 4 + lane; q < total; q += 32) dst[q] = rows[q];
+        __syncwarp();                                               // the stage may be rewritten
     };
 
     const int64_t num_tiles = (n + kFgTile - 1) / kFgTile;
@@ -218,18 +170,14 @@ dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __gri
         const int64_t i = tile * kFgTile + quad * 32 + lane;
         const uint64_t id = sample_id0 + (uint64_t)i;
 
-        // ---- 1. this thread's normals (Philox blocks kFgPer/4 * half ...), split into TF32 head and tail
-        float hi[kFgPer], lo[kFgPer];
+        // ---- 1. this thread's normals (Philox blocks 0 .. 7), split into TF32 head and tail
+        float hi[32], lo[32];
 #pragma unroll
-        for (int j = 0; j < kFgPer / 4; ++j) {
+        for (int j = 0; j < 8; ++j) {
             float z[4];
-#if RENV_FG_EXP_NOGEN
-            z[0] = (float)lane; z[1] = (float)j; z[2] = 1.0f; z[3] = (float)(id & 7);
-#else
-            // draw_block(seed, id, call, kTasks, slot) with the round keys as constant-bank operands
-            const uint32_t c1 = (uint32_t)(id >> 32) & 0xffffu, c3 = ((uint32_t)kTasks << 24) | (uint32_t)(kFgPer / 4 * half + j);
+            // draw_block(seed, id, call, kTasks, j) with the round keys as constant-bank operands
+            const uint32_t c1 = (uint32_t)(id >> 32) & 0xffffu, c3 = ((uint32_t)kTasks << 24) | (uint32_t)j;
             Num<float>::normals(philox4x32_10(make_uint4((uint32_t)id, c1, call, c3), ks), z);
-#endif
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 hi[4 * j + q] = __uint_as_float(__float_as_uint(z[q]) & 0xffffe000u);
@@ -238,13 +186,11 @@ dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __gri
         }
         // the previous tile's MMAs must have read Z before it is overwritten (they finished long ago: they ran while
         // the normals above were drawn); its accumulator is then ready for the epilogue further down
-#if !RENV_FG_TC_SINGLE_D
         if (it > 0) wait_mma((uint32_t)(it - 1) & 1u);
-#endif
 #pragma unroll
-        for (int q = 0; q < kFgPer; q += 8) {
-            fg_tmem_st8(lane_base + kFgColZhi + kFgPer * half + q, hi + q);
-            fg_tmem_st8(lane_base + kFgColZlo + kFgPer * half + q, lo + q);
+        for (int q = 0; q < 32; q += 8) {
+            fg_tmem_st8(lane_base + kFgColZhi + q, hi + q);
+            fg_tmem_st8(lane_base + kFgColZlo + q, lo + q);
         }
         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -253,50 +199,32 @@ dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __gri
         // ---- 2. D[it & 1] = Z F^T on the tensor core
         if (tid == 0) {
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint32_t d_col = RENV_FG_TC_SINGLE_D ? tmem_d : tmem_d + 32 * (it & 1);
+            const uint32_t d_col = tmem_d + 32 * (it & 1);
 #pragma unroll
             for (int s = 0; s < 4; ++s) {               // K-step s: columns 8 s .. 8 s + 7 of Z, 256 bytes further into B
                 const uint64_t off = (uint64_t)((256u * s) >> 4);
-#if RENV_FG_EXP_PASSES == 1
-                fg_mma(d_col, tmem + kFgColZhi + 8 * s, desc_hi + off, s > 0);
-#else
                 fg_mma(d_col, tmem + kFgColZlo + 8 * s, desc_hi + off, s > 0);
                 fg_mma(d_col, tmem + kFgColZhi + 8 * s, desc_lo + off, true);
                 fg_mma(d_col, tmem + kFgColZhi + 8 * s, desc_hi + off, true);
-#endif
             }
             asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(mbar) : "memory");
         }
 
-#if RENV_FG_TC_SINGLE_D
-        // ---- 3. wait for this tile's MMAs (the other four CTAs of the SM fill the gap), then its epilogue
-        wait_mma((uint32_t)it & 1u);
-        epilogue(tile, 0);
-#else
         // ---- 3. epilogue of the PREVIOUS tile while the tensor core works on this one
         if (it > 0) epilogue(prev_tile, (it - 1) & 1);
         prev_tile = tile;
-#endif
     }
-#if !RENV_FG_TC_SINGLE_D
     if (it > 0) {
         wait_mma((uint32_t)(it - 1) & 1u);
         epilogue(prev_tile, (it - 1) & 1);
     }
-#endif
 
     // ---- teardown
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (tid == 0 && sm.failed && counters) atomicAdd(counters + kCounterOrderTimeout, 1ull);
-    if (warp == 0) {
-#if RENV_FG_TC_SINGLE_D
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 64;" :: "r"(tmem) : "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 32;" :: "r"(tmem_d) : "memory");
-#else
+    if (warp == 0)
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "n"(kFgTmemCols) : "memory");
-#endif
-    }
 }
 
 }  // namespace renv

@@ -146,12 +146,7 @@ __device__ __forceinline__ void prefetch_l2(const void *p, uint32_t bytes)
 {
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" :: "l"(p), "r"(bytes) : "memory");
 }
-#ifndef RENV_ORDER_SPINS
-#define RENV_ORDER_SPINS (1 << 21)      // x ~40 ns: ~0.1 s, then the CTA proceeds and raises kCounterOrderTimeout
-#endif
-#ifndef RENV_TILE_PREFETCH
-#define RENV_TILE_PREFETCH 1
-#endif
+constexpr int kOrderSpins = 1 << 21;       // x ~40 ns: ~0.1 s, then the CTA proceeds and raises kCounterOrderTimeout
 
 template <typename T> struct StepArgs {
     EnvPtrs<T> env;
@@ -162,13 +157,8 @@ template <typename T> struct StepArgs {
     unsigned long long *counters;   // [kCounterGaussian], [kCounterBadAction]; may be nullptr
 };
 
-#ifndef RENV_STEP_THREADS
-#define RENV_STEP_THREADS 256
-#endif
-constexpr int kStepThreads = RENV_STEP_THREADS;
-#ifndef RENV_STEP_MIN_CTAS
-#define RENV_STEP_MIN_CTAS(T) ((sizeof(T) == 4 ? 4 : 3) * 256 / kStepThreads)
-#endif
+constexpr int kStepThreads = 256;          // x V envs = RENV_TILE_ENVS_F32 / _F64 (include/renv.h; checked in renv_abi.cu)
+template <typename T> constexpr int kStepMinCtas = sizeof(T) == 4 ? 4 : 3;     // resident CTAs per SM (register cap)
 
 // Tiles a CTA may own in one launch (tickets are kept in shared memory); the launcher sizes the grid accordingly.
 // kAutoReset = true is the hot kernel.  Finished envs are NOT reset by the thread that owns them (that would
@@ -211,7 +201,7 @@ constexpr int kStepThreads = RENV_STEP_THREADS;
 // episode that ended -- the xi row before its resample, the state the owner stored, the length and truncated bit the
 // owner staged in s_len -- into the episode log.  All of it precedes the tile's release / the end of the grid.
 template <typename T, bool kAutoReset, bool kNoisy = false, bool kLean = false>
-__global__ void __launch_bounds__(kStepThreads, kNoisy ? (sizeof(T) == 8 ? 2 : 3) : RENV_STEP_MIN_CTAS(T)) cartpole_step_kernel(const __grid_constant__ StepArgs<T> a)
+__global__ void __launch_bounds__(kStepThreads, kNoisy ? (sizeof(T) == 8 ? 2 : 3) : kStepMinCtas<T>) cartpole_step_kernel(const __grid_constant__ StepArgs<T> a)
 {
     constexpr bool kLog = false;
     const LogPtrs<T> log = {};
@@ -222,7 +212,7 @@ template <typename T> struct LoggedStepArgs { StepArgs<T> step; LogPtrs<T> log; 
 
 // The plain auto-reset step plus the episode log (a kernel of its own: the plain one keeps its parameter layout).
 template <typename T>
-__global__ void __launch_bounds__(kStepThreads, RENV_STEP_MIN_CTAS(T)) cartpole_step_logged_kernel(const __grid_constant__ LoggedStepArgs<T> args)
+__global__ void __launch_bounds__(kStepThreads, kStepMinCtas<T>) cartpole_step_logged_kernel(const __grid_constant__ LoggedStepArgs<T> args)
 {
     constexpr bool kAutoReset = true, kNoisy = false, kLean = false, kLog = true;
     const StepArgs<T> &a = args.step;
@@ -355,34 +345,13 @@ template <typename T> struct RolloutThread {
     bool refresh;       // ... and: parked for new action bits only, the episode goes on
 };
 
-#ifndef RENV_RESET_BATCH
-#define RENV_RESET_BATCH 4
-#endif
-#ifndef RENV_STEPS_PER_CHECK
-#define RENV_STEPS_PER_CHECK 8
-#endif
-#ifndef RENV_UNROLL_F64
-#define RENV_UNROLL_F64 2
-#endif
-constexpr int kResetBatch = RENV_RESET_BATCH;          // parked lanes per warp that trigger a reset pass
-constexpr int kStepsPerCheck = RENV_STEPS_PER_CHECK;   // env-steps between two warp votes
-constexpr int kUnrollF64 = RENV_UNROLL_F64;
+constexpr int kResetBatch = 4;             // parked lanes per warp that trigger a reset pass
+constexpr int kStepsPerCheck = 8;          // env-steps between two warp votes
+constexpr int kUnrollF64 = 2;
 // The fp32 random policy ends an episode every ~25 steps: its own vote period / batch size / unroll.  Measured at
 // 2^24 envs x 500 steps (check, batch -> 1e11 env-steps/s): (4,4) 2.48, (8,4) 2.92, (12,4) 3.05, (16,8) 3.11,
 // (16,12) 3.08, (20,12) 3.06, (24,12) 2.95, (32,16) 2.61; unroll 1 / 2 / 4 / 8 at (8,4): 2.79 / 2.92 / 2.81 / 2.75.
-#ifndef RENV_RANDOM_RESET_BATCH
-#define RENV_RANDOM_RESET_BATCH 8
-#endif
-#ifndef RENV_RANDOM_STEPS_PER_CHECK
-#define RENV_RANDOM_STEPS_PER_CHECK 16
-#endif
-#ifndef RENV_RANDOM_UNROLL
-#define RENV_RANDOM_UNROLL RENV_UNROLL_F64
-#endif
-constexpr int kRandomUnroll = RENV_RANDOM_UNROLL;
-#ifndef RENV_ROLLOUT_F64_CTAS
-#define RENV_ROLLOUT_F64_CTAS 3
-#endif
+constexpr int kRandomResetBatch = 8, kRandomStepsPerCheck = 16, kRandomUnroll = 2;
 
 // Bernoulli(1/2) action of env `id` at clock `step` (low 32 bits of the tick): bit (step & 127) of the env's OWN Philox
 // block (id, step >> 7) -- the bit random_actions_kernel writes for that env and tick, so a random-policy rollout equals
@@ -476,10 +445,11 @@ __device__ __forceinline__ void rollout_reset(RolloutThread<T> &t, const Rollout
 __device__ __forceinline__ float pin(float v) { asm volatile("" : "+f"(v)); return v; }
 __device__ __forceinline__ double pin(double v) { asm volatile("" : "+d"(v)); return v; }
 
-#define RENV_ROLLOUT_CTAS(T, kNoisy, kRandom) (sizeof(T) == 4 ? 3 : ((kNoisy) || (kRandom)) ? 2 : RENV_ROLLOUT_F64_CTAS)
+// Resident CTAs per SM (register cap) of the rollout kernels: 3, and 2 for the fp64 noisy / random-policy ones.
+template <typename T> constexpr int rollout_ctas(bool noisy, bool random) { return sizeof(T) == 4 || !(noisy || random) ? 3 : 2; }
 
 template <typename T, bool kEuler, bool kNoisy = false, bool kRandom = false>
-__global__ void __launch_bounds__(kRolloutThreads, RENV_ROLLOUT_CTAS(T, kNoisy, kRandom))
+__global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(kNoisy, kRandom))
 cartpole_rollout_kernel(const __grid_constant__ RolloutArgs<T> a)
 {
     constexpr bool kLog = false;
@@ -491,7 +461,7 @@ template <typename T> struct LoggedRolloutArgs { RolloutArgs<T> roll; LogPtrs<T>
 
 // The plain (not Noisy) rollout plus the episode log: fp64, and fp32 under the random policy.
 template <typename T, bool kEuler, bool kRandom>
-__global__ void __launch_bounds__(kRolloutThreads, RENV_ROLLOUT_CTAS(T, false, kRandom))
+__global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(false, kRandom))
 cartpole_rollout_logged_kernel(const __grid_constant__ LoggedRolloutArgs<T> args)
 {
     constexpr bool kNoisy = false, kLog = true;
@@ -644,13 +614,7 @@ __global__ void __launch_bounds__(kSampleThreads) dr_sample_kernel(T *__restrict
 //   * the transforms run on packed pairs (renv_dr.cuh: FFMA2 / FMUL2, the same rounding lane for lane);
 //   * attempt 0 only answers "did any dim fall below its floor" (4 FSETP); the retry loop of the reference, with
 //     its per-dim bookkeeping, is out of line.
-#ifndef RENV_SAMPLER_ILP
-#define RENV_SAMPLER_ILP 2
-#endif
-constexpr int kSamplerIlp = RENV_SAMPLER_ILP;
-#ifndef RENV_SAMPLER_F32_CTAS
-#define RENV_SAMPLER_F32_CTAS 2      // 90-94 registers: round keys, packed constants and parameters all stay resident
-#endif
+constexpr int kSamplerF32Ctas = 2;     // 90-94 registers: round keys, packed constants and parameters all stay resident
 // The reference's retry loop for one block whose first attempt left some dim below its floor (random_env.py:158-171,
 // 177-190): out of line, so that the per-block loop of the kernel stays Philox + packed transform + store.
 struct RedoneBlock { float v0, v1, v2, v3; unsigned viol; };      // returned in registers: no stack traffic in the loop
@@ -666,7 +630,7 @@ __device__ __noinline__ RedoneBlock sampler_redo_block(const DrCfgPrepared<float
 }
 
 template <int kDrType, int kStore>
-__global__ void __launch_bounds__(kSampleThreads, RENV_SAMPLER_F32_CTAS)
+__global__ void __launch_bounds__(kSampleThreads, kSamplerF32Ctas)
 dr_sample_f32_kernel(float *__restrict__ out, int64_t n, const __grid_constant__ DrCfgPrepared<float> cfg, uint64_t seed,
                      const __grid_constant__ PhiloxKeys ks, uint64_t sample_id0, uint32_t call,
                      unsigned long long *violations, int items)
@@ -708,7 +672,7 @@ dr_sample_f32_kernel(float *__restrict__ out, int64_t n, const __grid_constant__
             store_block<float, kStore>(dst, v, pb.valid);
         };
         int k = seg;
-        if (kSamplerIlp == 2 && kDrType != kDrUniform) {
+        if (kDrType != kDrUniform) {
             // the transcendental laws are LATENCY-bound (ncu: `wait` 31-36 % of stalls at 2 CTAs/SM: one serial Philox +
             // Horner chain per thread): two samples per iteration give the scheduler two independent chains
             // ... and both in ONE basic block (the rare floor check is taken once, after both transforms): with the
@@ -827,15 +791,12 @@ template <typename T> struct FullGaussCfg {
     T mean[32], lo[32], hi[32];
     T ft[32 * 32];               // ft[k * 32 + d] = F[d][k] (F F^T = cov), zero beyond dim: 4 KB fp32 / 8 KB fp64
 };
-#ifndef RENV_FULLGAUSS_CTAS
-#define RENV_FULLGAUSS_CTAS 4
-#endif
-constexpr int kFullGaussThreads = 128;
+constexpr int kFullGaussThreads = 128, kFullGaussCtas = 4;
 
 // D = dim rounded up to {4, 8, 16, 32}: accumulators and unrolled loops are sized for it (a 4-dim cart-pole sample is
 // 16 FMAs, not 1024).
 template <typename T, int D>
-__global__ void __launch_bounds__(kFullGaussThreads, RENV_FULLGAUSS_CTAS)
+__global__ void __launch_bounds__(kFullGaussThreads, kFullGaussCtas)
 dr_sample_fullgaussian_kernel(T *__restrict__ out, int64_t n, const __grid_constant__ FullGaussCfg<T> cfg, uint64_t seed,
                               uint64_t sample_id0, uint32_t call)
 {

@@ -51,7 +51,7 @@ __device__ __forceinline__ State<float> load_row(const float *rows, int64_t r)
 }
 
 template <int kAct>
-__global__ void __launch_bounds__(kMlpThreads, RENV_MLP_ROLLOUT_CTAS)
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_gae_mlp_kernel(const __grid_constant__ MlpGaeArgs a)
 {
     __shared__ MlpSmem sm;

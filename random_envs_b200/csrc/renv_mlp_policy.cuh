@@ -35,16 +35,9 @@ constexpr int kMlpParamFloats = 4612;     // 4610 rounded up to a multiple of 4 
 enum MlpAct : int { kMlpTanh = 0, kMlpRelu = 1 };
 
 constexpr int kMlpThreads = 128;
-#ifndef RENV_MLP_EXP_PASSES
-#define RENV_MLP_EXP_PASSES 3    // experiment knob (DESIGN.md section 4.9): 1 = head x head only, a third of the HMMAs
-#endif
-#ifndef RENV_MLP_CTAS
-#define RENV_MLP_CTAS 4          // policy_actions: 128 registers, 16 warps per SM
-#endif
-#ifndef RENV_MLP_ROLLOUT_CTAS
-#define RENV_MLP_ROLLOUT_CTAS 3  // the rollout keeps its env, task and statistics beside the policy: ~148 registers
-                                 // (at 4 CTAs = 128 registers it spills)
-#endif
+constexpr int kMlpCtas = 4;              // policy_actions: 128 registers, 16 warps per SM
+constexpr int kMlpRolloutCtas = 3;       // the rollout keeps its env, task and statistics beside the policy: ~148 registers
+                                         // (at 4 CTAs = 128 registers it spills)
 
 // The parameters as the fragments want them (filled by mlp_load_params; ~34 KB).
 struct __align__(16) MlpSmem {
@@ -143,10 +136,8 @@ __device__ __forceinline__ void mlp_logits(const MlpSmem &sm, const State<float>
             for (int nt = 0; nt < 8; ++nt) {
                 const float4 b = sm.w2[(j * 8 + nt) * 32 + lane];
                 const uint32_t bh0 = __float_as_uint(b.x), bh1 = __float_as_uint(b.y);
-#if RENV_MLP_EXP_PASSES == 3
                 mma_tf32(acc[nt], alo, bh0, bh1);
                 mma_tf32(acc[nt], ahi, __float_as_uint(b.z), __float_as_uint(b.w));
-#endif
                 mma_tf32(acc[nt], ahi, bh0, bh1);
             }
         }
@@ -226,7 +217,7 @@ struct MlpActionArgs {
 
 // Persistent CTAs (one wave): the parameters are staged once per CTA, not once per 256 envs.
 template <int kAct>
-__global__ void __launch_bounds__(kMlpThreads, RENV_MLP_CTAS)
+__global__ void __launch_bounds__(kMlpThreads, kMlpCtas)
 cartpole_policy_actions_mlp_kernel(const __grid_constant__ MlpActionArgs a)
 {
     __shared__ MlpSmem sm;
@@ -259,7 +250,7 @@ struct MlpLogpArgs {
 
 // 3 CTAs per SM as the rollout: at 4 (128 registers) the Philox block and log1p beside mlp_logits spill 16 bytes (Tanh).
 template <int kAct>
-__global__ void __launch_bounds__(kMlpThreads, RENV_MLP_ROLLOUT_CTAS)
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_policy_logp_mlp_kernel(const __grid_constant__ MlpLogpArgs args)
 {
     __shared__ MlpSmem sm;
@@ -299,7 +290,7 @@ struct MlpRolloutArgs {
 // (seed, global env id, tick) exactly as in cartpole_step_kernel, and the episode bookkeeping is that kernel's, so the
 // launch equals K x {renv_cartpole_policy_actions_mlp_f32; renv_cartpole_step_f32 (auto-reset)} bit for bit.
 template <int kAct, bool kEuler, bool kLog>
-__global__ void __launch_bounds__(kMlpThreads, RENV_MLP_ROLLOUT_CTAS)
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_rollout_mlp_kernel(const __grid_constant__ MlpRolloutArgs args)
 {
     constexpr bool kCollect = false;
@@ -326,7 +317,7 @@ struct MlpCollectArgs {
 // launch equals K x {record obs; renv_cartpole_policy_logp_mlp_f32; renv_cartpole_step_f32 (auto-reset)} bit for bit.
 // Greed / sampling is a runtime argument: one instance per (activation, integrator, log) as for the rollout.
 template <int kAct, bool kEuler, bool kLog>
-__global__ void __launch_bounds__(kMlpThreads, RENV_MLP_ROLLOUT_CTAS)
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_collect_mlp_kernel(const __grid_constant__ MlpCollectArgs args)
 {
     constexpr bool kCollect = true;

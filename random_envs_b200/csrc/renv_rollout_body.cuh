@@ -41,7 +41,7 @@
                 if (t.remaining > 0) rollout_step<T, kEuler, true, kNoisy, kRandom>(t, a, policy, limit, id);
         } else if (kRandom && sizeof(T) == 4) {
 #pragma unroll kRandomUnroll
-            for (int u = 0; u < RENV_RANDOM_STEPS_PER_CHECK; ++u)
+            for (int u = 0; u < kRandomStepsPerCheck; ++u)
                 if (t.remaining > 0) rollout_step<T, kEuler, true, kNoisy, kRandom>(t, a, policy, limit, id);
         } else {            // the fp64 / noisy step is ~10x the code of the fp32 one: keep the loop body inside the i-cache
 #pragma unroll kUnrollF64
@@ -50,7 +50,7 @@
         }
         const unsigned parked = __ballot_sync(0xffffffffu, t.parked >= 0);
         const unsigned running = __ballot_sync(0xffffffffu, t.remaining > 0);
-        if (parked != 0u && (__popc(parked) >= (kRandom && sizeof(T) == 4 ? RENV_RANDOM_RESET_BATCH : kResetBatch) || running == 0u)) {
+        if (parked != 0u && (__popc(parked) >= (kRandom && sizeof(T) == 4 ? kRandomResetBatch : kResetBatch) || running == 0u)) {
             if (t.parked >= 0) {
                 if (kLog && !(kRandom && t.refresh)) {      // t.s / t.p / t.el are still the ended episode's
                     log_episode(log, ld, il, log_count, t.p, t.s, t.el, !beyond_thresholds(t.s) && t.el >= limit,

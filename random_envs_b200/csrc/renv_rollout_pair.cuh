@@ -21,13 +21,9 @@
 
 namespace renv {
 
-#ifndef RENV_PAIR_RESET_BATCH
-#define RENV_PAIR_RESET_BATCH 16
-#endif
-#ifndef RENV_PAIR_CTAS
-#define RENV_PAIR_CTAS 3
-#endif
-constexpr int kPairResetBatch = RENV_PAIR_RESET_BATCH;   // parked slots (of 64) per warp that trigger a reset pass
+constexpr int kPairResetBatch = 16;      // parked slots (of 64) per warp that trigger a reset pass
+constexpr int kPairCtas = 3;             // resident CTAs per SM (register cap)
+constexpr int kPairSlots = 2;            // envs per thread: one packed pair
 constexpr int kInactive = 0x7fffffff;
 
 // Per-slot operands of the packed step, as scalars (the hot loop packs slot 0 / slot 1 into register pairs).
@@ -91,12 +87,6 @@ __device__ __forceinline__ void pair_step(PairSlot &s0, PairSlot &s1, const Pair
     }
     unpk(X, s0.x, s1.x); unpk(XD, s0.xd, s1.xd); unpk(TH, s0.th, s1.th); unpk(THD, s0.thd, s1.thd);
 }
-
-#ifndef RENV_PAIR_GROUPS
-#define RENV_PAIR_GROUPS 1
-#endif
-constexpr int kPairGroups = RENV_PAIR_GROUPS;    // env pairs per thread (independent packed chains: ILP)
-constexpr int kPairSlots = 2 * kPairGroups;
 
 // kLog: on_event stores an ended episode's terminal state and length like a finished env's (one more use of a store
 // the hot loop already has), and reset_slot -- in the warp's reset pass, outside the loop -- reads them back with the
@@ -203,8 +193,7 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
     for (;;) {
 #pragma unroll
         for (int u = 0; u < kStepsPerCheck; ++u) {
-#pragma unroll
-            for (int g = 0; g < kPairGroups; ++g) pair_step<kEuler>(q[2 * g], q[2 * g + 1], kc);
+            pair_step<kEuler>(q[0], q[1], kc);
             c += 1;
             bool term[S], any = false;
 #pragma unroll
@@ -227,7 +216,7 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
             parked = parked || q[k].parked >= 0;
         }
         const unsigned running = __ballot_sync(0xffffffffu, active);
-        if (nparked != 0 && (nparked >= kPairResetBatch * kPairGroups || running == 0u)) {
+        if (nparked != 0 && (nparked >= kPairResetBatch || running == 0u)) {
             if (parked) {
 #pragma unroll
                 for (int k = 0; k < S; ++k)
@@ -246,14 +235,14 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
 }
 
 template <bool kEuler>
-__global__ void __launch_bounds__(kRolloutThreads, RENV_PAIR_CTAS)
+__global__ void __launch_bounds__(kRolloutThreads, kPairCtas)
 cartpole_rollout_pair_kernel(const __grid_constant__ RolloutArgs<float> a)
 {
     rollout_pair_body<kEuler, false>(a, LogPtrs<float>{});
 }
 
 template <bool kEuler>
-__global__ void __launch_bounds__(kRolloutThreads, RENV_PAIR_CTAS)
+__global__ void __launch_bounds__(kRolloutThreads, kPairCtas)
 cartpole_rollout_pair_logged_kernel(const __grid_constant__ LoggedRolloutArgs<float> a)
 {
     rollout_pair_body<kEuler, true>(a.roll, a.log);

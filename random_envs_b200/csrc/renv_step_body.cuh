@@ -24,13 +24,13 @@
             uint32_t *const slot = a.env.progress + 2 * (size_t)blockIdx.x;
             ticket = atomicAdd(slot, 1u);
             uint32_t seen = ld_acquire_gpu(slot + 1);
-            for (int spin = 0; seen != ticket && spin < RENV_ORDER_SPINS; ++spin) {     // rare: the predecessor is still on this tile
+            for (int spin = 0; seen != ticket && spin < kOrderSpins; ++spin) {     // rare: the predecessor is still on this tile
                 __nanosleep(32);
                 seen = ld_acquire_gpu(slot + 1);
             }
             if (seen != ticket && a.counters) atomicAdd(a.counters + kCounterOrderTimeout, 1ull);
             if (kAutoReset) s_count = 0;
-        } else if (RENV_TILE_PREFETCH && block0 + kTile <= n && threadIdx.x >= 32 && threadIdx.x < 39) {
+        } else if (block0 + kTile <= n && threadIdx.x >= 32 && threadIdx.x < 39) {
             // while thread 0 waits for its L2 round trip the tile is pulled from HBM into L2 (never stale: L2 is the
             // point of coherence), so the loads below pay an L2 hit instead of a second DRAM latency
             const int q = threadIdx.x - 32;

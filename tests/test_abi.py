@@ -38,6 +38,8 @@ def test_header_constants_match_binding():
     text = open(HEADER).read()
     assert int(re.search(r"#define RENV_MAX_DIM (\d+)", text).group(1)) == _lib.MAX_DIM
     assert int(re.search(r"#define RENV_NUM_STATS (\d+)", text).group(1)) == _lib.NUM_STATS
+    assert int(re.search(r"#define RENV_TILE_ENVS_F32 (\d+)", text).group(1)) == _lib.TILE_ENVS["float32"]
+    assert int(re.search(r"#define RENV_TILE_ENVS_F64 (\d+)", text).group(1)) == _lib.TILE_ENVS["float64"]
     assert ctypes.sizeof(_lib.DrCfg) == 8 + 3 * 8 * _lib.MAX_DIM + 8 * _lib.MAX_DIM ** 2
     assert ctypes.sizeof(_lib.CartpoleEnv) == 7 * 8 + 4 * 8
 
