@@ -341,6 +341,40 @@ int renv_cartpole_gae_mlp_f32(const renv_cartpole_env *env, const renv_mlp_polic
                               int K, float gamma, float lambda, float *values, float *advantages, float *returns,
                               void *stream);
 
+/* Population evaluation: P policies, each on the env's E = n envs from a fresh start, with per-member statistics --
+ * ES / ARS / CEM over policy weights, population-based training, or the best of several checkpoints under a DR
+ * distribution, with common random numbers: member p and member q see the same tasks and initial states.
+ * For member p and env j (0 <= j < E), Philox id env_id0 + j for every member:
+ *   1. a fresh episode at tick `tick`, exactly as renv_cartpole_reset_f32 (mask NULL) starts one: the initial state
+ *      init_state(seed, id, tick); with an active DR config xi is drawn as that reset draws it, otherwise xi is row j of
+ *      env->xi;
+ *   2. K env-steps at ticks tick + 1 .. tick + K under policy p, with auto-reset, the TimeLimit `max_steps` and the DR
+ *      resample on reset, exactly as renv_cartpole_rollout_f32 runs them;
+ *   3. the member's finished episodes are ACCUMULATED into stats[p * RENV_NUM_STATS ..] (the rollout's 6 statistics;
+ *      the caller initialises each row to {0, 0, 0, +inf, -inf, 0}).
+ * Hence stats row p equals, bit for bit, the stats of renv_cartpole_reset_f32 at `tick` followed by
+ * renv_cartpole_rollout_f32(policy p, K) at tick + 1 on an env with the same n, seed, env_id0, xi table and DR config:
+ * the six values are exact in doubles (integer sums, min, max).  A row depends only on its policy and that
+ * configuration, not on P, the member's position or the launch; shards of E with env_id0 offsets combine per member as
+ * the rollout's statistics do.  Nothing is written into the env (only env->n, env_id0, seed and, without an active DR
+ * config, xi are read); gaussian DR failures are counted into `violations` (may be NULL) as everywhere else.
+ * Errors, all before any CUDA call: NULL env / policies / params / stats, or NULL xi when it is read, RENV_E_NULL;
+ * P < 1, n <= 0, K outside [1, 2^30] or P * n >= 2^31 RENV_E_SIZE; a misaligned pointer RENV_E_ALIGN (stats 8 bytes,
+ * xi 16); an unknown integrator RENV_E_INTEGRATOR; an unknown DR config RENV_E_DRTYPE / RENV_E_DIM.
+ *
+ * Linear policies: `policies` is P rows of 5 floats w0, w1, w2, w3, b (device, 4-byte aligned); the action is
+ * [fma(w3, theta_dot, fma(w2, theta, fma(w1, x_dot, fma(w0, x, b)))) > 0] in fp32 -- the action
+ * renv_cartpole_rollout_f32 takes for double w, b that round to these floats. */
+int renv_cartpole_population_linear_f32(const renv_cartpole_env *env, const float *policies, int P, int K,
+                                        int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                        double *stats, unsigned long long *violations, void *stream);
+/* MLP policies: `params` is P rows of RENV_MLP_PARAM_FLOATS floats in the layout of renv_mlp_policy (device; 18,448
+ * bytes a row, so every row is 16-byte aligned when the base is), with one `activation` for the whole population
+ * (unknown: RENV_E_ARG).  The action is renv_cartpole_rollout_mlp_f32's. */
+int renv_cartpole_population_mlp_f32(const renv_cartpole_env *env, const void *params, int activation, int P, int K,
+                                     int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                     double *stats, unsigned long long *violations, void *stream);
+
 /* Recorded cart-pole transitions for offline DR fitting (device pointers): transition i is (obs[i], action[i],
  * next_obs[i]), and `window` lists the W start indices t that are scored (t + lam <= T; windows crossing an episode
  * boundary are the caller's to leave out). */

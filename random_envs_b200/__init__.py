@@ -26,7 +26,7 @@ from . import gym_compat as gym
 from . import _lib
 from .distributed import allgather_stats, combine_stats, make_sharded_env, shard_range, summarize_stats
 from .episode_log import EpisodeLog
-from .mlp_policy import MLPPolicy
+from .mlp_policy import MLPPolicy, MLPPopulation
 from .offline_dr import TransitionDataset
 from .random_cartpole import RandomCartPoleEnv
 from .random_env import RandomEnv, TaskSampler
@@ -35,7 +35,7 @@ from .vector_env import RandomCartPoleVecEnv
 from .gym_vector import RandomCartPoleGymVectorEnv
 from .xi_tables import HUMANOID_NOMINAL, XI_TABLES
 
-__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "Trajectory", "TransitionDataset", "XI_TABLES",
+__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "MLPPopulation", "Trajectory", "TransitionDataset", "XI_TABLES",
            "HUMANOID_NOMINAL", "shard_range", "combine_stats", "summarize_stats", "allgather_stats",
            "make_sharded_env", "load_library"]
 

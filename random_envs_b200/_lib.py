@@ -110,6 +110,8 @@ SIGNATURES = {
     "renv_cartpole_collect_mlp_logged_f32": (_int, [_env_p, _log_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64, _cfg_p,
                                                     _vp, _vp, _vp]),
     "renv_cartpole_gae_mlp_f32": (_int, [_env_p, _mlp_p, _traj_p, _int, _flt, _flt, _vp, _vp, _vp, _vp]),
+    "renv_cartpole_population_linear_f32": (_int, [_env_p, _vp, _int, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
+    "renv_cartpole_population_mlp_f32": (_int, [_env_p, _vp, _int, _int, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
     "renv_cartpole_transition_loglik_f64": (_int, [_trans_p, _int, _int, _vp, _int, _int, ctypes.POINTER(_dbl), _vp, _vp,
                                                    _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),

@@ -571,6 +571,68 @@ int gae_mlp(const renv_cartpole_env *env, const renv_mlp_policy *critic, const r
     return launch_status();
 }
 
+// The checks and arguments both population entry points share, all before any CUDA call.  Only env->n, env_id0, seed
+// and, without an active DR config, xi are read.  `rows` holds the P policy rows, aligned to `row_align` bytes.  The
+// kernels start every episode at `tick` and step at tick + 1 .. tick + K (a->tick = tick + 1).
+int prepare_population(const renv_cartpole_env *env, const void *rows, size_t row_align, int P, int K, int integrator,
+                       int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
+                       unsigned long long *violations, RolloutArgs<float> *a, PopulationPtrs *pop)
+{
+    if (env == nullptr || rows == nullptr || stats == nullptr) return RENV_E_NULL;
+    // P n < 2^31: the flat (member, env) index and the MLP grid fit in 31 bits
+    if (P < 1 || env->n <= 0 || env->n >= (1LL << 31) || (int64_t)P * env->n >= (1LL << 31)) return RENV_E_SIZE;
+    const Policy<float> unused{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
+    const int rc = check_rollout<float>(stats, K, integrator, max_steps, tick + 1, dr, violations, unused, a);
+    if (rc) return rc;
+    const bool table = a->dr.dr_type == kDrNone;        // xi is row j of the env's table, else drawn at the fresh start
+    if (table && env->xi == nullptr) return RENV_E_NULL;
+    if ((table && !aligned(env->xi, 16)) || !aligned(rows, row_align)) return RENV_E_ALIGN;
+    a->env = EnvPtrs<float>{};
+    a->env.xi = table ? static_cast<float *>(env->xi) : nullptr;
+    a->env.n = env->n;
+    a->env.env_id0 = env->env_id0;
+    a->env.seed = env->seed;
+    *pop = PopulationPtrs{ static_cast<const float *>(rows), (int64_t)P * env->n,
+                           (uint32_t)((env->n + kMlpThreads - 1) / kMlpThreads) };
+    return RENV_OK;
+}
+
+int population_linear(const renv_cartpole_env *env, const float *policies, int P, int K, int integrator, int max_steps,
+                      uint64_t tick, const renv_dr_cfg *dr, double *stats, unsigned long long *violations, void *stream)
+{
+    PopulationArgs pa;
+    int rc = prepare_population(env, policies, 4, P, K, integrator, max_steps, tick, dr, stats, violations, &pa.roll, &pa.pop);
+    if (rc) return rc;
+    unsigned blocks = 0;
+    if ((rc = grid_for(pa.pop.total, kRolloutThreads, &blocks))) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_flag(pa.roll.euler, [&](auto euler) {
+        cartpole_population_linear_kernel<euler><<<blocks, kRolloutThreads, 0, st>>>(pa);
+    });
+    return launch_status();
+}
+
+int population_mlp(const renv_cartpole_env *env, const void *params, int activation, int P, int K, int integrator,
+                   int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats, unsigned long long *violations,
+                   void *stream)
+{
+    MlpPopulationArgs pa;
+    const int rc = prepare_population(env, params, 16, P, K, integrator, max_steps, tick, dr, stats, violations,
+                                      &pa.mlp.roll, &pa.pop);
+    if (rc) return rc;
+    if (activation != RENV_MLP_TANH && activation != RENV_MLP_RELU) return RENV_E_ARG;
+    pa.mlp.params = nullptr;
+    pa.mlp.log = LogPtrs<float>{};
+    const unsigned blocks = (unsigned)P * pa.pop.ctas;      // <= P n < 2^31
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_activation(activation, [&](auto act) {
+        with_flag(pa.mlp.roll.euler, [&](auto euler) {
+            cartpole_population_mlp_kernel<act, euler><<<blocks, kMlpThreads, 0, st>>>(pa);
+        });
+    });
+    return launch_status();
+}
+
 int check_transition_loglik(const renv_transitions *data, int lam, int integrator, const double *xi, int C, int M,
                             const double *eps, double *loglik, double *total, LoglikArgs *a, unsigned *blocks)
 {
@@ -798,6 +860,19 @@ int renv_cartpole_gae_mlp_f32(const renv_cartpole_env *env, const renv_mlp_polic
                               void *stream)
 {
     return gae_mlp(env, critic, traj, K, gamma, lambda, values, advantages, returns, stream);
+}
+
+int renv_cartpole_population_linear_f32(const renv_cartpole_env *env, const float *policies, int P, int K,
+                                        int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                        double *stats, unsigned long long *violations, void *stream)
+{
+    return population_linear(env, policies, P, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+int renv_cartpole_population_mlp_f32(const renv_cartpole_env *env, const void *params, int activation, int P, int K,
+                                     int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
+                                     double *stats, unsigned long long *violations, void *stream)
+{
+    return population_mlp(env, params, activation, P, K, integrator, max_steps, tick, dr, stats, violations, stream);
 }
 
 int renv_cartpole_transition_loglik_f64(const renv_transitions *data, int lam, int integrator, const double *xi, int C,

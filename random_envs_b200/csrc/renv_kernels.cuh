@@ -314,6 +314,41 @@ __device__ __forceinline__ void rollout_publish(double *stats, unsigned long lon
     }
 }
 
+// Statistics of a population launch (cartpole_population_linear_kernel), whose warps may serve two or more members:
+// a warp whose lanes all serve one member reduces by shuffles and lane 0 publishes into the member's row; in a warp
+// that straddles members every lane with a finished episode publishes into its own member's row.  The six values are
+// exact in doubles (integer sums below 2^53, min, max), so the order of the atomics does not change the bits.
+__device__ __forceinline__ void population_publish(double *stats, int64_t member, unsigned long long *violations,
+                                                   unsigned episodes, unsigned sum_len, unsigned sum_r_u,
+                                                   unsigned long long sum_r2_u, float min_r, float max_r, unsigned viol)
+{
+    double sum_r = (double)sum_r_u, sum_r2 = (double)sum_r2_u;
+    double cnt = (double)episodes, len = (double)sum_len;
+    const bool shared = __all_sync(0xffffffffu, member == __shfl_sync(0xffffffffu, member, 0));
+    if (shared) {
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
+            len += __shfl_xor_sync(0xffffffffu, len, off);
+            sum_r += __shfl_xor_sync(0xffffffffu, sum_r, off);
+            sum_r2 += __shfl_xor_sync(0xffffffffu, sum_r2, off);
+            min_r = fminf(min_r, __shfl_xor_sync(0xffffffffu, min_r, off));
+            max_r = fmaxf(max_r, __shfl_xor_sync(0xffffffffu, max_r, off));
+            viol += __shfl_xor_sync(0xffffffffu, viol, off);
+        }
+    }
+    if (shared && (threadIdx.x & 31) != 0) return;
+    if (cnt > 0.0) {
+        atomicAdd(stats + 0, cnt);
+        atomicAdd(stats + 1, sum_r);
+        atomicAdd(stats + 2, sum_r2);
+        atomic_min_f64(stats + 3, (double)min_r);
+        atomic_max_f64(stats + 4, (double)max_r);
+        atomicAdd(stats + 5, len);
+    }
+    if (viol && violations) atomicAdd(violations, (unsigned long long)viol);
+}
+
 template <typename T> struct RolloutArgs {
     EnvPtrs<T> env;
     Policy<T> policy;
@@ -448,12 +483,20 @@ __device__ __forceinline__ double pin(double v) { asm volatile("" : "+d"(v)); re
 // Resident CTAs per SM (register cap) of the rollout kernels: 3, and 2 for the fp64 noisy / random-policy ones.
 template <typename T> constexpr int rollout_ctas(bool noisy, bool random) { return sizeof(T) == 4 || !(noisy || random) ? 3 : 2; }
 
+// A population launch (renv_cartpole_population_*_f32): P policies, each on the env's n envs from a fresh start.
+struct PopulationPtrs {
+    const float *policies;      // member p's row: (P, 5) linear w0..w3, b, or (P, kMlpParamFloats) packed MLP parameters
+    int64_t total;              // linear kernel: P n, the flat (member, env) index range
+    uint32_t ctas;              // MLP kernel: CTAs per member, ceil(n / kMlpThreads)
+};
+
 template <typename T, bool kEuler, bool kNoisy = false, bool kRandom = false>
 __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(kNoisy, kRandom))
 cartpole_rollout_kernel(const __grid_constant__ RolloutArgs<T> a)
 {
-    constexpr bool kLog = false;
+    constexpr bool kLog = false, kPop = false;
     const LogPtrs<T> log = {};
+    constexpr PopulationPtrs pop = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -464,9 +507,27 @@ template <typename T, bool kEuler, bool kRandom>
 __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(false, kRandom))
 cartpole_rollout_logged_kernel(const __grid_constant__ LoggedRolloutArgs<T> args)
 {
-    constexpr bool kNoisy = false, kLog = true;
+    constexpr bool kNoisy = false, kLog = true, kPop = false;
     const RolloutArgs<T> &a = args.roll;
     const LogPtrs<T> &log = args.log;
+    constexpr PopulationPtrs pop = {};
+#include "renv_rollout_body.cuh"
+}
+
+struct PopulationArgs { RolloutArgs<float> roll; PopulationPtrs pop; };     // roll.policy is unused
+
+// P linear policies on the env's n envs, one (member, env) pair per thread over a flat index, so that a population of
+// many members with few envs each (ARS / ES: n of 1 to 64) still fills the GPU.  The generic one-env-per-thread body:
+// the FFMA2 pair body parks ended envs through the env's buffers, and this kernel writes nothing into the env.
+template <bool kEuler>
+__global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<float>(false, false))
+cartpole_population_linear_kernel(const __grid_constant__ PopulationArgs args)
+{
+    using T = float;
+    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true;
+    const RolloutArgs<T> &a = args.roll;
+    const LogPtrs<T> log = {};
+    const PopulationPtrs &pop = args.pop;
 #include "renv_rollout_body.cuh"
 }
 

@@ -293,9 +293,10 @@ template <int kAct, bool kEuler, bool kLog>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_rollout_mlp_kernel(const __grid_constant__ MlpRolloutArgs args)
 {
-    constexpr bool kCollect = false;
+    constexpr bool kCollect = false, kPop = false;
     constexpr MlpTrajPtrs traj = {};
     constexpr bool sample = false;
+    constexpr PopulationPtrs pop = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -320,9 +321,33 @@ template <int kAct, bool kEuler, bool kLog>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_collect_mlp_kernel(const __grid_constant__ MlpCollectArgs args)
 {
-    constexpr bool kCollect = true;
+    constexpr bool kCollect = true, kPop = false;
     const MlpTrajPtrs &traj = args.traj;
     const bool sample = args.sample != 0;
+    constexpr PopulationPtrs pop = {};
+#include "renv_mlp_rollout_body.cuh"
+}
+
+// ------------------------------------------------------------------------------------------------
+// Population evaluation: P MLP policies (one activation), each on the env's n envs from a fresh start
+// ------------------------------------------------------------------------------------------------
+struct MlpPopulationArgs {
+    MlpRolloutArgs mlp;        // mlp.roll.policy, mlp.params and mlp.log are unused
+    PopulationPtrs pop;        // pop.policies: (P, kMlpParamFloats) rows; pop.ctas = ceil(n / kMlpThreads)
+};
+
+// The rollout body with one member per CTA: the CTA stages its member's parameter row and runs ceil(n / 128) of its
+// envs.  P x ceil(n / 128) CTAs on a 1-D grid; lanes past n idle, so a launch keeps n / (128 ceil(n / 128)) of its
+// lanes busy (1 at n = 128 k, 0.5 at n = 64, 1 / 128 at n = 1).
+template <int kAct, bool kEuler>
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
+cartpole_population_mlp_kernel(const __grid_constant__ MlpPopulationArgs pa)
+{
+    constexpr bool kLog = false, kCollect = false, kPop = true;
+    constexpr MlpTrajPtrs traj = {};
+    constexpr bool sample = false;
+    const MlpRolloutArgs &args = pa.mlp;
+    const PopulationPtrs &pop = pa.pop;
 #include "renv_mlp_rollout_body.cuh"
 }
 

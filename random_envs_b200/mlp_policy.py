@@ -12,6 +12,9 @@ tensor cores as 3xTF32): ``max |logit - float64 logit| <= 1e-5 * max(1, max |flo
 
 A 1-output net packed the same way is a critic: ``V(s) = l1`` (``outputs == 1``), which
 ``RandomCartPoleVecEnv.gae(traj, critic)`` evaluates on a collected trajectory.
+
+``MLPPopulation`` stacks P such policies (one activation) for ``RandomCartPoleVecEnv.evaluate_population``, which
+evaluates them all on common tasks in one kernel.
 """
 import numpy as np
 
@@ -112,3 +115,53 @@ class MLPPolicy:
     def reference_logits(self, obs):
         """float64 logits of the packed (padded) net for (N, 4) observations."""
         return reference_logits(self.params, self.activation, obs.double())
+
+
+class MLPPopulation:
+    """P packed MLP policies with one activation, for ``RandomCartPoleVecEnv.evaluate_population``.  ``params`` is a
+    (P, PARAM_FLOATS) float32 device tensor whose row p is laid out as ``MLPPolicy.params``.  It may be edited in place
+    between evaluations, e.g. for ES perturbations of the weights; the padded entries of a net narrower than 64 units
+    must stay zero, otherwise the padded units stop being inert and the population is no longer the nets it was made
+    from."""
+
+    def __init__(self, params, activation, device=None):
+        t = _device.torch()
+        params = t.as_tensor(params, dtype=t.float32)
+        if params.dim() != 2 or params.shape[0] < 1 or params.shape[1] != PARAM_FLOATS:
+            raise ValueError("a population is a (P >= 1, %d) array of packed policies, got %s"
+                             % (PARAM_FLOATS, tuple(params.shape)))
+        if int(activation) not in (TANH, RELU):
+            raise ValueError("activation must be TANH (%d) or RELU (%d), got %r" % (TANH, RELU, activation))
+        self.activation = int(activation)
+        # rows of 18,448 bytes: each 16-byte aligned
+        self.params = params.to(device if device is not None else params.device).contiguous()
+        self.device = self.params.device        # with its index: "cuda" is the current device, as for the env's buffers
+
+    @classmethod
+    def from_modules(cls, modules, device=None):
+        """Validate and pack every module of ``modules``; they must share one activation (ValueError otherwise)."""
+        packed = [pack(m) for m in modules]
+        if not packed:
+            raise ValueError("a population needs at least one module")
+        acts = sorted({act for _, act in packed})
+        if len(acts) != 1:
+            raise ValueError("the modules of a population must share one activation (Tanh or ReLU), got both")
+        return cls(np.stack([p for p, _ in packed]), acts[0], _device.require_cuda(device))
+
+    @classmethod
+    def from_policies(cls, policies):
+        """Stack ``MLPPolicy`` objects of one activation and one device (copies their parameters)."""
+        policies = list(policies)
+        if not policies:
+            raise ValueError("a population needs at least one policy")
+        if len({p.activation for p in policies}) != 1 or len({p.device for p in policies}) != 1:
+            raise ValueError("the policies of a population must share one activation and one device")
+        t = _device.torch()
+        return cls(t.stack([p.params for p in policies]), policies[0].activation, policies[0].device)
+
+    def __len__(self):
+        return int(self.params.shape[0])
+
+    def member(self, p):
+        """An ``MLPPolicy`` viewing row ``p`` of ``params`` (no copy: in-place edits show through both ways)."""
+        return MLPPolicy(self.params[p], self.activation, self.device)

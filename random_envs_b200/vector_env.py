@@ -8,6 +8,7 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     step(actions)  -> obs (N, 4), reward (N,), done (N,) bool, info {'TimeLimit.truncated': (N,) bool}
     get_task()     -> (N, 4)            set_task(Tensor(N, 4) | g, m_c, m_p, l)
     rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0] or of an MLPPolicy)
+    evaluate_population(policies, K) -> (P, 6)   (P policies on common tasks from fresh starts; the env is untouched)
     policy_actions(policy) -> (N,)      (the MLPPolicy's actions for the current observations, ready for step)
     collect(policy, K) -> Trajectory    (K fused steps under the sampled policy, every step recorded for training)
     gae(traj, critic) -> Trajectory     (values, GAE advantages and returns of that trajectory under an MLP critic)
@@ -31,7 +32,7 @@ import numpy as np
 
 from . import _device, _lib
 from .episode_log import EpisodeLog
-from .mlp_policy import MLPPolicy
+from .mlp_policy import PARAM_FLOATS, MLPPolicy, MLPPopulation
 from .random_env import RandomEnv
 from .trajectory import Trajectory
 from .xi_tables import get_table
@@ -496,6 +497,53 @@ class RandomCartPoleVecEnv(RandomEnv):
         self._launch(fn, *head, *policy_args, int(num_steps), self._integrator(), self.max_episode_steps, self._tick,
                      self._active_dr_cfg(), _device.ptr(buf["stats"]), _device.ptr(viol))
         self._tick += int(num_steps)
+
+    def evaluate_population(self, policies, num_steps=MAX_EPISODE_STEPS):
+        """Evaluate P policies on this env's tasks with common random numbers, in one kernel: ``policies`` is an
+        ``MLPPopulation`` or a float32 (P, 5) tensor of linear policies (w0, w1, w2, w3, b: a = [w.s + b > 0]) on the
+        env's device.  Returns a (P, 6) float64 device tensor: row p holds the statistics of member p's finished
+        episodes (``distributed.STAT_NAMES``, as ``stats_tensor``).
+
+        Member p runs what a fresh twin of this env (same seed, env_id0, task table, DR config, integrator and
+        TimeLimit) would run under ``reset()`` then ``rollout(policy_p, num_steps)`` on zeroed statistics, and its row
+        equals that twin's ``stats_tensor`` bit for bit: every member sees the same initial states and tasks, so
+        differences between rows come from the policies alone.  A row does not depend on P or on the member's
+        position.  The env itself is left untouched -- state, tasks, TimeLimit counters, episode counters, statistics,
+        an attached episode log -- except for its step clock, which advances by ``num_steps + 1`` so that the next
+        call draws new tasks and initial states.  A gaussian DR failure is raised by the next synchronising call, as
+        for ``rollout``.  float32 envs without observation noise only."""
+        b = self._alloc()
+        t = _device.torch()
+        if self._dtype_name != "float32" or self.noisy:
+            raise ValueError("evaluate_population() needs a float32 env without observation noise")
+        K = int(num_steps)
+        if K < 1:
+            raise ValueError("num_steps must be >= 1, got %d" % K)
+        if isinstance(policies, MLPPopulation):
+            rows, width = policies.params, PARAM_FLOATS
+        elif isinstance(policies, t.Tensor):
+            if policies.dtype != t.float32:
+                raise ValueError("linear policies must be a float32 (P, 5) tensor, got %s" % policies.dtype)
+            rows, width = policies, 5
+        else:
+            raise TypeError("evaluate_population() takes an MLPPopulation or a float32 (P, 5) tensor of linear policies")
+        if rows.dim() != 2 or rows.shape[0] < 1 or rows.shape[1] != width or rows.dtype != t.float32:
+            raise ValueError("the population must be (P >= 1, %d) float32, got %s %s"
+                             % (width, tuple(rows.shape), rows.dtype))
+        if rows.device != b["device"]:
+            raise ValueError("the population lives on %s, the env on %s" % (rows.device, b["device"]))
+        rows = rows.contiguous()
+        P = int(rows.shape[0])
+        stats = t.tensor([0.0, 0.0, 0.0, math.inf, -math.inf, 0.0], dtype=t.float64, device=b["device"]).repeat(P, 1)
+        if width == 5:
+            fn, policy_args = "renv_cartpole_population_linear_f32", (_device.ptr(rows), P)
+        else:
+            fn, policy_args = "renv_cartpole_population_mlp_f32", (_device.ptr(rows), policies.activation, P)
+        viol = self._violation_counter(b["device"])
+        self._launch(fn, ctypes.byref(b["env"]), *policy_args, K, self._integrator(), self.max_episode_steps, self._tick,
+                     self._active_dr_cfg(), _device.ptr(stats), _device.ptr(viol))
+        self._tick += K + 1             # the fresh start at the current tick, then K steps
+        return stats
 
     # ---- episode log ----------------------------------------------------------------------------------
     def start_episode_log(self, capacity=1):
