@@ -97,9 +97,14 @@ typedef struct renv_cartpole_env {
     int32_t *elapsed;            /* (n) TimeLimit._elapsed_steps (gym 0.21)                 */
     uint32_t *episode;           /* (n) episodes started per env (statistics only; may be NULL)   */
     int32_t *beyond;             /* (n) steps_beyond_done, -1 == None (:207-222); may be NULL when auto_reset */
-    uint16_t *elapsed16;         /* (n) the same TimeLimit counter as uint16 for renv_cartpole_step_lean_f32 (16-byte
-                                    aligned); NULL otherwise.  reset zeroes whichever of elapsed / elapsed16 is set;
-                                    `elapsed` may be NULL only for an env that is stepped through the lean entry. */
+    uint16_t *elapsed16;         /* (n) the same TimeLimit counter as uint16 (16-byte aligned; fp32 only, max_steps
+                                    <= 65535), or NULL.  renv_cartpole_step_lean_f32 steps it; reset zeroes whichever
+                                    of elapsed / elapsed16 is set.  `elapsed` may be NULL wherever elapsed16 is set:
+                                    in the lean step, reset, the fp32 rollouts (linear, random, MLP, _logged and
+                                    _noisy forms), collect and renv_cartpole_step_logged_f32 (then give it
+                                    reward = NULL: the lean step's 54 bytes).  These use the int32 counter when
+                                    `elapsed` is set, else elapsed16, and return RENV_E_SIZE for max_steps > 65535
+                                    with elapsed16 alone.  The population entry points use neither. */
     uint32_t *progress;          /* step-to-step ordering at TILE granularity, or NULL for plain stream order.
                                     2 * ceil(n / RENV_TILE_ENVS_F32 | _F64) uint32, 8-byte aligned, zero-initialised ONCE
                                     by the caller and afterwards touched only by the step entry points: word 2b counts

@@ -51,6 +51,7 @@ template <typename T> int to_cfg4(const renv_dr_cfg *dr, DrCfg4<T> *out)
 }
 
 enum ElapsedKind { kNeedElapsed32, kNeedElapsed16, kNeedEitherElapsed };
+// kNeedEitherElapsed: the kernels take the int32 counter when env->elapsed is set, else the uint16 one.
 template <typename T>
 int check_env(const renv_cartpole_env *env, bool need_beyond, EnvPtrs<T> *out, ElapsedKind elapsed = kNeedElapsed32)
 {
@@ -327,7 +328,8 @@ int cartpole_step(const renv_cartpole_env *env, const renv_obs_noise *noise, con
                   const renv_episode_log *log = nullptr, bool logged = false)
 {
     StepArgs<T> a;
-    int rc = check_env<T>(env, !auto_reset, &a.env, kLean ? kNeedElapsed16 : kNeedElapsed32);
+    const ElapsedKind counter = kLean ? kNeedElapsed16 : logged && sizeof(T) == 4 ? kNeedEitherElapsed : kNeedElapsed32;
+    int rc = check_env<T>(env, !auto_reset, &a.env, counter);
     if (rc) return rc;
     rc = attach_noise<T>(noise, &a.env);
     if (rc) return rc;
@@ -339,7 +341,7 @@ int cartpole_step(const renv_cartpole_env *env, const renv_obs_noise *noise, con
         return RENV_E_ALIGN;
     if (counters && !aligned(counters, 8)) return RENV_E_ALIGN;
     if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
-    if (kLean && max_steps > 65535) return RENV_E_SIZE;
+    if ((kLean || env->elapsed == nullptr) && max_steps > 65535) return RENV_E_SIZE;
     rc = to_cfg4<T>(auto_reset ? dr : nullptr, &a.dr);
     if (rc) return rc;
     a.action = action; a.reward = reward; a.done = done; a.truncated = truncated;
@@ -421,7 +423,7 @@ int cartpole_rollout(const renv_cartpole_env *env, const renv_obs_noise *noise, 
                      bool logged = false)
 {
     LoggedRolloutArgs<T> la;
-    int rc = check_env<T>(env, false, &la.roll.env);
+    int rc = check_env<T>(env, false, &la.roll.env, sizeof(T) == 4 ? kNeedEitherElapsed : kNeedElapsed32);
     if (rc) return rc;
     rc = attach_noise<T>(noise, &la.roll.env);
     if (rc) return rc;
@@ -431,6 +433,7 @@ int cartpole_rollout(const renv_cartpole_env *env, const renv_obs_noise *noise, 
     const Policy<T> policy = w ? Policy<T>{ (T)w[0], (T)w[1], (T)w[2], (T)w[3], (T)b } : Policy<T>{ T(0), T(0), T(0), T(0), T(0) };
     rc = check_rollout<T>(stats, K, integrator, max_steps, tick, dr, violations, policy, &la.roll);
     if (rc) return rc;
+    if (env->elapsed == nullptr && max_steps > 65535) return RENV_E_SIZE;     // the uint16 counter
     return launch_rollout(la, logged, w == nullptr, static_cast<cudaStream_t>(stream));
 }
 
@@ -481,7 +484,7 @@ int prepare_rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *lo
                         int K, int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr, double *stats,
                         unsigned long long *violations, A *a, unsigned *blocks)
 {
-    int rc = check_env<float>(env, false, &a->roll.env);
+    int rc = check_env<float>(env, false, &a->roll.env, kNeedEitherElapsed);
     if (rc) return rc;
     if (logged && (rc = check_log<float>(log, &a->log))) return rc;
     if (!logged) a->log = LogPtrs<float>{};
@@ -489,6 +492,7 @@ int prepare_rollout_mlp(const renv_cartpole_env *env, const renv_episode_log *lo
     if (stats == nullptr) return RENV_E_NULL;
     const Policy<float> unused{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
     if ((rc = check_rollout<float>(stats, K, integrator, max_steps, tick, dr, violations, unused, &a->roll))) return rc;
+    if (env->elapsed == nullptr && max_steps > 65535) return RENV_E_SIZE;     // the uint16 counter
     a->params = static_cast<const float *>(p->params);
     return grid_for(env->n, kMlpThreads, blocks);
 }

@@ -67,11 +67,24 @@ __device__ __forceinline__ void store_xi(double *xi, int64_t i, const Xi<double>
 
 template <typename T> struct EnvPtrs {
     T *state; T *xi; int32_t *elapsed; uint32_t *episode; int32_t *beyond;
-    uint16_t *elapsed16;      // lean step only: the TimeLimit counter as uint16 (then `elapsed` may be nullptr)
+    uint16_t *elapsed16;      // the TimeLimit counter as uint16 (fp32): the lean step, and wherever `elapsed` is nullptr
     uint32_t *progress;       // tile-granular step ordering (see cartpole_step_kernel); nullptr: the stream orders steps
     int64_t n, ld; uint64_t env_id0, seed;
     T *obs; T noise_std;      // "Noisy" variants: obs (4, ld) = state + noise_std * N(0, I); obs == nullptr: obs IS state
 };
+
+// TimeLimit counter of env i in whichever layout the env has: the int32 array when `elapsed` is set, else the uint16
+// one (fp32 only: an fp64 env always has the int32 counter).  The fused rollouts read it when an env enters and write
+// it when it leaves, outside their step loops.
+template <typename T> __device__ __forceinline__ int32_t load_elapsed(const EnvPtrs<T> &env, int64_t i)
+{
+    return sizeof(T) == 8 || env.elapsed ? env.elapsed[i] : (int32_t)env.elapsed16[i];
+}
+template <typename T> __device__ __forceinline__ void store_elapsed(const EnvPtrs<T> &env, int64_t i, int32_t el)
+{
+    if (sizeof(T) == 8 || env.elapsed) env.elapsed[i] = el;
+    else env.elapsed16[i] = (uint16_t)el;
+}
 
 // RandomCartPoleEnv.reset (+ set_random_task) of env i at clock `tick`; scalar stores.
 template <typename T>
@@ -211,10 +224,14 @@ __global__ void __launch_bounds__(kStepThreads, kNoisy ? (sizeof(T) == 8 ? 2 : 3
 template <typename T> struct LoggedStepArgs { StepArgs<T> step; LogPtrs<T> log; };
 
 // The plain auto-reset step plus the episode log (a kernel of its own: the plain one keeps its parameter layout).
+// The fp32 one serves both counter layouts: the int32 counter when a.env.elapsed is set, else the uint16 one (the
+// lean step's loads and stores; a.reward == nullptr drops the reward store), chosen per launch -- one kernel per
+// element type, whichever layout the env has.
 template <typename T>
 __global__ void __launch_bounds__(kStepThreads, kStepMinCtas<T>) cartpole_step_logged_kernel(const __grid_constant__ LoggedStepArgs<T> args)
 {
-    constexpr bool kAutoReset = true, kNoisy = false, kLean = false, kLog = true;
+    constexpr bool kAutoReset = true, kNoisy = false, kLog = true;
+    const bool kLean = sizeof(T) == 4 && args.step.env.elapsed == nullptr;
     const StepArgs<T> &a = args.step;
     const LogPtrs<T> &log = args.log;
 #include "renv_step_body.cuh"

@@ -39,7 +39,7 @@
         p = load_xi(a.env.xi, il);
     }
     Derived<float> d = derive(p);
-    int32_t el = kPop ? 0 : a.env.elapsed[il];
+    int32_t el = kPop ? 0 : load_elapsed(a.env, il);
     uint32_t log_count = kLog ? (uint32_t)args.log.count[il] : 0u;
     unsigned episodes = 0, sum_len = 0, viol = fresh_viol;   // return == length (:207-212): sum_len is also sum R
     unsigned long long sum_r2 = 0;
@@ -100,7 +100,7 @@
     if (live && !kPop) {
         a.env.state[i] = s.x; a.env.state[ld + i] = s.x_dot; a.env.state[2 * ld + i] = s.theta; a.env.state[3 * ld + i] = s.theta_dot;
         if (xi_dirty) store_xi(a.env.xi, i, p);
-        a.env.elapsed[i] = el;
+        store_elapsed(a.env, i, el);
         if (kLog) args.log.count[i] = (int32_t)log_count;
         if (a.env.episode && episodes) a.env.episode[i] += episodes;      // one started per episode that ended
     }

@@ -35,7 +35,7 @@
         t.p = load_xi(a.env.xi, il);
     }
     t.d = derive(t.p);
-    t.el = kPop ? 0 : a.env.elapsed[il];
+    t.el = kPop ? 0 : load_elapsed(a.env, il);
     t.new_episodes = 0; t.xi_dirty = false; t.parked = -1;
     t.obs_loaded = kNoisy; t.after_reset = 0u;
     t.act.group = (uint32_t)a.tick >> 7; t.act.r = make_uint4(0, 0, 0, 0); t.refresh = false;
@@ -88,7 +88,7 @@
         a.env.state[i] = t.s.x; a.env.state[ld + i] = t.s.x_dot; a.env.state[2 * ld + i] = t.s.theta;
         a.env.state[3 * ld + i] = t.s.theta_dot;
         if (t.xi_dirty) store_xi(a.env.xi, i, t.p);
-        a.env.elapsed[i] = t.el;
+        store_elapsed(a.env, i, t.el);
         if (kLog) log.count[i] = (int32_t)log_count;
         if (a.env.episode && t.new_episodes) a.env.episode[i] += t.new_episodes;
         if (kNoisy) {       // leave the obs buffer as K calls of step() would: the observation of the last step / reset

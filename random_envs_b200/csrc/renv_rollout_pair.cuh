@@ -30,7 +30,8 @@ constexpr int kInactive = 0x7fffffff;
 struct PairSlot {
     float x, xd, th, thd;                       // state
     float ng, fot, pmlot, l43, nlpm;            // -gravity, F/M, pml/M, l*4/3, -(l*m_p/M)   (Derived<float>)
-    int B, E, L, parked;                        // see the header comment; parked = env-steps done when parked, -1 = not
+    int B, E, L, parked;                        // see the header comment; parked = env-steps done when parked, -1 = not;
+                                                // an inactive slot's E is the counter itself (see on_event)
     uint32_t log_count;                         // logged kernel only: episode-log records of the env (stored at exit)
 };
 
@@ -113,12 +114,13 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
         const long long lk = min((long long)K - s.B, (long long)limit - s.E);
         s.L = (int)min(lk, (long long)(kInactive - 1));
     };
-    auto store_env = [&](const PairSlot &s, int64_t i, int elapsed) {
+    auto store_state = [&](const PairSlot &s, int64_t i) {
         a.env.state[i] = s.x; a.env.state[ld + i] = s.xd; a.env.state[2 * ld + i] = s.th; a.env.state[3 * ld + i] = s.thd;
-        a.env.elapsed[i] = elapsed;
     };
     // slot reached `terminated || c >= L`: the episode ended (-> statistics, park for the deferred reset) or the
-    // env has done its K steps in a still-running episode (-> store it, slot goes inactive)
+    // env has done its K steps in a still-running episode (-> store its state, slot goes inactive).  Either way E
+    // takes the counter's value: the ended episode's length (the reset pass logs it) or the env's final count, which
+    // the kernel stores once at exit -- the counter is read at entry and written at exit, never in the loop
     auto on_event = [&](PairSlot &s, int64_t i, bool terminated) {
         const int steps_done = s.B + c, el = s.E + c;
         if (terminated || el >= limit) {
@@ -126,10 +128,11 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
             episodes += 1; sum_r += (unsigned)el; sum_r2 += (unsigned long long)el * (unsigned)el;   // reward is 1.0/step
             min_r = fminf(min_r, ret); max_r = fmaxf(max_r, ret);
             s.parked = steps_done;
-            if (kLog) store_env(s, i, el);
+            if (kLog) store_state(s, i);
         } else {
-            store_env(s, i, el);
+            store_state(s, i);
         }
+        s.E = el;
         deactivate(s);
     };
     // RandomCartPoleEnv.reset (+ set_random_task) at the clock tick of the step that ended the episode
@@ -138,7 +141,7 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
         const uint64_t tick = a.tick + (uint64_t)(s.parked - 1);
         if (kLog) {
             const State<float> fs = { a.env.state[i], a.env.state[ld + i], a.env.state[2 * ld + i], a.env.state[3 * ld + i] };
-            const int32_t len = a.env.elapsed[i];
+            const int32_t len = s.E;
             log_episode(log, ld, i, s.log_count, load_xi(a.env.xi, i), fs, len, !beyond_thresholds(fs) && len >= limit, tick);
             s.log_count += 1u;
         }
@@ -154,7 +157,7 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
         if (a.env.episode) atomicAdd(a.env.episode + i, 1u);
         const int steps_done = s.parked;
         s.parked = -1;
-        if (steps_done >= K) { store_env(s, i, 0); deactivate(s); }      // the episode ended on the launch's last step
+        if (steps_done >= K) { store_state(s, i); s.E = 0; deactivate(s); }   // the episode ended on the launch's last step
         else activate(s, steps_done, 0);
     };
 
@@ -174,7 +177,7 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
             slot_params(s, p);
             term0[k] = dynamics<false>(st, p, derive(p), policy_action(policy, st), kEuler);
             s.x = st.x; s.xd = st.x_dot; s.th = st.theta; s.thd = st.theta_dot;
-            activate(s, 0, a.env.elapsed[i]);
+            activate(s, 0, load_elapsed(a.env, i));
             if (kLog) s.log_count = (uint32_t)log.count[i];     // in a register: no DRAM round trip in the reset pass
         } else {
             deactivate(s);
@@ -226,10 +229,12 @@ __device__ __forceinline__ void rollout_pair_body(const RolloutArgs<float> &a, c
         }
         if (running == 0u) break;
     }
-    if (kLog) {
 #pragma unroll
-        for (int k = 0; k < S; ++k)
-            if (i0 + k < n) log.count[i0 + k] = (int32_t)q[k].log_count;
+    for (int k = 0; k < S; ++k) {        // every slot of an env has finished: E is its counter
+        if (i0 + k < n) {
+            store_elapsed(a.env, i0 + k, q[k].E);
+            if (kLog) log.count[i0 + k] = (int32_t)q[k].log_count;
+        }
     }
     rollout_publish(a.stats, a.violations, episodes, sum_r, sum_r, sum_r2, min_r, max_r, viol);
 }

@@ -1,7 +1,8 @@
 // Body of cartpole_step_kernel and cartpole_step_logged_kernel (renv_kernels.cuh), included textually into both
 // __global__ functions rather than called as an inlined device function: an inlined body schedules the plain kernels'
 // code differently, and the plain kernels must stay exactly what they were.  The including function defines
-//     T, kAutoReset, kNoisy, kLean, kLog       (template parameters or constexpr)
+//     T, kAutoReset, kNoisy, kLean, kLog       (template parameters or constexpr; kLean is a per-launch constant in
+//                                             the logged kernel)
 //     a    const StepArgs<T> &    the launch arguments
 //     log  const LogPtrs<T> &     the episode log (read only when kLog)
 // No include guard: included once per kernel.

@@ -57,7 +57,7 @@ class RandomCartPoleVecEnv(RandomEnv):
     def __init__(self, num_envs, dtype="float32", device=None, seed=0, env_id0=0,
                  max_episode_steps=MAX_EPISODE_STEPS, auto_reset=True, kinematics_integrator="euler",
                  track_truncated=True, validate_actions=True, track_episodes=True, noisy=False, noise_level=1e-4,
-                 lean=False, tile_ordering="auto", pack_host_flags=True):
+                 lean=False, tile_ordering="auto", pack_host_flags=True, _int32_counter=False):
         RandomEnv.__init__(self)
         if num_envs <= 0:
             raise ValueError("num_envs must be positive")
@@ -82,8 +82,11 @@ class RandomCartPoleVecEnv(RandomEnv):
         if self.noise_level < 0:
             raise ValueError("noise_level must be >= 0")
         # lean step (include/renv.h renv_cartpole_step_lean_f32): uint16 TimeLimit counter, no reward store -- 54 instead
-        # of 62 bytes of HBM traffic per env-step; state / done / truncated bit-identical
+        # of 62 bytes of HBM traffic per env-step; state / done / truncated bit-identical.  The default env takes the
+        # same step whenever it can (see _counter16_fits); lean=True only insists on it, and keeps rollout(), collect()
+        # and the episode log refused as they were before the default took that step.
         self.lean = bool(lean)
+        self._int32_counter = bool(_int32_counter) and not self.lean     # tests: the int32 layout whatever the settings
         if self.lean and (self._dtype_name != "float32" or not self.auto_reset or self.noisy
                           or not 0 < self.max_episode_steps <= 65535):
             raise ValueError("lean=True needs float32, auto_reset, no observation noise and 0 < max_episode_steps <= 65535")
@@ -121,6 +124,23 @@ class RandomCartPoleVecEnv(RandomEnv):
         return _TABLE.lower_bounds[index]
 
     # ---- buffers ----------------------------------------------------------------------------------
+    def _counter16_fits(self):
+        """The env's settings allow the uint16 TimeLimit counter: float32, auto-reset, no observation noise and
+        0 < max_episode_steps <= 65535.  Then the counter never exceeds 65535 and the reward is 1.0 on every step, so
+        ``step`` moves 54 instead of 62 bytes per env (no reward store) with bit-identical results."""
+        return self._dtype_name == "float32" and self.auto_reset and not self.noisy \
+            and 0 < self.max_episode_steps <= 65535
+
+    def _check_counter(self):
+        """Widen the uint16 counter to int32 once a setting changed since allocation rules it out (auto_reset,
+        noisy and max_episode_steps are plain attributes).  One-way: a widened counter may have counted past 65535."""
+        b = self._buffers
+        if b["elapsed16"] is not None and not self.lean and not self._counter16_fits():
+            t = _device.torch()
+            b["elapsed"] = b["elapsed16"].to(t.int32) & 0xFFFF
+            b["elapsed16"] = None
+            self._refresh_env_struct()
+
     @property
     def torch_dtype(self):
         t = _device.torch()
@@ -141,11 +161,12 @@ class RandomCartPoleVecEnv(RandomEnv):
         b = dict(device=dev, ld=ld)
         b["state"] = t.zeros((4, ld), dtype=dt, device=dev)
         b["xi"] = t.tensor(NOMINAL_TASK, dtype=dt, device=dev).reshape(1, 4).repeat(ld, 1).contiguous()   # (ld, 4) rows
-        b["elapsed"] = None if self.lean else t.zeros(ld, dtype=t.int32, device=dev)
-        b["elapsed16"] = t.zeros(ld, dtype=t.int16, device=dev) if self.lean else None     # uint16 bit pattern
+        counter16 = self.lean or (self._counter16_fits() and not self._int32_counter)
+        b["elapsed16"] = t.zeros(ld, dtype=t.int16, device=dev) if counter16 else None     # uint16 bit pattern
+        b["elapsed"] = b["elapsed16"] if counter16 else t.zeros(ld, dtype=t.int32, device=dev)  # the counter, either layout
         b["episode"] = t.zeros(ld, dtype=t.int32, device=dev)       # uint32 bit pattern
         b["beyond"] = t.full((ld,), -1, dtype=t.int32, device=dev)
-        b["reward"] = t.ones(ld, dtype=dt, device=dev)      # lean: never written, 1.0 on every step (:207-212)
+        b["reward"] = t.ones(ld, dtype=dt, device=dev)      # uint16 counter: never written, 1.0 on every step (:207-212)
         b["done"] = t.zeros(ld, dtype=t.uint8, device=dev)
         b["truncated"] = t.zeros(ld, dtype=t.uint8, device=dev)
         b["action"] = t.zeros(ld, dtype=t.uint8, device=dev)
@@ -162,8 +183,8 @@ class RandomCartPoleVecEnv(RandomEnv):
         b = self._buffers
         env = _lib.CartpoleEnv()
         env.state, env.xi = b["state"].data_ptr(), b["xi"].data_ptr()
-        env.elapsed = None if self.lean else b["elapsed"].data_ptr()
-        env.elapsed16 = b["elapsed16"].data_ptr() if self.lean else None
+        env.elapsed = b["elapsed"].data_ptr() if b["elapsed16"] is None else None
+        env.elapsed16 = b["elapsed16"].data_ptr() if b["elapsed16"] is not None else None
         env.beyond = b["beyond"].data_ptr()
         env.progress = b["progress"].data_ptr() if b["progress"] is not None else None
         env.episode = b["episode"].data_ptr() if self.track_episodes else None
@@ -282,17 +303,22 @@ class RandomCartPoleVecEnv(RandomEnv):
         pointers of the persistent buffers and the views handed back.  Rebuilt when a layout-affecting attribute
         changes.  (A 2^20-env step is an 11 us kernel: per-call Python work has to stay below that.)"""
         b = self._buffers
-        key = (self.noisy, self.track_truncated, self._dtype_name, self.lean, self._episode_log, self.auto_reset)
+        key = (self.noisy, self.track_truncated, self._dtype_name, self.lean, self._episode_log, self.auto_reset,
+               self.max_episode_steps)
         plan = b.get("step_plan")
         if plan is not None and plan["key"] == key:
             return plan
+        self._check_counter()
         t = _device.torch()
         n = self.num_envs
-        fn, head = self._resolve("step_lean" if self.lean else "step")
+        counter16 = b["elapsed16"] is not None
+        # the uint16 counter: the lean step, or with a log attached the logged step on that counter without a reward store
+        fn, head = self._resolve("step_lean" if counter16 and self._episode_log is None else "step")
         info = {"TimeLimit.truncated": b["truncated"][:n].view(t.bool)} if self.track_truncated else {}
         viol = self._violation_counter(b["device"])
         plan = dict(key=key, fn=getattr(_lib.load(), fn), name=fn, head=head, logged=self._episode_log is not None,
-                    reward=_device.ptr(b["reward"]), done=_device.ptr(b["done"]),
+                    lean=counter16 and self._episode_log is None,
+                    reward=None if counter16 else _device.ptr(b["reward"]), done=_device.ptr(b["done"]),
                     truncated=_device.ptr(b["truncated"]) if self.track_truncated else None,
                     out=(self.obs, b["reward"][:n], b["done"][:n].view(t.bool)), info=info,
                     device_index=b["device"].index, viol=ctypes.c_void_p(viol.data_ptr()), viol_tensor=viol,
@@ -321,7 +347,7 @@ class RandomCartPoleVecEnv(RandomEnv):
         if self.noisy:
             b["noise"].std = math.sqrt(self.noise_level)
         idx = plan["device_index"]
-        if self.lean:
+        if plan["lean"]:
             args = plan["head"] + (action_ptr, plan["done"], plan["truncated"], self._integrator(), self.max_episode_steps,
                                    self._tick, self._active_dr_cfg(), plan["viol"], ctypes.c_void_p(_device.raw_stream(idx)))
         elif plan["logged"]:        # auto-reset is implied
@@ -415,10 +441,11 @@ class RandomCartPoleVecEnv(RandomEnv):
         ``sample=False`` takes argmax and leaves the env, statistics and episode log exactly as ``rollout(policy, K)``.
         One kernel; bit for bit the K x {obs; policy_actions(policy, sample=sample, return_logp=True); step} loop.
         Advances the step clock by K; afterwards ``obs`` is the observation after the last step (the bootstrap
-        observation).  float32 envs without observation noise or lean=True only."""
+        observation).  float32 envs without observation noise, and not lean=True."""
         buf = self._alloc()
         if self.lean:
             raise ValueError("collect() keeps the int32 TimeLimit counter: build the env without lean=True")
+        self._check_counter()
         self._check_mlp_supported(policy, "collect()")
         K = int(num_steps)
         if K < 1:
@@ -482,6 +509,7 @@ class RandomCartPoleVecEnv(RandomEnv):
         buf = self._alloc()
         if self.lean:
             raise ValueError("rollout() keeps the int32 TimeLimit counter: build the env without lean=True")
+        self._check_counter()
         if isinstance(w, MLPPolicy):
             self._check_mlp_supported(w, "rollout()")
             if float(b) != 0.0:
@@ -735,8 +763,9 @@ class RandomCartPoleVecEnv(RandomEnv):
 
     # ---- checkpoint / resume --------------------------------------------------------------------------
     def _tensor_keys(self):
-        return ("state", "xi", "elapsed16" if self.lean else "elapsed", "episode", "beyond", "stats") + \
-               (("obs",) if self.noisy else ())
+        """The buffers a state_dict holds; the TimeLimit counter goes under the key of the env's layout."""
+        return ("state", "xi", "elapsed16" if self._alloc()["elapsed16"] is not None else "elapsed", "episode", "beyond",
+                "stats") + (("obs",) if self.noisy else ())
 
     def state_dict(self):
         """Everything a resumed run needs to continue bit for bit: env buffers, the Philox key and step clock, the DR
@@ -753,11 +782,22 @@ class RandomCartPoleVecEnv(RandomEnv):
         return out
 
     def load_state_dict(self, sd):
-        if sd["num_envs"] != self.num_envs or sd["dtype"] != self._dtype_name or sd.get("lean", False) != self.lean:
-            raise ValueError("state_dict is for %d %s envs%s" % (sd["num_envs"], sd["dtype"], " (lean)" if sd.get("lean") else ""))
+        """Restore a ``state_dict`` of an env of the same size and dtype, whichever TimeLimit counter layout either env
+        has (int32 ``elapsed`` or uint16 ``elapsed16``): the counter is converted."""
+        if sd["num_envs"] != self.num_envs or sd["dtype"] != self._dtype_name:
+            raise ValueError("state_dict is for %d %s envs" % (sd["num_envs"], sd["dtype"]))
+        t = _device.torch()
         b = self._alloc()
+        counter = sd["elapsed16"].to(t.int32) & 0xFFFF if "elapsed16" in sd else sd["elapsed"]
+        if b["elapsed16"] is not None and "elapsed16" not in sd and int(counter.max()) > 0xFFFF:
+            if self.lean:       # counted without a TimeLimit: the uint16 counter cannot hold it
+                raise ValueError("the state_dict's TimeLimit counters exceed 65535: load it into an env without lean=True")
+            b["elapsed"], b["elapsed16"] = t.zeros_like(b["elapsed16"], dtype=t.int32), None
         for k in self._tensor_keys():
-            b[k].copy_(sd[k])
+            if k == "elapsed16":
+                b[k].copy_(counter.to(b[k].device).to(t.int16))
+            else:
+                b[k].copy_(counter if k == "elapsed" else sd[k])
         self._seed, self.env_id0, self._tick = sd["seed"], sd["env_id0"], sd["tick"]
         dr = sd.get("dr")
         if dr is not None:
@@ -774,7 +814,7 @@ class RandomCartPoleVecEnv(RandomEnv):
     @property
     def elapsed(self):
         b = self._alloc()
-        if self.lean:
+        if b["elapsed16"] is not None:
             t = _device.torch()
             return b["elapsed16"][:self.num_envs].to(t.int32) & 0xFFFF
         return b["elapsed"][:self.num_envs]
@@ -796,7 +836,7 @@ class RandomCartPoleVecEnv(RandomEnv):
         b["beyond"].fill_(-1)
         if elapsed is not None:
             el = t.as_tensor(elapsed, device=b["device"]).to(t.int32)
-            if self.lean:
+            if b["elapsed16"] is not None:
                 b["elapsed16"][:self.num_envs].copy_(el.to(t.int16))
             else:
                 b["elapsed"][:self.num_envs].copy_(el)
