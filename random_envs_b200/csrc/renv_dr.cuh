@@ -11,9 +11,10 @@
 //
 // double: library normcdfinv / log / sincospi with explicitly rounded affine maps (parity path).
 // float:  the truncation to [-2, 2] keeps the inverse CDF in its central region, so Phi^-1 is one MUFU.LG2 and a
-//         degree-6 polynomial (no tail branches, no sign select, max abs error ~5e-7 at |z| = 2); Box-Muller uses the
-//         MUFU lg2 / sqrt / sin / cos approximations (abs error ~2^-21, far below anything a DR law can resolve).
-//         Both transforms start from the integer draw (r >> 8): the 2^-24 scale is folded into their first FMA.
+//         degree-6 polynomial (no tail branches, no sign select, max abs error 7e-7); Box-Muller takes its radius
+//         from MUFU.LG2, or a series of ln(1 - v) near u1 = 1 (max abs error 2e-6), and its angle from MUFU sin / cos
+//         (max abs error 1e-6, angle rounding included).  Both transforms start from the integer draw (r >> 8).  These bounds hold over all 2^24 inputs
+//         (tests/test_gpu_normal_transforms.py) and are the ones oracle/f32_draws.py checks every fp32 draw against.
 #pragma once
 #include "renv_philox.cuh"
 #include "renv_pack.cuh"
@@ -40,7 +41,7 @@ template <typename T> struct DrCfg4 {
 };
 
 template <typename T> struct Num;
-// MUFU.LG2 without the denormal-input scaling of lg2.approx.f32 (3 extra instructions): arguments here are >= 0.089.
+// MUFU.LG2 without the denormal-input scaling of lg2.approx.f32 (3 extra instructions): arguments here are >= 2^-24.
 __device__ __forceinline__ float lg2_approx(float x)
 {
     float r;
@@ -61,6 +62,8 @@ template <> struct Num<float> {
     // x = 2p - 1 = X (2u - 1) in [-X, X):  z = sqrt(2) erfinv(x) = x * g(w), w = -ln(1 - x^2) in [0, 2.42]; g is fitted
     // (Chebyshev nodes, degree 6 in t = w - 1.25, max abs error of z 2.9e-7).  1 - x^2 >= 0.089, so forming it with
     // one FMA loses nothing that matters (<= 2e-7 in z).  11 FMA-pipe + 1 MUFU + 2 ALU instructions per value.
+    // Max abs error of z over all 2^24 inputs, float(Phi(2) - Phi(-2)) included: 7e-7 (measured 6.1e-7 on the B200,
+    // tests/test_gpu_normal_transforms.py).
     __device__ static __forceinline__ float tn_z_bits(uint32_t r)
     {
         const float X = (float)kPhiSpan;
@@ -79,13 +82,32 @@ template <> struct Num<float> {
     {
         z[0] = tn_z_bits(r.x); z[1] = tn_z_bits(r.y); z[2] = tn_z_bits(r.z); z[3] = tn_z_bits(r.w);
     }
+    // Box-Muller radius sqrt(-2 ln u1), u1 = ((r >> 8) + 1) 2^-24 in (0, 1].  Near u1 = 1 the radius -> 0 and the square
+    // root turns an absolute error e of the logarithm into sqrt(2 e), so MUFU.LG2 (absolute error ~2^-22 there) cannot
+    // be used on its own: for v = 1 - u1 < 1/16 (exact: v = (~r >> 8) 2^-24) -ln(1 - v) is its series to v^6 (relative
+    // truncation error v^6 / 7 < 1e-8); below, lg2(u1) <= -0.093 and MUFU.LG2's absolute error is harmless.  (The
+    // former (24 - lg2(k)) 2 ln 2, k = 2^24 u1, cancelled near k = 2^24: off by up to 1.28e-3 on the B200.)  Max abs
+    // error over all 2^24 inputs: 2e-6 (measured 6.3e-7 on the B200, tests/test_gpu_normal_transforms.py).  Cost:
+    // 5 FFMA + FMUL + FSETP + FSEL more per pair than the cancelling form, 11 % of the gaussian sampler's rate.
+    __device__ static __forceinline__ float bm_radius(uint32_t ra)
+    {
+        const float v = __fmul_rn((float)(~ra >> 8), 1.0f / 16777216.0f);
+        float p = fmaf(v, 1.0f / 6.0f, 0.2f);
+        p = fmaf(p, v, 0.25f);
+        p = fmaf(p, v, 1.0f / 3.0f);
+        p = fmaf(p, v, 0.5f);
+        p = fmaf(p, v, 1.0f);
+        const float near1 = __fmul_rn(2.0f * v, p);                                         // -2 ln(1 - v)
+        const float far = __fmul_rn(lg2_approx(__fsub_rn(1.0f, v)), -1.3862943611198906f);  // -2 ln 2 lg2(u1)
+        return sqrt_approx(v < 0.0625f ? near1 : far);
+    }
     // 4 standard normals from one Philox block: Box-Muller on the pairs (x,y) and (z,w), both branches used.
-    // radius^2 = -2 ln u1 with u1 = ((r >> 8) + 1) 2^-24 in (0, 1]  ==  (24 - lg2(k)) * 2 ln 2, k = (r >> 8) + 1;
-    // angle = 2 pi (u2 - 1/2).  MUFU lg2 / sqrt / sin / cos (abs error ~2^-21, far below what a DR law resolves).
+    // angle = 2 pi (u2 - 1/2), u2 = (r >> 8) 2^-24, with MUFU sin / cos: together with the rounding of the angle, off
+    // by at most 1e-6 absolute; each normal is within 2e-6 + 1e-6 rad (+ its own rounding) of the float64 value.
     __device__ static __forceinline__ void normal_pair(uint32_t ra, uint32_t rb, float *z)
     {
-        const float two_ln2 = 1.3862943611198906f, two_pi = 6.283185307179586f;
-        const float rad = sqrt_approx(fmaf(lg2_approx((float)((ra >> 8) + 1u)), -two_ln2, 24.0f * two_ln2));
+        const float two_pi = 6.283185307179586f;
+        const float rad = bm_radius(ra);
         const float ang = fmaf((float)(rb >> 8), two_pi / 16777216.0f, -0.5f * two_pi);
         z[0] = __fmul_rn(rad, __cosf(ang));
         z[1] = __fmul_rn(rad, __sinf(ang));
@@ -301,8 +323,8 @@ __device__ __forceinline__ u64 truncnorm_pair(uint32_t ra, uint32_t rb, u64 std2
 // Num<float>::normal_pair for one (radius, angle) draw pair, then the affine map
 __device__ __forceinline__ u64 gaussian_pair(uint32_t ra, uint32_t rb, u64 std2, u64 mean2)
 {
-    const float two_ln2 = 1.3862943611198906f, two_pi = 6.283185307179586f;
-    const float rad = sqrt_approx(fmaf(lg2_approx((float)((ra >> 8) + 1u)), -two_ln2, 24.0f * two_ln2));
+    const float two_pi = 6.283185307179586f;
+    const float rad = Num<float>::bm_radius(ra);
     const float ang = fmaf((float)(rb >> 8), two_pi / 16777216.0f, -0.5f * two_pi);
     return fma2(std2, mul2(splat(rad), pk(__cosf(ang), __sinf(ang))), mean2);
 }

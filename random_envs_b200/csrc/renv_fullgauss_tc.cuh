@@ -145,11 +145,12 @@ dr_sample_fullgaussian_tc_kernel(float *__restrict__ out, int64_t n, const __gri
         float *row = rows + lane * dim;
 #pragma unroll
         for (int d = 0; d < 32; ++d) {
-            // (clip(mean + x, 0, 4) * width) / 4 + lo (random_env.py:194-198, 205-220) in two instructions: scaling by
-            // 1/4 is exact and commutes with rounding, so sat(x / 4 + mean / 4) == clip(fl(mean + x), 0, 4) / 4 and
-            // fl(q * width) == fl(p * width) / 4 bit for bit; the host passes mean / 4 and width = hi - lo
+            // (clip(mean + x, 0, 4) * width) / 4 + lo (random_env.py:194-198, 205-220): scaling by 1/4 is exact and
+            // commutes with rounding, so sat(x / 4 + mean / 4) == clip(fl(mean + x), 0, 4) / 4 and
+            // fl(q4 * width) == fl(p * width) / 4; rounding that product before adding lo makes the result
+            // denormalize(fl(mean + x), lo, hi) bit for bit.  The host passes mean / 4 and width = hi - lo.
             const float q4 = __saturatef(fmaf(x[d], 0.25f, cfg.mean[d]));
-            if (d < dim) row[d] = fmaf(q4, cfg.hi[d], cfg.lo[d]);
+            if (d < dim) row[d] = __fadd_rn(__fmul_rn(q4, cfg.hi[d]), cfg.lo[d]);
         }
         __syncwarp();
         const int64_t quad_first = tile * kFgTile + quad * 32;

@@ -70,8 +70,7 @@ __device__ __forceinline__ double u01(uint32_t hi, uint32_t lo)
     return __dmul_rn(__dadd_rn(__dmul_rn((double)(hi >> 5), 67108864.0), (double)(lo >> 6)),
                      1.0 / 9007199254740992.0);
 }
-// (0,1] variants for log() in Box-Muller.
-__device__ __forceinline__ float u01_open0(uint32_t r) { return (float)((r >> 8) + 1u) * (1.0f / 16777216.0f); }
+// (0,1] variant for log() in the fp64 Box-Muller.
 __device__ __forceinline__ double u01_open0(uint32_t hi, uint32_t lo)
 {
     return __dmul_rn(__dadd_rn(__dadd_rn(__dmul_rn((double)(hi >> 5), 67108864.0), (double)(lo >> 6)), 1.0),
@@ -98,17 +97,7 @@ template <> struct Pack<float> {
         out[2] = fmaf(scale[2], (float)(r.z >> 8), off[2]);
         out[3] = fmaf(scale[3], (float)(r.w >> 8), off[3]);
     }
-    // 4 standard normals: Box-Muller on the pairs (x,y) and (z,w), both branches used
-    __device__ static __forceinline__ void normals(uint4 r, float z[4])
-    {
-        float s, c;
-        float rad = sqrtf(-2.0f * logf(u01_open0(r.x)));
-        sincospif(2.0f * u01(r.y), &s, &c);
-        z[0] = rad * c; z[1] = rad * s;
-        rad = sqrtf(-2.0f * logf(u01_open0(r.z)));
-        sincospif(2.0f * u01(r.w), &s, &c);
-        z[2] = rad * c; z[3] = rad * s;
-    }
+    // (fp32 standard normals: Num<float>::normals in renv_dr.cuh)
 };
 template <> struct Pack<double> {
     static constexpr int kPerBlock = 2;

@@ -11,7 +11,7 @@ from scipy import stats
 
 import random_envs_b200 as random_envs
 from random_envs_b200.random_env import covariance_factor
-from oracle import c_oracle, dr_port
+from oracle import c_oracle, dr_port, f32_draws
 
 pytestmark = pytest.mark.gpu
 
@@ -138,8 +138,10 @@ def test_tensor_core_contraction_matches_the_fma_chain_kernel(env_id, n):
     assert np.max(np.abs(xt - xc) / (hi - lo)) <= 4e-6 and np.max(np.abs(yt - yc) / (hi - lo)) <= 4e-6
     assert not np.array_equal(xt, yt)
     assert np.mean(xt == xc) > 0.2          # many entries even agree to the last bit
-    # and against the fp64 contract (fp64 Box-Muller vs MUFU lg2/sin/cos: 2e-5 of the width is the fp32 kernels' bound)
-    s64 = random_envs.TaskSampler(env_id); s64.seed_dr(21)
-    s64.set_dr_distribution("fullgaussian", {"mean": mean, "cov": cov})
-    x64 = s64.sample_tasks_tensor(n, dtype=torch.float64).cpu().numpy()
-    assert x64.shape == xt.shape
+    # and both against the float64 restatement of the fp32 contract (fp32 takes 4 normals per Philox block, fp64 2,
+    # so the fp64 sampler draws other values): every entry within its stated bound
+    f = covariance_factor(cov)
+    for got, tick, tc in ((xt, 0, True), (yt, 1, True), (xc, 0, False), (yc, 1, False)):
+        value, bound = f32_draws.fullgaussian_sample(21, np.arange(n, dtype=np.uint64), tick, f32_draws.PURPOSE_TASKS,
+                                                     mean, f, lo, hi, tensor_core=tc)
+        assert np.all(np.abs(got - value) <= bound), (tick, tc, np.max(np.abs(got - value) - bound))
