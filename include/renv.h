@@ -380,6 +380,53 @@ int renv_cartpole_population_mlp_f32(const renv_cartpole_env *env, const void *p
                                      int integrator, int max_steps, uint64_t tick, const renv_dr_cfg *dr,
                                      double *stats, unsigned long long *violations, void *stream);
 
+/* Evaluation grids: P policies x C task scenarios in one launch, with statistics per (policy, scenario) cell -- a
+ * return map over the task space, the check of a policy at each boundary of the current ADR ranges, or the choice of a
+ * checkpoint over several test distributions.
+ *
+ * A scenario is a row of RENV_SCENARIO_FLOATS floats (128 bytes, 16-byte aligned in device memory) holding the image of
+ * one DR config in the kernels' element type, as renv_scenario_pack_f32 writes it:
+ *   float index  0      dr_type (int32 bits): RENV_DR_NONE for a fixed task, else one of the four laws
+ *                1      dim (int32 bits, 4)
+ *                2..5   a[4]       uniform: lo; truncnorm / gaussian: mean; fullgaussian: mean (normalised space);
+ *                                  fixed task: the task (gravity, cart_mass, pole_mass, pole_length)
+ *                6..9   b[4]       uniform: float(float(hi) - float(lo)) * 2^-24; truncnorm / gaussian: std;
+ *                                  fullgaussian: search-bound lo
+ *               10..13  floor[4]   truncnorm: lower bound; gaussian: 0.1; fullgaussian: search-bound hi
+ *               14..29  factor[16] fullgaussian: row-major 4 x 4 F with F F^T = cov
+ *               30..31  padding (zero) */
+#define RENV_SCENARIO_FLOATS 32
+
+/* Host only (no CUDA call, no allocation): scenario row `out` of `dr`, or of the fixed task `task` when `dr` is NULL or
+ * RENV_DR_NONE (`task` is not read otherwise).  A distribution row holds exactly the float parameters a launch with
+ * that `dr` passes to its kernels, so a grid cell sees the draws a population launch with `dr` sees.  Errors: NULL out,
+ * or NULL task for a fixed task, RENV_E_NULL; a non-finite task RENV_E_ARG; an unknown dr_type RENV_E_DRTYPE; dim != 4
+ * RENV_E_DIM. */
+int renv_scenario_pack_f32(const renv_dr_cfg *dr, const double task[4], float out[RENV_SCENARIO_FLOATS]);
+
+/* With E = env->n: for policy p < P, scenario c < C and env j < E, Philox id env_id0 + j whatever p and c, the cell
+ * (p, c) runs what renv_cartpole_population_*_f32 runs for policy row p alone at the same `tick` (a fresh episode at
+ * `tick`, then K steps at tick + 1 .. tick + K with auto-reset, the TimeLimit `max_steps` and the resample on reset),
+ * with xi taken from scenario row c:
+ *   - a row whose dr_type is one of the four laws: as a population launch with `dr` = the config it was packed from;
+ *   - any other row (a fixed task): as a population launch with dr = NULL on an xi table whose every row is its task
+ *     a[0..3]; the task stays across resets.
+ * The cell's finished episodes are ACCUMULATED into stats[(p * C + c) * RENV_NUM_STATS ..] (caller-initialised to
+ * {0, 0, 0, +inf, -inf, 0}) and equal, bit for bit, that population launch's row p.  Every cell sees the same initial
+ * states and, under one law, the same draws (common random numbers across policies and scenarios); a cell depends on
+ * neither P, C nor its position in the grid.  Nothing is written into the env, and only env->n, env_id0 and seed are
+ * read (not xi).  Gaussian DR failures are counted into `violations` (may be NULL).
+ * Errors, all before any CUDA call: NULL env / policies / params / scenarios / stats RENV_E_NULL; P < 1, C < 1, n <= 0,
+ * K outside [1, 2^30] or P * C * n >= 2^31 RENV_E_SIZE; a misaligned pointer RENV_E_ALIGN (scenarios 16 bytes, stats 8,
+ * linear policies 4, MLP params 16); an unknown integrator RENV_E_INTEGRATOR; an unknown activation RENV_E_ARG.
+ * The policy rows are those of renv_cartpole_population_linear_f32 / renv_cartpole_population_mlp_f32. */
+int renv_cartpole_grid_linear_f32(const renv_cartpole_env *env, const float *policies, int P, const float *scenarios,
+                                  int C, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                                  unsigned long long *violations, void *stream);
+int renv_cartpole_grid_mlp_f32(const renv_cartpole_env *env, const void *params, int activation, int P,
+                               const float *scenarios, int C, int K, int integrator, int max_steps, uint64_t tick,
+                               double *stats, unsigned long long *violations, void *stream);
+
 /* Recorded cart-pole transitions for offline DR fitting (device pointers): transition i is (obs[i], action[i],
  * next_obs[i]), and `window` lists the W start indices t that are scored (t + lam <= T; windows crossing an episode
  * boundary are the caller's to leave out). */

@@ -30,12 +30,13 @@ from .mlp_policy import MLPPolicy, MLPPopulation
 from .offline_dr import TransitionDataset
 from .random_cartpole import RandomCartPoleEnv
 from .random_env import RandomEnv, TaskSampler
+from .scenarios import Scenarios
 from .trajectory import Trajectory
 from .vector_env import RandomCartPoleVecEnv
 from .gym_vector import RandomCartPoleGymVectorEnv
 from .xi_tables import HUMANOID_NOMINAL, XI_TABLES
 
-__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "MLPPopulation", "Trajectory", "TransitionDataset", "XI_TABLES",
+__all__ = ["gym", "RandomEnv", "TaskSampler", "RandomCartPoleEnv", "RandomCartPoleVecEnv", "RandomCartPoleGymVectorEnv", "EpisodeLog", "MLPPolicy", "MLPPopulation", "Scenarios", "Trajectory", "TransitionDataset", "XI_TABLES",
            "HUMANOID_NOMINAL", "shard_range", "combine_stats", "summarize_stats", "allgather_stats",
            "make_sharded_env", "load_library"]
 

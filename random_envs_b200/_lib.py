@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(_HERE, "librenv_b200.so")
 ABI_VERSION = 6
 MAX_DIM = 32
 NUM_STATS = 6
+SCENARIO_FLOATS = 32      # RENV_SCENARIO_FLOATS
 SCALAR_SAVE_BYTES = 512     # RENV_SCALAR_SAVE_BYTES
 COUNTER_GAUSSIAN, COUNTER_BAD_ACTION, COUNTER_ORDER_TIMEOUT = 0, 1, 2
 TILE_ENVS = {'float32': 1024, 'float64': 512}      # RENV_TILE_ENVS_F32 / _F64
@@ -112,6 +113,9 @@ SIGNATURES = {
     "renv_cartpole_gae_mlp_f32": (_int, [_env_p, _mlp_p, _traj_p, _int, _flt, _flt, _vp, _vp, _vp, _vp]),
     "renv_cartpole_population_linear_f32": (_int, [_env_p, _vp, _int, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
     "renv_cartpole_population_mlp_f32": (_int, [_env_p, _vp, _int, _int, _int, _int, _int, _u64, _cfg_p, _vp, _vp, _vp]),
+    "renv_scenario_pack_f32": (_int, [_cfg_p, ctypes.POINTER(_dbl), _vp]),
+    "renv_cartpole_grid_linear_f32": (_int, [_env_p, _vp, _int, _vp, _int, _int, _int, _int, _u64, _vp, _vp, _vp]),
+    "renv_cartpole_grid_mlp_f32": (_int, [_env_p, _vp, _int, _int, _vp, _int, _int, _int, _int, _u64, _vp, _vp, _vp]),
     "renv_cartpole_transition_loglik_f64": (_int, [_trans_p, _int, _int, _vp, _int, _int, ctypes.POINTER(_dbl), _vp, _vp,
                                                    _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),

@@ -9,7 +9,9 @@
 #include "renv_mlp_gae.cuh"
 #include "renv_transition_loglik.cuh"
 #include "renv_scalar_server.cuh"
+#include <stddef.h>
 #include <stdlib.h>
+#include <string.h>
 #include <type_traits>
 
 using namespace renv;
@@ -637,6 +639,94 @@ int population_mlp(const renv_cartpole_env *env, const void *params, int activat
     return launch_status();
 }
 
+// A scenario row (include/renv.h RENV_SCENARIO_FLOATS) is the DrCfg4<float> image the kernels take, zero-padded.
+static_assert(kScenarioFloats == RENV_SCENARIO_FLOATS, "scenario row size differs from include/renv.h");
+static_assert(offsetof(DrCfg4<float>, dr_type) == 0 && offsetof(DrCfg4<float>, dim) == 4 &&
+              offsetof(DrCfg4<float>, a) == 8 && offsetof(DrCfg4<float>, b) == 24 &&
+              offsetof(DrCfg4<float>, floor) == 40 && offsetof(DrCfg4<float>, factor) == 56 &&
+              sizeof(DrCfg4<float>) == 120, "scenario row layout differs from include/renv.h");
+
+int scenario_pack(const renv_dr_cfg *dr, const double *task, float *out)
+{
+    if (out == nullptr) return RENV_E_NULL;
+    DrCfg4<float> cfg;
+    const int rc = to_cfg4<float>(dr, &cfg);
+    if (rc) return rc;
+    if (cfg.dr_type == kDrNone) {           // a fixed task: a = the task, kept across resets
+        if (task == nullptr) return RENV_E_NULL;
+        for (int k = 0; k < 4; ++k)
+            if (!std::isfinite(task[k])) return RENV_E_ARG;
+        for (int k = 0; k < 4; ++k) cfg.a[k] = (float)task[k];
+    }
+    float row[kScenarioFloats] = {};
+    memcpy(row, &cfg, sizeof(cfg));
+    memcpy(out, row, sizeof(row));
+    return RENV_OK;
+}
+
+// The checks and arguments both grid entry points share, all before any CUDA call: those of a population launch on
+// P C n (policy, scenario, env) triples, plus the scenario rows.  Neither env->xi nor a DR config is read.
+int prepare_grid(const renv_cartpole_env *env, const void *rows, size_t row_align, int P, const float *scenarios, int C,
+                 int K, int integrator, int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+                 RolloutArgs<float> *a, PopulationPtrs *pop, GridPtrs *grid)
+{
+    if (env == nullptr || rows == nullptr || scenarios == nullptr || stats == nullptr) return RENV_E_NULL;
+    // P C n < 2^31: the flat (policy, scenario, env) index, a member's (scenario, env) range and the MLP grid fit in 31 bits
+    if (P < 1 || C < 1 || env->n <= 0 || env->n >= (1LL << 31) || (int64_t)P * C >= (1LL << 31) ||
+        (int64_t)P * C * env->n >= (1LL << 31))
+        return RENV_E_SIZE;
+    const Policy<float> unused{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
+    const int rc = check_rollout<float>(stats, K, integrator, max_steps, tick + 1, nullptr, violations, unused, a);
+    if (rc) return rc;
+    if (!aligned(rows, row_align) || !aligned(scenarios, 16)) return RENV_E_ALIGN;
+    a->env = EnvPtrs<float>{};
+    a->env.n = env->n;
+    a->env.env_id0 = env->env_id0;
+    a->env.seed = env->seed;
+    const int64_t span = (int64_t)C * env->n;
+    *pop = PopulationPtrs{ static_cast<const float *>(rows), (int64_t)P * span,
+                           (uint32_t)((span + kMlpThreads - 1) / kMlpThreads) };
+    *grid = GridPtrs{ scenarios, (uint32_t)C, (uint32_t)span };
+    return RENV_OK;
+}
+
+int grid_linear(const renv_cartpole_env *env, const float *policies, int P, const float *scenarios, int C, int K,
+                int integrator, int max_steps, uint64_t tick, double *stats, unsigned long long *violations, void *stream)
+{
+    GridArgs ga;
+    int rc = prepare_grid(env, policies, 4, P, scenarios, C, K, integrator, max_steps, tick, stats, violations, &ga.roll,
+                          &ga.pop, &ga.grid);
+    if (rc) return rc;
+    unsigned blocks = 0;
+    if ((rc = grid_for(ga.pop.total, kRolloutThreads, &blocks))) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_flag(ga.roll.euler, [&](auto euler) {
+        cartpole_grid_linear_kernel<euler><<<blocks, kRolloutThreads, 0, st>>>(ga);
+    });
+    return launch_status();
+}
+
+int grid_mlp(const renv_cartpole_env *env, const void *params, int activation, int P, const float *scenarios, int C,
+             int K, int integrator, int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+             void *stream)
+{
+    MlpGridArgs ga;
+    const int rc = prepare_grid(env, params, 16, P, scenarios, C, K, integrator, max_steps, tick, stats, violations,
+                                &ga.mlp.roll, &ga.pop, &ga.grid);
+    if (rc) return rc;
+    if (activation != RENV_MLP_TANH && activation != RENV_MLP_RELU) return RENV_E_ARG;
+    ga.mlp.params = nullptr;
+    ga.mlp.log = LogPtrs<float>{};
+    const unsigned blocks = (unsigned)P * ga.pop.ctas;      // <= P C n < 2^31
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_activation(activation, [&](auto act) {
+        with_flag(ga.mlp.roll.euler, [&](auto euler) {
+            cartpole_grid_mlp_kernel<act, euler><<<blocks, kMlpThreads, 0, st>>>(ga);
+        });
+    });
+    return launch_status();
+}
+
 int check_transition_loglik(const renv_transitions *data, int lam, int integrator, const double *xi, int C, int M,
                             const double *eps, double *loglik, double *total, LoglikArgs *a, unsigned *blocks)
 {
@@ -877,6 +967,23 @@ int renv_cartpole_population_mlp_f32(const renv_cartpole_env *env, const void *p
                                      double *stats, unsigned long long *violations, void *stream)
 {
     return population_mlp(env, params, activation, P, K, integrator, max_steps, tick, dr, stats, violations, stream);
+}
+
+int renv_scenario_pack_f32(const renv_dr_cfg *dr, const double task[4], float out[RENV_SCENARIO_FLOATS])
+{
+    return scenario_pack(dr, task, out);
+}
+int renv_cartpole_grid_linear_f32(const renv_cartpole_env *env, const float *policies, int P, const float *scenarios,
+                                  int C, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                                  unsigned long long *violations, void *stream)
+{
+    return grid_linear(env, policies, P, scenarios, C, K, integrator, max_steps, tick, stats, violations, stream);
+}
+int renv_cartpole_grid_mlp_f32(const renv_cartpole_env *env, const void *params, int activation, int P,
+                               const float *scenarios, int C, int K, int integrator, int max_steps, uint64_t tick,
+                               double *stats, unsigned long long *violations, void *stream)
+{
+    return grid_mlp(env, params, activation, P, scenarios, C, K, integrator, max_steps, tick, stats, violations, stream);
 }
 
 int renv_cartpole_transition_loglik_f64(const renv_transitions *data, int lam, int integrator, const double *xi, int C,

@@ -459,8 +459,17 @@ __device__ __forceinline__ void rollout_step(RolloutThread<T> &t, const RolloutA
     t.remaining = park ? 0 : t.remaining - 1;
 }
 
-template <typename T, bool kRandom = false>
-__device__ __forceinline__ void rollout_reset(RolloutThread<T> &t, const RolloutArgs<T> &a, uint64_t id)
+// Whether a reset draws xi from `dr`: any active DR config of a launch; for a grid scenario row (kGrid) one of the four
+// laws only, any other dr_type being a fixed task that the env keeps across resets.
+template <bool kGrid> __device__ __forceinline__ bool draws_xi(int dr_type)
+{
+    return kGrid ? (unsigned)(dr_type - kDrUniform) <= (unsigned)(kDrFullGaussian - kDrUniform) : dr_type != kDrNone;
+}
+
+// A grid launch (kGrid) passes the lane's scenario row `scen`, which replaces a.dr.
+template <typename T, bool kRandom = false, bool kGrid = false>
+__device__ __forceinline__ void rollout_reset(RolloutThread<T> &t, const RolloutArgs<T> &a, uint64_t id,
+                                              const DrCfg4<T> *scen = nullptr)
 {
     if (!(kRandom && t.refresh)) {
         // the episode that just ended (return == length: the reward is 1.0 on every step, :207-212)
@@ -471,9 +480,10 @@ __device__ __forceinline__ void rollout_reset(RolloutThread<T> &t, const Rollout
         t.new_episodes += 1; t.el = 0;
         // the clock value a single step() would have used for the step that ended it: t.parked steps were left after it
         const uint64_t reset_tick = a.tick + (uint64_t)(a.K - t.parked - 1);
-        if (a.dr.dr_type != kDrNone) {
+        const DrCfg4<T> &dr = kGrid ? *scen : a.dr;
+        if (draws_xi<kGrid>(dr.dr_type)) {
             t.p = Xi<T>{ T(0), T(0), T(0), T(0) };
-            t.viol += sample_xi(t.p, a.dr, a.env.seed, id, reset_tick);
+            t.viol += sample_xi(t.p, dr, a.env.seed, id, reset_tick);
             t.d = derive(t.p);
             t.xi_dirty = true;
         }
@@ -507,13 +517,30 @@ struct PopulationPtrs {
     uint32_t ctas;              // MLP kernel: CTAs per member, ceil(n / kMlpThreads)
 };
 
+// A grid launch (renv_cartpole_grid_*_f32): P policies x C scenarios, each cell (p, c) on the env's n envs from a fresh
+// start.  Scenario row c is kScenarioFloats floats holding the DrCfg4<float> image of its DR config, or of a fixed task
+// (dr_type none, a = the task): the layout of RENV_SCENARIO_FLOATS in include/renv.h.
+constexpr int kScenarioFloats = 32;
+static_assert(sizeof(DrCfg4<float>) <= kScenarioFloats * sizeof(float), "a scenario row holds a DrCfg4<float>");
+struct GridPtrs {
+    const float *scenarios;     // (C, kScenarioFloats) rows, 16-byte aligned
+    uint32_t C;                 // scenarios
+    uint32_t span;              // MLP kernel: C n, a member's flat (scenario, env) index range
+};
+// Row c of a grid's scenarios, in global memory: read through L1 at the fresh start and at resets (the cold path) only.
+template <typename T> __device__ __forceinline__ const DrCfg4<T> &grid_scenario(const GridPtrs &g, uint32_t c)
+{
+    return *reinterpret_cast<const DrCfg4<T> *>(g.scenarios + (size_t)c * kScenarioFloats);
+}
+
 template <typename T, bool kEuler, bool kNoisy = false, bool kRandom = false>
 __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(kNoisy, kRandom))
 cartpole_rollout_kernel(const __grid_constant__ RolloutArgs<T> a)
 {
-    constexpr bool kLog = false, kPop = false;
+    constexpr bool kLog = false, kPop = false, kGrid = false;
     const LogPtrs<T> log = {};
     constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -524,10 +551,11 @@ template <typename T, bool kEuler, bool kRandom>
 __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(false, kRandom))
 cartpole_rollout_logged_kernel(const __grid_constant__ LoggedRolloutArgs<T> args)
 {
-    constexpr bool kNoisy = false, kLog = true, kPop = false;
+    constexpr bool kNoisy = false, kLog = true, kPop = false, kGrid = false;
     const RolloutArgs<T> &a = args.roll;
     const LogPtrs<T> &log = args.log;
     constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -541,10 +569,29 @@ __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<float>(false, fa
 cartpole_population_linear_kernel(const __grid_constant__ PopulationArgs args)
 {
     using T = float;
-    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true;
+    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true, kGrid = false;
     const RolloutArgs<T> &a = args.roll;
     const LogPtrs<T> log = {};
     const PopulationPtrs &pop = args.pop;
+    constexpr GridPtrs grid = {};
+#include "renv_rollout_body.cuh"
+}
+
+struct GridArgs { RolloutArgs<float> roll; PopulationPtrs pop; GridPtrs grid; };     // roll.policy and roll.dr are unused
+
+// P linear policies x C scenarios on the env's n envs: the population kernel with one (policy, scenario, env) triple
+// per thread over the flat index ((p C + c) n + j), so that a robustness map of many scenarios with few envs each
+// still fills the GPU.  pop.total = P C n; a lane takes xi from its scenario row instead of the launch's DR config.
+template <bool kEuler>
+__global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<float>(false, false))
+cartpole_grid_linear_kernel(const __grid_constant__ GridArgs args)
+{
+    using T = float;
+    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true, kGrid = true;
+    const RolloutArgs<T> &a = args.roll;
+    const LogPtrs<T> log = {};
+    const PopulationPtrs &pop = args.pop;
+    const GridPtrs &grid = args.grid;
 #include "renv_rollout_body.cuh"
 }
 

@@ -293,10 +293,11 @@ template <int kAct, bool kEuler, bool kLog>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_rollout_mlp_kernel(const __grid_constant__ MlpRolloutArgs args)
 {
-    constexpr bool kCollect = false, kPop = false;
+    constexpr bool kCollect = false, kPop = false, kGrid = false;
     constexpr MlpTrajPtrs traj = {};
     constexpr bool sample = false;
     constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -321,10 +322,11 @@ template <int kAct, bool kEuler, bool kLog>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_collect_mlp_kernel(const __grid_constant__ MlpCollectArgs args)
 {
-    constexpr bool kCollect = true, kPop = false;
+    constexpr bool kCollect = true, kPop = false, kGrid = false;
     const MlpTrajPtrs &traj = args.traj;
     const bool sample = args.sample != 0;
     constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -343,11 +345,38 @@ template <int kAct, bool kEuler>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_population_mlp_kernel(const __grid_constant__ MlpPopulationArgs pa)
 {
-    constexpr bool kLog = false, kCollect = false, kPop = true;
+    constexpr bool kLog = false, kCollect = false, kPop = true, kGrid = false;
     constexpr MlpTrajPtrs traj = {};
     constexpr bool sample = false;
     const MlpRolloutArgs &args = pa.mlp;
     const PopulationPtrs &pop = pa.pop;
+    constexpr GridPtrs grid = {};
+#include "renv_mlp_rollout_body.cuh"
+}
+
+// ------------------------------------------------------------------------------------------------
+// Evaluation grid: P MLP policies (one activation) x C scenarios, each cell on the env's n envs from a fresh start
+// ------------------------------------------------------------------------------------------------
+struct MlpGridArgs {
+    MlpRolloutArgs mlp;        // mlp.roll.policy, mlp.roll.dr, mlp.params and mlp.log are unused
+    PopulationPtrs pop;        // pop.policies: (P, kMlpParamFloats) rows; pop.ctas = ceil(C n / kMlpThreads)
+    GridPtrs grid;             // grid.span = C n
+};
+
+// The population kernel over a member's flat (scenario, env) range: CTA b stages member b / pop.ctas's parameters and
+// runs 128 consecutive indices of its C n (scenario, env) pairs, each lane with its own scenario row.  P x
+// ceil(C n / 128) CTAs on a 1-D grid; no lane idles whenever C n is a multiple of 128, whatever n (the robustness map:
+// thousands of scenarios with n = 1 .. 32 envs each).
+template <int kAct, bool kEuler>
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
+cartpole_grid_mlp_kernel(const __grid_constant__ MlpGridArgs pa)
+{
+    constexpr bool kLog = false, kCollect = false, kPop = true, kGrid = true;
+    constexpr MlpTrajPtrs traj = {};
+    constexpr bool sample = false;
+    const MlpRolloutArgs &args = pa.mlp;
+    const PopulationPtrs &pop = pa.pop;
+    const GridPtrs &grid = pa.grid;
 #include "renv_mlp_rollout_body.cuh"
 }
 

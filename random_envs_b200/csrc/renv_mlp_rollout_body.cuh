@@ -1,8 +1,8 @@
-// Body of cartpole_rollout_mlp_kernel, cartpole_collect_mlp_kernel and cartpole_population_mlp_kernel
-// (renv_mlp_policy.cuh), included textually into each of these __global__ functions so that the rollout compiles to
-// exactly the code it had before the other kernels existed (an inlined device function would not guarantee that:
-// DESIGN.md section 4.8).  The including function defines
-//     kAct, kEuler, kLog, kCollect, kPop   (template parameters or constexpr)
+// Body of cartpole_rollout_mlp_kernel, cartpole_collect_mlp_kernel, cartpole_population_mlp_kernel and
+// cartpole_grid_mlp_kernel (renv_mlp_policy.cuh), included textually into each of these __global__ functions so that
+// the rollout compiles to exactly the code it had before the other kernels existed (an inlined device function would
+// not guarantee that: DESIGN.md section 4.8).  The including function defines
+//     kAct, kEuler, kLog, kCollect, kPop, kGrid   (template parameters or constexpr)
 //     args     the launch arguments: .roll (RolloutArgs<float>), .params, .log (read only when kLog)
 //     traj     const MlpTrajPtrs &: the per-step record (read only when kCollect)
 //     sample   bool: sample the action from softmax(l0, l1) instead of taking the argmax (read only when kCollect)
@@ -10,6 +10,10 @@
 //                 (b % pop.ctas) * kMlpThreads + threadIdx.x of member b / pop.ctas, whose parameters are row
 //                 b / pop.ctas of pop.policies, from a fresh episode started in registers at tick a.tick - 1; it stores
 //                 nothing into the env and publishes into the member's stats row
+//     kGrid, grid cartpole_grid_mlp_kernel (with kPop; GridPtrs, read only when kGrid): pop.ctas = ceil(C n / 128), and
+//                 the CTA's index i runs over the member's flat (scenario, env) range, i < grid.span = C n: lane i serves
+//                 env j = i % n under scenario c = i / n, whose row replaces a.dr / the env's table, and publishes
+//                 into cell p C + c's stats row by population_publish (a CTA may span several cells)
 // No include guard: included once per kernel.
     __shared__ MlpSmem sm;
     const uint32_t member = kPop ? blockIdx.x / pop.ctas : 0u;
@@ -17,19 +21,24 @@
     const RolloutArgs<float> &a = args.roll;
     const int64_t i = (int64_t)(kPop ? blockIdx.x - member * pop.ctas : blockIdx.x) * blockDim.x + threadIdx.x;
     const int64_t ld = a.env.ld;
-    const bool live = i < a.env.n;
-    const int64_t il = live ? i : 0;
+    const bool live = i < (kGrid ? (int64_t)grid.span : a.env.n);
+    // kGrid: lanes past C n shadow the last scenario (C n < 2^31: 32-bit division)
+    const uint32_t scenario = kGrid ? (uint32_t)(live ? i : grid.span - 1) / (uint32_t)a.env.n : 0u;
+    const int64_t il = kGrid ? (live ? i - (int64_t)scenario * a.env.n : 0) : live ? i : 0;
     const uint64_t id = a.env.env_id0 + (uint64_t)il;
+    const DrCfg4<float> &dr = kGrid ? grid_scenario<float>(grid, scenario) : a.dr;
 
     State<float> s;
     Xi<float> p;
     unsigned fresh_viol = 0;
     if (kPop) {         // renv_cartpole_reset_f32 at tick a.tick - 1, in registers (lanes past n shadow env 0)
         init_state(s, a.env.seed, id, a.tick - 1);
-        if (a.dr.dr_type != kDrNone) {
+        if (draws_xi<kGrid>(dr.dr_type)) {
             p = Xi<float>{ 0.0f, 0.0f, 0.0f, 0.0f };
-            const unsigned v = sample_xi(p, a.dr, a.env.seed, id, a.tick - 1);
+            const unsigned v = sample_xi(p, dr, a.env.seed, id, a.tick - 1);
             fresh_viol = live ? v : 0u;
+        } else if (kGrid) {     // a fixed-task scenario: its task, kept across resets
+            p = Xi<float>{ dr.a[0], dr.a[1], dr.a[2], dr.a[3] };
         } else {
             p = load_xi(a.env.xi, il);
         }
@@ -84,9 +93,9 @@
                         log_count += 1u;
                     }
                     el = 0;
-                    if (a.dr.dr_type != kDrNone) {                         // reset_env: set_random_task, then reset
+                    if (draws_xi<kGrid>(dr.dr_type)) {                     // reset_env: set_random_task, then reset
                         p = Xi<float>{ 0.0f, 0.0f, 0.0f, 0.0f };
-                        viol += sample_xi(p, a.dr, a.env.seed, id, tick);
+                        viol += sample_xi(p, dr, a.env.seed, id, tick);
                         d = derive(p);
                         xi_dirty = true;
                     }
@@ -104,4 +113,9 @@
         if (kLog) args.log.count[i] = (int32_t)log_count;
         if (a.env.episode && episodes) a.env.episode[i] += episodes;      // one started per episode that ended
     }
-    rollout_publish(kPop ? a.stats + 6 * member : a.stats, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
+    if (kGrid) {
+        const int64_t cell = (int64_t)member * grid.C + scenario;
+        population_publish(a.stats + 6 * cell, cell, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
+    } else {
+        rollout_publish(kPop ? a.stats + 6 * member : a.stats, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
+    }

@@ -1,13 +1,17 @@
-// Body of cartpole_rollout_kernel, cartpole_rollout_logged_kernel and cartpole_population_linear_kernel
-// (renv_kernels.cuh), included textually into each of these __global__ functions for the reason given in
-// renv_step_body.cuh.  The including function defines
-//     T, kEuler, kNoisy, kRandom, kLog, kPop   (template parameters or constexpr)
+// Body of cartpole_rollout_kernel, cartpole_rollout_logged_kernel, cartpole_population_linear_kernel and
+// cartpole_grid_linear_kernel (renv_kernels.cuh), included textually into each of these __global__ functions for the
+// reason given in renv_step_body.cuh.  The including function defines
+//     T, kEuler, kNoisy, kRandom, kLog, kPop, kGrid   (template parameters or constexpr)
 //     a    const RolloutArgs<T> &  the launch arguments
 //     log  const LogPtrs<T> &      the episode log (read only when kLog): an ended episode's record is written in the
 //                                  warp's reset pass, before rollout_reset overwrites t.s / t.p / t.el
 //     kPop (constexpr), pop (PopulationPtrs, read only when kPop): cartpole_population_linear_kernel.  Thread i serves
 //          env j = i % n of member i / n (i < pop.total = P n), from a fresh episode started in registers at tick
 //          a.tick - 1, under member's policy row; it stores nothing into the env and publishes into member's stats row.
+//     kGrid (constexpr, with kPop), grid (GridPtrs, read only when kGrid): cartpole_grid_linear_kernel.  pop.total is
+//          P C n and "member" i / n is the cell p C + c: the policy row is p = cell / C, and the lane's xi comes from
+//          scenario row c = cell % C (a DrCfg4<float> image in global memory, read at the fresh start and at resets
+//          only) instead of a.dr / the env's table.  The stats row is the cell's.
 // No include guard: included once per kernel.
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t ld = a.env.ld;
@@ -15,6 +19,9 @@
     // dead lanes of the last warp shadow the last member's env 0 with zero steps to do (P n < 2^31: 32-bit division)
     const int64_t member = kPop ? (int64_t)((uint32_t)(live ? i : pop.total - 1) / (uint32_t)a.env.n) : 0;
     const int64_t il = kPop ? (live ? i - member * a.env.n : 0) : live ? i : 0;
+    // kGrid: member is the cell p C + c (P C n < 2^31: 32-bit division)
+    const uint32_t policy_row = kGrid ? (uint32_t)member / grid.C : (uint32_t)member;
+    const DrCfg4<T> *const scen = kGrid ? &grid_scenario<T>(grid, (uint32_t)member - policy_row * grid.C) : nullptr;
 
     // per-thread episode statistics (return == length here: reward is 1.0 on every step, :207-212)
     RolloutThread<T> t;
@@ -23,10 +30,13 @@
     t.episodes = 0; t.sum_len = 0; t.viol = 0;
     if (kPop) {         // renv_cartpole_reset_f32 at tick a.tick - 1, in registers
         init_state(t.s, a.env.seed, a.env.env_id0 + (uint64_t)il, a.tick - 1);
-        if (a.dr.dr_type != kDrNone) {
+        const DrCfg4<T> &dr = kGrid ? *scen : a.dr;
+        if (draws_xi<kGrid>(dr.dr_type)) {
             t.p = Xi<T>{ T(0), T(0), T(0), T(0) };
-            const unsigned v = sample_xi(t.p, a.dr, a.env.seed, a.env.env_id0 + (uint64_t)il, a.tick - 1);
+            const unsigned v = sample_xi(t.p, dr, a.env.seed, a.env.env_id0 + (uint64_t)il, a.tick - 1);
             t.viol = live ? v : 0u;
+        } else if (kGrid) {     // a fixed-task scenario: its task, kept across resets
+            t.p = Xi<T>{ dr.a[0], dr.a[1], dr.a[2], dr.a[3] };
         } else {
             t.p = load_xi(a.env.xi, il);
         }
@@ -46,7 +56,7 @@
     const int32_t limit = a.max_steps > 0 ? a.max_steps : 0x7fffffff;
     uint32_t log_count = kLog ? (uint32_t)log.count[il] : 0u;    // episode-log records of this env
     t.remaining = live ? a.K : 0;
-    const float *const row = pop.policies + 5 * member;
+    const float *const row = pop.policies + 5 * (kGrid ? (int64_t)policy_row : member);
     const Policy<T> policy = kPop ? Policy<T>{ pin(row[0]), pin(row[1]), pin(row[2]), pin(row[3]), pin(row[4]) }
                                   : Policy<T>{ pin(a.policy.w0), pin(a.policy.w1), pin(a.policy.w2), pin(a.policy.w3), pin(a.policy.b) };
 
@@ -77,7 +87,7 @@
                                 a.tick + (uint64_t)(a.K - t.parked - 1));
                     log_count += 1u;
                 }
-                rollout_reset<T, kRandom>(t, a, id);
+                rollout_reset<T, kRandom, kGrid>(t, a, id, scen);
             }
             continue;                       // revived lanes may still have steps to do
         }

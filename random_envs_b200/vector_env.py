@@ -9,6 +9,7 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     get_task()     -> (N, 4)            set_task(Tensor(N, 4) | g, m_c, m_p, l)
     rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0] or of an MLPPolicy)
     evaluate_population(policies, K) -> (P, 6)   (P policies on common tasks from fresh starts; the env is untouched)
+    evaluate_grid(policies, scenarios, K) -> (P, C, 6)   (the same for each of C task scenarios, in one kernel)
     policy_actions(policy) -> (N,)      (the MLPPolicy's actions for the current observations, ready for step)
     collect(policy, K) -> Trajectory    (K fused steps under the sampled policy, every step recorded for training)
     gae(traj, critic) -> Trajectory     (values, GAE advantages and returns of that trajectory under an MLP critic)
@@ -542,8 +543,56 @@ class RandomCartPoleVecEnv(RandomEnv):
         for ``rollout``.  float32 envs without observation noise only."""
         b = self._alloc()
         t = _device.torch()
+        K, rows, P, kind, policy_args = self._population_rows(policies, num_steps, "evaluate_population()")
+        stats = t.tensor([0.0, 0.0, 0.0, math.inf, -math.inf, 0.0], dtype=t.float64, device=b["device"]).repeat(P, 1)
+        viol = self._violation_counter(b["device"])
+        self._launch("renv_cartpole_population_%s_f32" % kind, ctypes.byref(b["env"]), *policy_args, P, K,
+                     self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(), _device.ptr(stats),
+                     _device.ptr(viol))
+        self._tick += K + 1             # the fresh start at the current tick, then K steps
+        return stats
+
+    def evaluate_grid(self, policies, scenarios, num_steps=MAX_EPISODE_STEPS):
+        """Evaluate P policies on C task scenarios in one kernel: ``policies`` as for ``evaluate_population``,
+        ``scenarios`` a ``Scenarios`` (fixed tasks and / or DR distributions) on the env's device.  Returns a (P, C, 6)
+        float64 device tensor: [p, c] holds the statistics of policy p's finished episodes under scenario c
+        (``distributed.STAT_NAMES``).
+
+        Cell [p, c] equals, bit for bit, ``evaluate_population(policies)[p]`` of a twin of this env (same seed,
+        env_id0, integrator and TimeLimit, and the same step clock) configured with scenario c: for a distribution,
+        ``set_dr_distribution`` with it and ``set_dr_training(True)``; for a fixed task, ``set_task`` with it and no
+        DR.  Every cell sees the same initial states and, under one law, the same draws, so differences between cells
+        come from the policies and the scenarios alone; a cell depends on neither P, C nor its position.  The env's
+        own tasks and DR config are not used, and the env is left untouched except for its step clock, which advances
+        by ``num_steps + 1``.  A gaussian DR failure is raised by the next synchronising call.  float32 envs without
+        observation noise only."""
+        from .scenarios import Scenarios
+        b = self._alloc()
+        t = _device.torch()
+        K, rows, P, kind, policy_args = self._population_rows(policies, num_steps, "evaluate_grid()")
+        if not isinstance(scenarios, Scenarios):
+            raise TypeError("evaluate_grid() takes its scenarios as a Scenarios (Scenarios.tasks / .distributions)")
+        if scenarios.device != b["device"]:
+            raise ValueError("the scenarios live on %s, the env on %s" % (scenarios.device, b["device"]))
+        C = len(scenarios)
+        if P * C * self.num_envs >= 1 << 31:
+            raise ValueError("P * C * num_envs = %d: a grid launch takes fewer than 2^31 (policy, scenario, env) triples"
+                             % (P * C * self.num_envs))
+        stats = t.tensor([0.0, 0.0, 0.0, math.inf, -math.inf, 0.0], dtype=t.float64, device=b["device"]).repeat(P * C, 1)
+        viol = self._violation_counter(b["device"])
+        self._launch("renv_cartpole_grid_%s_f32" % kind, ctypes.byref(b["env"]), *policy_args, P,
+                     _device.ptr(scenarios.rows), C, K, self._integrator(), self.max_episode_steps, self._tick,
+                     _device.ptr(stats), _device.ptr(viol))
+        self._tick += K + 1             # the fresh start at the current tick, then K steps
+        return stats.view(P, C, _lib.NUM_STATS)
+
+    def _population_rows(self, policies, num_steps, what):
+        """The checks ``evaluate_population`` and ``evaluate_grid`` share: (K, rows, P, "linear" | "mlp", the policy
+        arguments of the C entry point before P)."""
+        b = self._buffers
+        t = _device.torch()
         if self._dtype_name != "float32" or self.noisy:
-            raise ValueError("evaluate_population() needs a float32 env without observation noise")
+            raise ValueError("%s needs a float32 env without observation noise" % what)
         K = int(num_steps)
         if K < 1:
             raise ValueError("num_steps must be >= 1, got %d" % K)
@@ -554,24 +603,16 @@ class RandomCartPoleVecEnv(RandomEnv):
                 raise ValueError("linear policies must be a float32 (P, 5) tensor, got %s" % policies.dtype)
             rows, width = policies, 5
         else:
-            raise TypeError("evaluate_population() takes an MLPPopulation or a float32 (P, 5) tensor of linear policies")
+            raise TypeError("%s takes an MLPPopulation or a float32 (P, 5) tensor of linear policies" % what)
         if rows.dim() != 2 or rows.shape[0] < 1 or rows.shape[1] != width or rows.dtype != t.float32:
             raise ValueError("the population must be (P >= 1, %d) float32, got %s %s"
                              % (width, tuple(rows.shape), rows.dtype))
         if rows.device != b["device"]:
             raise ValueError("the population lives on %s, the env on %s" % (rows.device, b["device"]))
         rows = rows.contiguous()
-        P = int(rows.shape[0])
-        stats = t.tensor([0.0, 0.0, 0.0, math.inf, -math.inf, 0.0], dtype=t.float64, device=b["device"]).repeat(P, 1)
         if width == 5:
-            fn, policy_args = "renv_cartpole_population_linear_f32", (_device.ptr(rows), P)
-        else:
-            fn, policy_args = "renv_cartpole_population_mlp_f32", (_device.ptr(rows), policies.activation, P)
-        viol = self._violation_counter(b["device"])
-        self._launch(fn, ctypes.byref(b["env"]), *policy_args, K, self._integrator(), self.max_episode_steps, self._tick,
-                     self._active_dr_cfg(), _device.ptr(stats), _device.ptr(viol))
-        self._tick += K + 1             # the fresh start at the current tick, then K steps
-        return stats
+            return K, rows, int(rows.shape[0]), "linear", (_device.ptr(rows),)
+        return K, rows, int(rows.shape[0]), "mlp", (_device.ptr(rows), policies.activation)
 
     # ---- episode log ----------------------------------------------------------------------------------
     def start_episode_log(self, capacity=1):
