@@ -427,6 +427,56 @@ int renv_cartpole_grid_mlp_f32(const renv_cartpole_env *env, const void *params,
                                const float *scenarios, int C, int K, int integrator, int max_steps, uint64_t tick,
                                double *stats, unsigned long long *violations, void *stream);
 
+/* Per-env task scenarios in the training path: env i has a fixed scenario index of_env[i], and every reset of env i --
+ * in reset, in the auto-reset of a step, or inside a rollout or collect -- takes its task from scenario row c = of_env[i]
+ * (the rows of the evaluation grids above):
+ *   - a row with one of the four laws: xi drawn by the law with Philox (seed, env_id0 + i, tick, purpose 1), exactly as
+ *     a launch with the config the row was packed from draws it;
+ *   - any other row (a fixed task): xi = the row's a[0..3].
+ * So every per-env output of env i -- state, xi, elapsed, episode counters, done / truncated, trajectory rows, logp,
+ * episode-log records -- equals, bit for bit, that of a twin env with the same n, seed, env_id0, integrator, TimeLimit
+ * and clock whose launches pass the row's law as `dr` (a fixed task: dr = NULL, with the task in every xi row).  Env i
+ * depends only on its own row, never on the other envs' assignment or on C.  Several DR distributions (ADR boundary
+ * sampling, curricula, mixtures, an empirical task set) thus train in one batch of one launch.
+ *
+ * The kernels read row min(of_env[i], C - 1), so memory stays in bounds; validating the indices is the caller's job.
+ * Rollout and collect accumulate the finished episodes of the envs of scenario c into stats[c * RENV_NUM_STATS ..], a
+ * (C, RENV_NUM_STATS) array initialised like the plain stats; each row is exact in doubles (integer sums, a min and a
+ * max), whatever the order of the atomics.  fp32 only; `log` may be NULL, otherwise it is checked and written as by the
+ * _logged forms.  Errors, all before any CUDA call: every check of the corresponding plain entry point with its code,
+ * then NULL scen, rows or of_env RENV_E_NULL; C outside [1, 65535] RENV_E_SIZE; misaligned rows or of_env
+ * RENV_E_ALIGN. */
+typedef struct renv_env_scenarios {
+    const float *rows;        /* (C, RENV_SCENARIO_FLOATS) device rows, 16-byte aligned, as renv_scenario_pack_f32 writes them */
+    const uint16_t *of_env;   /* (n) device, 4-byte aligned: the scenario of env i, < C */
+    int32_t C;                /* 1 <= C <= 65535 */
+} renv_env_scenarios;
+
+/* renv_cartpole_reset_f32 with env i's row in place of `dr`. */
+int renv_cartpole_reset_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen, const uint8_t *mask,
+                                 uint64_t tick, unsigned long long *violations, void *stream);
+/* The auto-reset step: the int32 TimeLimit counter when env->elapsed is set, else the uint16 one (max_steps <= 65535);
+ * reward == NULL drops the reward store (with the uint16 counter: the 54-byte step of renv_cartpole_step_lean_f32).
+ * With `log`, the step of renv_cartpole_step_logged_f32.  Only the CTA reset pass reads of_env and the rows. */
+int renv_cartpole_step_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+                                const uint8_t *action, float *reward, uint8_t *done, uint8_t *truncated, int integrator,
+                                int max_steps, uint64_t tick, unsigned long long *counters, void *stream);
+/* renv_cartpole_rollout_f32 (linear policy, or the random policy with w == NULL), statistics per scenario. */
+int renv_cartpole_rollout_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
+                                   const renv_episode_log *log, const double w[4], double b, int K, int integrator,
+                                   int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+                                   void *stream);
+/* renv_cartpole_rollout_mlp_f32, statistics per scenario. */
+int renv_cartpole_rollout_mlp_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
+                                       const renv_episode_log *log, const renv_mlp_policy *p, int K, int integrator,
+                                       int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+                                       void *stream);
+/* renv_cartpole_collect_mlp_f32, statistics per scenario. */
+int renv_cartpole_collect_mlp_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
+                                       const renv_episode_log *log, const renv_mlp_policy *p, const renv_trajectory *traj,
+                                       int sample, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                                       unsigned long long *violations, void *stream);
+
 /* Recorded cart-pole transitions for offline DR fitting (device pointers): transition i is (obs[i], action[i],
  * next_obs[i]), and `window` lists the W start indices t that are scored (t + lam <= T; windows crossing an episode
  * boundary are the caller's to leave out). */

@@ -65,6 +65,11 @@ class Trajectory(ctypes.Structure):
                 ("capacity", ctypes.c_int32)]
 
 
+class EnvScenarios(ctypes.Structure):
+    """struct renv_env_scenarios (include/renv.h)."""
+    _fields_ = [("rows", ctypes.c_void_p), ("of_env", ctypes.c_void_p), ("C", ctypes.c_int32)]
+
+
 class Transitions(ctypes.Structure):
     """struct renv_transitions (include/renv.h)."""
     _fields_ = [("obs", ctypes.c_void_p), ("next_obs", ctypes.c_void_p), ("action", ctypes.c_void_p),
@@ -79,6 +84,7 @@ _log_p = ctypes.POINTER(EpisodeLog)
 _mlp_p = ctypes.POINTER(MlpPolicy)
 _traj_p = ctypes.POINTER(Trajectory)
 _trans_p = ctypes.POINTER(Transitions)
+_scen_p = ctypes.POINTER(EnvScenarios)
 
 # name -> (restype, argtypes); must list every function declared in include/renv.h
 SIGNATURES = {
@@ -116,6 +122,13 @@ SIGNATURES = {
     "renv_scenario_pack_f32": (_int, [_cfg_p, ctypes.POINTER(_dbl), _vp]),
     "renv_cartpole_grid_linear_f32": (_int, [_env_p, _vp, _int, _vp, _int, _int, _int, _int, _u64, _vp, _vp, _vp]),
     "renv_cartpole_grid_mlp_f32": (_int, [_env_p, _vp, _int, _int, _vp, _int, _int, _int, _int, _u64, _vp, _vp, _vp]),
+    "renv_cartpole_reset_scen_f32": (_int, [_env_p, _scen_p, _vp, _u64, _vp, _vp]),
+    "renv_cartpole_step_scen_f32": (_int, [_env_p, _scen_p, _log_p, _vp, _vp, _vp, _vp, _int, _int, _u64, _vp, _vp]),
+    "renv_cartpole_rollout_scen_f32": (_int, [_env_p, _scen_p, _log_p, ctypes.POINTER(_dbl), _dbl, _int, _int, _int, _u64,
+                                              _vp, _vp, _vp]),
+    "renv_cartpole_rollout_mlp_scen_f32": (_int, [_env_p, _scen_p, _log_p, _mlp_p, _int, _int, _int, _u64, _vp, _vp, _vp]),
+    "renv_cartpole_collect_mlp_scen_f32": (_int, [_env_p, _scen_p, _log_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64,
+                                                  _vp, _vp, _vp]),
     "renv_cartpole_transition_loglik_f64": (_int, [_trans_p, _int, _int, _vp, _int, _int, ctypes.POINTER(_dbl), _vp, _vp,
                                                    _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),

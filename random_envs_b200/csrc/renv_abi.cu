@@ -727,6 +727,134 @@ int grid_mlp(const renv_cartpole_env *env, const void *params, int activation, i
     return launch_status();
 }
 
+// The per-env scenarios of the training entry points (include/renv.h renv_env_scenarios), checked after every check
+// of the corresponding plain entry point.
+int check_env_scenarios(const renv_env_scenarios *scen, EnvScenPtrs *out)
+{
+    if (scen == nullptr || scen->rows == nullptr || scen->of_env == nullptr) return RENV_E_NULL;
+    if (scen->C < 1 || scen->C > 65535) return RENV_E_SIZE;
+    if (!aligned(scen->rows, 16) || !aligned(scen->of_env, 4)) return RENV_E_ALIGN;
+    *out = EnvScenPtrs{ scen->rows, scen->of_env, (uint32_t)scen->C };
+    return RENV_OK;
+}
+
+int reset_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const uint8_t *mask, uint64_t tick,
+               unsigned long long *violations, void *stream)
+{
+    ScenResetArgs a;
+    int rc = check_env<float>(env, false, &a.reset.env, kNeedEitherElapsed);
+    if (rc) return rc;
+    if ((rc = to_cfg4<float>(nullptr, &a.reset.dr))) return rc;
+    a.reset.mask = mask;
+    a.reset.tick = tick;
+    a.reset.violations = violations;
+    unsigned blocks = 0;
+    if ((rc = grid_for(env->n, 256, &blocks))) return rc;
+    if ((rc = check_env_scenarios(scen, &a.scen))) return rc;
+    cartpole_scen_reset_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    return launch_status();
+}
+
+// The auto-reset step (renv_cartpole_step_f32 / _lean_f32 / _logged_f32, whichever the env's counter and `log` make
+// it) with per-env scenarios.
+int step_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+              const uint8_t *action, float *reward, uint8_t *done, uint8_t *truncated, int integrator, int max_steps,
+              uint64_t tick, unsigned long long *counters, void *stream)
+{
+    ScenStepArgs sa;
+    StepArgs<float> &a = sa.step;
+    int rc = check_env<float>(env, false, &a.env, kNeedEitherElapsed);
+    if (rc) return rc;
+    sa.log = LogPtrs<float>{};
+    if (log && (rc = check_log<float>(log, &sa.log))) return rc;
+    if (action == nullptr || done == nullptr) return RENV_E_NULL;
+    if (!aligned(action, 4) || !aligned(reward, 16) || !aligned(done, 4) || (truncated && !aligned(truncated, 4)))
+        return RENV_E_ALIGN;
+    if (counters && !aligned(counters, 8)) return RENV_E_ALIGN;
+    if (integrator != RENV_EULER && integrator != RENV_SEMI_IMPLICIT) return RENV_E_INTEGRATOR;
+    const bool lean = env->elapsed == nullptr;          // the uint16 counter
+    if (lean && max_steps > 65535) return RENV_E_SIZE;
+    if ((rc = to_cfg4<float>(nullptr, &a.dr))) return rc;
+    a.action = action; a.reward = reward; a.done = done; a.truncated = truncated;
+    a.euler = integrator == RENV_EULER;
+    a.max_steps = max_steps;
+    a.tick = tick;
+    a.counters = counters;
+    unsigned blocks = 0;
+    if ((rc = grid_for(env->n, (int64_t)kStepThreads * VecTraits<float>::V, &blocks))) return rc;
+    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_flag(lean, [&](auto ln) {
+        with_flag(log != nullptr, [&](auto lg) { rc = launch_pdl(cartpole_scen_step_kernel<ln, lg>, blocks, kStepThreads, st, sa); });
+    });
+    return rc;
+}
+
+int rollout_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+                 const double w[4], double b, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                 unsigned long long *violations, void *stream)
+{
+    ScenRolloutArgs sa;
+    int rc = check_env<float>(env, false, &sa.roll.env, kNeedEitherElapsed);
+    if (rc) return rc;
+    sa.log = LogPtrs<float>{};
+    if (log && (rc = check_log<float>(log, &sa.log))) return rc;
+    if (stats == nullptr) return RENV_E_NULL;
+    const Policy<float> policy = w ? Policy<float>{ (float)w[0], (float)w[1], (float)w[2], (float)w[3], (float)b }
+                                   : Policy<float>{ 0.0f, 0.0f, 0.0f, 0.0f, 0.0f };
+    if ((rc = check_rollout<float>(stats, K, integrator, max_steps, tick, nullptr, violations, policy, &sa.roll))) return rc;
+    if (env->elapsed == nullptr && max_steps > 65535) return RENV_E_SIZE;     // the uint16 counter
+    unsigned blocks = 0;
+    if ((rc = grid_for(env->n, kRolloutThreads, &blocks))) return rc;
+    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_flag(sa.roll.euler, [&](auto euler) {
+        with_flag(w == nullptr, [&](auto random) {
+            with_flag(log != nullptr, [&](auto lg) {
+                cartpole_scen_rollout_kernel<euler, random, lg><<<blocks, kRolloutThreads, 0, st>>>(sa);
+            });
+        });
+    });
+    return launch_status();
+}
+
+int rollout_mlp_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+                     const renv_mlp_policy *p, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                     unsigned long long *violations, void *stream)
+{
+    MlpScenRolloutArgs sa;
+    unsigned blocks = 0;
+    int rc = prepare_rollout_mlp(env, log, log != nullptr, p, K, integrator, max_steps, tick, nullptr, stats, violations,
+                                 &sa.mlp, &blocks);
+    if (rc) return rc;
+    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_mlp_instance(p->activation, sa.mlp.roll.euler, log != nullptr, [&](auto act, auto euler, auto lg) {
+        cartpole_scen_rollout_mlp_kernel<act, euler, lg><<<blocks, kMlpThreads, 0, st>>>(sa);
+    });
+    return launch_status();
+}
+
+int collect_mlp_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+                     const renv_mlp_policy *p, const renv_trajectory *traj, int sample, int K, int integrator,
+                     int max_steps, uint64_t tick, double *stats, unsigned long long *violations, void *stream)
+{
+    MlpScenCollectArgs sa;
+    unsigned blocks = 0;
+    int rc = prepare_rollout_mlp(env, log, log != nullptr, p, K, integrator, max_steps, tick, nullptr, stats, violations,
+                                 &sa.mlp, &blocks);
+    if (rc) return rc;
+    if ((rc = check_traj(traj, K, &sa.mlp.traj))) return rc;
+    if (sample != 0 && sample != 1) return RENV_E_ARG;
+    sa.mlp.sample = sample;
+    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    with_mlp_instance(p->activation, sa.mlp.roll.euler, log != nullptr, [&](auto act, auto euler, auto lg) {
+        cartpole_scen_collect_mlp_kernel<act, euler, lg><<<blocks, kMlpThreads, 0, st>>>(sa);
+    });
+    return launch_status();
+}
+
 int check_transition_loglik(const renv_transitions *data, int lam, int integrator, const double *xi, int C, int M,
                             const double *eps, double *loglik, double *total, LoglikArgs *a, unsigned *blocks)
 {
@@ -984,6 +1112,39 @@ int renv_cartpole_grid_mlp_f32(const renv_cartpole_env *env, const void *params,
                                double *stats, unsigned long long *violations, void *stream)
 {
     return grid_mlp(env, params, activation, P, scenarios, C, K, integrator, max_steps, tick, stats, violations, stream);
+}
+
+int renv_cartpole_reset_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen, const uint8_t *mask,
+                                 uint64_t tick, unsigned long long *violations, void *stream)
+{
+    return reset_scen(env, scen, mask, tick, violations, stream);
+}
+int renv_cartpole_step_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+                                const uint8_t *action, float *reward, uint8_t *done, uint8_t *truncated, int integrator,
+                                int max_steps, uint64_t tick, unsigned long long *counters, void *stream)
+{
+    return step_scen(env, scen, log, action, reward, done, truncated, integrator, max_steps, tick, counters, stream);
+}
+int renv_cartpole_rollout_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
+                                   const renv_episode_log *log, const double w[4], double b, int K, int integrator,
+                                   int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+                                   void *stream)
+{
+    return rollout_scen(env, scen, log, w, b, K, integrator, max_steps, tick, stats, violations, stream);
+}
+int renv_cartpole_rollout_mlp_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
+                                       const renv_episode_log *log, const renv_mlp_policy *p, int K, int integrator,
+                                       int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+                                       void *stream)
+{
+    return rollout_mlp_scen(env, scen, log, p, K, integrator, max_steps, tick, stats, violations, stream);
+}
+int renv_cartpole_collect_mlp_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
+                                       const renv_episode_log *log, const renv_mlp_policy *p, const renv_trajectory *traj,
+                                       int sample, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                                       unsigned long long *violations, void *stream)
+{
+    return collect_mlp_scen(env, scen, log, p, traj, sample, K, integrator, max_steps, tick, stats, violations, stream);
 }
 
 int renv_cartpole_transition_loglik_f64(const renv_transitions *data, int lam, int integrator, const double *xi, int C,

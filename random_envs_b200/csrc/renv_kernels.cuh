@@ -86,8 +86,37 @@ template <typename T> __device__ __forceinline__ void store_elapsed(const EnvPtr
     else env.elapsed16[i] = (uint16_t)el;
 }
 
-// RandomCartPoleEnv.reset (+ set_random_task) of env i at clock `tick`; scalar stores.
-template <typename T>
+// Whether a reset draws xi from `dr`: any active DR config of a launch; for a scenario row (kGrid: an evaluation grid's,
+// or a training env's) one of the four laws only, any other dr_type being a fixed task.
+template <bool kGrid> __device__ __forceinline__ bool draws_xi(int dr_type)
+{
+    return kGrid ? (unsigned)(dr_type - kDrUniform) <= (unsigned)(kDrFullGaussian - kDrUniform) : dr_type != kDrNone;
+}
+
+// A scenario row (include/renv.h RENV_SCENARIO_FLOATS): kScenarioFloats floats holding the DrCfg4<float> image of a DR
+// config, or of a fixed task (dr_type none, a = the task).
+constexpr int kScenarioFloats = 32;
+static_assert(sizeof(DrCfg4<float>) <= kScenarioFloats * sizeof(float), "a scenario row holds a DrCfg4<float>");
+template <typename T> __device__ __forceinline__ const DrCfg4<T> &scenario_row(const float *rows, uint32_t c)
+{
+    return *reinterpret_cast<const DrCfg4<T> *>(rows + (size_t)c * kScenarioFloats);
+}
+
+// Per-env scenarios of the training path (include/renv.h renv_env_scenarios): every reset of env i draws from row
+// env_scenario(sc, i).  The index is clamped so that a bad one stays inside the rows; validating it is the caller's job.
+struct EnvScenPtrs {
+    const float *rows;          // (C, kScenarioFloats), 16-byte aligned
+    const uint16_t *of_env;     // (n): the scenario of env i
+    uint32_t C;
+};
+__device__ __forceinline__ uint32_t env_scenario(const EnvScenPtrs &sc, int64_t i)
+{
+    return min((uint32_t)sc.of_env[i], sc.C - 1u);
+}
+
+// RandomCartPoleEnv.reset (+ set_random_task) of env i at clock `tick`; scalar stores.  kScen: `dr` is env i's scenario
+// row, and a fixed-task row writes its task into xi.
+template <typename T, bool kScen = false>
 __device__ __forceinline__ unsigned reset_env(const EnvPtrs<T> &env, const DrCfg4<T> &dr, int64_t i, uint64_t tick, uint64_t seed)
 {
     const int64_t ld = env.ld;
@@ -102,10 +131,12 @@ __device__ __forceinline__ unsigned reset_env(const EnvPtrs<T> &env, const DrCfg
         env.obs[0 * ld + i] = o[0]; env.obs[1 * ld + i] = o[1]; env.obs[2 * ld + i] = o[2]; env.obs[3 * ld + i] = o[3];
     }
     unsigned viol = 0;
-    if (dr.dr_type != kDrNone) {
+    if (draws_xi<kScen>(dr.dr_type)) {
         Xi<T> xi = { T(0), T(0), T(0), T(0) };
         viol = sample_xi(xi, dr, seed, id, tick);
         store_xi(env.xi, i, xi);
+    } else if (kScen) {
+        store_xi(env.xi, i, Xi<T>{ dr.a[0], dr.a[1], dr.a[2], dr.a[3] });
     }
     if (env.episode) atomicAdd(env.episode + i, 1u);      // optional episode count: fire-and-forget RED, no load stall
     return viol;
@@ -216,8 +247,9 @@ template <typename T> constexpr int kStepMinCtas = sizeof(T) == 4 ? 4 : 3;     /
 template <typename T, bool kAutoReset, bool kNoisy = false, bool kLean = false>
 __global__ void __launch_bounds__(kStepThreads, kNoisy ? (sizeof(T) == 8 ? 2 : 3) : kStepMinCtas<T>) cartpole_step_kernel(const __grid_constant__ StepArgs<T> a)
 {
-    constexpr bool kLog = false;
+    constexpr bool kLog = false, kScen = false;
     const LogPtrs<T> log = {};
+    constexpr EnvScenPtrs env_scen = {};
 #include "renv_step_body.cuh"
 }
 
@@ -230,10 +262,28 @@ template <typename T> struct LoggedStepArgs { StepArgs<T> step; LogPtrs<T> log; 
 template <typename T>
 __global__ void __launch_bounds__(kStepThreads, kStepMinCtas<T>) cartpole_step_logged_kernel(const __grid_constant__ LoggedStepArgs<T> args)
 {
-    constexpr bool kAutoReset = true, kNoisy = false, kLog = true;
+    constexpr bool kAutoReset = true, kNoisy = false, kLog = true, kScen = false;
     const bool kLean = sizeof(T) == 4 && args.step.env.elapsed == nullptr;
     const StepArgs<T> &a = args.step;
     const LogPtrs<T> &log = args.log;
+    constexpr EnvScenPtrs env_scen = {};
+#include "renv_step_body.cuh"
+}
+
+struct ScenStepArgs { StepArgs<float> step; LogPtrs<float> log; EnvScenPtrs scen; };     // step.dr is unused
+
+// The fp32 auto-reset step with per-env scenarios (renv_cartpole_step_scen_f32): the plain step body, whose CTA reset
+// pass reads env i's scenario index and row for each env it resets -- nothing else changes, so the streamed bytes are
+// those of the plain step.  kLean: the uint16 counter (a.reward == nullptr drops the reward store in either layout);
+// kLog: the episode log, as in cartpole_step_logged_kernel.
+template <bool kLean, bool kLog>
+__global__ void __launch_bounds__(kStepThreads, kStepMinCtas<float>) cartpole_scen_step_kernel(const __grid_constant__ ScenStepArgs args)
+{
+    using T = float;
+    constexpr bool kAutoReset = true, kNoisy = false, kScen = true;
+    const StepArgs<T> &a = args.step;
+    const LogPtrs<T> &log = args.log;
+    const EnvScenPtrs &env_scen = args.scen;
 #include "renv_step_body.cuh"
 }
 
@@ -257,6 +307,23 @@ template <typename T> __global__ void __launch_bounds__(256) cartpole_reset_kern
     if (a.env.elapsed16) a.env.elapsed16[i] = 0;
     if (a.env.beyond) a.env.beyond[i] = -1;
     const unsigned viol = reset_env(a.env, a.dr, i, a.tick, a.env.seed);
+    if (viol && a.violations) atomicAdd(a.violations, (unsigned long long)viol);
+}
+
+struct ScenResetArgs { ResetArgs<float> reset; EnvScenPtrs scen; };     // reset.dr is unused
+
+// cartpole_reset_kernel with env i's scenario row in place of the launch's DR config (renv_cartpole_reset_scen_f32).
+__global__ void __launch_bounds__(256) cartpole_scen_reset_kernel(const __grid_constant__ ScenResetArgs args)
+{
+    const ResetArgs<float> &a = args.reset;
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.env.n) return;
+    if (a.mask && !a.mask[i]) return;
+    if (a.env.elapsed) a.env.elapsed[i] = 0;
+    if (a.env.elapsed16) a.env.elapsed16[i] = 0;
+    if (a.env.beyond) a.env.beyond[i] = -1;
+    const DrCfg4<float> &row = scenario_row<float>(args.scen.rows, env_scenario(args.scen, i));
+    const unsigned viol = reset_env<float, true>(a.env, row, i, a.tick, a.env.seed);
     if (viol && a.violations) atomicAdd(a.violations, (unsigned long long)viol);
 }
 
@@ -366,6 +433,52 @@ __device__ __forceinline__ void population_publish(double *stats, int64_t member
     if (viol && violations) atomicAdd(violations, (unsigned long long)viol);
 }
 
+// Statistics of a per-env scenario launch (cartpole_scen_*), whose CTAs may serve any of C scenarios in any pattern:
+// publishing per lane sends up to one set of six double atomics per lane into a few rows, and the CAS loops of min / max
+// serialise on them (measured: the random-policy rollout at half its rate).  With C <= kScenSmemRows the CTA reduces
+// into a shared table first -- integer atomics, exact: returns and lengths are integers -- and one thread per row
+// publishes it; beyond that each lane publishes by population_publish.  Every thread of the CTA must call it.  Out of
+// line: it runs once per thread, and inline it cost the random-policy logged rollout a spill.
+constexpr int kScenSmemRows = 64;
+struct ScenStatsRow { unsigned long long episodes, sum_len, sum_r, sum_r2; unsigned min_r, max_r; };
+__device__ __noinline__ void scenario_publish(double *stats, uint32_t C, uint32_t c, unsigned long long *violations,
+                                                 unsigned episodes, unsigned sum_len, unsigned sum_r_u,
+                                                 unsigned long long sum_r2_u, float min_r, float max_r, unsigned viol)
+{
+    if (C > (uint32_t)kScenSmemRows) {          // uniform: C is a launch argument
+        population_publish(stats + 6 * (int64_t)c, c, violations, episodes, sum_len, sum_r_u, sum_r2_u, min_r, max_r, viol);
+        return;
+    }
+    __shared__ ScenStatsRow tab[kScenSmemRows];
+    __shared__ unsigned tab_viol;
+    for (uint32_t r = threadIdx.x; r < C; r += blockDim.x) tab[r] = ScenStatsRow{ 0ull, 0ull, 0ull, 0ull, 0xffffffffu, 0u };
+    if (threadIdx.x == 0) tab_viol = 0u;
+    __syncthreads();
+    if (episodes) {
+        atomicAdd(&tab[c].episodes, (unsigned long long)episodes);
+        atomicAdd(&tab[c].sum_len, (unsigned long long)sum_len);
+        atomicAdd(&tab[c].sum_r, (unsigned long long)sum_r_u);
+        atomicAdd(&tab[c].sum_r2, sum_r2_u);
+        atomicMin(&tab[c].min_r, (unsigned)min_r);
+        atomicMax(&tab[c].max_r, (unsigned)max_r);
+    }
+    if (viol) atomicAdd(&tab_viol, viol);
+    __syncthreads();
+    for (uint32_t r = threadIdx.x; r < C; r += blockDim.x) {
+        const ScenStatsRow e = tab[r];
+        if (e.episodes) {
+            double *row = stats + 6 * (size_t)r;
+            atomicAdd(row + 0, (double)e.episodes);
+            atomicAdd(row + 1, (double)e.sum_r);
+            atomicAdd(row + 2, (double)e.sum_r2);
+            atomic_min_f64(row + 3, (double)e.min_r);
+            atomic_max_f64(row + 4, (double)e.max_r);
+            atomicAdd(row + 5, (double)e.sum_len);
+        }
+    }
+    if (threadIdx.x == 0 && tab_viol && violations) atomicAdd(violations, (unsigned long long)tab_viol);
+}
+
 template <typename T> struct RolloutArgs {
     EnvPtrs<T> env;
     Policy<T> policy;
@@ -459,15 +572,9 @@ __device__ __forceinline__ void rollout_step(RolloutThread<T> &t, const RolloutA
     t.remaining = park ? 0 : t.remaining - 1;
 }
 
-// Whether a reset draws xi from `dr`: any active DR config of a launch; for a grid scenario row (kGrid) one of the four
-// laws only, any other dr_type being a fixed task that the env keeps across resets.
-template <bool kGrid> __device__ __forceinline__ bool draws_xi(int dr_type)
-{
-    return kGrid ? (unsigned)(dr_type - kDrUniform) <= (unsigned)(kDrFullGaussian - kDrUniform) : dr_type != kDrNone;
-}
-
-// A grid launch (kGrid) passes the lane's scenario row `scen`, which replaces a.dr.
-template <typename T, bool kRandom = false, bool kGrid = false>
+// A grid launch (kGrid) or a per-env scenario launch (kScen) passes the lane's scenario row `scen`, which replaces
+// a.dr.  A grid lane keeps a fixed task across resets (it took it at its fresh start); a kScen lane takes it here.
+template <typename T, bool kRandom = false, bool kGrid = false, bool kScen = false>
 __device__ __forceinline__ void rollout_reset(RolloutThread<T> &t, const RolloutArgs<T> &a, uint64_t id,
                                               const DrCfg4<T> *scen = nullptr)
 {
@@ -480,10 +587,14 @@ __device__ __forceinline__ void rollout_reset(RolloutThread<T> &t, const Rollout
         t.new_episodes += 1; t.el = 0;
         // the clock value a single step() would have used for the step that ended it: t.parked steps were left after it
         const uint64_t reset_tick = a.tick + (uint64_t)(a.K - t.parked - 1);
-        const DrCfg4<T> &dr = kGrid ? *scen : a.dr;
-        if (draws_xi<kGrid>(dr.dr_type)) {
+        const DrCfg4<T> &dr = kGrid || kScen ? *scen : a.dr;
+        if (draws_xi<kGrid || kScen>(dr.dr_type)) {
             t.p = Xi<T>{ T(0), T(0), T(0), T(0) };
             t.viol += sample_xi(t.p, dr, a.env.seed, id, reset_tick);
+            t.d = derive(t.p);
+            t.xi_dirty = true;
+        } else if (kScen) {
+            t.p = Xi<T>{ dr.a[0], dr.a[1], dr.a[2], dr.a[3] };
             t.d = derive(t.p);
             t.xi_dirty = true;
         }
@@ -520,8 +631,6 @@ struct PopulationPtrs {
 // A grid launch (renv_cartpole_grid_*_f32): P policies x C scenarios, each cell (p, c) on the env's n envs from a fresh
 // start.  Scenario row c is kScenarioFloats floats holding the DrCfg4<float> image of its DR config, or of a fixed task
 // (dr_type none, a = the task): the layout of RENV_SCENARIO_FLOATS in include/renv.h.
-constexpr int kScenarioFloats = 32;
-static_assert(sizeof(DrCfg4<float>) <= kScenarioFloats * sizeof(float), "a scenario row holds a DrCfg4<float>");
 struct GridPtrs {
     const float *scenarios;     // (C, kScenarioFloats) rows, 16-byte aligned
     uint32_t C;                 // scenarios
@@ -530,17 +639,18 @@ struct GridPtrs {
 // Row c of a grid's scenarios, in global memory: read through L1 at the fresh start and at resets (the cold path) only.
 template <typename T> __device__ __forceinline__ const DrCfg4<T> &grid_scenario(const GridPtrs &g, uint32_t c)
 {
-    return *reinterpret_cast<const DrCfg4<T> *>(g.scenarios + (size_t)c * kScenarioFloats);
+    return scenario_row<T>(g.scenarios, c);
 }
 
 template <typename T, bool kEuler, bool kNoisy = false, bool kRandom = false>
 __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(kNoisy, kRandom))
 cartpole_rollout_kernel(const __grid_constant__ RolloutArgs<T> a)
 {
-    constexpr bool kLog = false, kPop = false, kGrid = false;
+    constexpr bool kLog = false, kPop = false, kGrid = false, kScen = false;
     const LogPtrs<T> log = {};
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -551,11 +661,12 @@ template <typename T, bool kEuler, bool kRandom>
 __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<T>(false, kRandom))
 cartpole_rollout_logged_kernel(const __grid_constant__ LoggedRolloutArgs<T> args)
 {
-    constexpr bool kNoisy = false, kLog = true, kPop = false, kGrid = false;
+    constexpr bool kNoisy = false, kLog = true, kPop = false, kGrid = false, kScen = false;
     const RolloutArgs<T> &a = args.roll;
     const LogPtrs<T> &log = args.log;
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -569,11 +680,12 @@ __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<float>(false, fa
 cartpole_population_linear_kernel(const __grid_constant__ PopulationArgs args)
 {
     using T = float;
-    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true, kGrid = false;
+    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true, kGrid = false, kScen = false;
     const RolloutArgs<T> &a = args.roll;
     const LogPtrs<T> log = {};
     const PopulationPtrs &pop = args.pop;
     constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -587,11 +699,32 @@ __global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<float>(false, fa
 cartpole_grid_linear_kernel(const __grid_constant__ GridArgs args)
 {
     using T = float;
-    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true, kGrid = true;
+    constexpr bool kNoisy = false, kRandom = false, kLog = false, kPop = true, kGrid = true, kScen = false;
     const RolloutArgs<T> &a = args.roll;
     const LogPtrs<T> log = {};
     const PopulationPtrs &pop = args.pop;
     const GridPtrs &grid = args.grid;
+    constexpr EnvScenPtrs env_scen = {};
+#include "renv_rollout_body.cuh"
+}
+
+struct ScenRolloutArgs { RolloutArgs<float> roll; LogPtrs<float> log; EnvScenPtrs scen; };     // roll.dr is unused
+
+// The fp32 linear-policy (kRandom: random-policy) rollout with per-env scenarios (renv_cartpole_rollout_scen_f32): the
+// generic one-env-per-thread body, whose lanes take their scenario row at every reset and publish their episodes into
+// their scenario's statistics row.  (The FFMA2 pair kernel parks ended envs through the env's buffers and resets them
+// in a pass of its own; it has no per-lane row to read.)
+template <bool kEuler, bool kRandom, bool kLog>
+__global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<float>(false, kRandom))
+cartpole_scen_rollout_kernel(const __grid_constant__ ScenRolloutArgs args)
+{
+    using T = float;
+    constexpr bool kNoisy = false, kPop = false, kGrid = false, kScen = true;
+    const RolloutArgs<T> &a = args.roll;
+    const LogPtrs<T> &log = args.log;
+    constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
+    const EnvScenPtrs &env_scen = args.scen;
 #include "renv_rollout_body.cuh"
 }
 

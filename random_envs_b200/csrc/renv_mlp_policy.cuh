@@ -293,11 +293,12 @@ template <int kAct, bool kEuler, bool kLog>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_rollout_mlp_kernel(const __grid_constant__ MlpRolloutArgs args)
 {
-    constexpr bool kCollect = false, kPop = false, kGrid = false;
+    constexpr bool kCollect = false, kPop = false, kGrid = false, kScen = false;
     constexpr MlpTrajPtrs traj = {};
     constexpr bool sample = false;
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -322,11 +323,12 @@ template <int kAct, bool kEuler, bool kLog>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_collect_mlp_kernel(const __grid_constant__ MlpCollectArgs args)
 {
-    constexpr bool kCollect = true, kPop = false, kGrid = false;
+    constexpr bool kCollect = true, kPop = false, kGrid = false, kScen = false;
     const MlpTrajPtrs &traj = args.traj;
     const bool sample = args.sample != 0;
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -345,12 +347,13 @@ template <int kAct, bool kEuler>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_population_mlp_kernel(const __grid_constant__ MlpPopulationArgs pa)
 {
-    constexpr bool kLog = false, kCollect = false, kPop = true, kGrid = false;
+    constexpr bool kLog = false, kCollect = false, kPop = true, kGrid = false, kScen = false;
     constexpr MlpTrajPtrs traj = {};
     constexpr bool sample = false;
     const MlpRolloutArgs &args = pa.mlp;
     const PopulationPtrs &pop = pa.pop;
     constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -371,12 +374,50 @@ template <int kAct, bool kEuler>
 __global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
 cartpole_grid_mlp_kernel(const __grid_constant__ MlpGridArgs pa)
 {
-    constexpr bool kLog = false, kCollect = false, kPop = true, kGrid = true;
+    constexpr bool kLog = false, kCollect = false, kPop = true, kGrid = true, kScen = false;
     constexpr MlpTrajPtrs traj = {};
     constexpr bool sample = false;
     const MlpRolloutArgs &args = pa.mlp;
     const PopulationPtrs &pop = pa.pop;
     const GridPtrs &grid = pa.grid;
+    constexpr EnvScenPtrs env_scen = {};
+#include "renv_mlp_rollout_body.cuh"
+}
+
+// ------------------------------------------------------------------------------------------------
+// Per-env task scenarios: the MLP rollout and collection with env i resetting from its own scenario row
+// ------------------------------------------------------------------------------------------------
+struct MlpScenRolloutArgs { MlpRolloutArgs mlp; EnvScenPtrs scen; };     // mlp.roll.dr is unused
+struct MlpScenCollectArgs { MlpCollectArgs mlp; EnvScenPtrs scen; };     // mlp.roll.dr is unused
+
+// cartpole_rollout_mlp_kernel / cartpole_collect_mlp_kernel (the same body) with per-env scenarios
+// (renv_cartpole_rollout_mlp_scen_f32 / renv_cartpole_collect_mlp_scen_f32): a lane reads its env's scenario index at
+// kernel start and the row at its resets; its episodes go to the scenario's statistics row.
+template <int kAct, bool kEuler, bool kLog>
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
+cartpole_scen_rollout_mlp_kernel(const __grid_constant__ MlpScenRolloutArgs sa)
+{
+    constexpr bool kCollect = false, kPop = false, kGrid = false, kScen = true;
+    constexpr MlpTrajPtrs traj = {};
+    constexpr bool sample = false;
+    const MlpRolloutArgs &args = sa.mlp;
+    constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
+    const EnvScenPtrs &env_scen = sa.scen;
+#include "renv_mlp_rollout_body.cuh"
+}
+
+template <int kAct, bool kEuler, bool kLog>
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
+cartpole_scen_collect_mlp_kernel(const __grid_constant__ MlpScenCollectArgs sa)
+{
+    constexpr bool kCollect = true, kPop = false, kGrid = false, kScen = true;
+    const MlpCollectArgs &args = sa.mlp;
+    const MlpTrajPtrs &traj = args.traj;
+    const bool sample = args.sample != 0;
+    constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
+    const EnvScenPtrs &env_scen = sa.scen;
 #include "renv_mlp_rollout_body.cuh"
 }
 

@@ -1,8 +1,9 @@
-// Body of cartpole_rollout_mlp_kernel, cartpole_collect_mlp_kernel, cartpole_population_mlp_kernel and
-// cartpole_grid_mlp_kernel (renv_mlp_policy.cuh), included textually into each of these __global__ functions so that
-// the rollout compiles to exactly the code it had before the other kernels existed (an inlined device function would
-// not guarantee that: DESIGN.md section 4.8).  The including function defines
-//     kAct, kEuler, kLog, kCollect, kPop, kGrid   (template parameters or constexpr)
+// Body of cartpole_rollout_mlp_kernel, cartpole_collect_mlp_kernel, cartpole_population_mlp_kernel,
+// cartpole_grid_mlp_kernel, cartpole_scen_rollout_mlp_kernel and cartpole_scen_collect_mlp_kernel (renv_mlp_policy.cuh),
+// included textually into each of these __global__ functions so that the rollout compiles to exactly the code it had
+// before the other kernels existed (an inlined device function would not guarantee that: DESIGN.md section 4.8).  The
+// including function defines
+//     kAct, kEuler, kLog, kCollect, kPop, kGrid, kScen   (template parameters or constexpr)
 //     args     the launch arguments: .roll (RolloutArgs<float>), .params, .log (read only when kLog)
 //     traj     const MlpTrajPtrs &: the per-step record (read only when kCollect)
 //     sample   bool: sample the action from softmax(l0, l1) instead of taking the argmax (read only when kCollect)
@@ -14,6 +15,9 @@
 //                 the CTA's index i runs over the member's flat (scenario, env) range, i < grid.span = C n: lane i serves
 //                 env j = i % n under scenario c = i / n, whose row replaces a.dr / the env's table, and publishes
 //                 into cell p C + c's stats row by population_publish (a CTA may span several cells)
+//     kScen, env_scen  the per-env scenario kernels (EnvScenPtrs, read only when kScen): lane i reads env i's scenario
+//                 index once here and its row (global memory) at resets only; the row replaces a.dr, a fixed-task row's
+//                 task replaces the env's xi at each reset, and statistics go to the scenario's row (scenario_publish)
 // No include guard: included once per kernel.
     __shared__ MlpSmem sm;
     const uint32_t member = kPop ? blockIdx.x / pop.ctas : 0u;
@@ -23,10 +27,12 @@
     const int64_t ld = a.env.ld;
     const bool live = i < (kGrid ? (int64_t)grid.span : a.env.n);
     // kGrid: lanes past C n shadow the last scenario (C n < 2^31: 32-bit division)
-    const uint32_t scenario = kGrid ? (uint32_t)(live ? i : grid.span - 1) / (uint32_t)a.env.n : 0u;
-    const int64_t il = kGrid ? (live ? i - (int64_t)scenario * a.env.n : 0) : live ? i : 0;
+    const uint32_t grid_scenario_of = kGrid ? (uint32_t)(live ? i : grid.span - 1) / (uint32_t)a.env.n : 0u;
+    const int64_t il = kGrid ? (live ? i - (int64_t)grid_scenario_of * a.env.n : 0) : live ? i : 0;
+    const uint32_t scenario = kScen ? env_scenario(env_scen, il) : grid_scenario_of;
     const uint64_t id = a.env.env_id0 + (uint64_t)il;
-    const DrCfg4<float> &dr = kGrid ? grid_scenario<float>(grid, scenario) : a.dr;
+    const DrCfg4<float> &dr = kGrid ? grid_scenario<float>(grid, scenario)
+                            : kScen ? scenario_row<float>(env_scen.rows, scenario) : a.dr;
 
     State<float> s;
     Xi<float> p;
@@ -93,9 +99,13 @@
                         log_count += 1u;
                     }
                     el = 0;
-                    if (draws_xi<kGrid>(dr.dr_type)) {                     // reset_env: set_random_task, then reset
+                    if (draws_xi<kGrid || kScen>(dr.dr_type)) {            // reset_env: set_random_task, then reset
                         p = Xi<float>{ 0.0f, 0.0f, 0.0f, 0.0f };
                         viol += sample_xi(p, dr, a.env.seed, id, tick);
+                        d = derive(p);
+                        xi_dirty = true;
+                    } else if (kScen) {                                    // a fixed-task row: its task
+                        p = Xi<float>{ dr.a[0], dr.a[1], dr.a[2], dr.a[3] };
                         d = derive(p);
                         xi_dirty = true;
                     }
@@ -116,6 +126,8 @@
     if (kGrid) {
         const int64_t cell = (int64_t)member * grid.C + scenario;
         population_publish(a.stats + 6 * cell, cell, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
+    } else if (kScen) {
+        scenario_publish(a.stats, env_scen.C, scenario, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
     } else {
         rollout_publish(kPop ? a.stats + 6 * member : a.stats, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
     }

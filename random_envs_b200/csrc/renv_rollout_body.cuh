@@ -1,7 +1,7 @@
-// Body of cartpole_rollout_kernel, cartpole_rollout_logged_kernel, cartpole_population_linear_kernel and
-// cartpole_grid_linear_kernel (renv_kernels.cuh), included textually into each of these __global__ functions for the
-// reason given in renv_step_body.cuh.  The including function defines
-//     T, kEuler, kNoisy, kRandom, kLog, kPop, kGrid   (template parameters or constexpr)
+// Body of cartpole_rollout_kernel, cartpole_rollout_logged_kernel, cartpole_population_linear_kernel,
+// cartpole_grid_linear_kernel and cartpole_scen_rollout_kernel (renv_kernels.cuh), included textually into each of these
+// __global__ functions for the reason given in renv_step_body.cuh.  The including function defines
+//     T, kEuler, kNoisy, kRandom, kLog, kPop, kGrid, kScen   (template parameters or constexpr)
 //     a    const RolloutArgs<T> &  the launch arguments
 //     log  const LogPtrs<T> &      the episode log (read only when kLog): an ended episode's record is written in the
 //                                  warp's reset pass, before rollout_reset overwrites t.s / t.p / t.el
@@ -12,6 +12,9 @@
 //          P C n and "member" i / n is the cell p C + c: the policy row is p = cell / C, and the lane's xi comes from
 //          scenario row c = cell % C (a DrCfg4<float> image in global memory, read at the fresh start and at resets
 //          only) instead of a.dr / the env's table.  The stats row is the cell's.
+//     kScen (constexpr), env_scen (EnvScenPtrs, read only when kScen): cartpole_scen_rollout_kernel.  Env i reads its
+//          scenario index once here and its row (in global memory) at resets only: the row replaces a.dr, and a
+//          fixed-task row's task replaces the env's xi at each reset.  Statistics go to the scenario's row (scenario_publish).
 // No include guard: included once per kernel.
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t ld = a.env.ld;
@@ -22,6 +25,7 @@
     // kGrid: member is the cell p C + c (P C n < 2^31: 32-bit division)
     const uint32_t policy_row = kGrid ? (uint32_t)member / grid.C : (uint32_t)member;
     const DrCfg4<T> *const scen = kGrid ? &grid_scenario<T>(grid, (uint32_t)member - policy_row * grid.C) : nullptr;
+    const uint32_t scenario = kScen ? env_scenario(env_scen, il) : 0u;     // kScen: its row is found at each reset
 
     // per-thread episode statistics (return == length here: reward is 1.0 on every step, :207-212)
     RolloutThread<T> t;
@@ -87,7 +91,8 @@
                                 a.tick + (uint64_t)(a.K - t.parked - 1));
                     log_count += 1u;
                 }
-                rollout_reset<T, kRandom, kGrid>(t, a, id, scen);
+                rollout_reset<T, kRandom, kGrid, kScen>(t, a, id,
+                                                        kScen ? &scenario_row<T>(env_scen.rows, scenario) : scen);
             }
             continue;                       // revived lanes may still have steps to do
         }
@@ -107,7 +112,10 @@
             a.env.obs[i] = ov[0]; a.env.obs[ld + i] = ov[1]; a.env.obs[2 * ld + i] = ov[2]; a.env.obs[3 * ld + i] = ov[3];
         }
     }
-    if (kPop)
+    if (kScen)
+        scenario_publish(a.stats, env_scen.C, scenario, a.violations, t.episodes, t.sum_len, t.sum_r, t.sum_r2, t.min_r,
+                         t.max_r, t.viol);
+    else if (kPop)
         population_publish(a.stats + 6 * member, member, a.violations, t.episodes, t.sum_len, t.sum_r, t.sum_r2, t.min_r,
                            t.max_r, t.viol);
     else

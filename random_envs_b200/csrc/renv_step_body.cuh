@@ -1,15 +1,19 @@
-// Body of cartpole_step_kernel and cartpole_step_logged_kernel (renv_kernels.cuh), included textually into both
-// __global__ functions rather than called as an inlined device function: an inlined body schedules the plain kernels'
-// code differently, and the plain kernels must stay exactly what they were.  The including function defines
-//     T, kAutoReset, kNoisy, kLean, kLog       (template parameters or constexpr; kLean is a per-launch constant in
-//                                             the logged kernel)
+// Body of cartpole_step_kernel, cartpole_step_logged_kernel and cartpole_scen_step_kernel (renv_kernels.cuh), included
+// textually into each __global__ function rather than called as an inlined device function: an inlined body schedules
+// the plain kernels' code differently, and the plain kernels must stay exactly what they were.  The including function
+// defines
+//     T, kAutoReset, kNoisy, kLean, kLog, kScen   (template parameters or constexpr; kLean is a per-launch constant
+//                                                in the logged kernel)
 //     a    const StepArgs<T> &    the launch arguments
 //     log  const LogPtrs<T> &     the episode log (read only when kLog)
+//     env_scen  const EnvScenPtrs &  per-env scenarios (read only when kScen): the reset pass takes env i's row in
+//                                    place of a.dr
 // No include guard: included once per kernel.
     using VT = VecTraits<T>;
     constexpr int V = VT::V;
     constexpr int kTile = kStepThreads * V;
     __shared__ unsigned s_count;
+    __shared__ uint32_t s_ticket;                          // kScen: the ticket waits here across the reset pass
     __shared__ uint16_t s_list[kAutoReset ? kTile : 1];
     __shared__ int32_t s_len[kLog ? kTile : 1];          // length of the ended episode, negated when truncated
     const int64_t block0 = (int64_t)blockIdx.x * kTile;
@@ -30,6 +34,7 @@
                 seen = ld_acquire_gpu(slot + 1);
             }
             if (seen != ticket && a.counters) atomicAdd(a.counters + kCounterOrderTimeout, 1ull);
+            if (kScen) s_ticket = ticket;
             if (kAutoReset) s_count = 0;
         } else if (block0 + kTile <= n && threadIdx.x >= 32 && threadIdx.x < 39) {
             // while thread 0 waits for its L2 round trip the tile is pulled from HBM into L2 (never stale: L2 is the
@@ -189,14 +194,20 @@
                 log_episode(log, ld, i, c, load_xi(a.env.xi, i), fs, len < 0 ? -len : len, len < 0, a.tick);
                 log.count[i] = (int32_t)(c + 1u);
             }
-            viol += reset_env(a.env, a.dr, block0 + s_list[j], a.tick, a.env.seed);
+            if (kScen) {        // env i's scenario row, read here only (through L1: few distinct rows per CTA)
+                const int64_t i = block0 + s_list[j];
+                viol += reset_env<T, true>(a.env, scenario_row<T>(env_scen.rows, env_scenario(env_scen, i)), i, a.tick,
+                                           a.env.seed);
+            } else {
+                viol += reset_env(a.env, a.dr, block0 + s_list[j], a.tick, a.env.seed);
+            }
         }
         if (viol && a.counters) atomicAdd(a.counters + kCounterGaussian, (unsigned long long)viol);
     }
     if (tracked) {
         __syncthreads();                    // every store of the CTA precedes (happens-before) thread 0's release
         if (threadIdx.x == 0) {
-            st_release_gpu(a.env.progress + 2 * (size_t)blockIdx.x + 1, ticket + 1u);
+            st_release_gpu(a.env.progress + 2 * (size_t)blockIdx.x + 1, (kScen ? s_ticket : ticket) + 1u);
             asm volatile("griddepcontrol.wait;" ::: "memory");     // do not complete before the previous grid has
         }
     }

@@ -1,4 +1,5 @@
-"""Task scenarios: the columns of an evaluation grid (``RandomCartPoleVecEnv.evaluate_grid``).
+"""Task scenarios: the columns of an evaluation grid (``RandomCartPoleVecEnv.evaluate_grid``), and the per-env task
+configurations of training (``RandomCartPoleVecEnv.set_scenarios``).
 
 A scenario is either a fixed task (gravity, cart_mass, pole_mass, pole_length), kept by every episode, or a DR
 distribution that every episode draws its task from.  Each is one row of ``RENV_SCENARIO_FLOATS`` float32 values in
@@ -21,7 +22,7 @@ def _pack(cfg, task, out):
 
 
 class Scenarios:
-    """C scenario rows for ``RandomCartPoleVecEnv.evaluate_grid``: ``rows`` is a (C, SCENARIO_FLOATS) float32 tensor on
+    """C scenario rows for ``RandomCartPoleVecEnv.evaluate_grid`` and ``set_scenarios``: ``rows`` is a (C, SCENARIO_FLOATS) float32 tensor on
     ``device``.  Build them with ``Scenarios.tasks`` (fixed tasks) or ``Scenarios.distributions`` (DR distributions)
     and join them with ``Scenarios.cat``.
 
@@ -76,6 +77,24 @@ class Scenarios:
             sampler.set_dr_distribution(dr_type, distr)
             _pack(sampler.dr_config(), None, host[c])
         return cls._place(host, device)
+
+    @classmethod
+    def adr_boundaries(cls, low, high, device=None):
+        """The 1 + 2 x 4 uniform rows of an ADR iteration over the box [low, high] (two length-4 sequences): row 0 is
+        the box itself, row 1 + 2k the box with dim k pinned at ``low[k]`` and row 2 + 2k the box with dim k pinned at
+        ``high[k]`` (width 0: see the class docstring).  Built through ``Scenarios.distributions``, so the ranges are
+        validated as ``set_dr_distribution("uniform", ...)`` validates them.  How the ranges grow or shrink from the
+        returns of each row is left to the caller."""
+        lo, hi = np.asarray(low, dtype=np.float64), np.asarray(high, dtype=np.float64)
+        if lo.shape != (4,) or hi.shape != (4,):
+            raise ValueError("low and high are 4 values each (gravity, cart_mass, pole_mass, pole_length)")
+        boxes = [(lo, hi)]
+        for k in range(4):
+            for v in (lo[k], hi[k]):
+                pl, ph = lo.copy(), hi.copy()
+                pl[k] = ph[k] = v
+                boxes.append((pl, ph))
+        return cls.distributions("uniform", [np.stack([pl, ph], 1).reshape(-1).tolist() for pl, ph in boxes], device)
 
     @classmethod
     def cat(cls, *parts):

@@ -10,6 +10,8 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     rollout(w, b, K) -> None            (K fused steps of the linear policy a = [w.s + b > 0] or of an MLPPolicy)
     evaluate_population(policies, K) -> (P, 6)   (P policies on common tasks from fresh starts; the env is untouched)
     evaluate_grid(policies, scenarios, K) -> (P, C, 6)   (the same for each of C task scenarios, in one kernel)
+    set_scenarios(scenarios, assignment)  (env i resets from scenario assignment[i] in reset / step / rollout / collect)
+    scenario_stats() -> (C, 6)          (returns of the episodes finished inside rollouts, per scenario)
     policy_actions(policy) -> (N,)      (the MLPPolicy's actions for the current observations, ready for step)
     collect(policy, K) -> Trajectory    (K fused steps under the sampled policy, every step recorded for training)
     gae(traj, critic) -> Trajectory     (values, GAE advantages and returns of that trajectory under an MLP critic)
@@ -46,6 +48,17 @@ MAX_EPISODE_STEPS = 500                            # :294
 # entry points that end episodes: a _logged variant (taking the log after env) runs them while a log is attached
 _LOGGED_ENTRIES = ("step", "step_lean", "rollout", "rollout_mlp", "collect_mlp")
 _NOISY_ENTRIES = ("reset", "step", "rollout")       # a _noisy variant takes the obs-noise block after env
+
+
+_EMPTY_STATS = [0.0, 0.0, 0.0, math.inf, -math.inf, 0.0]
+
+
+def _combine_stats(rows):
+    """(R, 6) statistics rows -> their 6-vector combination (sum, sum, sum, min, max, sum), on their device.  Exact:
+    the sums are of integers below 2^53."""
+    t = _device.torch()
+    return t.stack([rows[:, 0].sum(), rows[:, 1].sum(), rows[:, 2].sum(), rows[:, 3].min(), rows[:, 4].max(),
+                    rows[:, 5].sum()])
 
 
 def _round_up(x, m):
@@ -112,6 +125,8 @@ class RandomCartPoleVecEnv(RandomEnv):
         self.polemass_length = 0.05     # frozen, as in the reference (:79 vs :157-166)
         self._buffers = None
         self._episode_log = None        # EpisodeLog attached by start_episode_log
+        self._scen = None               # per-env scenarios (set_scenarios): rows, of_env, stats, the C struct
+        self._scen_version = 0          # bumped whenever _scen changes (the step plan holds a pointer to its struct)
         self._cfg_cache = None
         self._cfg_key = None
         self._tick = 0                  # step clock: Philox episode key; +1 per reset/step, +K per rollout
@@ -213,6 +228,18 @@ class RandomCartPoleVecEnv(RandomEnv):
             return "renv_cartpole_%s_noisy_%s" % (name, suffix), head + (ctypes.byref(b["noise"]),)
         return "renv_cartpole_%s_%s" % (name, suffix), head
 
+    def _resolve_scen(self, name):
+        """(C function, leading arguments) of the per-env scenario form of ``name`` ("reset", "step", "rollout",
+        "rollout_mlp", "collect_mlp"): env, scenarios and -- except for reset -- the episode log or NULL."""
+        if self.noisy or self._dtype_name != "float32":
+            raise ValueError("per-env scenarios need a float32 env without observation noise")
+        head = (ctypes.byref(self._buffers["env"]), ctypes.byref(self._scen["struct"]))
+        if name != "reset":
+            if self._episode_log is not None:
+                self._check_log_supported()
+            head += (ctypes.byref(self._episode_log.struct) if self._episode_log is not None else None,)
+        return "renv_cartpole_%s_scen_f32" % name, head
+
     def _launch(self, fn, *args):
         """Call the C function ``fn`` with ``args`` on the env's device and current stream (the last argument)."""
         dev = self._buffers["device"]
@@ -260,8 +287,12 @@ class RandomCartPoleVecEnv(RandomEnv):
             assert mask.shape == (self.num_envs,)
             mask_ptr = _device.ptr(mask)
         viol = self._violation_counter(b["device"])
-        fn, head = self._resolve("reset")
-        self._launch(fn, *head, mask_ptr, self._tick, self._active_dr_cfg(), _device.ptr(viol))
+        if self._scen is not None:
+            fn, head = self._resolve_scen("reset")
+            self._launch(fn, *head, mask_ptr, self._tick, _device.ptr(viol))
+        else:
+            fn, head = self._resolve("reset")
+            self._launch(fn, *head, mask_ptr, self._tick, self._active_dr_cfg(), _device.ptr(viol))
         self._tick += 1
         return self.obs
 
@@ -305,7 +336,7 @@ class RandomCartPoleVecEnv(RandomEnv):
         changes.  (A 2^20-env step is an 11 us kernel: per-call Python work has to stay below that.)"""
         b = self._buffers
         key = (self.noisy, self.track_truncated, self._dtype_name, self.lean, self._episode_log, self.auto_reset,
-               self.max_episode_steps)
+               self.max_episode_steps, self._scen_version)
         plan = b.get("step_plan")
         if plan is not None and plan["key"] == key:
             return plan
@@ -314,11 +345,17 @@ class RandomCartPoleVecEnv(RandomEnv):
         n = self.num_envs
         counter16 = b["elapsed16"] is not None
         # the uint16 counter: the lean step, or with a log attached the logged step on that counter without a reward store
-        fn, head = self._resolve("step_lean" if counter16 and self._episode_log is None else "step")
+        scen = self._scen is not None
+        if scen and not self.auto_reset:
+            raise ValueError("per-env scenarios act at resets: step() with scenarios needs auto_reset")
+        if scen:        # one entry point for every layout: the counter of the env, reward NULL with the uint16 one
+            fn, head = self._resolve_scen("step")
+        else:
+            fn, head = self._resolve("step_lean" if counter16 and self._episode_log is None else "step")
         info = {"TimeLimit.truncated": b["truncated"][:n].view(t.bool)} if self.track_truncated else {}
         viol = self._violation_counter(b["device"])
         plan = dict(key=key, fn=getattr(_lib.load(), fn), name=fn, head=head, logged=self._episode_log is not None,
-                    lean=counter16 and self._episode_log is None,
+                    lean=counter16 and self._episode_log is None, scen=scen,
                     reward=None if counter16 else _device.ptr(b["reward"]), done=_device.ptr(b["done"]),
                     truncated=_device.ptr(b["truncated"]) if self.track_truncated else None,
                     out=(self.obs, b["reward"][:n], b["done"][:n].view(t.bool)), info=info,
@@ -348,7 +385,10 @@ class RandomCartPoleVecEnv(RandomEnv):
         if self.noisy:
             b["noise"].std = math.sqrt(self.noise_level)
         idx = plan["device_index"]
-        if plan["lean"]:
+        if plan["scen"]:
+            args = plan["head"] + (action_ptr, plan["reward"], plan["done"], plan["truncated"], self._integrator(),
+                                   self.max_episode_steps, self._tick, plan["viol"], ctypes.c_void_p(_device.raw_stream(idx)))
+        elif plan["lean"]:
             args = plan["head"] + (action_ptr, plan["done"], plan["truncated"], self._integrator(), self.max_episode_steps,
                                    self._tick, self._active_dr_cfg(), plan["viol"], ctypes.c_void_p(_device.raw_stream(idx)))
         elif plan["logged"]:        # auto-reset is implied
@@ -458,11 +498,17 @@ class RandomCartPoleVecEnv(RandomEnv):
             raise ValueError("out is not a trajectory buffer of this env's shape and device: use trajectory_buffer()")
         elif out.capacity < K:
             raise ValueError("out holds %d steps, collect() was asked for %d" % (out.capacity, K))
-        fn, head = self._resolve("collect_mlp")
         viol = self._violation_counter(buf["device"])
-        self._launch(fn, *head, ctypes.byref(policy.struct), ctypes.byref(out.struct), int(bool(sample)), K,
-                     self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(),
-                     _device.ptr(buf["stats"]), _device.ptr(viol))
+        if self._scen is not None:
+            fn, head = self._resolve_scen("collect_mlp")
+            self._launch(fn, *head, ctypes.byref(policy.struct), ctypes.byref(out.struct), int(bool(sample)), K,
+                         self._integrator(), self.max_episode_steps, self._tick, _device.ptr(self._scen["stats"]),
+                         _device.ptr(viol))
+        else:
+            fn, head = self._resolve("collect_mlp")
+            self._launch(fn, *head, ctypes.byref(policy.struct), ctypes.byref(out.struct), int(bool(sample)), K,
+                         self._integrator(), self.max_episode_steps, self._tick, self._active_dr_cfg(),
+                         _device.ptr(buf["stats"]), _device.ptr(viol))
         out.tick0, out.num_steps = self._tick, K
         self._tick += K
         return out
@@ -521,10 +567,15 @@ class RandomCartPoleVecEnv(RandomEnv):
                 raise ValueError("the random policy ignores observations: use a noise-free env")
             w_arr = None if w is None else (ctypes.c_double * 4)(*[float(v) for v in w])
             name, policy_args = "rollout", (w_arr, float(b))    # Noisy variant: the policy acts on the noisy observation
-        fn, head = self._resolve(name)
         viol = self._violation_counter(buf["device"])
-        self._launch(fn, *head, *policy_args, int(num_steps), self._integrator(), self.max_episode_steps, self._tick,
-                     self._active_dr_cfg(), _device.ptr(buf["stats"]), _device.ptr(viol))
+        if self._scen is not None:
+            fn, head = self._resolve_scen(name)
+            self._launch(fn, *head, *policy_args, int(num_steps), self._integrator(), self.max_episode_steps, self._tick,
+                         _device.ptr(self._scen["stats"]), _device.ptr(viol))
+        else:
+            fn, head = self._resolve(name)
+            self._launch(fn, *head, *policy_args, int(num_steps), self._integrator(), self.max_episode_steps, self._tick,
+                         self._active_dr_cfg(), _device.ptr(buf["stats"]), _device.ptr(viol))
         self._tick += int(num_steps)
 
     def evaluate_population(self, policies, num_steps=MAX_EPISODE_STEPS):
@@ -543,6 +594,9 @@ class RandomCartPoleVecEnv(RandomEnv):
         for ``rollout``.  float32 envs without observation noise only."""
         b = self._alloc()
         t = _device.torch()
+        if self._scen is not None:
+            raise ValueError("evaluate_population() runs the env's own DR config or task table, which per-env scenarios "
+                             "replace: call set_scenarios(None) first, or use evaluate_grid()")
         K, rows, P, kind, policy_args = self._population_rows(policies, num_steps, "evaluate_population()")
         stats = t.tensor([0.0, 0.0, 0.0, math.inf, -math.inf, 0.0], dtype=t.float64, device=b["device"]).repeat(P, 1)
         viol = self._violation_counter(b["device"])
@@ -644,12 +698,114 @@ class RandomCartPoleVecEnv(RandomEnv):
 
     @property
     def stats_tensor(self):
-        """Device tensor [episodes, sum R, sum R^2, min R, max R, sum length] (float64)."""
-        return self._alloc()["stats"]
+        """Device tensor [episodes, sum R, sum R^2, min R, max R, sum length] (float64).  While per-env scenarios are
+        set, a new tensor: the env-wide combination of ``scenario_stats()`` and what was accumulated before."""
+        b = self._alloc()
+        if self._scen is None:
+            return b["stats"]
+        return _combine_stats(_device.torch().cat([b["stats"].view(1, -1), self._scen["stats"]]))
 
     def reset_stats(self):
         t = _device.torch()
-        self._alloc()["stats"].copy_(t.tensor([0.0, 0.0, 0.0, math.inf, -math.inf, 0.0], dtype=t.float64))
+        self._alloc()["stats"].copy_(t.tensor(_EMPTY_STATS, dtype=t.float64))
+        if self._scen is not None:
+            self._scen["stats"].copy_(t.tensor(_EMPTY_STATS, dtype=t.float64).expand_as(self._scen["stats"]))
+
+    # ---- per-env task scenarios -----------------------------------------------------------------------
+    def set_scenarios(self, scenarios, assignment=None):
+        """Give env i the task scenario ``assignment[i]`` of ``scenarios`` (a ``Scenarios`` on the env's device; C
+        rows): from now on every reset of env i -- in ``reset()``, the auto-reset of ``step()``, and inside
+        ``rollout()`` and ``collect()`` -- takes its task from that row, and rollouts and collect accumulate the
+        finished episodes of each scenario's envs into its row of ``scenario_stats()``.  A distribution row draws as a
+        twin env with ``set_dr_distribution`` of it and ``set_dr_training(True)`` would; a fixed-task row gives the
+        task, as ``set_task`` of it without DR would.  Env i's results depend on its own row only, so several DR
+        distributions -- ADR boundaries, a curriculum, a mixture, an empirical task set -- train in one batch.
+
+        ``assignment`` is N integers in [0, C) (a sequence, a numpy array, or a tensor on the CPU or the env's
+        device); it is checked here, with one synchronisation, and copied into the env.  While scenarios are set, the
+        DR config, ``dr_training`` and the task table do not decide what a reset draws; ``set_random_task`` and
+        ``evaluate_population`` are refused.  Running episodes keep their task until their next reset.
+        ``set_scenarios(None)`` restores the env's own configuration.  float32 envs without observation noise."""
+        from .scenarios import Scenarios
+        t = _device.torch()
+        if scenarios is None:
+            if assignment is not None:
+                raise ValueError("set_scenarios(None) takes no assignment")
+            self._clear_scenarios()
+            return
+        # every argument check that needs no device comes first: nothing is allocated for a refused call
+        if self._dtype_name != "float32" or self.noisy:
+            raise ValueError("per-env scenarios need a float32 env without observation noise")
+        if not isinstance(scenarios, Scenarios):
+            raise TypeError("set_scenarios() takes its scenarios as a Scenarios (Scenarios.tasks / .distributions)")
+        if scenarios.device.type != "cuda":
+            raise ValueError("the scenarios live on %s: move them to the env's device" % scenarios.device)
+        C = len(scenarios)
+        if C > 65535:
+            raise ValueError("at most 65535 scenarios, got %d" % C)
+        if assignment is None:
+            raise ValueError("set_scenarios() needs an assignment: the scenario of each env")
+        a = assignment if isinstance(assignment, t.Tensor) else t.as_tensor(np.asarray(assignment))
+        if a.dtype.is_floating_point or a.dtype.is_complex or a.dtype == t.bool:
+            raise ValueError("the assignment holds integer scenario indices, got %s" % a.dtype)
+        if tuple(a.shape) != (self.num_envs,):
+            raise ValueError("the assignment must have shape (%d,), got %s" % (self.num_envs, tuple(a.shape)))
+        on_device = a.is_cuda
+        if not on_device:
+            self._check_assignment_range(a, C)
+        b = self._alloc()
+        for what, dev in (("scenarios", scenarios.device), ("assignment", a.device if on_device else None)):
+            if dev is not None and dev != b["device"]:
+                raise ValueError("the %s live on %s, the env on %s" % (what, dev, b["device"]))
+        a = a.to(b["device"], t.int64)
+        if on_device:
+            self._check_assignment_range(a, C)          # the one synchronisation
+        self._install_scenarios(scenarios.rows.clone(), a.to(t.int32).to(t.int16),
+                                t.tensor(_EMPTY_STATS, dtype=t.float64, device=b["device"]).repeat(C, 1))
+
+    @staticmethod
+    def _check_assignment_range(a, C):
+        t = _device.torch()
+        lo, hi = (int(v) for v in t.stack([a.min(), a.max()]).cpu())
+        if lo < 0 or hi >= C:
+            raise ValueError("scenario indices must lie in [0, %d), got [%d, %d]" % (C, lo, hi))
+
+    def _install_scenarios(self, rows, of_env, stats):
+        """Set the env-owned scenario buffers: rows (C, SCENARIO_FLOATS) float32, of_env (N,) int16 holding the uint16
+        indices, stats (C, 6) float64 -- all on the env's device and already checked."""
+        t = _device.torch()
+        b = self._buffers
+        self._clear_scenarios()
+        idx = t.zeros(b["ld"], dtype=t.int16, device=b["device"])
+        idx[:self.num_envs].copy_(of_env)
+        rows = rows.contiguous()
+        st = _lib.EnvScenarios()
+        st.rows, st.of_env, st.C = rows.data_ptr(), idx.data_ptr(), int(rows.shape[0])
+        self._scen = dict(rows=rows, of_env=idx, stats=stats.contiguous(), struct=st)
+        self._scen_version += 1
+
+    def _clear_scenarios(self):
+        """Drop the scenarios, folding their statistics into the env-wide row."""
+        if self._scen is not None:
+            self._buffers["stats"].copy_(self.stats_tensor)
+            self._scen = None
+            self._scen_version += 1
+
+    @property
+    def scenarios(self):
+        """(rows (C, SCENARIO_FLOATS) float32, assignment (N,) int64) of the env's scenarios, or None."""
+        if self._scen is None:
+            return None
+        return self._scen["rows"], self._scen["of_env"][:self.num_envs].to(_device.torch().int64) & 0xFFFF
+
+    def scenario_stats(self):
+        """(C, 6) float64 device tensor: row c holds the statistics (``distributed.STAT_NAMES``) of the episodes that
+        the envs of scenario c finished inside ``rollout()`` and ``collect()`` since ``set_scenarios`` or
+        ``reset_stats()``.  Each row is exact (integer sums, a min and a max); shards combine row by row as
+        ``distributed.combine_stats`` combines ranks, and the rows combined are ``stats_tensor``."""
+        if self._scen is None:
+            raise ValueError("no scenarios are set (set_scenarios)")
+        return self._scen["stats"]
 
     def allgather_stats(self, group=None):
         """The per-iteration collective (distributed.allgather_stats) on this env's statistics; like every call that
@@ -697,6 +853,9 @@ class RandomCartPoleVecEnv(RandomEnv):
 
     def set_random_task(self):
         """Resample xi of every env now (random_env.py:37-39)."""
+        if self._scen is not None:
+            raise ValueError("set_random_task() draws from the env's own DR config, which per-env scenarios replace: "
+                             "call set_scenarios(None) first")
         # sample i of the call is keyed by the GLOBAL env id, so a sharded env draws what the unsharded one would
         self.set_task(self.sample_tasks_tensor(self.num_envs, dtype=self.torch_dtype, device=self._alloc()["device"],
                                                sample_id0=self.env_id0))
@@ -819,6 +978,9 @@ class RandomCartPoleVecEnv(RandomEnv):
                            min_task=self.min_task.copy(), max_task=self.max_task.copy(), mean_task=self.mean_task.copy(),
                            stdev_task=self.stdev_task.copy(),
                            cov_task=np.copy(self.cov_task) if getattr(self, "cov_task", None) is not None else None))
+        sc = self._scen
+        out["scenarios"] = None if sc is None else dict(rows=sc["rows"].clone(), of_env=sc["of_env"][:self.num_envs].clone(),
+                                                        stats=sc["stats"].clone())
         self.check_dr_violations()          # synchronises; a checkpoint must not hide an error the reference raises
         return out
 
@@ -850,6 +1012,12 @@ class RandomCartPoleVecEnv(RandomEnv):
                 self.cov_task = np.copy(dr["cov_task"])
             self._on_distribution_change()
         self._refresh_env_struct()
+        self._scen = None
+        self._scen_version += 1
+        sc = sd.get("scenarios")
+        if sc is not None:
+            dev = b["device"]
+            self._install_scenarios(sc["rows"].to(dev), sc["of_env"].to(dev), sc["stats"].to(dev).clone())
 
     # ---- introspection used by tests -------------------------------------------------------------------
     @property
