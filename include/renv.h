@@ -29,7 +29,8 @@
  *                    were not in the state the protocol leaves them in (see there); the step still ran.
  *     The host reads them at its next synchronisation point and raises the reference's exception.
  *   - RNG: counter-based Philox4x32-10, key = seed, counter = (global env id, tick, purpose|slot), purpose 0 initial
- *     state, 1 xi, 2 random action, 3 sample_tasks, 4 observation noise, 5 MLP policy sample.  `tick` is
+ *     state, 1 xi, 2 random action, 3 sample_tasks, 4 observation noise, 5 MLP policy sample, 6 scenario-mixture
+ *     row.  `tick` is
  *     the caller's step clock (48 bits used): pass a value that grows by 1 per reset/step call and by K per
  *     K-step rollout (step k of a rollout uses tick + k).  An env starts at most one episode per tick, so
  *     (seed, env_id0 + i, tick) names the episode; results never depend on launch geometry or sharding,
@@ -476,6 +477,57 @@ int renv_cartpole_collect_mlp_scen_f32(const renv_cartpole_env *env, const renv_
                                        const renv_episode_log *log, const renv_mlp_policy *p, const renv_trajectory *traj,
                                        int sample, int K, int integrator, int max_steps, uint64_t tick, double *stats,
                                        unsigned long long *violations, void *stream);
+
+/* Scenario mixtures in the training path: every reset of env i -- in reset, in the auto-reset of a step, or inside a
+ * rollout or collect -- at clock tick t draws its scenario row c from a C-entry alias table:
+ *   (x, y) = words 0 and 1 of the Philox block (seed, env_id0 + i, t, purpose 6, slot 0);
+ *   j = (uint64_t)x * C >> 32;   c = y < table[j].q ? j : table[j].alias.
+ * Row c is P(c) = sum over j of [j == c] (q_j / 2^32) / C + [alias_j == c] (1 - q_j / 2^32) / C, an integer count over
+ * 2^64.  The reset is then exactly the per-env scenario reset above with row c (a law row draws xi with purpose 1 at
+ * (env_id0 + i, t), a fixed row gives its task), and of_env[i] = c is stored.  So every per-env output of env i equals,
+ * bit for bit, that of a renv_env_scenarios twin whose of_env[i] is set to the drawn row before each reset.
+ *
+ * of_env[i] holds the row of env i's running episode; the kernels write it.  C marks an episode that began before the
+ * mixture was installed.  Rollout and collect accumulate each finished episode into stats[min(of_env, C) *
+ * RENV_NUM_STATS ..] of the reset that began it: a (C + 1, RENV_NUM_STATS) array, initialised like the plain stats,
+ * whose row C holds the episodes that began before the mixture.  Each row is exact in doubles.  A bad alias is clamped
+ * to C - 1; building the table is the caller's job.  fp32 only; `log` may be NULL or an episode log.  Errors, all before
+ * any CUDA call: every check of the corresponding plain entry point with its code, then NULL mix, rows, table or of_env
+ * RENV_E_NULL; C outside [1, 65535] RENV_E_SIZE; misaligned rows, table or of_env RENV_E_ALIGN. */
+typedef struct renv_alias_entry {
+    uint32_t q;               /* column j keeps row j when y < q */
+    uint16_t alias;           /* ... and gives row alias otherwise */
+    uint16_t pad;
+} renv_alias_entry;
+
+typedef struct renv_env_mixture {
+    const float *rows;                /* (C, RENV_SCENARIO_FLOATS) device rows, 16-byte aligned */
+    const renv_alias_entry *table;    /* (C) device, 8-byte aligned */
+    uint16_t *of_env;                 /* (n) device, 4-byte aligned: the row of env i's running episode (written) */
+    int32_t C;                        /* 1 <= C <= 65535 */
+} renv_env_mixture;
+
+/* renv_cartpole_reset_scen_f32 with the drawn row. */
+int renv_cartpole_reset_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix, const uint8_t *mask,
+                                uint64_t tick, unsigned long long *violations, void *stream);
+/* renv_cartpole_step_scen_f32 with the drawn row: only the CTA reset pass draws and reads the table and rows. */
+int renv_cartpole_step_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix, const renv_episode_log *log,
+                               const uint8_t *action, float *reward, uint8_t *done, uint8_t *truncated, int integrator,
+                               int max_steps, uint64_t tick, unsigned long long *counters, void *stream);
+/* renv_cartpole_rollout_scen_f32 with the drawn rows, statistics per row into (C + 1, RENV_NUM_STATS). */
+int renv_cartpole_rollout_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix, const renv_episode_log *log,
+                                  const double w[4], double b, int K, int integrator, int max_steps, uint64_t tick,
+                                  double *stats, unsigned long long *violations, void *stream);
+/* renv_cartpole_rollout_mlp_scen_f32 with the drawn rows. */
+int renv_cartpole_rollout_mlp_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix,
+                                      const renv_episode_log *log, const renv_mlp_policy *p, int K, int integrator,
+                                      int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+                                      void *stream);
+/* renv_cartpole_collect_mlp_scen_f32 with the drawn rows. */
+int renv_cartpole_collect_mlp_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix,
+                                      const renv_episode_log *log, const renv_mlp_policy *p, const renv_trajectory *traj,
+                                      int sample, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                                      unsigned long long *violations, void *stream);
 
 /* Recorded cart-pole transitions for offline DR fitting (device pointers): transition i is (obs[i], action[i],
  * next_obs[i]), and `window` lists the W start indices t that are scored (t + lam <= T; windows crossing an episode

@@ -70,6 +70,11 @@ class EnvScenarios(ctypes.Structure):
     _fields_ = [("rows", ctypes.c_void_p), ("of_env", ctypes.c_void_p), ("C", ctypes.c_int32)]
 
 
+class EnvMixture(ctypes.Structure):
+    """struct renv_env_mixture (include/renv.h)."""
+    _fields_ = [("rows", ctypes.c_void_p), ("table", ctypes.c_void_p), ("of_env", ctypes.c_void_p), ("C", ctypes.c_int32)]
+
+
 class Transitions(ctypes.Structure):
     """struct renv_transitions (include/renv.h)."""
     _fields_ = [("obs", ctypes.c_void_p), ("next_obs", ctypes.c_void_p), ("action", ctypes.c_void_p),
@@ -85,6 +90,7 @@ _mlp_p = ctypes.POINTER(MlpPolicy)
 _traj_p = ctypes.POINTER(Trajectory)
 _trans_p = ctypes.POINTER(Transitions)
 _scen_p = ctypes.POINTER(EnvScenarios)
+_mix_p = ctypes.POINTER(EnvMixture)
 
 # name -> (restype, argtypes); must list every function declared in include/renv.h
 SIGNATURES = {
@@ -129,6 +135,13 @@ SIGNATURES = {
     "renv_cartpole_rollout_mlp_scen_f32": (_int, [_env_p, _scen_p, _log_p, _mlp_p, _int, _int, _int, _u64, _vp, _vp, _vp]),
     "renv_cartpole_collect_mlp_scen_f32": (_int, [_env_p, _scen_p, _log_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64,
                                                   _vp, _vp, _vp]),
+    "renv_cartpole_reset_mix_f32": (_int, [_env_p, _mix_p, _vp, _u64, _vp, _vp]),
+    "renv_cartpole_step_mix_f32": (_int, [_env_p, _mix_p, _log_p, _vp, _vp, _vp, _vp, _int, _int, _u64, _vp, _vp]),
+    "renv_cartpole_rollout_mix_f32": (_int, [_env_p, _mix_p, _log_p, ctypes.POINTER(_dbl), _dbl, _int, _int, _int, _u64,
+                                             _vp, _vp, _vp]),
+    "renv_cartpole_rollout_mlp_mix_f32": (_int, [_env_p, _mix_p, _log_p, _mlp_p, _int, _int, _int, _u64, _vp, _vp, _vp]),
+    "renv_cartpole_collect_mlp_mix_f32": (_int, [_env_p, _mix_p, _log_p, _mlp_p, _traj_p, _int, _int, _int, _int, _u64,
+                                                 _vp, _vp, _vp]),
     "renv_cartpole_transition_loglik_f64": (_int, [_trans_p, _int, _int, _vp, _int, _int, ctypes.POINTER(_dbl), _vp, _vp,
                                                    _vp]),
     "renv_cartpole_scalar_serve": (_int, [_vp, _vp, _u32, _u64, _vp]),

@@ -737,11 +737,46 @@ int check_env_scenarios(const renv_env_scenarios *scen, EnvScenPtrs *out)
     *out = EnvScenPtrs{ scen->rows, scen->of_env, (uint32_t)scen->C };
     return RENV_OK;
 }
+static_assert(sizeof(renv_alias_entry) == sizeof(uint2) && offsetof(renv_alias_entry, q) == 0 &&
+              offsetof(renv_alias_entry, alias) == 4, "alias entry layout differs from MixPtrs::table");
+int check_env_scenarios(const renv_env_mixture *mix, MixPtrs *out)
+{
+    if (mix == nullptr || mix->rows == nullptr || mix->table == nullptr || mix->of_env == nullptr) return RENV_E_NULL;
+    if (mix->C < 1 || mix->C > 65535) return RENV_E_SIZE;
+    if (!aligned(mix->rows, 16) || !aligned(mix->table, 8) || !aligned(mix->of_env, 4)) return RENV_E_ALIGN;
+    *out = MixPtrs{ mix->rows, reinterpret_cast<const uint2 *>(mix->table), mix->of_env, (uint32_t)mix->C };
+    return RENV_OK;
+}
 
-int reset_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const uint8_t *mask, uint64_t tick,
+// The training entry points with per-env rows: per-env scenarios (renv_env_scenarios, the cartpole_scen_* kernels) or
+// a scenario mixture (renv_env_mixture, the cartpole_mix_* kernels).  The two forms share every check and launch.
+template <bool kMixture> struct RowForm;
+template <> struct RowForm<false> {
+    using ResetA = ScenResetArgs; using StepA = ScenStepArgs; using RolloutA = ScenRolloutArgs;
+    using MlpRolloutA = MlpScenRolloutArgs; using MlpCollectA = MlpScenCollectArgs;
+    static auto reset() { return cartpole_scen_reset_kernel; }
+    template <bool ln, bool lg> static auto step() { return cartpole_scen_step_kernel<ln, lg>; }
+    template <bool e, bool r, bool lg> static auto rollout() { return cartpole_scen_rollout_kernel<e, r, lg>; }
+    template <int act, bool e, bool lg> static auto rollout_mlp() { return cartpole_scen_rollout_mlp_kernel<act, e, lg>; }
+    template <int act, bool e, bool lg> static auto collect_mlp() { return cartpole_scen_collect_mlp_kernel<act, e, lg>; }
+    template <class A> static auto &rows(A &a) { return a.scen; }
+};
+template <> struct RowForm<true> {
+    using ResetA = MixResetArgs; using StepA = MixStepArgs; using RolloutA = MixRolloutArgs;
+    using MlpRolloutA = MlpMixRolloutArgs; using MlpCollectA = MlpMixCollectArgs;
+    static auto reset() { return cartpole_mix_reset_kernel; }
+    template <bool ln, bool lg> static auto step() { return cartpole_mix_step_kernel<ln, lg>; }
+    template <bool e, bool r, bool lg> static auto rollout() { return cartpole_mix_rollout_kernel<e, r, lg>; }
+    template <int act, bool e, bool lg> static auto rollout_mlp() { return cartpole_mix_rollout_mlp_kernel<act, e, lg>; }
+    template <int act, bool e, bool lg> static auto collect_mlp() { return cartpole_mix_collect_mlp_kernel<act, e, lg>; }
+    template <class A> static auto &rows(A &a) { return a.mix; }
+};
+
+template <class F, class B>
+int reset_rows(const renv_cartpole_env *env, const B *scen, const uint8_t *mask, uint64_t tick,
                unsigned long long *violations, void *stream)
 {
-    ScenResetArgs a;
+    typename F::ResetA a;
     int rc = check_env<float>(env, false, &a.reset.env, kNeedEitherElapsed);
     if (rc) return rc;
     if ((rc = to_cfg4<float>(nullptr, &a.reset.dr))) return rc;
@@ -750,18 +785,19 @@ int reset_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, con
     a.reset.violations = violations;
     unsigned blocks = 0;
     if ((rc = grid_for(env->n, 256, &blocks))) return rc;
-    if ((rc = check_env_scenarios(scen, &a.scen))) return rc;
-    cartpole_scen_reset_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    if ((rc = check_env_scenarios(scen, &F::rows(a)))) return rc;
+    F::reset()<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
     return launch_status();
 }
 
 // The auto-reset step (renv_cartpole_step_f32 / _lean_f32 / _logged_f32, whichever the env's counter and `log` make
-// it) with per-env scenarios.
-int step_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+// it) with per-env rows.
+template <class F, class B>
+int step_rows(const renv_cartpole_env *env, const B *scen, const renv_episode_log *log,
               const uint8_t *action, float *reward, uint8_t *done, uint8_t *truncated, int integrator, int max_steps,
               uint64_t tick, unsigned long long *counters, void *stream)
 {
-    ScenStepArgs sa;
+    typename F::StepA sa;
     StepArgs<float> &a = sa.step;
     int rc = check_env<float>(env, false, &a.env, kNeedEitherElapsed);
     if (rc) return rc;
@@ -782,19 +818,22 @@ int step_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, cons
     a.counters = counters;
     unsigned blocks = 0;
     if ((rc = grid_for(env->n, (int64_t)kStepThreads * VecTraits<float>::V, &blocks))) return rc;
-    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    if ((rc = check_env_scenarios(scen, &F::rows(sa)))) return rc;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     with_flag(lean, [&](auto ln) {
-        with_flag(log != nullptr, [&](auto lg) { rc = launch_pdl(cartpole_scen_step_kernel<ln, lg>, blocks, kStepThreads, st, sa); });
+        with_flag(log != nullptr, [&](auto lg) {
+            rc = launch_pdl(F::template step<ln, lg>(), blocks, kStepThreads, st, sa);
+        });
     });
     return rc;
 }
 
-int rollout_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+template <class F, class B>
+int rollout_rows(const renv_cartpole_env *env, const B *scen, const renv_episode_log *log,
                  const double w[4], double b, int K, int integrator, int max_steps, uint64_t tick, double *stats,
                  unsigned long long *violations, void *stream)
 {
-    ScenRolloutArgs sa;
+    typename F::RolloutA sa;
     int rc = check_env<float>(env, false, &sa.roll.env, kNeedEitherElapsed);
     if (rc) return rc;
     sa.log = LogPtrs<float>{};
@@ -806,40 +845,42 @@ int rollout_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, c
     if (env->elapsed == nullptr && max_steps > 65535) return RENV_E_SIZE;     // the uint16 counter
     unsigned blocks = 0;
     if ((rc = grid_for(env->n, kRolloutThreads, &blocks))) return rc;
-    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    if ((rc = check_env_scenarios(scen, &F::rows(sa)))) return rc;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     with_flag(sa.roll.euler, [&](auto euler) {
         with_flag(w == nullptr, [&](auto random) {
             with_flag(log != nullptr, [&](auto lg) {
-                cartpole_scen_rollout_kernel<euler, random, lg><<<blocks, kRolloutThreads, 0, st>>>(sa);
+                F::template rollout<euler, random, lg>()<<<blocks, kRolloutThreads, 0, st>>>(sa);
             });
         });
     });
     return launch_status();
 }
 
-int rollout_mlp_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+template <class F, class B>
+int rollout_mlp_rows(const renv_cartpole_env *env, const B *scen, const renv_episode_log *log,
                      const renv_mlp_policy *p, int K, int integrator, int max_steps, uint64_t tick, double *stats,
                      unsigned long long *violations, void *stream)
 {
-    MlpScenRolloutArgs sa;
+    typename F::MlpRolloutA sa;
     unsigned blocks = 0;
     int rc = prepare_rollout_mlp(env, log, log != nullptr, p, K, integrator, max_steps, tick, nullptr, stats, violations,
                                  &sa.mlp, &blocks);
     if (rc) return rc;
-    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    if ((rc = check_env_scenarios(scen, &F::rows(sa)))) return rc;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     with_mlp_instance(p->activation, sa.mlp.roll.euler, log != nullptr, [&](auto act, auto euler, auto lg) {
-        cartpole_scen_rollout_mlp_kernel<act, euler, lg><<<blocks, kMlpThreads, 0, st>>>(sa);
+        F::template rollout_mlp<act, euler, lg>()<<<blocks, kMlpThreads, 0, st>>>(sa);
     });
     return launch_status();
 }
 
-int collect_mlp_scen(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
+template <class F, class B>
+int collect_mlp_rows(const renv_cartpole_env *env, const B *scen, const renv_episode_log *log,
                      const renv_mlp_policy *p, const renv_trajectory *traj, int sample, int K, int integrator,
                      int max_steps, uint64_t tick, double *stats, unsigned long long *violations, void *stream)
 {
-    MlpScenCollectArgs sa;
+    typename F::MlpCollectA sa;
     unsigned blocks = 0;
     int rc = prepare_rollout_mlp(env, log, log != nullptr, p, K, integrator, max_steps, tick, nullptr, stats, violations,
                                  &sa.mlp, &blocks);
@@ -847,10 +888,10 @@ int collect_mlp_scen(const renv_cartpole_env *env, const renv_env_scenarios *sce
     if ((rc = check_traj(traj, K, &sa.mlp.traj))) return rc;
     if (sample != 0 && sample != 1) return RENV_E_ARG;
     sa.mlp.sample = sample;
-    if ((rc = check_env_scenarios(scen, &sa.scen))) return rc;
+    if ((rc = check_env_scenarios(scen, &F::rows(sa)))) return rc;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     with_mlp_instance(p->activation, sa.mlp.roll.euler, log != nullptr, [&](auto act, auto euler, auto lg) {
-        cartpole_scen_collect_mlp_kernel<act, euler, lg><<<blocks, kMlpThreads, 0, st>>>(sa);
+        F::template collect_mlp<act, euler, lg>()<<<blocks, kMlpThreads, 0, st>>>(sa);
     });
     return launch_status();
 }
@@ -1117,34 +1158,68 @@ int renv_cartpole_grid_mlp_f32(const renv_cartpole_env *env, const void *params,
 int renv_cartpole_reset_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen, const uint8_t *mask,
                                  uint64_t tick, unsigned long long *violations, void *stream)
 {
-    return reset_scen(env, scen, mask, tick, violations, stream);
+    return reset_rows<RowForm<false>>(env, scen, mask, tick, violations, stream);
 }
 int renv_cartpole_step_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen, const renv_episode_log *log,
                                 const uint8_t *action, float *reward, uint8_t *done, uint8_t *truncated, int integrator,
                                 int max_steps, uint64_t tick, unsigned long long *counters, void *stream)
 {
-    return step_scen(env, scen, log, action, reward, done, truncated, integrator, max_steps, tick, counters, stream);
+    return step_rows<RowForm<false>>(env, scen, log, action, reward, done, truncated, integrator, max_steps, tick, counters, stream);
 }
 int renv_cartpole_rollout_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
                                    const renv_episode_log *log, const double w[4], double b, int K, int integrator,
                                    int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
                                    void *stream)
 {
-    return rollout_scen(env, scen, log, w, b, K, integrator, max_steps, tick, stats, violations, stream);
+    return rollout_rows<RowForm<false>>(env, scen, log, w, b, K, integrator, max_steps, tick, stats, violations, stream);
 }
 int renv_cartpole_rollout_mlp_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
                                        const renv_episode_log *log, const renv_mlp_policy *p, int K, int integrator,
                                        int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
                                        void *stream)
 {
-    return rollout_mlp_scen(env, scen, log, p, K, integrator, max_steps, tick, stats, violations, stream);
+    return rollout_mlp_rows<RowForm<false>>(env, scen, log, p, K, integrator, max_steps, tick, stats, violations, stream);
 }
 int renv_cartpole_collect_mlp_scen_f32(const renv_cartpole_env *env, const renv_env_scenarios *scen,
                                        const renv_episode_log *log, const renv_mlp_policy *p, const renv_trajectory *traj,
                                        int sample, int K, int integrator, int max_steps, uint64_t tick, double *stats,
                                        unsigned long long *violations, void *stream)
 {
-    return collect_mlp_scen(env, scen, log, p, traj, sample, K, integrator, max_steps, tick, stats, violations, stream);
+    return collect_mlp_rows<RowForm<false>>(env, scen, log, p, traj, sample, K, integrator, max_steps, tick, stats, violations, stream);
+}
+
+int renv_cartpole_reset_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix, const uint8_t *mask,
+                                uint64_t tick, unsigned long long *violations, void *stream)
+{
+    return reset_rows<RowForm<true>>(env, mix, mask, tick, violations, stream);
+}
+int renv_cartpole_step_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix, const renv_episode_log *log,
+                               const uint8_t *action, float *reward, uint8_t *done, uint8_t *truncated, int integrator,
+                               int max_steps, uint64_t tick, unsigned long long *counters, void *stream)
+{
+    return step_rows<RowForm<true>>(env, mix, log, action, reward, done, truncated, integrator, max_steps, tick, counters,
+                                    stream);
+}
+int renv_cartpole_rollout_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix, const renv_episode_log *log,
+                                  const double w[4], double b, int K, int integrator, int max_steps, uint64_t tick,
+                                  double *stats, unsigned long long *violations, void *stream)
+{
+    return rollout_rows<RowForm<true>>(env, mix, log, w, b, K, integrator, max_steps, tick, stats, violations, stream);
+}
+int renv_cartpole_rollout_mlp_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix,
+                                      const renv_episode_log *log, const renv_mlp_policy *p, int K, int integrator,
+                                      int max_steps, uint64_t tick, double *stats, unsigned long long *violations,
+                                      void *stream)
+{
+    return rollout_mlp_rows<RowForm<true>>(env, mix, log, p, K, integrator, max_steps, tick, stats, violations, stream);
+}
+int renv_cartpole_collect_mlp_mix_f32(const renv_cartpole_env *env, const renv_env_mixture *mix,
+                                      const renv_episode_log *log, const renv_mlp_policy *p, const renv_trajectory *traj,
+                                      int sample, int K, int integrator, int max_steps, uint64_t tick, double *stats,
+                                      unsigned long long *violations, void *stream)
+{
+    return collect_mlp_rows<RowForm<true>>(env, mix, log, p, traj, sample, K, integrator, max_steps, tick, stats,
+                                           violations, stream);
 }
 
 int renv_cartpole_transition_loglik_f64(const renv_transitions *data, int lam, int integrator, const double *xi, int C,

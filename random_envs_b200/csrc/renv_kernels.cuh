@@ -114,6 +114,27 @@ __device__ __forceinline__ uint32_t env_scenario(const EnvScenPtrs &sc, int64_t 
     return min((uint32_t)sc.of_env[i], sc.C - 1u);
 }
 
+// A scenario mixture of the training path (include/renv.h renv_env_mixture): every reset of env i draws its row from
+// the C-entry alias table with Philox (seed, id, tick, purpose 6, slot 0), words x and y: column j = x C >> 32, row
+// j when y < table[j].q, else table[j].alias.  of_env[i] holds the row of env i's running episode (C: one that began
+// before the mixture was installed); the kernels write it.  A bad alias is clamped so that the row load stays inside
+// the rows; building the table is the caller's job.
+struct MixPtrs {
+    const float *rows;          // (C, kScenarioFloats), 16-byte aligned
+    const uint2 *table;         // (C): x = q, y = alias (low 16 bits)
+    uint16_t *of_env;           // (n): the row of env i's running episode
+    uint32_t C;
+};
+__device__ __forceinline__ uint32_t mixture_draw(const MixPtrs &m, uint64_t seed, uint64_t id, uint64_t tick)
+{
+    const uint4 r = draw_block(seed, id, tick, kMixture, 0);
+    const uint32_t j = (uint32_t)(((uint64_t)r.x * m.C) >> 32);
+    const uint2 e = m.table[j];
+    // a row is below C <= 65535; the 16-bit type says so, and keeps an index of unbounded range away from
+    // scenario_row, which would otherwise change how scenario_publish of the per-env scenario kernels compiles
+    return (uint16_t)(r.y < e.x ? j : min(e.y & 0xffffu, m.C - 1u));
+}
+
 // RandomCartPoleEnv.reset (+ set_random_task) of env i at clock `tick`; scalar stores.  kScen: `dr` is env i's scenario
 // row, and a fixed-task row writes its task into xi.
 template <typename T, bool kScen = false>
@@ -250,6 +271,8 @@ __global__ void __launch_bounds__(kStepThreads, kNoisy ? (sizeof(T) == 8 ? 2 : 3
     constexpr bool kLog = false, kScen = false;
     const LogPtrs<T> log = {};
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_step_body.cuh"
 }
 
@@ -267,6 +290,8 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinCtas<T>) cartpole_step_l
     const StepArgs<T> &a = args.step;
     const LogPtrs<T> &log = args.log;
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_step_body.cuh"
 }
 
@@ -284,6 +309,26 @@ __global__ void __launch_bounds__(kStepThreads, kStepMinCtas<float>) cartpole_sc
     const StepArgs<T> &a = args.step;
     const LogPtrs<T> &log = args.log;
     const EnvScenPtrs &env_scen = args.scen;
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
+#include "renv_step_body.cuh"
+}
+
+struct MixStepArgs { StepArgs<float> step; LogPtrs<float> log; MixPtrs mix; };     // step.dr is unused
+
+// The fp32 auto-reset step under a scenario mixture (renv_cartpole_step_mix_f32): the plain step body, whose CTA reset
+// pass draws each resetting env's row from the alias table, resets it from that row and stores the row in of_env --
+// nothing else changes, so the streamed bytes are those of the plain step.  kLean and kLog as in
+// cartpole_scen_step_kernel.
+template <bool kLean, bool kLog>
+__global__ void __launch_bounds__(kStepThreads, kStepMinCtas<float>) cartpole_mix_step_kernel(const __grid_constant__ MixStepArgs args)
+{
+    using T = float;
+    constexpr bool kAutoReset = true, kNoisy = false, kScen = false, kMix = true;
+    const StepArgs<T> &a = args.step;
+    const LogPtrs<T> &log = args.log;
+    constexpr EnvScenPtrs env_scen = {};
+    const MixPtrs &mix = args.mix;
 #include "renv_step_body.cuh"
 }
 
@@ -324,6 +369,25 @@ __global__ void __launch_bounds__(256) cartpole_scen_reset_kernel(const __grid_c
     if (a.env.beyond) a.env.beyond[i] = -1;
     const DrCfg4<float> &row = scenario_row<float>(args.scen.rows, env_scenario(args.scen, i));
     const unsigned viol = reset_env<float, true>(a.env, row, i, a.tick, a.env.seed);
+    if (viol && a.violations) atomicAdd(a.violations, (unsigned long long)viol);
+}
+
+struct MixResetArgs { ResetArgs<float> reset; MixPtrs mix; };     // reset.dr is unused
+
+// cartpole_reset_kernel with a row drawn from the mixture in place of the launch's DR config
+// (renv_cartpole_reset_mix_f32); the row goes to of_env.
+__global__ void __launch_bounds__(256) cartpole_mix_reset_kernel(const __grid_constant__ MixResetArgs args)
+{
+    const ResetArgs<float> &a = args.reset;
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.env.n) return;
+    if (a.mask && !a.mask[i]) return;
+    if (a.env.elapsed) a.env.elapsed[i] = 0;
+    if (a.env.elapsed16) a.env.elapsed16[i] = 0;
+    if (a.env.beyond) a.env.beyond[i] = -1;
+    const uint32_t c = mixture_draw(args.mix, a.env.seed, a.env.env_id0 + (uint64_t)i, a.tick);
+    const unsigned viol = reset_env<float, true>(a.env, scenario_row<float>(args.mix.rows, c), i, a.tick, a.env.seed);
+    args.mix.of_env[i] = (uint16_t)c;
     if (viol && a.violations) atomicAdd(a.violations, (unsigned long long)viol);
 }
 
@@ -477,6 +541,68 @@ __device__ __noinline__ void scenario_publish(double *stats, uint32_t C, uint32_
         }
     }
     if (threadIdx.x == 0 && tab_viol && violations) atomicAdd(violations, (unsigned long long)tab_viol);
+}
+
+// Statistics of a mixture launch (cartpole_mix_*): a lane's episodes in one launch may belong to different rows, so a
+// lane keeps running sums for the row of its current episode and flushes them (mixture_stats_add) whenever a reset
+// draws another row, and once at the end.  With C <= kScenSmemRows the flushes go into a shared table of C + 1 rows
+// (exact integer atomics) that mixture_stats_end publishes with one thread per row; beyond that each flush is a set of
+// six double atomics into stats.  Row C collects the episodes that began before the mixture was installed.
+// mixture_stats_begin and mixture_stats_end must be called by every thread of the CTA.
+__device__ __forceinline__ ScenStatsRow *mixture_table()
+{
+    __shared__ ScenStatsRow tab[kScenSmemRows + 1];
+    return tab;
+}
+__device__ __forceinline__ void mixture_stats_begin(uint32_t C)
+{
+    if (C > (uint32_t)kScenSmemRows) return;    // uniform: C is a launch argument
+    ScenStatsRow *tab = mixture_table();
+    for (uint32_t r = threadIdx.x; r <= C; r += blockDim.x) tab[r] = ScenStatsRow{ 0ull, 0ull, 0ull, 0ull, 0xffffffffu, 0u };
+    __syncthreads();
+}
+__device__ __noinline__ void mixture_stats_add(double *stats, uint32_t C, uint32_t row, unsigned episodes,
+                                               unsigned sum_len, unsigned sum_r_u, unsigned long long sum_r2_u,
+                                               float min_r, float max_r)
+{
+    if (episodes == 0u) return;
+    if (C <= (uint32_t)kScenSmemRows) {
+        ScenStatsRow &e = mixture_table()[row];
+        atomicAdd(&e.episodes, (unsigned long long)episodes);
+        atomicAdd(&e.sum_len, (unsigned long long)sum_len);
+        atomicAdd(&e.sum_r, (unsigned long long)sum_r_u);
+        atomicAdd(&e.sum_r2, sum_r2_u);
+        atomicMin(&e.min_r, (unsigned)min_r);
+        atomicMax(&e.max_r, (unsigned)max_r);
+    } else {
+        double *s = stats + 6 * (size_t)row;
+        atomicAdd(s + 0, (double)episodes);
+        atomicAdd(s + 1, (double)sum_r_u);
+        atomicAdd(s + 2, (double)sum_r2_u);
+        atomic_min_f64(s + 3, (double)min_r);
+        atomic_max_f64(s + 4, (double)max_r);
+        atomicAdd(s + 5, (double)sum_len);
+    }
+}
+__device__ __noinline__ void mixture_stats_end(double *stats, uint32_t C, unsigned long long *violations, unsigned viol)
+{
+    viol = __reduce_add_sync(0xffffffffu, viol);
+    if ((threadIdx.x & 31) == 0 && viol && violations) atomicAdd(violations, (unsigned long long)viol);
+    if (C > (uint32_t)kScenSmemRows) return;
+    __syncthreads();
+    const ScenStatsRow *tab = mixture_table();
+    for (uint32_t r = threadIdx.x; r <= C; r += blockDim.x) {
+        const ScenStatsRow e = tab[r];
+        if (e.episodes) {
+            double *row = stats + 6 * (size_t)r;
+            atomicAdd(row + 0, (double)e.episodes);
+            atomicAdd(row + 1, (double)e.sum_r);
+            atomicAdd(row + 2, (double)e.sum_r2);
+            atomic_min_f64(row + 3, (double)e.min_r);
+            atomic_max_f64(row + 4, (double)e.max_r);
+            atomicAdd(row + 5, (double)e.sum_len);
+        }
+    }
 }
 
 template <typename T> struct RolloutArgs {
@@ -651,6 +777,8 @@ cartpole_rollout_kernel(const __grid_constant__ RolloutArgs<T> a)
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -667,6 +795,8 @@ cartpole_rollout_logged_kernel(const __grid_constant__ LoggedRolloutArgs<T> args
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -686,6 +816,8 @@ cartpole_population_linear_kernel(const __grid_constant__ PopulationArgs args)
     const PopulationPtrs &pop = args.pop;
     constexpr GridPtrs grid = {};
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -705,6 +837,8 @@ cartpole_grid_linear_kernel(const __grid_constant__ GridArgs args)
     const PopulationPtrs &pop = args.pop;
     const GridPtrs &grid = args.grid;
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_rollout_body.cuh"
 }
 
@@ -725,6 +859,28 @@ cartpole_scen_rollout_kernel(const __grid_constant__ ScenRolloutArgs args)
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
     const EnvScenPtrs &env_scen = args.scen;
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
+#include "renv_rollout_body.cuh"
+}
+
+struct MixRolloutArgs { RolloutArgs<float> roll; LogPtrs<float> log; MixPtrs mix; };     // roll.dr is unused
+
+// The fp32 linear-policy (kRandom: random-policy) rollout under a scenario mixture (renv_cartpole_rollout_mix_f32): the
+// generic body of cartpole_scen_rollout_kernel, whose lanes draw their row at every reset and flush their statistics
+// into the row of the episodes they belong to (mixture_stats_add).
+template <bool kEuler, bool kRandom, bool kLog>
+__global__ void __launch_bounds__(kRolloutThreads, rollout_ctas<float>(false, kRandom))
+cartpole_mix_rollout_kernel(const __grid_constant__ MixRolloutArgs args)
+{
+    using T = float;
+    constexpr bool kNoisy = false, kPop = false, kGrid = false, kScen = false, kMix = true;
+    const RolloutArgs<T> &a = args.roll;
+    const LogPtrs<T> &log = args.log;
+    constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
+    const MixPtrs &mix = args.mix;
 #include "renv_rollout_body.cuh"
 }
 

@@ -299,6 +299,8 @@ cartpole_rollout_mlp_kernel(const __grid_constant__ MlpRolloutArgs args)
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -329,6 +331,8 @@ cartpole_collect_mlp_kernel(const __grid_constant__ MlpCollectArgs args)
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -354,6 +358,8 @@ cartpole_population_mlp_kernel(const __grid_constant__ MlpPopulationArgs pa)
     const PopulationPtrs &pop = pa.pop;
     constexpr GridPtrs grid = {};
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -381,6 +387,8 @@ cartpole_grid_mlp_kernel(const __grid_constant__ MlpGridArgs pa)
     const PopulationPtrs &pop = pa.pop;
     const GridPtrs &grid = pa.grid;
     constexpr EnvScenPtrs env_scen = {};
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -404,6 +412,8 @@ cartpole_scen_rollout_mlp_kernel(const __grid_constant__ MlpScenRolloutArgs sa)
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
     const EnvScenPtrs &env_scen = sa.scen;
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
 #include "renv_mlp_rollout_body.cuh"
 }
 
@@ -418,6 +428,47 @@ cartpole_scen_collect_mlp_kernel(const __grid_constant__ MlpScenCollectArgs sa)
     constexpr PopulationPtrs pop = {};
     constexpr GridPtrs grid = {};
     const EnvScenPtrs &env_scen = sa.scen;
+    constexpr bool kMix = false;
+    constexpr MixPtrs mix = {};
+#include "renv_mlp_rollout_body.cuh"
+}
+
+// ------------------------------------------------------------------------------------------------
+// Scenario mixtures: the MLP rollout and collection with every reset drawing its row from a weighted table
+// ------------------------------------------------------------------------------------------------
+struct MlpMixRolloutArgs { MlpRolloutArgs mlp; MixPtrs mix; };     // mlp.roll.dr is unused
+struct MlpMixCollectArgs { MlpCollectArgs mlp; MixPtrs mix; };     // mlp.roll.dr is unused
+
+// cartpole_rollout_mlp_kernel / cartpole_collect_mlp_kernel (the same body) under a scenario mixture
+// (renv_cartpole_rollout_mlp_mix_f32 / renv_cartpole_collect_mlp_mix_f32): a lane draws its row at each reset, and its
+// episodes go to the statistics row of the reset that began them.
+template <int kAct, bool kEuler, bool kLog>
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
+cartpole_mix_rollout_mlp_kernel(const __grid_constant__ MlpMixRolloutArgs sa)
+{
+    constexpr bool kCollect = false, kPop = false, kGrid = false, kScen = false, kMix = true;
+    constexpr MlpTrajPtrs traj = {};
+    constexpr bool sample = false;
+    const MlpRolloutArgs &args = sa.mlp;
+    constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
+    const MixPtrs &mix = sa.mix;
+#include "renv_mlp_rollout_body.cuh"
+}
+
+template <int kAct, bool kEuler, bool kLog>
+__global__ void __launch_bounds__(kMlpThreads, kMlpRolloutCtas)
+cartpole_mix_collect_mlp_kernel(const __grid_constant__ MlpMixCollectArgs sa)
+{
+    constexpr bool kCollect = true, kPop = false, kGrid = false, kScen = false, kMix = true;
+    const MlpCollectArgs &args = sa.mlp;
+    const MlpTrajPtrs &traj = args.traj;
+    const bool sample = args.sample != 0;
+    constexpr PopulationPtrs pop = {};
+    constexpr GridPtrs grid = {};
+    constexpr EnvScenPtrs env_scen = {};
+    const MixPtrs &mix = sa.mix;
 #include "renv_mlp_rollout_body.cuh"
 }
 

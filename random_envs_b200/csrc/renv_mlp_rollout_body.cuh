@@ -1,9 +1,9 @@
 // Body of cartpole_rollout_mlp_kernel, cartpole_collect_mlp_kernel, cartpole_population_mlp_kernel,
-// cartpole_grid_mlp_kernel, cartpole_scen_rollout_mlp_kernel and cartpole_scen_collect_mlp_kernel (renv_mlp_policy.cuh),
-// included textually into each of these __global__ functions so that the rollout compiles to exactly the code it had
-// before the other kernels existed (an inlined device function would not guarantee that: DESIGN.md section 4.8).  The
-// including function defines
-//     kAct, kEuler, kLog, kCollect, kPop, kGrid, kScen   (template parameters or constexpr)
+// cartpole_grid_mlp_kernel, cartpole_scen_rollout_mlp_kernel, cartpole_scen_collect_mlp_kernel,
+// cartpole_mix_rollout_mlp_kernel and cartpole_mix_collect_mlp_kernel (renv_mlp_policy.cuh), included textually into
+// each of these __global__ functions so that the rollout compiles to exactly the code it had before the other kernels
+// existed (an inlined device function would not guarantee that: DESIGN.md section 4.8).  The including function defines
+//     kAct, kEuler, kLog, kCollect, kPop, kGrid, kScen, kMix   (template parameters or constexpr)
 //     args     the launch arguments: .roll (RolloutArgs<float>), .params, .log (read only when kLog)
 //     traj     const MlpTrajPtrs &: the per-step record (read only when kCollect)
 //     sample   bool: sample the action from softmax(l0, l1) instead of taking the argmax (read only when kCollect)
@@ -18,6 +18,9 @@
 //     kScen, env_scen  the per-env scenario kernels (EnvScenPtrs, read only when kScen): lane i reads env i's scenario
 //                 index once here and its row (global memory) at resets only; the row replaces a.dr, a fixed-task row's
 //                 task replaces the env's xi at each reset, and statistics go to the scenario's row (scenario_publish)
+//     kMix, mix   the mixture kernels (MixPtrs, read only when kMix): each reset draws the lane's row (mixture_draw),
+//                 which then acts as a kScen row; the running sums belong to the row of the current episode and are
+//                 flushed when a reset draws another row (mixture_stats_add); of_env is stored at the end
 // No include guard: included once per kernel.
     __shared__ MlpSmem sm;
     const uint32_t member = kPop ? blockIdx.x / pop.ctas : 0u;
@@ -33,6 +36,9 @@
     const uint64_t id = a.env.env_id0 + (uint64_t)il;
     const DrCfg4<float> &dr = kGrid ? grid_scenario<float>(grid, scenario)
                             : kScen ? scenario_row<float>(env_scen.rows, scenario) : a.dr;
+    uint32_t mix_row = kMix ? min((uint32_t)mix.of_env[il], mix.C) : 0u;    // kMix: the row of the running episode
+    unsigned mix_ended = 0;                 // kMix: episodes ended (the running sums restart at each flush)
+    if (kMix) mixture_stats_begin(mix.C);
 
     State<float> s;
     Xi<float> p;
@@ -99,17 +105,26 @@
                         log_count += 1u;
                     }
                     el = 0;
-                    if (draws_xi<kGrid || kScen>(dr.dr_type)) {            // reset_env: set_random_task, then reset
+                    if (kMix) mix_ended += 1u;
+                    const uint32_t c = kMix ? mixture_draw(mix, a.env.seed, id, tick) : 0u;
+                    const DrCfg4<float> &rdr = kMix ? scenario_row<float>(mix.rows, c) : dr;
+                    if (draws_xi<kGrid || kScen || kMix>(rdr.dr_type)) {   // reset_env: set_random_task, then reset
                         p = Xi<float>{ 0.0f, 0.0f, 0.0f, 0.0f };
-                        viol += sample_xi(p, dr, a.env.seed, id, tick);
+                        viol += sample_xi(p, rdr, a.env.seed, id, tick);
                         d = derive(p);
                         xi_dirty = true;
-                    } else if (kScen) {                                    // a fixed-task row: its task
-                        p = Xi<float>{ dr.a[0], dr.a[1], dr.a[2], dr.a[3] };
+                    } else if (kScen || kMix) {                            // a fixed-task row: its task
+                        p = Xi<float>{ rdr.a[0], rdr.a[1], rdr.a[2], rdr.a[3] };
                         d = derive(p);
                         xi_dirty = true;
                     }
                     init_state(s, a.env.seed, id, tick);
+                    if (kMix && c != mix_row) {     // the ended episode was the last of row mix_row in this run
+                        mixture_stats_add(a.stats, mix.C, mix_row, episodes, sum_len, sum_len, sum_r2, min_r, max_r);
+                        episodes = 0; sum_len = 0; sum_r2 = 0;
+                        min_r = __int_as_float(0x7f800000); max_r = __int_as_float(0xff800000);
+                        mix_row = c;
+                    }
                 }
             }
             __syncwarp();
@@ -121,11 +136,17 @@
         if (xi_dirty) store_xi(a.env.xi, i, p);
         store_elapsed(a.env, i, el);
         if (kLog) args.log.count[i] = (int32_t)log_count;
-        if (a.env.episode && episodes) a.env.episode[i] += episodes;      // one started per episode that ended
+        if (kMix) mix.of_env[i] = (uint16_t)mix_row;
+        if (kMix) {
+            if (a.env.episode && mix_ended) a.env.episode[i] += mix_ended;
+        } else if (a.env.episode && episodes) a.env.episode[i] += episodes;      // one started per episode that ended
     }
     if (kGrid) {
         const int64_t cell = (int64_t)member * grid.C + scenario;
         population_publish(a.stats + 6 * cell, cell, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
+    } else if (kMix) {
+        mixture_stats_add(a.stats, mix.C, mix_row, episodes, sum_len, sum_len, sum_r2, min_r, max_r);
+        mixture_stats_end(a.stats, mix.C, a.violations, viol);
     } else if (kScen) {
         scenario_publish(a.stats, env_scen.C, scenario, a.violations, episodes, sum_len, sum_len, sum_r2, min_r, max_r, viol);
     } else {

@@ -1,7 +1,8 @@
 // Body of cartpole_rollout_kernel, cartpole_rollout_logged_kernel, cartpole_population_linear_kernel,
-// cartpole_grid_linear_kernel and cartpole_scen_rollout_kernel (renv_kernels.cuh), included textually into each of these
-// __global__ functions for the reason given in renv_step_body.cuh.  The including function defines
-//     T, kEuler, kNoisy, kRandom, kLog, kPop, kGrid, kScen   (template parameters or constexpr)
+// cartpole_grid_linear_kernel, cartpole_scen_rollout_kernel and cartpole_mix_rollout_kernel (renv_kernels.cuh), included
+// textually into each of these __global__ functions for the reason given in renv_step_body.cuh.  The including function
+// defines
+//     T, kEuler, kNoisy, kRandom, kLog, kPop, kGrid, kScen, kMix   (template parameters or constexpr)
 //     a    const RolloutArgs<T> &  the launch arguments
 //     log  const LogPtrs<T> &      the episode log (read only when kLog): an ended episode's record is written in the
 //                                  warp's reset pass, before rollout_reset overwrites t.s / t.p / t.el
@@ -15,6 +16,9 @@
 //     kScen (constexpr), env_scen (EnvScenPtrs, read only when kScen): cartpole_scen_rollout_kernel.  Env i reads its
 //          scenario index once here and its row (in global memory) at resets only: the row replaces a.dr, and a
 //          fixed-task row's task replaces the env's xi at each reset.  Statistics go to the scenario's row (scenario_publish).
+//     kMix (constexpr), mix (MixPtrs, read only when kMix): cartpole_mix_rollout_kernel.  Each reset draws env i's row
+//          (mixture_draw), which then acts as a kScen row; the lane's running sums belong to the row of its current
+//          episode and are flushed when a reset draws another row (mixture_stats_add).  of_env is stored at the end.
 // No include guard: included once per kernel.
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t ld = a.env.ld;
@@ -26,6 +30,8 @@
     const uint32_t policy_row = kGrid ? (uint32_t)member / grid.C : (uint32_t)member;
     const DrCfg4<T> *const scen = kGrid ? &grid_scenario<T>(grid, (uint32_t)member - policy_row * grid.C) : nullptr;
     const uint32_t scenario = kScen ? env_scenario(env_scen, il) : 0u;     // kScen: its row is found at each reset
+    uint32_t mix_row = kMix ? min((uint32_t)mix.of_env[il], mix.C) : 0u;    // kMix: the row of the running episode
+    if (kMix) mixture_stats_begin(mix.C);
 
     // per-thread episode statistics (return == length here: reward is 1.0 on every step, :207-212)
     RolloutThread<T> t;
@@ -91,8 +97,22 @@
                                 a.tick + (uint64_t)(a.K - t.parked - 1));
                     log_count += 1u;
                 }
-                rollout_reset<T, kRandom, kGrid, kScen>(t, a, id,
-                                                        kScen ? &scenario_row<T>(env_scen.rows, scenario) : scen);
+                if (kMix) {
+                    const bool ends = !(kRandom && t.refresh);     // a refresh keeps the episode and its row
+                    const uint32_t c = ends ? mixture_draw(mix, a.env.seed, id, a.tick + (uint64_t)(a.K - t.parked - 1))
+                                            : mix_row;
+                    rollout_reset<T, kRandom, kGrid, true>(t, a, id, &scenario_row<T>(mix.rows, (uint16_t)min(c, mix.C - 1u)));
+                    if (c != mix_row) {     // the ended episode was the last of row mix_row in this run of the lane
+                        mixture_stats_add(a.stats, mix.C, mix_row, t.episodes, t.sum_len, t.sum_r, t.sum_r2, t.min_r,
+                                          t.max_r);
+                        t.episodes = 0; t.sum_len = 0; t.sum_r = 0; t.sum_r2 = 0;
+                        t.min_r = __int_as_float(0x7f800000); t.max_r = __int_as_float(0xff800000);
+                        mix_row = c;
+                    }
+                } else {
+                    rollout_reset<T, kRandom, kGrid, kScen>(t, a, id,
+                                                            kScen ? &scenario_row<T>(env_scen.rows, scenario) : scen);
+                }
             }
             continue;                       // revived lanes may still have steps to do
         }
@@ -105,6 +125,7 @@
         if (t.xi_dirty) store_xi(a.env.xi, i, t.p);
         store_elapsed(a.env, i, t.el);
         if (kLog) log.count[i] = (int32_t)log_count;
+        if (kMix) mix.of_env[i] = (uint16_t)mix_row;
         if (a.env.episode && t.new_episodes) a.env.episode[i] += t.new_episodes;
         if (kNoisy) {       // leave the obs buffer as K calls of step() would: the observation of the last step / reset
             T ov[4];
@@ -112,7 +133,10 @@
             a.env.obs[i] = ov[0]; a.env.obs[ld + i] = ov[1]; a.env.obs[2 * ld + i] = ov[2]; a.env.obs[3 * ld + i] = ov[3];
         }
     }
-    if (kScen)
+    if (kMix) {
+        mixture_stats_add(a.stats, mix.C, mix_row, t.episodes, t.sum_len, t.sum_r, t.sum_r2, t.min_r, t.max_r);
+        mixture_stats_end(a.stats, mix.C, a.violations, t.viol);
+    } else if (kScen)
         scenario_publish(a.stats, env_scen.C, scenario, a.violations, t.episodes, t.sum_len, t.sum_r, t.sum_r2, t.min_r,
                          t.max_r, t.viol);
     else if (kPop)

@@ -1,19 +1,21 @@
-// Body of cartpole_step_kernel, cartpole_step_logged_kernel and cartpole_scen_step_kernel (renv_kernels.cuh), included
-// textually into each __global__ function rather than called as an inlined device function: an inlined body schedules
-// the plain kernels' code differently, and the plain kernels must stay exactly what they were.  The including function
-// defines
-//     T, kAutoReset, kNoisy, kLean, kLog, kScen   (template parameters or constexpr; kLean is a per-launch constant
-//                                                in the logged kernel)
+// Body of cartpole_step_kernel, cartpole_step_logged_kernel, cartpole_scen_step_kernel and cartpole_mix_step_kernel
+// (renv_kernels.cuh), included textually into each __global__ function rather than called as an inlined device
+// function: an inlined body schedules the plain kernels' code differently, and the plain kernels must stay exactly what
+// they were.  The including function defines
+//     T, kAutoReset, kNoisy, kLean, kLog, kScen, kMix   (template parameters or constexpr; kLean is a per-launch
+//                                                      constant in the logged kernel)
 //     a    const StepArgs<T> &    the launch arguments
 //     log  const LogPtrs<T> &     the episode log (read only when kLog)
 //     env_scen  const EnvScenPtrs &  per-env scenarios (read only when kScen): the reset pass takes env i's row in
 //                                    place of a.dr
+//     mix  const MixPtrs &        a scenario mixture (read only when kMix): the reset pass draws env i's row, resets
+//                                 from it and stores it in of_env
 // No include guard: included once per kernel.
     using VT = VecTraits<T>;
     constexpr int V = VT::V;
     constexpr int kTile = kStepThreads * V;
     __shared__ unsigned s_count;
-    __shared__ uint32_t s_ticket;                          // kScen: the ticket waits here across the reset pass
+    __shared__ uint32_t s_ticket;                          // kScen, kMix: the ticket waits here across the reset pass
     __shared__ uint16_t s_list[kAutoReset ? kTile : 1];
     __shared__ int32_t s_len[kLog ? kTile : 1];          // length of the ended episode, negated when truncated
     const int64_t block0 = (int64_t)blockIdx.x * kTile;
@@ -34,7 +36,7 @@
                 seen = ld_acquire_gpu(slot + 1);
             }
             if (seen != ticket && a.counters) atomicAdd(a.counters + kCounterOrderTimeout, 1ull);
-            if (kScen) s_ticket = ticket;
+            if (kScen || kMix) s_ticket = ticket;
             if (kAutoReset) s_count = 0;
         } else if (block0 + kTile <= n && threadIdx.x >= 32 && threadIdx.x < 39) {
             // while thread 0 waits for its L2 round trip the tile is pulled from HBM into L2 (never stale: L2 is the
@@ -198,6 +200,11 @@
                 const int64_t i = block0 + s_list[j];
                 viol += reset_env<T, true>(a.env, scenario_row<T>(env_scen.rows, env_scenario(env_scen, i)), i, a.tick,
                                            a.env.seed);
+            } else if (kMix) {  // the drawn row: one more Philox block and one 8-byte table load per reset
+                const int64_t i = block0 + s_list[j];
+                const uint32_t c = mixture_draw(mix, a.env.seed, a.env.env_id0 + (uint64_t)i, a.tick);
+                viol += reset_env<T, true>(a.env, scenario_row<T>(mix.rows, c), i, a.tick, a.env.seed);
+                mix.of_env[i] = (uint16_t)c;
             } else {
                 viol += reset_env(a.env, a.dr, block0 + s_list[j], a.tick, a.env.seed);
             }
@@ -207,7 +214,7 @@
     if (tracked) {
         __syncthreads();                    // every store of the CTA precedes (happens-before) thread 0's release
         if (threadIdx.x == 0) {
-            st_release_gpu(a.env.progress + 2 * (size_t)blockIdx.x + 1, (kScen ? s_ticket : ticket) + 1u);
+            st_release_gpu(a.env.progress + 2 * (size_t)blockIdx.x + 1, (kScen || kMix ? s_ticket : ticket) + 1u);
             asm volatile("griddepcontrol.wait;" ::: "memory");     // do not complete before the previous grid has
         }
     }

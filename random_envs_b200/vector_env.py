@@ -11,6 +11,8 @@ Same method names as the reference's single env (random_cartpole.py / random_env
     evaluate_population(policies, K) -> (P, 6)   (P policies on common tasks from fresh starts; the env is untouched)
     evaluate_grid(policies, scenarios, K) -> (P, C, 6)   (the same for each of C task scenarios, in one kernel)
     set_scenarios(scenarios, assignment)  (env i resets from scenario assignment[i] in reset / step / rollout / collect)
+    set_scenario_mixture(scenarios, weights)  (every reset draws its scenario from the weighted rows, on the device)
+    set_mixture_weights(weights)        (new weights for the next resets; rows, running episodes and statistics kept)
     scenario_stats() -> (C, 6)          (returns of the episodes finished inside rollouts, per scenario)
     policy_actions(policy) -> (N,)      (the MLPPolicy's actions for the current observations, ready for step)
     collect(policy, K) -> Trajectory    (K fused steps under the sampled policy, every step recorded for training)
@@ -59,6 +61,44 @@ def _combine_stats(rows):
     t = _device.torch()
     return t.stack([rows[:, 0].sum(), rows[:, 1].sum(), rows[:, 2].sum(), rows[:, 3].min(), rows[:, 4].max(),
                     rows[:, 5].sum()])
+
+
+def _mixture_table(weights, C):
+    """(weights as a float64 numpy array, the (C,) int64 alias table of include/renv.h renv_env_mixture) of C mixture
+    weights; raises ValueError on bad weights.  Vose's method in float64, then q rounded to an integer over 2^32; two
+    rules hold exactly: a weight-0 row is never drawn (its q is 0 and no column aliases it), and a column that keeps
+    all its mass aliases itself (so y < q failing at y = 2^32 - 1 still draws it).  Entry j is q | alias << 32."""
+    t = _device.torch()
+    if isinstance(weights, t.Tensor):
+        weights = weights.detach().to("cpu", t.float64).numpy()        # the one synchronisation of a device tensor
+    w = np.array(weights, dtype=np.float64)
+    if w.shape != (C,):
+        raise ValueError("the mixture weights must have shape (%d,), got %s" % (C, w.shape))
+    if not np.all(np.isfinite(w)) or np.any(w < 0):
+        raise ValueError("the mixture weights must be finite and >= 0")
+    total = w.sum()
+    if not total > 0:
+        raise ValueError("the mixture weights must have a positive sum")
+    p = w * (C / total)
+    q = np.ones(C, dtype=np.float64)
+    alias = np.arange(C, dtype=np.int64)
+    small = [j for j in range(C) if p[j] < 1.0]
+    large = [j for j in range(C) if p[j] >= 1.0]
+    while small and large:
+        s, l = small.pop(), large.pop()
+        q[s], alias[s] = p[s], l
+        p[l] -= 1.0 - p[s]
+        (small if p[l] < 1.0 else large).append(l)
+    # left over by rounding: columns whose mass is (nearly) 1 keep it, except a weight-0 row, which gives it away
+    heaviest = int(np.argmax(w))
+    for j in small + large:
+        q[j], alias[j] = (1.0, j) if w[j] > 0 else (0.0, heaviest)
+    qi = np.minimum(np.rint(q * 2.0 ** 32), 2.0 ** 32).astype(np.int64)
+    qi[w == 0] = 0
+    keep = qi >= 2 ** 32
+    alias[keep] = np.nonzero(keep)[0]
+    qi[keep] = 2 ** 32 - 1
+    return w, qi | (alias << 32)
 
 
 def _round_up(x, m):
@@ -125,7 +165,8 @@ class RandomCartPoleVecEnv(RandomEnv):
         self.polemass_length = 0.05     # frozen, as in the reference (:79 vs :157-166)
         self._buffers = None
         self._episode_log = None        # EpisodeLog attached by start_episode_log
-        self._scen = None               # per-env scenarios (set_scenarios): rows, of_env, stats, the C struct
+        self._scen = None               # per-env scenarios (set_scenarios) or a mixture (set_scenario_mixture): rows,
+                                        # of_env, stats, the C struct; a mixture also its weights and alias table
         self._scen_version = 0          # bumped whenever _scen changes (the step plan holds a pointer to its struct)
         self._cfg_cache = None
         self._cfg_key = None
@@ -228,17 +269,22 @@ class RandomCartPoleVecEnv(RandomEnv):
             return "renv_cartpole_%s_noisy_%s" % (name, suffix), head + (ctypes.byref(b["noise"]),)
         return "renv_cartpole_%s_%s" % (name, suffix), head
 
+    def _scen_what(self):
+        return "a scenario mixture" if "table" in self._scen else "per-env scenarios"
+
     def _resolve_scen(self, name):
-        """(C function, leading arguments) of the per-env scenario form of ``name`` ("reset", "step", "rollout",
-        "rollout_mlp", "collect_mlp"): env, scenarios and -- except for reset -- the episode log or NULL."""
+        """(C function, leading arguments) of the per-env scenario or mixture form of ``name`` ("reset", "step",
+        "rollout", "rollout_mlp", "collect_mlp"): env, scenarios or mixture and -- except for reset -- the episode log
+        or NULL."""
         if self.noisy or self._dtype_name != "float32":
-            raise ValueError("per-env scenarios need a float32 env without observation noise")
+            raise ValueError("%s need%s a float32 env without observation noise"
+                             % (self._scen_what(), "s" if "table" in self._scen else ""))
         head = (ctypes.byref(self._buffers["env"]), ctypes.byref(self._scen["struct"]))
         if name != "reset":
             if self._episode_log is not None:
                 self._check_log_supported()
             head += (ctypes.byref(self._episode_log.struct) if self._episode_log is not None else None,)
-        return "renv_cartpole_%s_scen_f32" % name, head
+        return "renv_cartpole_%s_%s_f32" % (name, "mix" if "table" in self._scen else "scen"), head
 
     def _launch(self, fn, *args):
         """Call the C function ``fn`` with ``args`` on the env's device and current stream (the last argument)."""
@@ -347,6 +393,8 @@ class RandomCartPoleVecEnv(RandomEnv):
         # the uint16 counter: the lean step, or with a log attached the logged step on that counter without a reward store
         scen = self._scen is not None
         if scen and not self.auto_reset:
+            if "table" in self._scen:
+                raise ValueError("a scenario mixture acts at resets: step() with a mixture needs auto_reset")
             raise ValueError("per-env scenarios act at resets: step() with scenarios needs auto_reset")
         if scen:        # one entry point for every layout: the counter of the env, reward NULL with the uint16 one
             fn, head = self._resolve_scen("step")
@@ -595,8 +643,9 @@ class RandomCartPoleVecEnv(RandomEnv):
         b = self._alloc()
         t = _device.torch()
         if self._scen is not None:
-            raise ValueError("evaluate_population() runs the env's own DR config or task table, which per-env scenarios "
-                             "replace: call set_scenarios(None) first, or use evaluate_grid()")
+            raise ValueError("evaluate_population() runs the env's own DR config or task table, which %s "
+                             "replace%s: call set_scenarios(None) first, or use evaluate_grid()"
+                             % (self._scen_what(), "s" if "table" in self._scen else ""))
         K, rows, P, kind, policy_args = self._population_rows(policies, num_steps, "evaluate_population()")
         stats = t.tensor([0.0, 0.0, 0.0, math.inf, -math.inf, 0.0], dtype=t.float64, device=b["device"]).repeat(P, 1)
         viol = self._violation_counter(b["device"])
@@ -802,10 +851,81 @@ class RandomCartPoleVecEnv(RandomEnv):
         """(C, 6) float64 device tensor: row c holds the statistics (``distributed.STAT_NAMES``) of the episodes that
         the envs of scenario c finished inside ``rollout()`` and ``collect()`` since ``set_scenarios`` or
         ``reset_stats()``.  Each row is exact (integer sums, a min and a max); shards combine row by row as
-        ``distributed.combine_stats`` combines ranks, and the rows combined are ``stats_tensor``."""
+        ``distributed.combine_stats`` combines ranks, and the rows combined are ``stats_tensor``.  Under a mixture,
+        row c holds the episodes whose reset drew row c; the episodes that were running when the mixture was installed
+        are in ``stats_tensor`` only."""
         if self._scen is None:
             raise ValueError("no scenarios are set (set_scenarios)")
-        return self._scen["stats"]
+        return self._scen["stats"][:self._scen["rows"].shape[0]]
+
+    # ---- scenario mixtures ------------------------------------------------------------------------------
+    def set_scenario_mixture(self, scenarios, weights):
+        """Draw the task scenario of every episode from the C rows of ``scenarios`` (a ``Scenarios`` on the env's
+        device) with probabilities proportional to ``weights`` (C finite values >= 0 with a positive sum: a sequence,
+        a numpy array or a tensor).  From now on every reset of env i at clock tick t -- in ``reset()``, the
+        auto-reset of ``step()``, and inside ``rollout()`` and ``collect()`` -- draws its row on the device from
+        Philox (seed, id, t, purpose 6) and an alias table, then resets from that row exactly as ``set_scenarios``
+        would with that row assigned to env i.  Successive episodes of an env thus run i.i.d. tasks of the mixture:
+        ADR boundary sampling (``Scenarios.adr_boundaries`` with weights ``[1 - p_b] + [p_b / 8] * 8``), weighted
+        curricula, an empirical task set.  A weight-0 row is never drawn.
+
+        Rollouts and collect accumulate each finished episode into the ``scenario_stats()`` row its reset drew; the
+        episodes running now keep their task and count in ``stats_tensor`` only.  ``scenarios`` holds the rows and
+        the row of each env's running episode.  Replaces per-env scenarios or an earlier mixture;
+        ``set_scenarios(None)`` clears it.  ``set_mixture_weights`` changes the weights alone.  At most one
+        synchronisation.  float32 envs without observation noise; ``set_random_task``, ``evaluate_population`` and
+        ``step()`` without auto-reset are refused while a mixture is set."""
+        from .scenarios import Scenarios
+        t = _device.torch()
+        if self._dtype_name != "float32" or self.noisy:
+            raise ValueError("a scenario mixture needs a float32 env without observation noise")
+        if not isinstance(scenarios, Scenarios):
+            raise TypeError("set_scenario_mixture() takes its scenarios as a Scenarios (Scenarios.tasks / .distributions)")
+        if scenarios.device.type != "cuda":
+            raise ValueError("the scenarios live on %s: move them to the env's device" % scenarios.device)
+        C = len(scenarios)
+        if C > 65535:
+            raise ValueError("at most 65535 scenarios, got %d" % C)
+        w, table = _mixture_table(weights, C)
+        b = self._alloc()
+        if scenarios.device != b["device"]:
+            raise ValueError("the scenarios live on %s, the env on %s" % (scenarios.device, b["device"]))
+        of_env = t.full((self.num_envs,), C, dtype=t.int32, device=b["device"]).to(t.int16)
+        self._install_mixture(scenarios.rows.clone(), w, t.from_numpy(table).to(b["device"]), of_env,
+                              t.tensor(_EMPTY_STATS, dtype=t.float64, device=b["device"]).repeat(C + 1, 1))
+
+    def set_mixture_weights(self, weights):
+        """New weights for the installed mixture (C values, as ``set_scenario_mixture`` takes them): only the alias
+        table is rebuilt.  The rows, the row of every running episode and the statistics are kept, so the next resets
+        draw from the new weights while running episodes finish under the row they drew.  The per-iteration call of a
+        curriculum or ADR loop; at most one synchronisation."""
+        if self._scen is None or "table" not in self._scen:
+            raise ValueError("no scenario mixture is set (set_scenario_mixture)")
+        w, table = _mixture_table(weights, self._scen["rows"].shape[0])
+        self._scen["table"].copy_(_device.torch().from_numpy(table))
+        self._scen["weights"] = w
+
+    @property
+    def scenario_weights(self):
+        """The weights of the installed mixture as given (float64 numpy array of C values), or None."""
+        if self._scen is None or "table" not in self._scen:
+            return None
+        return self._scen["weights"].copy()
+
+    def _install_mixture(self, rows, weights, table, of_env, stats):
+        """Set the env-owned mixture buffers: rows (C, SCENARIO_FLOATS) float32, weights (C,) float64 numpy, table (C,)
+        int64 alias entries, of_env (N,) int16 holding uint16 rows (C: running since before the mixture), stats
+        (C + 1, 6) float64 -- all checked, the tensors on the env's device."""
+        t = _device.torch()
+        b = self._buffers
+        self._clear_scenarios()
+        idx = t.zeros(b["ld"], dtype=t.int16, device=b["device"])
+        idx[:self.num_envs].copy_(of_env)
+        rows, table = rows.contiguous(), table.contiguous()
+        st = _lib.EnvMixture()
+        st.rows, st.table, st.of_env, st.C = rows.data_ptr(), table.data_ptr(), idx.data_ptr(), int(rows.shape[0])
+        self._scen = dict(rows=rows, of_env=idx, stats=stats.contiguous(), struct=st, table=table, weights=weights)
+        self._scen_version += 1
 
     def allgather_stats(self, group=None):
         """The per-iteration collective (distributed.allgather_stats) on this env's statistics; like every call that
@@ -854,8 +974,8 @@ class RandomCartPoleVecEnv(RandomEnv):
     def set_random_task(self):
         """Resample xi of every env now (random_env.py:37-39)."""
         if self._scen is not None:
-            raise ValueError("set_random_task() draws from the env's own DR config, which per-env scenarios replace: "
-                             "call set_scenarios(None) first")
+            raise ValueError("set_random_task() draws from the env's own DR config, which %s replace%s: "
+                             "call set_scenarios(None) first" % (self._scen_what(), "s" if "table" in self._scen else ""))
         # sample i of the call is keyed by the GLOBAL env id, so a sharded env draws what the unsharded one would
         self.set_task(self.sample_tasks_tensor(self.num_envs, dtype=self.torch_dtype, device=self._alloc()["device"],
                                                sample_id0=self.env_id0))
@@ -979,8 +1099,13 @@ class RandomCartPoleVecEnv(RandomEnv):
                            stdev_task=self.stdev_task.copy(),
                            cov_task=np.copy(self.cov_task) if getattr(self, "cov_task", None) is not None else None))
         sc = self._scen
-        out["scenarios"] = None if sc is None else dict(rows=sc["rows"].clone(), of_env=sc["of_env"][:self.num_envs].clone(),
-                                                        stats=sc["stats"].clone())
+        mixture = sc is not None and "table" in sc
+        out["scenarios"] = None if sc is None or mixture else dict(rows=sc["rows"].clone(),
+                                                                   of_env=sc["of_env"][:self.num_envs].clone(),
+                                                                   stats=sc["stats"].clone())
+        if mixture:
+            out["mixture"] = dict(rows=sc["rows"].clone(), weights=sc["weights"].copy(), table=sc["table"].clone(),
+                                  of_env=sc["of_env"][:self.num_envs].clone(), stats=sc["stats"].clone())
         self.check_dr_violations()          # synchronises; a checkpoint must not hide an error the reference raises
         return out
 
@@ -1018,6 +1143,12 @@ class RandomCartPoleVecEnv(RandomEnv):
         if sc is not None:
             dev = b["device"]
             self._install_scenarios(sc["rows"].to(dev), sc["of_env"].to(dev), sc["stats"].to(dev).clone())
+        mx = sd.get("mixture")
+        if mx is not None:
+            dev = b["device"]
+            # clones: set_mixture_weights rewrites the table in place, which must not reach the caller's state_dict
+            self._install_mixture(mx["rows"].to(dev).clone(), np.array(mx["weights"], dtype=np.float64),
+                                  mx["table"].to(dev).clone(), mx["of_env"].to(dev), mx["stats"].to(dev).clone())
 
     # ---- introspection used by tests -------------------------------------------------------------------
     @property
